@@ -2,7 +2,7 @@
 """Benchmark of the Illumina read-generation hot path (BASELINE.json metric:
 Illumina PE150 read pairs/s, HS25).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload ("human_pe150_hs25", BASELINE.json configs[4] / SURVEY.md section 8d config 5):
@@ -321,6 +321,41 @@ def parity_slices(J, ctx, genome, n_reads, L, seed, kw, n_slice=2048):
     return "ok", checked
 
 
+# ------------------------------------------------------------ outputs of the timed leg ---
+
+DUMP_BYTES_PER_END, DUMP_WINDOWS_PER_BATCH = 4 << 20, 4       # 32 MB of float32 for both ends
+
+
+def dump_outputs(J, ctx, genome, st, n_reads, L, seed, kw, B, launches, step, n_steps, out_dir):
+    """What the device-resident leg computed in its last step, as DIR/<name>.npy.  That leg leaves its FASTQ in HBM and
+    drops it; a pair's bytes depend only on the seed and its index, so the step -- shard `step` of the `n_steps` equal
+    steps of the timed job, cut into the same `launches` launches of B pairs -- is generated again through the stream
+    sink (the same kernels, plus the copy out).
+      r1_fastq, r2_fastq  DUMP_WINDOWS_PER_BATCH windows at seeded offsets in every batch's FASTQ, one byte per float32
+      step                pairs, batches and FASTQ bytes per end of the regenerated step
+      timed_call          pairs and FASTQ bytes per end of the whole timed call (its caller's results, timing aside)"""
+    win = max(1, DUMP_BYTES_PER_END // (DUMP_WINDOWS_PER_BATCH * launches))
+    parts, calls = ([], []), [0, 0]
+
+    def sink(job, end, buf):
+        n, w = len(buf), min(win, len(buf))
+        offsets = np.random.default_rng([seed, end, calls[end]]).integers(0, n - w + 1, DUMP_WINDOWS_PER_BATCH) if w else []
+        calls[end] += 1
+        for o in np.sort(offsets):
+            parts[end].append(buf[int(o):int(o) + w])
+
+    ss = J.illumina(genome, "", n_reads, L, True, seed=seed, ctx=ctx, sink=sink, batch_pairs=B, shard=(step, n_steps), **kw)
+    assert ss["pairs"] == B * launches and ss["batches"] == launches, ss
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"r1_fastq": np.frombuffer(b"".join(parts[0]), np.uint8).astype(np.float32),
+              "r2_fastq": np.frombuffer(b"".join(parts[1]), np.uint8).astype(np.float32),
+              "step": np.array([ss["pairs"], ss["batches"], ss["bytes_out"][0], ss["bytes_out"][1]], dtype=np.float64),
+              "timed_call": np.array([st["pairs"], st["bytes_out"][0], st["bytes_out"][1]], dtype=np.float64)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    return {name: list(arr.shape) for name, arr in arrays.items()}
+
+
 # -------------------------------------------------- BASELINE.json configs[0..3] (rank 0, N = 1) ---
 
 def extra_workloads(J, ctx, seed, log):
@@ -448,7 +483,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip BASELINE configs[0..3], files, PacBio and the full-job legs")
     ap.add_argument("--seed", type=int, default=20261018)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, generate the last step of the device-resident "
+                    "leg again and write a fixed sample of its FASTQ to DIR/*.npy (rank 0; see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else max(a.warmup, 1)
     rank, local_rank, world = dist_env()
     if a.impl == "reference" and rank != 0:
@@ -761,6 +802,11 @@ def main():
             log("[bench] parity slices vs the oracle: %s (%.1f s)" % (verdict, time.perf_counter() - t0))
         except Exception as e:
             out["parity_slice"] = "error: " + str(e)[:200]
+        if a.dump_outputs:
+            t0 = time.perf_counter()
+            out["dumped_outputs"] = dump_outputs(J, ctx, genome, st, job_reads, L, a.seed, kw, B, a.launches_per_step,
+                                                 rank * a.steps + a.steps - 1, a.steps * world, a.dump_outputs)
+            log("[bench] outputs of the last step written to %s (%.1f s)" % (a.dump_outputs, time.perf_counter() - t0))
         if extras is not None:
             out["extra_workloads"] = extras
         if not a.no_cpu_baseline and world == 1:

@@ -44,3 +44,15 @@ def load(name):
     import os
     d = np.load(os.path.join(os.path.dirname(__file__), name + ".npz"))
     return d["r1"].tobytes(), d["r2"].tobytes(), d["counts"]
+
+
+def assert_oracle_reproduces(name):
+    """The oracle's run of case `name` is the reference's stored FASTQ byte for byte (pairs per group included);
+    returns (r1, r2) for further checks."""
+    from oracle.compare import oracle_run
+    make, n_reads, L, paired, seed, kw = CASES[name]
+    r1, r2, counts = load(name)
+    o = oracle_run(make(), n_reads, L, paired, seed, **kw)
+    assert np.array_equal(o["groups"].counts, counts)
+    assert o["r1"] == r1 and o["r2"] == r2
+    return r1, r2

@@ -12,7 +12,7 @@ import pytest
 
 import jackalope_b200 as J
 from jackalope_b200 import _lib
-from golden.cases import CASES, load
+from golden.cases import CASES, assert_oracle_reproduces
 from oracle import harness as H
 from oracle.compare import fastq_records, frag_table, oracle_run
 
@@ -328,11 +328,8 @@ def test_params_struct_matches_the_header():
 
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_oracle_reproduces_golden(name):
-    make, n_reads, L, paired, seed, kw = CASES[name]
-    r1, r2, counts = load(name)
-    o = oracle_run(make(), n_reads, L, paired, seed, **kw)
-    assert np.array_equal(o["groups"].counts, counts)
-    assert o["r1"] == r1 and o["r2"] == r2
+    _, n_reads, _, paired, _, _ = CASES[name]
+    r1, r2 = assert_oracle_reproduces(name)
     recs = fastq_records(r1)
     assert len(recs) == n_reads // (2 if paired else 1)
     assert all(r[0].startswith(b"@") and r[2] == b"+" and len(r[1]) == len(r[3]) for r in recs)

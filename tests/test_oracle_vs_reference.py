@@ -13,6 +13,8 @@
   expressions.
 
 Skipped where neither /root/reference nor a prebuilt oracle/_ref exists.
+The replay tests are not: without the reference they check the oracle against the reference's FASTQ stored for the
+same scenario (tests/golden, written by make_golden.py only where the reference consumed exactly the draw ledger).
 """
 import numpy as np
 import pytest
@@ -20,9 +22,11 @@ import pytest
 import jackalope_b200 as J
 from jackalope_b200 import _lib
 from oracle import harness as H
+from golden.cases import assert_oracle_reproduces
 from oracle.compare import hap_sequences, oracle_run
 
-needs_ref = pytest.mark.skipif(not (H.have_ref(True) and H.have_ref(False)), reason="oracle/_ref not built")
+HAVE_REF = H.have_ref(True) and H.have_ref(False)
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 
 
 def genome_with_n(seed=1, n=3, length=5000):
@@ -73,33 +77,44 @@ def replay_check(obj, n_reads, L, paired, seed, ref_obj=None, **kw):
     return o
 
 
-@needs_ref
 @pytest.mark.parametrize("paired,matepair", [(False, False), (True, False), (True, True)])
 def test_replay_ref_default_args(paired, matepair):
+    if not HAVE_REF:
+        assert_oracle_reproduces({False: "se100_default", True: "mp100_default" if matepair else "pe100_default"}[paired])
+        return
     replay_check(genome_with_n(), 1200, 100, paired, seed=11, matepair=matepair)
 
 
-@needs_ref
 def test_replay_pe150_hs25():
+    if not HAVE_REF:
+        assert_oracle_reproduces("pe150_hs25")
+        return
     replay_check(genome_with_n(seed=2, n=4, length=9000), 1500, 150, True, seed=12, seq_sys="HS25")
 
 
-@needs_ref
 def test_replay_high_indels_dups_barcode():
+    if not HAVE_REF:
+        assert_oracle_reproduces("pe100_indels_dups_barcode")
+        return
     replay_check(genome_with_n(seed=4), 1500, 100, True, seed=13, ins_prob1=0.02, del_prob1=0.03, ins_prob2=0.05,
                  del_prob2=0.01, prob_dup=0.4, read_pool_size=14, barcodes=["ACGTTG"])
 
 
-@needs_ref
 def test_replay_short_fragments_and_chromosomes():
+    if not HAVE_REF:
+        assert_oracle_reproduces("pe100_short_fragments")
+        return
     g = J.RefGenome(["a", "b", "c"], [J.random_genome(1, 60, seed=5).seqs[0], J.random_genome(1, 4000, seed=6).seqs[0],
                                       J.random_genome(1, 130, seed=7).seqs[0]])
     replay_check(g, 1500, 100, True, seed=14, frag_mean=120, frag_sd=40, frag_len_min=20, ins_prob1=0.01,
                  del_prob1=0.01)
 
 
-@needs_ref
 def test_replay_haplotypes():
+    if not HAVE_REF:
+        assert_oracle_reproduces("hap_pe100_pooled")
+        assert_oracle_reproduces("hap_se100_sep_files")
+        return
     g = J.random_genome(3, 6000, seed=8)
     haps, edits = J.random_haplotypes(g, 3, sub_rate=0.02, indel_rate=0.005, seed=9, return_edits=True)
     hs = to_ref_haps(haps, edits, replay=True)
