@@ -62,10 +62,29 @@ class RunStats(C.Structure):
                     z_bytes=list(self.z_bytes), bgzf_ms=self.bgzf_ms)
 
 
+class MutationParams(C.Structure):
+    _fields_ = [
+        ("Q", C.c_double * 16), ("invariant", C.c_double), ("n_rates", C.c_uint32), ("rates", f64p),
+        ("n_nodes", C.c_uint32), ("parent", C.POINTER(C.c_int32)), ("branch_len", f64p), ("n_tips", C.c_uint32),
+        ("tip_node", u32p), ("tip_names", C.POINTER(C.c_char_p)), ("seed", C.c_uint64),
+    ]
+
+
+class MutationStats(C.Structure):
+    _fields_ = [
+        ("count_ms", C.c_double), ("scan_ms", C.c_double), ("write_ms", C.c_double), ("store_ms", C.c_double),
+        ("total_ms", C.c_double), ("records", C.c_uint64), ("d2h_bytes", C.c_uint64), ("table_bytes", C.c_uint64),
+        ("table_in_smem", C.c_int), ("max_slots", C.c_uint32),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/jlp_b200.h declares
 SYMBOLS = [
     "jlp_ctx_create", "jlp_ctx_create_multi", "jlp_ctx_n_devices", "jlp_materialize_haplotypes", "jlp_ctx_destroy", "jlp_last_error", "jlp_set_genome", "jlp_set_genome_async", "jlp_genome_sync", "jlp_create_genome", "jlp_get_genome", "jlp_genome_draw", "jlp_clear_haplotypes",
-    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
+    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_get_haplotype_muts", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
     "jlp_illumina_to_memory", "jlp_illumina_stream", "jlp_illumina_device_only", "jlp_illumina_group_counts", "jlp_apportion", "jlp_shard_range", "jlp_deflate", "jlp_bgzf_device", "jlp_pacbio", "jlp_pacbio_to_memory", "jlp_pacbio_read_plan", "jlp_pacbio_sample", "jlp_reads_per_group", "jlp_alias_build",
     "jlp_threshold", "jlp_unif_expr", "jlp_frag_table", "jlp_philox4x32_10", "jlp_draw_pos", "jlp_draw_pair",
     "jlp_version",
@@ -103,6 +122,10 @@ def lib():
     L.jlp_add_haplotype.argtypes = [C.c_void_p, C.c_char_p, u64p, C.POINTER(u64p), C.POINTER(u64p),
                                     C.POINTER(u64p), C.POINTER(C.c_void_p), u64p, u64p, u64p]
     L.jlp_get_haplotype_chrom.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint64, u64p]
+    L.jlp_create_haplotypes.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(MutationStats)]
+    L.jlp_get_haplotype_muts.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, u64p, u64p, u64p, C.c_void_p, C.c_uint64,
+                                         C.c_uint64, u64p, u64p, u64p]
+    L.jlp_transition_matrix.argtypes = [f64p, C.c_double, f64p]
     L.jlp_set_profile.argtypes = [C.c_void_p, C.c_int, C.c_uint64, u32p, f64p, u8p]
     L.jlp_illumina_ref.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(RunStats)]
     L.jlp_illumina_hap.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(RunStats)]

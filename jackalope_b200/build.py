@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libjlp_b200.so")
-SOURCES = ["jlp_api.cu", "jlp_kernels.cu", "jlp_bgzf.cu", "jlp_pacbio.cu", "jlp_pacbio.cpp", "jlp_host.cpp", "jlp_deflate.cpp"]
+SOURCES = ["jlp_api.cu", "jlp_kernels.cu", "jlp_bgzf.cu", "jlp_pacbio.cu", "jlp_mutate.cu", "jlp_pacbio.cpp", "jlp_host.cpp", "jlp_deflate.cpp"]
 HEADERS = ["jlp_draws.h", "jlp_host.h", "jlp_kernels.cuh", "jlp_deflate.h", "jlp_pacbio.h", os.path.join("..", "..", "include", "jlp_b200.h")]
 
 

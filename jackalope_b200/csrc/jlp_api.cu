@@ -15,6 +15,7 @@
 #include <atomic>
 #include <cerrno>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <deque>
 #include <functional>
@@ -1717,6 +1718,267 @@ int jlp_get_haplotype_chrom(jlp_ctx* c, uint64_t hap, uint64_t chrom, char* out,
     });
 }
 
+int jlp_get_haplotype_muts(jlp_ctx* c, uint64_t hap, uint64_t chrom, uint64_t* old_pos, uint64_t* new_pos,
+                           uint64_t* nuc_off, char* pool, uint64_t cap_muts, uint64_t cap_pool, uint64_t* n_muts,
+                           uint64_t* pool_len, uint64_t* chrom_size) {
+    if (!c) return JLP_ERR_ARG;
+    return guarded(c, [&]() {
+        if (hap >= c->haps.size() || chrom >= c->haps[hap].store->chrom.size()) throw ArgErr("haplotype / chromosome index out of range");
+        const HapChromHost& H = c->haps[hap].store->chrom[chrom];
+        const uint64_t M = H.n_muts;
+        if (n_muts) *n_muts = M;
+        if (pool_len) *pool_len = H.pool_bytes;
+        if (chrom_size) *chrom_size = H.size;
+        if (!old_pos) return;
+        if (M > cap_muts || H.pool_bytes > cap_pool) throw ArgErr("output arrays too small");
+        if (M && (!new_pos || !nuc_off)) throw ArgErr("new_pos / nuc_off is NULL");
+        if (H.pool_bytes && !pool) throw ArgErr("pool is NULL");
+        const uint64_t* w = H.packed.data();
+        if (M) {
+            std::memcpy(old_pos, w, M * 8);
+            std::memcpy(new_pos, w + M, M * 8);
+            std::memcpy(nuc_off, w + 2 * M, M * 8);
+        }
+        if (H.pool_bytes) std::memcpy(pool, w + 4 * M, H.pool_bytes);
+    });
+}
+
+// ---------------------------------------------------------------- create_haplotypes ---
+
+namespace {
+
+// The visiting order of the tree and the node-state slots (k_mutate): preorder with the child of fewer tips first, a
+// parent's slot freed when its last child is visited (before that child takes one), so at most about log2(tips) + 2
+// slots are live.  Childless nodes that are not tips are left out.
+std::vector<MutNode> mut_schedule(const jlp_mutation_params* p, const std::vector<int32_t>& tip_of, uint32_t n_cat,
+                                  uint32_t& max_slots) {
+    const uint32_t n = p->n_nodes;
+    std::vector<std::vector<uint32_t>> kids(n);
+    for (uint32_t i = 1; i < n; i++) kids[p->parent[i]].push_back(i);
+    std::vector<uint64_t> tips(n, 0);
+    for (uint32_t i = n; i-- > 0;) {
+        if (kids[i].empty()) tips[i] = tip_of[i] >= 0 ? 1 : 0;
+        if (i) tips[p->parent[i]] += tips[i];
+    }
+    for (auto& k : kids) std::stable_sort(k.begin(), k.end(), [&](uint32_t a, uint32_t b) { return tips[a] < tips[b]; });
+    std::vector<uint32_t> left(n), slot(n, 0), free_slots;
+    for (uint32_t i = 0; i < n; i++) left[i] = (uint32_t)kids[i].size();
+    for (uint32_t s = kMutSlots; s-- > 1;) free_slots.push_back((uint32_t)s);
+    max_slots = 1;
+    std::vector<MutNode> out;
+    std::vector<uint32_t> stack(kids[0].rbegin(), kids[0].rend());
+    while (!stack.empty()) {
+        const uint32_t v = stack.back();
+        stack.pop_back();
+        const uint32_t par = (uint32_t)p->parent[v];
+        MutNode m;
+        m.node = v;
+        m.tab = v * n_cat * 4;
+        m.tip = tip_of[v];
+        m.pslot = (uint16_t)slot[par];
+        m.slot = 0;
+        if (--left[par] == 0) free_slots.push_back(slot[par]);
+        if (!kids[v].empty()) {
+            if (free_slots.empty()) throw ArgErr("tree too deep for the node-state slots");
+            slot[v] = free_slots.back();
+            free_slots.pop_back();
+            m.slot = (uint16_t)slot[v];
+            max_slots = std::max<uint32_t>(max_slots, kMutSlots - (uint32_t)free_slots.size());
+            for (auto it = kids[v].rbegin(); it != kids[v].rend(); ++it) stack.push_back(*it);
+        }
+        if (!kids[v].empty() || m.tip >= 0) out.push_back(m);
+    }
+    return out;
+}
+
+struct EventSet {
+    cudaEvent_t e[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    EventSet() { for (cudaEvent_t& x : e) CK(cudaEventCreate(&x)); }
+    ~EventSet() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+    float ms(int a, int b) const { float t = 0; cudaEventElapsedTime(&t, e[a], e[b]); return t; }
+};
+
+}  // namespace
+
+int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation_stats* stats) {
+    if (!c || !p) return JLP_ERR_ARG;
+    return guarded(c, [&]() {
+        const auto t0 = std::chrono::steady_clock::now();
+        if (c->chrom_off.size() < 2) throw ArgErr("set the reference genome first");
+        for (int i = 0; i < 16; i++)
+            if (i % 5 && !(std::isfinite(p->Q[i]) && p->Q[i] >= 0)) throw ArgErr("the off-diagonal rates of Q must be finite and >= 0");
+        if (!(p->invariant >= 0 && p->invariant < 1)) throw ArgErr("invariant must be >= 0 and < 1");
+        if (p->n_rates < 1 || p->n_rates > 255 || !p->rates) throw ArgErr("n_rates must be 1..255 (rates not NULL)");
+        for (uint32_t k = 0; k < p->n_rates; k++)
+            if (!(std::isfinite(p->rates[k]) && p->rates[k] >= 0)) throw ArgErr("category rates must be finite and >= 0");
+        const uint32_t n = p->n_nodes;
+        if (n < 2 || n > kMutMaxNodes || !p->parent || !p->branch_len)
+            throw ArgErr("the tree needs 2 to " + std::to_string(kMutMaxNodes) + " nodes (parent / branch_len not NULL)");
+        if (p->parent[0] != -1) throw ArgErr("parent[0] must be -1 (the root comes first)");
+        std::vector<char> has_kid(n, 0);
+        for (uint32_t i = 1; i < n; i++) {
+            if (p->parent[i] < 0 || (uint32_t)p->parent[i] >= i) throw ArgErr("the tree must be in preorder: 0 <= parent[i] < i");
+            if (!(std::isfinite(p->branch_len[i]) && p->branch_len[i] >= 0)) throw ArgErr("branch lengths must be finite and >= 0");
+            has_kid[p->parent[i]] = 1;
+        }
+        if (p->n_tips < 1 || p->n_tips > kMutMaxTips)
+            throw ArgErr("a tree of " + std::to_string(p->n_tips) + " tips: 1 to " + std::to_string(kMutMaxTips) + " tips are supported");
+        if (!p->tip_node || !p->tip_names) throw ArgErr("tip_node / tip_names is NULL");
+        std::vector<int32_t> tip_of(n, -1);
+        for (uint32_t t = 0; t < p->n_tips; t++) {
+            const uint32_t v = p->tip_node[t];
+            if (v >= n || has_kid[v] || tip_of[v] >= 0) throw ArgErr("tip_node must list distinct childless nodes");
+            if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
+            tip_of[v] = (int32_t)t;
+        }
+        const uint64_t nc = c->chrom_off.size() - 1;
+        std::vector<uint32_t> tile0(nc + 1, 0);
+        for (uint64_t ci = 0; ci < nc; ci++) {
+            const uint64_t len = c->chrom_off[ci + 1] - c->chrom_off[ci];
+            if (len >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
+            const uint64_t t = tile0[ci] + (len + kMutTile - 1) / kMutTile;
+            if (t >> 32) throw ArgErr("genome too large");
+            tile0[ci + 1] = (uint32_t)t;
+        }
+        const uint32_t K = p->n_rates, n_tips = p->n_tips, n_tiles = tile0[nc];
+
+        // host tables: the schedule, per (node, category, parent state) the row thresholds, the category thresholds
+        uint32_t max_slots = 0;
+        const std::vector<MutNode> sched = mut_schedule(p, tip_of, K, max_slots);
+        const uint64_t rows = (uint64_t)n * K * 4;
+        std::vector<uint4> thr_hi(rows, make_uint4(0, 0, 0, 0)), thr_lo(rows, make_uint4(0, 0, 0, 0));
+        for (const MutNode& m : sched)
+            for (uint32_t k = 0; k < K; k++) {
+                double P[16];
+                transition_matrix(p->Q, p->rates[k] * p->branch_len[m.node], P);
+                for (uint32_t a = 0; a < 4; a++) {
+                    uint64_t t[3];
+                    row_thresholds(P + 4 * a, t);
+                    const uint64_t r = m.tab + 4ull * k + a;
+                    thr_hi[r] = make_uint4((uint32_t)(t[0] >> 32), (uint32_t)(t[1] >> 32), (uint32_t)(t[2] >> 32), 0);
+                    thr_lo[r] = make_uint4((uint32_t)t[0], (uint32_t)t[1], (uint32_t)t[2], 0);
+                }
+            }
+        std::vector<uint64_t> cat_thr(K);
+        cat_thr[0] = prob_threshold(p->invariant);
+        for (uint32_t j = 1; j < K; j++) cat_thr[j] = prob_threshold(p->invariant + j * (1 - p->invariant) / K);
+
+        jlp_ctx* d = first_device(c);
+        finish_upload(d);
+        cudaStream_t s = d->s_compute;
+        DevBuf<uint64_t> d_off, d_cat, d_region, d_region_n, d_out;
+        DevBuf<uint32_t> d_tile0, d_cnt;
+        DevBuf<MutNode> d_sched;
+        DevBuf<uint4> d_hi, d_lo;
+        d_off.upload(d->chrom_off, s);
+        d_tile0.upload(tile0, s);
+        d_sched.upload(sched, s);
+        d_cat.upload(cat_thr, s);
+        d_hi.upload(thr_hi, s);
+        d_lo.upload(thr_lo, s);
+        const size_t n_cnt = (size_t)n_tips * n_tiles;
+        d_cnt.ensure(n_cnt);
+        if (n_cnt) CK(cudaMemsetAsync(d_cnt.p, 0, n_cnt * 4, s));
+        d_region_n.ensure((size_t)n_tips * nc);
+        MutParams mp{};
+        mp.seed = p->seed;
+        mp.genome = d->genome.p + kPad;
+        mp.chrom_off = d_off.p;
+        mp.tile0 = d_tile0.p;
+        mp.n_chroms = (uint32_t)nc; mp.n_tiles = n_tiles; mp.n_tips = n_tips; mp.n_sched = (uint32_t)sched.size();
+        mp.sched = d_sched.p;
+        mp.n_cat = K;
+        mp.cat_thr = d_cat.p;
+        mp.thr_hi = d_hi.p; mp.thr_lo = d_lo.p;
+        mp.tab_rows = (uint32_t)rows;
+        mp.tab_smem = mut_smem_bytes((uint32_t)rows) <= (64u << 10);
+        mp.cnt = d_cnt.p;
+        EventSet ev;
+        CK(cudaEventRecord(ev.e[0], s));
+        CK(launch_mutate(mp, false, s));
+        CK(cudaEventRecord(ev.e[1], s));
+        CK(launch_mut_scan(mp, d_region_n.p, s));
+        CK(cudaEventRecord(ev.e[2], s));
+        std::vector<uint64_t> region_n((size_t)n_tips * nc), region((size_t)n_tips * nc);
+        CK(cudaMemcpyAsync(region_n.data(), d_region_n.p, region_n.size() * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        uint64_t words = 0, records = 0;
+        for (size_t r = 0; r < region.size(); r++) {
+            region[r] = words;
+            words += 4 * region_n[r] + (region_n[r] + 7) / 8;
+            records += region_n[r];
+        }
+        d_region.upload(region, s);
+        mp.region = d_region.p;
+        mp.region_n = d_region_n.p;              // k_mut_scan left the totals there
+        d_out.ensure(words);
+        if (words) CK(cudaMemsetAsync(d_out.p, 0, words * 8, s));
+        mp.out = d_out.p;
+        CK(cudaEventRecord(ev.e[3], s));
+        if (records) CK(launch_mutate(mp, true, s));
+        CK(cudaEventRecord(ev.e[4], s));
+        CK(cudaStreamSynchronize(s));
+        const float count_ms = ev.ms(0, 1), scan_ms = ev.ms(1, 2), write_ms = ev.ms(3, 4);
+        const auto t_gen = std::chrono::steady_clock::now();
+
+        // the records into one HapStore per tip, copied straight into the packed arrays by a few host threads
+        std::vector<std::shared_ptr<HapStore>> stores(n_tips);
+        for (uint32_t t = 0; t < n_tips; t++) {
+            stores[t] = std::make_shared<HapStore>();
+            stores[t]->name = p->tip_names[t];
+            stores[t]->chrom.resize(nc);
+        }
+        const size_t n_items = (size_t)n_tips * nc;
+        std::atomic<size_t> next{0};
+        std::mutex err_mu;
+        std::string err;
+        const int dev = d->device;
+        auto work = [&]() {
+            try {
+                CK(cudaSetDevice(dev));
+                for (size_t r; (r = next.fetch_add(1)) < n_items;) {
+                    HapChromHost& H = stores[r / nc]->chrom[r % nc];
+                    const uint64_t M = region_n[r];
+                    H.size = c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
+                    H.n_muts = M;
+                    H.pool_bytes = M;
+                    if (!M) continue;
+                    H.packed.resize(4 * M + (M + 7) / 8);
+                    CK(cudaMemcpy(H.packed.data(), d_out.p + region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
+                }
+            } catch (const std::exception& e) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = e.what(); }
+        };
+        const unsigned nt = records < (1u << 16) ? 1u
+                            : (unsigned)std::min<uint64_t>(std::min<uint64_t>(n_items, 16), std::max(1u, std::thread::hardware_concurrency()));
+        std::vector<std::thread> th;
+        for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
+        work();
+        for (std::thread& t : th) t.join();
+        if (!err.empty()) throw CudaErr(err);
+        CK(cudaSetDevice(dev));
+
+        for_each_device(c, [](jlp_ctx* k) { free_haps(k); });
+        c->haps.clear();
+        for (const auto& S : stores) {
+            attach_hap(c, S);
+            for (jlp_ctx* k : c->kids) attach_hap(k, S);
+        }
+        if (stats) {
+            const auto t1 = std::chrono::steady_clock::now();
+            stats->count_ms = count_ms;
+            stats->scan_ms = scan_ms;
+            stats->write_ms = write_ms;
+            stats->store_ms = std::chrono::duration<double, std::milli>(t1 - t_gen).count();
+            stats->total_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
+            stats->records = records;
+            stats->d2h_bytes = words * 8;
+            stats->table_bytes = rows * 2 * sizeof(uint4);
+            stats->table_in_smem = (int)mp.tab_smem;
+            stats->max_slots = max_slots;
+        }
+    });
+}
+
 int jlp_set_profile(jlp_ctx* c, int end, uint64_t read_length, const uint32_t* nq, const double* probs,
                     const uint8_t* quals) {
     if (!c) return JLP_ERR_ARG;
@@ -2310,6 +2572,11 @@ int jlp_reads_per_group(uint64_t n_reads, const double* probs, uint64_t n, uint6
     if (!probs || !out) return JLP_ERR_ARG;
     std::vector<uint64_t> r = reads_per_group(n_reads, std::vector<double>(probs, probs + n), seed);
     std::copy(r.begin(), r.end(), out);
+    return JLP_OK;
+}
+int jlp_transition_matrix(const double Q[16], double t, double P[16]) {
+    if (!Q || !P || !(t >= 0) || !std::isfinite(t)) return JLP_ERR_ARG;
+    transition_matrix(Q, t, P);
     return JLP_OK;
 }
 int jlp_alias_build(const double* probs, uint64_t n, double* prob_out, uint64_t* alias_out) {

@@ -38,7 +38,8 @@
 
 namespace jlp {
 
-enum Plane : uint32_t { PL_PAIR = 0, PL_INDEL = 1, PL_QUAL = 2, PL_SLOW = 3, PL_GENOME = 4, PL_GSLOW = 5 };
+// plane 6 is the oracle's PacBio plane
+enum Plane : uint32_t { PL_PAIR = 0, PL_INDEL = 1, PL_QUAL = 2, PL_SLOW = 3, PL_GENOME = 4, PL_GSLOW = 5, PL_MUT = 7, PL_MSLOW = 8 };
 enum Purpose : uint32_t { PU_INDEL = 0, PU_DIE = 1, PU_COIN = 2, PU_MIS = 3, PU_SUB = 4, PU_INS = 5 };
 
 struct U4 { uint32_t w0, w1, w2, w3; };
@@ -157,6 +158,23 @@ JLP_HD uint64_t genome_draw(uint64_t seed, uint32_t chrom, uint64_t b, uint32_t 
     const uint64_t s = genome_slow(seed, chrom, b, which);
     if (which == 0) return ((uint64_t)(w >> 30) << 62) | (s & (~0ull >> 2));
     return ((uint64_t)((w >> 14) & 0xffffu) << 48) | (s & (~0ull >> 16));
+}
+
+// ---- draws of the haplotype mutator (create_haplotypes): chromosome c, site b, tree node v ----
+//   X(c, b, v) is one 64-bit draw; node 0 (the root, which has no branch) gives the site's rate-category draw,
+//   node v >= 1 the transition draw of the branch above v.  v < 2^24.
+//   plane MUT  : counter (b>>2 lo, b>>2 hi, c, PL_MUT | v<<8), word b&3 = high 32 bits of X(c, b, v)
+//   plane MSLOW: counter (b lo, b hi, c, PL_MSLOW | v<<8), w0 = low 32 bits of X(c, b, v)
+//   Decisions compare the high word with the thresholds' high words and fetch the MSLOW block only on equality.
+JLP_HD U4 mut_block(uint64_t seed, uint32_t chrom, uint64_t b4, uint32_t node) {
+    return philox4x32_10((uint32_t)b4, (uint32_t)(b4 >> 32), chrom, PL_MUT | (node << 8), (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+JLP_HD uint32_t mut_low(uint64_t seed, uint32_t chrom, uint64_t b, uint32_t node) {
+    return philox4x32_10((uint32_t)b, (uint32_t)(b >> 32), chrom, PL_MSLOW | (node << 8), (uint32_t)seed, (uint32_t)(seed >> 32)).w0;
+}
+JLP_HD uint64_t mut_draw(uint64_t seed, uint32_t chrom, uint64_t b, uint32_t node) {
+    const uint32_t h = genome_word(mut_block(seed, chrom, b >> 2, node), (uint32_t)b & 3u);
+    return ((uint64_t)h << 32) | mut_low(seed, chrom, b, node);
 }
 
 // ---- exact restatements of the reference's uses of u = runif_01(x) ----

@@ -289,4 +289,61 @@ std::vector<uint64_t> split_int(uint64_t x, uint64_t n) {
     return out;
 }
 
+// --- substitution model (create_haplotypes) ------------------------------------
+
+void transition_matrix(const double Q[16], double t, double P[16]) {
+    for (int i = 0; i < 16; i++) P[i] = (i % 5 == 0) ? 1.0 : 0.0;
+    if (t == 0) return;
+    // A = Q t with the diagonal made minus the row sum; scaled by 2^-s so that ||A||_1 <= 1, Taylor series to
+    // 30 terms (remainder < 1/30!), then squared s times
+    double A[16], norm = 0;
+    for (int i = 0; i < 4; i++) {
+        double row = 0;
+        for (int j = 0; j < 4; j++) if (j != i) { A[4 * i + j] = Q[4 * i + j] * t; row += A[4 * i + j]; }
+        A[5 * i] = -row;
+    }
+    for (int j = 0; j < 4; j++) {
+        double col = 0;
+        for (int i = 0; i < 4; i++) col += std::fabs(A[4 * i + j]);
+        norm = std::max(norm, col);
+    }
+    int s = 0;
+    if (norm > 1) s = std::min(1000, (int)std::ceil(std::log2(norm)));
+    const double sc = std::ldexp(1.0, -s);
+    for (double& a : A) a *= sc;
+    double term[16], next[16];
+    for (int i = 0; i < 16; i++) term[i] = P[i];
+    for (int k = 1; k <= 30; k++) {
+        for (int i = 0; i < 4; i++)
+            for (int j = 0; j < 4; j++) {
+                double acc = 0;
+                for (int m = 0; m < 4; m++) acc += term[4 * i + m] * A[4 * m + j];
+                next[4 * i + j] = acc / k;
+            }
+        for (int i = 0; i < 16; i++) { term[i] = next[i]; P[i] += next[i]; }
+    }
+    for (int r = 0; r < s; r++) {
+        for (int i = 0; i < 4; i++)
+            for (int j = 0; j < 4; j++) {
+                double acc = 0;
+                for (int m = 0; m < 4; m++) acc += P[4 * i + m] * P[4 * m + j];
+                next[4 * i + j] = acc;
+            }
+        for (int i = 0; i < 16; i++) P[i] = next[i];
+    }
+}
+
+uint64_t prob_threshold(double c) {
+    if (!(c > 0)) return 0;
+    if (c >= 1) return ~0ull;
+    return (uint64_t)std::ldexp(c, 64);
+}
+
+void row_thresholds(const double* row, uint64_t thr[3]) {
+    double p[4], sum = 0;
+    for (int j = 0; j < 4; j++) { p[j] = row[j] > 0 ? row[j] : 0.0; sum += p[j]; }
+    double c = 0;
+    for (int j = 0; j < 3; j++) { c += p[j] / sum; thr[j] = prob_threshold(c); }
+}
+
 }  // namespace jlp

@@ -67,5 +67,14 @@ std::vector<uint64_t> reads_per_group(uint64_t n_reads, std::vector<double> prob
 // split_int, src/util.h:245-258
 std::vector<uint64_t> split_int(uint64_t x, uint64_t n);
 
+// --- substitution model (create_haplotypes) -------------------------------------
+// P = expm(Q t), 4x4 in T,C,A,G, Q's diagonal taken as minus the off-diagonal row sum; t == 0 gives exactly I
+void transition_matrix(const double Q[16], double t, double P[16]);
+// a cumulative probability as a draw threshold: floor(c 2^64), 0 for c <= 0, 2^64 - 1 for c >= 1
+uint64_t prob_threshold(double c);
+// one row of P as the thresholds of a 64-bit draw X: new state = #{j < 3 : X >= thr[j]}; the row is clipped at 0
+// and renormalised, thr[j] = prob_threshold(p[0] + ... + p[j])
+void row_thresholds(const double* row, uint64_t thr[3]);
+
 }  // namespace jlp
 #endif

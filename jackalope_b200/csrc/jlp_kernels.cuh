@@ -96,6 +96,48 @@ struct GenomeTables {
 cudaError_t launch_create_chrom(uint8_t* out, uint64_t len, uint32_t chrom, uint64_t seed, const GenomeTables& t,
                                 cudaStream_t s);
 
+// create_haplotypes: substitutions along a tree (jlp_mutate.cu).  A warp owns a tile of kMutTile consecutive sites
+// of one chromosome, a lane 4 consecutive sites per 128-site step; the states of the live internal nodes sit in
+// shared memory, 2 bits per site, one byte per (slot, lane).
+constexpr uint32_t kMutWarps = 8;                  // warps per CTA
+constexpr uint32_t kMutSteps = 64;                 // 128-site steps per tile
+constexpr uint32_t kMutTile = 128 * kMutSteps;     // sites per tile
+constexpr uint32_t kMutSlots = 32;                 // node-state slots per lane
+constexpr uint32_t kMutMaxTips = 4096;
+constexpr uint32_t kMutMaxNodes = 65536;
+
+struct MutNode {          // a non-root node in visiting order
+    uint32_t node;        // index in the caller's preorder: addresses the draws
+    uint32_t tab;         // its first threshold row: row = tab + 4 * category + parent state
+    int32_t tip;          // tip index, or -1 for an internal node
+    uint16_t pslot;       // slot holding the parent's states
+    uint16_t slot;        // slot receiving this node's states (internal nodes)
+};
+
+struct MutParams {
+    uint64_t seed;
+    const uint8_t* genome;       // reference bases; chromosome c at chrom_off[c]
+    const uint64_t* chrom_off;   // [n_chroms + 1]
+    const uint32_t* tile0;       // [n_chroms + 1] first tile of each chromosome
+    uint32_t n_chroms, n_tiles, n_tips, n_sched;
+    const MutNode* sched;        // [n_sched]
+    uint32_t n_cat;              // rate categories of the variable sites
+    const uint64_t* cat_thr;     // [n_cat]: index = #{j : X_cat >= cat_thr[j]}; 0 = invariant, k = category k - 1
+    const uint4* thr_hi;         // [rows] high words of the three thresholds of a row (.w unused)
+    const uint4* thr_lo;         // [rows] low words
+    uint32_t tab_rows;
+    uint32_t tab_smem;           // 1: stage thr_hi in shared memory (thr_lo, read only on ties, stays in global memory)
+    uint32_t* cnt;               // [n_tips][n_tiles]: pass 1 counts; after k_mut_scan each tile's first record in its region
+    uint64_t* out;               // pass 2: the packed regions (HapChromHost::packed layout)
+    const uint64_t* region;      // [n_tips][n_chroms] word offset of the region in `out`
+    const uint64_t* region_n;    // [n_tips][n_chroms] records of the region
+};
+// pass 1 (write = false): records per (tip, tile) added into cnt; pass 2 (write = true): records written
+cudaError_t launch_mutate(const MutParams& p, bool write, cudaStream_t s);
+// exclusive scan of every (tip, chromosome) run of cnt in place; region_n receives the totals
+cudaError_t launch_mut_scan(const MutParams& p, uint64_t* region_n, cudaStream_t s);
+size_t mut_smem_bytes(uint32_t tab_rows);
+
 // fragment placement + indel summary + record lengths, one thread per read end
 cudaError_t launch_place(const GenParams& p, cudaStream_t s);
 
