@@ -5,7 +5,6 @@
 
 #include <cuda_runtime.h>
 #include <fcntl.h>
-#include <sys/mman.h>
 #include <sys/stat.h>
 #include <sys/statvfs.h>
 #include <unistd.h>
@@ -16,7 +15,6 @@
 #include <cerrno>
 #include <chrono>
 #include <cmath>
-#include <condition_variable>
 #include <deque>
 #include <functional>
 #include <mutex>
@@ -33,6 +31,7 @@
 #include "jlp_draws.h"
 #include "jlp_host.h"
 #include "jlp_kernels.cuh"
+#include "jlp_output.h"
 #include "jlp_pacbio.h"
 
 using namespace jlp;
@@ -44,22 +43,6 @@ std::string g_create_error;
 // Bytes of padding in front of and behind every sequence allocation: the read kernel
 // fetches template bases as aligned words and may touch a few bytes outside a chromosome.
 constexpr size_t kPad = 64;
-
-struct CudaErr : std::runtime_error {
-    explicit CudaErr(const std::string& m) : std::runtime_error(m) {}
-};
-struct ArgErr : std::runtime_error {
-    explicit ArgErr(const std::string& m) : std::runtime_error(m) {}
-};
-struct IoErr : std::runtime_error {
-    explicit IoErr(const std::string& m) : std::runtime_error(m) {}
-};
-struct Unsupported : std::runtime_error {
-    explicit Unsupported(const std::string& m) : std::runtime_error(m) {}
-};
-struct Aborted : std::runtime_error {
-    Aborted() : std::runtime_error("aborted by user") {}
-};
 
 #define CK(call)                                                                          \
     do {                                                                                  \
@@ -98,96 +81,6 @@ template <typename T> struct PinBuf {
     }
     ~PinBuf() { if (p) cudaFreeHost(p); }
 };
-
-// Host writer threads: the FASTQ of a batch sits in a pinned buffer; its slices are written
-// with pwrite() at their final file offsets while the GPU generates and copies the next
-// batch (the reference's threads serialise on one omp critical per pool instead,
-// src/hts.h:401-416).
-class WriterPool {
-public:
-    // a task returns an error text (empty = fine); `pending` counts the tasks of one batch slot
-    struct Task { std::function<std::string()> run; std::atomic<int>* pending; };
-    ~WriterPool() { stop(); }
-    void start(size_t n_threads) {
-        if (th.size() == n_threads) return;
-        stop();
-        quit = false;
-        for (size_t i = 0; i < n_threads; i++) th.emplace_back([this]() { loop(); });
-    }
-    void stop() {
-        { std::lock_guard<std::mutex> l(m); quit = true; }
-        cv.notify_all();
-        for (std::thread& t : th) t.join();
-        th.clear();
-    }
-    void submit(std::atomic<int>* pending, std::function<std::string()> f) {
-        pending->fetch_add(1);
-        { std::lock_guard<std::mutex> l(m); q.push_back(Task{std::move(f), pending}); }
-        cv.notify_one();
-    }
-    // wait until every task counted by `pending` is done; returns the first error text (empty = none)
-    std::string wait(std::atomic<int>& pending) {
-        std::unique_lock<std::mutex> l(m);
-        cv_done.wait(l, [&]() { return pending.load() == 0; });
-        return err;
-    }
-    void clear_error() { std::lock_guard<std::mutex> l(m); err.clear(); }
-private:
-    void loop() {
-        for (;;) {
-            Task t;
-            {
-                std::unique_lock<std::mutex> l(m);
-                cv.wait(l, [&]() { return quit || !q.empty(); });
-                if (q.empty()) return;
-                t = std::move(q.front()); q.pop_front();
-            }
-            std::string e = t.run();
-            {
-                std::lock_guard<std::mutex> l(m);
-                if (!e.empty() && err.empty()) err = e;
-                t.pending->fetch_sub(1);
-            }
-            cv_done.notify_all();
-        }
-    }
-    std::vector<std::thread> th;
-    std::mutex m;
-    std::condition_variable cv, cv_done;
-    std::deque<Task> q;
-    std::string err;
-    bool quit = false;
-};
-
-std::string pwrite_all(int fd, const uint8_t* p, uint64_t n, uint64_t off) {
-    while (n) {
-        ssize_t w = ::pwrite(fd, p, n > (1u << 30) ? (1u << 30) : n, (off_t)off);
-        if (w < 0) { if (errno == EINTR) continue; return std::strerror(errno); }
-        p += w; n -= (uint64_t)w; off += (uint64_t)w;
-    }
-    return std::string();
-}
-
-// Files are also written through shared mappings: the main thread extends the file by a batch and maps the new
-// range once, the writer threads copy their slices into the mapping (page-cache pages are allocated and filled by
-// the copying thread, so the threads do not queue on the inode lock that serialises write() calls on one file;
-// measured on the B200 box's tmpfs: 7.4 GB/s with pwrite from any number of threads, 14 GB/s with 16 threads
-// copying into mappings, tools/write_probe.cpp), and the range is unmapped when the batch's slices are done --
-// one munmap per batch and file, not one TLB shoot-down per slice.
-struct Mapping {
-    void* base = nullptr;
-    size_t len = 0;
-    uint8_t* at = nullptr;      // where the batch's first byte goes
-    void unmap() { if (base) ::munmap(base, len); base = nullptr; len = 0; at = nullptr; }
-};
-bool map_range(int fd, uint64_t off, uint64_t n, Mapping& m) {
-    static const uint64_t page = (uint64_t)sysconf(_SC_PAGESIZE);
-    const uint64_t a0 = off / page * page;
-    void* p = ::mmap(nullptr, (size_t)(off + n - a0), PROT_READ | PROT_WRITE, MAP_SHARED, fd, (off_t)a0);
-    if (p == MAP_FAILED) return false;
-    m.base = p; m.len = (size_t)(off + n - a0); m.at = static_cast<uint8_t*>(p) + (off - a0);
-    return true;
-}
 
 // AllMutations of one haplotype chromosome (src/hap_classes.h:100-104) as the library keeps them on the host:
 // a haplotype chromosome is materialised on a device only when a run's pair range touches it (SURVEY.md 8e:
@@ -238,10 +131,7 @@ struct Slot {
     uint64_t tot[2] = {0, 0};     // FASTQ bytes of the batch per file (read back from the device)
     uint64_t ztot[2] = {0, 0};    // compressed bytes of the batch per file (device BGZF)
     bool busy = false;
-    std::atomic<int> writes{0};   // slices of h_out still being written to / compressed for the files
-    std::vector<std::vector<uint8_t>> zout[2];   // compressed slices of the batch, in file order
-    Mapping map[2];               // the file ranges this batch is being copied into
-    uint64_t file_end[2] = {0, 0};  // where this batch ends in the files (plain FASTQ)
+    HostBatch host;               // h_out on its way into the files
 };
 
 }  // namespace
@@ -282,13 +172,8 @@ struct jlp_ctx {
     uint64_t h2d_bytes = 0;
     // scratch of the haplotype materialisation (mutation records of one chromosome)
     HapArena hap_mem;
-    // PacBio driver: FASTQ of a batch on the device, its compressed form, and the two pinned host buffers batches alternate between
-    DevBuf<uint8_t> pb_out, pb_zslots, pb_zout, pb_strpool, pb_zcode;
+    // PacBio driver: the per-read plan of a batch (its other buffers are those of the slots)
     DevBuf<PbRead> pb_reads;
-    DevBuf<GroupDev> pb_groups;
-    DevBuf<uint32_t> pb_rec_len, pb_rec_local, pb_zlen;
-    DevBuf<uint64_t> pb_block_tot, pb_block_base, pb_totals, pb_zoff;
-    PinBuf<uint8_t> pb_h_buf[2];
     // PacBioPassSampler's outlier thresholds (one chi-squared quantile per read length up to chi2_params_n[2]) of the last call
     std::shared_ptr<std::atomic<double>[]> pb_qcache;
     double pb_qcache_key[3] = {0, 0, 0};
@@ -389,28 +274,6 @@ void finish_upload(jlp_ctx* c) {
 
 // ---------------------------------------------------------------- the run ---
 
-enum SinkKind { SINK_FILES, SINK_MEMORY, SINK_STREAM, SINK_NONE };
-
-struct Sink {
-    SinkKind kind = SINK_NONE;
-    // memory
-    char* mem[2] = {nullptr, nullptr};
-    uint64_t cap[2] = {0, 0}, len[2] = {0, 0};
-    // stream
-    jlp_chunk_cb chunk_cb = nullptr;
-    void* chunk_user = nullptr;
-    // files
-    int fd[2] = {-1, -1};
-    uint64_t pos[2] = {0, 0};        // where the next batch goes
-    uint64_t done[2] = {0, 0};       // end of the last batch known to be completely written (error paths truncate back to it)
-    bool own_size[2] = {false, false};   // this call extends the file itself (not a pre-sized file shared with other devices)
-    std::string names[2];
-    void close_files() {
-        for (int e = 0; e < 2; e++) if (fd[e] >= 0) { ::close(fd[e]); fd[e] = -1; }
-    }
-    ~Sink() { close_files(); }
-};
-
 struct Job {
     uint64_t lo, hi;          // pair-instance range
     std::string file_prefix;  // <prefix> or <prefix>_<hap>
@@ -455,17 +318,35 @@ std::vector<std::vector<uint64_t>> apportion_sizes(uint64_t seed, uint64_t n_pai
     return out;
 }
 
+// What a run's groups and jobs depend on besides the context, from the parameters of either driver (which name these
+// fields alike); Illumina adds its barcodes.
+struct LayoutSpec {
+    uint64_t seed;
+    uint64_t n_units;                          // pairs (Illumina: floor(n_reads / n_ends)) or reads (PacBio)
+    bool use_haps;                             // the haplotypes, else the reference
+    const double* hap_probs;
+    const char* const* barcodes = nullptr;     // one per haplotype (one for the reference), or NULL
+    uint32_t read_len = 0;                     // a barcode must be shorter than the read
+    bool sep_files;                            // one job per haplotype
+    const char* prefix;
+    template <typename Params> LayoutSpec(bool haps, const Params* P, uint64_t units)
+        : seed(P->seed), n_units(units), use_haps(haps), hap_probs(P->haplotype_probs), sep_files(P->sep_files != 0),
+          prefix(P->out_prefix) {}
+};
+
 // needs only the sizes: works on a multi-GPU parent context (metadata, no device state) as well
-std::vector<std::vector<uint64_t>> apportion(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, uint64_t n_pairs) {
+std::vector<std::vector<uint64_t>> apportion(const jlp_ctx* c, const LayoutSpec& S) {
+    if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
+    if (S.use_haps && c->haps.empty()) throw ArgErr("no haplotypes have been added");
     const uint64_t n_chroms = c->chrom_off.size() - 1;
     std::vector<uint64_t> sizes;
-    if (!use_haps) {
+    if (!S.use_haps) {
         for (uint64_t i = 0; i < n_chroms; i++) sizes.push_back(c->chrom_off[i + 1] - c->chrom_off[i]);
-        return apportion_sizes(P->seed, n_pairs, 1, n_chroms, nullptr, sizes.data());
+        return apportion_sizes(S.seed, S.n_units, 1, n_chroms, nullptr, sizes.data());
     }
-    if (!P->haplotype_probs) throw ArgErr("haplotype_probs is NULL");
+    if (!S.hap_probs) throw ArgErr("haplotype_probs is NULL");
     for (const HapDev& h : c->haps) sizes.insert(sizes.end(), h.len.begin(), h.len.end());
-    return apportion_sizes(P->seed, n_pairs, c->haps.size(), n_chroms, P->haplotype_probs, sizes.data());
+    return apportion_sizes(S.seed, S.n_units, c->haps.size(), n_chroms, S.hap_probs, sizes.data());
 }
 
 // How a run's compressed output is produced (write_reads_cpp_, src/hts.h:441-500): compressed + one thread -> the
@@ -476,11 +357,6 @@ std::vector<std::vector<uint64_t>> apportion(const jlp_ctx* c, bool use_haps, co
 // would write BGZF (comp_method "bgzip", or several threads) at levels 1..6; a gzip request with one thread is a
 // gzip stream from zlib (FileGZ, src/io.h:140-236).  Memory and stream sinks receive compressed bytes only when the
 // device coder is asked for explicitly.
-struct Compression {
-    bool dev_z = false;       // BGZF on the device
-    int zmethod = -1;         // host zlib: DEFLATE_BGZF / DEFLATE_GZIP; -1 = none
-    bool want_gz = false;     // file names get ".gz"
-};
 Compression compression_of(const jlp_illumina_params* P, SinkKind kind) {
     Compression z;
     if (P->compress <= 0) return z;
@@ -530,7 +406,6 @@ void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P,
 // jobs (= sets of output files).  A pure function of the parameters and of the sizes the context knows, so every
 // device of a multi-GPU run builds the same one.
 struct Layout {
-    int n_ends = 1;
     uint64_t n_pairs = 0;
     std::vector<uint64_t> group_off;      // [n_groups + 1]
     std::vector<GroupDev> groups;         // seq is filled in per device
@@ -539,26 +414,24 @@ struct Layout {
     std::vector<Job> jobs;
 };
 
-Layout make_layout(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P) {
+Layout make_layout(const jlp_ctx* c, const LayoutSpec& S) {
     Layout Y;
-    Y.n_ends = P->paired || P->matepair ? 2 : 1;
-    const uint32_t L = (uint32_t)c->tab[0].L;
     const uint64_t n_haps = c->haps.size(), n_chroms = c->chrom_off.size() - 1;
-    const bool sep = use_haps && P->sep_files;
+    const bool use_haps = S.use_haps, sep = use_haps && S.sep_files;
     // --- barcodes (T/C/A/G only, R/hts_illumina.R:385-391)
     std::vector<std::string> barcodes(use_haps ? n_haps : 1);
-    if (P->barcodes)
-        for (size_t i = 0; i < barcodes.size(); i++) barcodes[i] = P->barcodes[i] ? P->barcodes[i] : "";
-    for (const std::string& bcs : barcodes) {
-        for (char ch : bcs)
-            if (ch != 'T' && ch != 'C' && ch != 'A' && ch != 'G') throw ArgErr("barcodes may only contain T, C, A, G");
-        if (bcs.size() >= L) throw ArgErr("a barcode is as long as the read");
-    }
+    if (S.barcodes)
+        for (size_t i = 0; i < barcodes.size(); i++) {
+            barcodes[i] = S.barcodes[i] ? S.barcodes[i] : "";
+            for (char ch : barcodes[i])
+                if (ch != 'T' && ch != 'C' && ch != 'A' && ch != 'G') throw ArgErr("barcodes may only contain T, C, A, G");
+            if (barcodes[i].size() >= S.read_len) throw ArgErr("a barcode is as long as the read");
+        }
     // --- apportion pairs: threads -> haplotypes -> chromosomes
     //     (write_reads_one_filetype_ src/hts.h:334-353, add_n_reads src/hts_illumina.h:410-418, :620-644,
-    //      write_reads_cpp_sep_files_ src/hts.h:527-529); one "thread", n_pairs = floor(n_reads / n_ends)
-    Y.n_pairs = P->n_reads / Y.n_ends;
-    const std::vector<std::vector<uint64_t>> counts = apportion(c, use_haps, P, Y.n_pairs);
+    //      write_reads_cpp_sep_files_ src/hts.h:527-529; PacBioOneGenome::add_n_reads, src/hts_pacbio.h); one "thread"
+    Y.n_pairs = S.n_units;
+    const std::vector<std::vector<uint64_t>> counts = apportion(c, S);
     Y.group_off.assign(1, 0);
     auto add_group = [&](const std::string& gname, uint32_t hap, uint64_t chrom, uint64_t len, const std::string& bc, uint64_t count) {
         GroupDev g;
@@ -573,7 +446,7 @@ Layout make_layout(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P
         Y.group_off.push_back(Y.group_off.back() + count);
         if (count > 0 && len == 0) throw ArgErr("a chromosome of length 0 was given reads");
     };
-    const std::string prefix = P->out_prefix ? P->out_prefix : "";
+    const std::string prefix = S.prefix ? S.prefix : "";
     if (!use_haps) {
         for (uint64_t i = 0; i < n_chroms; i++)
             add_group(c->genome_name, 0, i, c->chrom_off[i + 1] - c->chrom_off[i], barcodes[0], counts[0][i]);
@@ -591,13 +464,20 @@ Layout make_layout(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P
     return Y;
 }
 
+LayoutSpec illumina_spec(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P) {
+    LayoutSpec S(use_haps, P, P->n_reads / (P->paired || P->matepair ? 2 : 1));
+    S.barcodes = P->barcodes;
+    S.read_len = (uint32_t)c->tab[0].L;
+    return S;
+}
+
 // name of output file `e` of a job (src/hts.h:344; ".gz" appended by FileGZ / FileBGZF, src/io.h:126,217).
 // A process that generates one shard of a run (shard_count > 1, one process per GPU) writes its own files,
 // <prefix>[_<hap>]_R<k>.fq[.gz].shard<i>of<n>: concatenated in shard order they are the unsharded run's file.
 std::string file_name(const Job& job, int e, bool gz, const jlp_illumina_params* P) {
     std::string n = job.file_prefix + "_R" + std::to_string(e + 1) + ".fq";
     if (gz) n += ".gz";
-    if (P->shard_count > 1) n += ".shard" + std::to_string(P->shard_index) + "of" + std::to_string(P->shard_count);
+    if (P && P->shard_count > 1) n += ".shard" + std::to_string(P->shard_index) + "of" + std::to_string(P->shard_count);
     return n;
 }
 
@@ -639,28 +519,44 @@ struct RunExtras {
     PerJobBytes* sizes_out = nullptr;     // size pass: only count the FASTQ bytes per job and end of those ranges
     const PerJobBytes* base = nullptr;    // [jobs] where this call's bytes start in each job's files / in the memory sink
     bool shared_files = false;            // the files exist, created and sized by the caller: open without truncating, no EOF block
-    std::string part_suffix;              // compressed multi-GPU runs: this call writes <name><suffix>, joined by the caller
-    bool no_eof = false;                  // ... and the caller appends the BGZF end-of-file block
-    const std::vector<std::string>* job_suffix = nullptr;   // [jobs] the same per job (overrides part_suffix)
+    // [jobs] compressed multi-GPU runs: this call writes <name><suffix>, joined by the caller, who appends the BGZF
+    // end-of-file block
+    const std::vector<std::string>* job_suffix = nullptr;
     PerJobBytes* zsizes_out = nullptr;    // the compressed bytes per job and end this call produced (device coder)
     bool dry_files = false;               // generate and compress as for files, deliver nothing (sink NONE): the compressed size pass
 };
 
-void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jlp_run_stats* stats, const RunExtras& X = RunExtras()) {
+// If a run ends by an exception, nothing of it may stay in flight: kernels and copies still use the slots, writer
+// tasks still hold the file descriptors the caller's Output is about to close.  Files the run extends itself are cut
+// back to the last completely written batch (an extended, never filled tail would otherwise stay behind as zero bytes).
+struct Quiesce {
+    jlp_ctx* c;
+    Output* out;
+    bool armed = true;
+    ~Quiesce() {
+        if (!armed) return;
+        cudaStreamSynchronize(c->s_compute);
+        cudaStreamSynchronize(c->s_copy);
+        HostBatch* b[3];
+        for (int k = 0; k < 3; k++) { c->slot[k].busy = false; b[k] = &c->slot[k].host; }
+        out->abandon(b, 3);
+    }
+};
+
+void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, jlp_run_stats* stats, const RunExtras& X = RunExtras()) {
     check_params(c, use_haps, P, sink.kind);
     const int n_ends = P->paired || P->matepair ? 2 : 1;
     const bool matepair = P->matepair != 0;
     if (use_haps) finish_upload(c);
     const uint64_t h2d_before = c->h2d_bytes;
     const Compression Z = compression_of(P, X.dry_files ? SINK_FILES : sink.kind);
-    const bool dev_z = Z.dev_z, want_gz = Z.want_gz;
-    const int zmethod = Z.zmethod;
+    const bool dev_z = Z.dev_z;
     const bool sizes_only = X.sizes_out != nullptr;
     if (X.zsizes_out) X.zsizes_out->assign(X.ranges ? X.ranges->size() : 0, std::array<uint64_t, 2>{0, 0});
     const double insp[2] = {P->ins_prob1, P->ins_prob2}, delp[2] = {P->del_prob1, P->del_prob2};
     const uint32_t L = (uint32_t)c->tab[0].L;
 
-    Layout Y = make_layout(c, use_haps, P);
+    Layout Y = make_layout(c, illumina_spec(c, use_haps, P));
     const std::vector<uint64_t>& group_off = Y.group_off;
     std::vector<GroupDev>& groups = Y.groups;
     const std::vector<Job>& jobs = Y.jobs;
@@ -781,51 +677,9 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
     jlp_run_stats st;
     std::memset(&st, 0, sizeof st);
 
-    // If the run ends by an exception, nothing of it may stay in flight: kernels and copies still use the
-    // slots, writer tasks still hold the file descriptors the caller's Sink is about to close.  Files this call
-    // extends itself are cut back to the last completely written batch (an extended, never filled tail would
-    // otherwise stay behind as zero bytes).
-    struct Quiesce {
-        jlp_ctx* c;
-        Sink* sink;
-        bool armed = true;
-        ~Quiesce() {
-            if (!armed) return;
-            cudaStreamSynchronize(c->s_compute);
-            cudaStreamSynchronize(c->s_copy);
-            for (Slot& s : c->slot) {
-                c->writers.wait(s.writes);
-                for (Mapping& m : s.map) m.unmap();
-                s.busy = false;
-                s.zout[0].clear(); s.zout[1].clear();
-            }
-            c->writers.clear_error();
-            if (sink->kind == SINK_FILES)
-                for (int e = 0; e < 2; e++)
-                    if (sink->fd[e] >= 0 && sink->own_size[e] && ::ftruncate(sink->fd[e], (off_t)sink->done[e]) != 0) { /* best effort */ }
-        }
-    } quiesce{c, &sink};
-
-    auto wait_writes = [&](Slot& s) {
-        if (sink.kind != SINK_FILES) return;
-        std::string e = c->writers.wait(s.writes);
-        for (Mapping& m : s.map) m.unmap();
-        if (!e.empty()) { c->writers.clear_error(); throw IoErr("Error writing to file " + sink.names[0] + " / " + sink.names[1] + ": " + e); }
-        // compressed slices of the slot's batch go to the files in order
-        for (int k = 0; k < n_ends; k++) {
-            for (std::vector<uint8_t>& v : s.zout[k]) {
-                std::string w = pwrite_all(sink.fd[k], v.data(), v.size(), sink.pos[k]);
-                if (!w.empty()) throw IoErr("Error writing to file " + sink.names[k] + ": " + w);
-                sink.pos[k] += v.size();
-            }
-            s.zout[k].clear();
-            if (s.file_end[k] > sink.done[k]) sink.done[k] = s.file_end[k];
-            if (zmethod >= 0) sink.done[k] = sink.pos[k];
-        }
-    };
-    if (sink.kind == SINK_FILES && !sizes_only) c->writers.start((size_t)std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 1), 64));
+    sink.begin(Z, P->compress, P->n_threads, c->writers);
+    Quiesce quiesce{c, &sink};
     uint64_t job_index = 0;
-    Slot* z_pending = nullptr;      // the batch whose compressed slices are not in the files yet
     // stage 2 of a batch: its kernels are done -> statistics, then its FASTQ starts its way to the host
     // (queued right behind the previous batch's copy, so the bus never idles)
     auto issue_copy = [&](Slot& s) {
@@ -845,8 +699,7 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
         st.pairs += s.pairs;
         st.batches++;
         if (!need_host) return;
-        if (z_pending == &s) { wait_writes(s); z_pending = nullptr; }
-        wait_writes(s);                         // the pinned buffers of this slot are free again
+        sink.settle(s.host);                    // the pinned buffers of this slot are free again
         for (int e = 0; e < n_ends; e++) {
             const uint64_t nb = dev_z ? s.ztot[e] : s.tot[e];
             CK(cudaMemcpyAsync(s.h_out[e].p, dev_z ? s.zdev[e].p : s.out[e].p, nb, cudaMemcpyDeviceToHost, c->s_copy));
@@ -858,77 +711,9 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
     auto deliver = [&](Slot& s) {
         if (need_host) {
             CK(cudaEventSynchronize(s.ev[4]));
-            if (zmethod >= 0 && z_pending) { wait_writes(*z_pending); z_pending = nullptr; }   // files stay in batch order
-            for (int e = 0; e < n_ends; e++) {
-                const uint64_t n = dev_z ? s.ztot[e] : s.tot[e];
-                s.file_end[e] = 0;
-                if (sink.kind == SINK_FILES && zmethod < 0) {
-                    // R1 and R2 stay record-aligned: both files receive the same batches in the same order.
-                    // With several writer threads the file is extended and the batch's range mapped; ONE task per file
-                    // reserves the range's pages (posix_fallocate: a full file system is an error in that task, not a
-                    // SIGBUS later) and then hands the 8 MiB slices to the pool, which copies them into the mapping.
-                    // Page allocation is what the kernel serialises per file and it costs more than the copy, so it
-                    // must neither sit on the driver thread nor be fought over by all the writers (tools/fill_probe.cpp,
-                    // tools/files_probe.py; tmpfs, 16 threads: reserved by the driver thread 11.1 GB/s, by every writer
-                    // for its own slice 8.5, by page faults in the copies 9.2, this way 13.3).
-                    // With one thread, or when the range cannot be mapped, plain pwrite.
-                    bool mapped = P->n_threads > 1 && n > 0;
-                    if (mapped) {
-                        if (sink.own_size[e]) mapped = ::ftruncate(sink.fd[e], (off_t)(sink.pos[e] + n)) == 0;
-                        mapped = mapped && map_range(sink.fd[e], sink.pos[e], n, s.map[e]);
-                    }
-                    const uint64_t slice = 8ull << 20;
-                    if (mapped) {
-                        const int fd = sink.fd[e];
-                        const uint8_t* src0 = s.h_out[e].p;
-                        uint8_t* dst0 = s.map[e].at;
-                        const uint64_t off0 = sink.pos[e];
-                        WriterPool* pool = &c->writers;
-                        std::atomic<int>* pend = &s.writes;
-                        c->writers.submit(&s.writes, [fd, src0, dst0, off0, n, slice, pool, pend]() {
-                            const int rc = ::posix_fallocate(fd, (off_t)off0, (off_t)n);
-                            if (rc != 0 && rc != EOPNOTSUPP && rc != EINVAL) return std::string(std::strerror(rc));
-                            for (uint64_t o = 0; o < n; o += slice) {
-                                uint8_t* dst = dst0 + o;
-                                const uint8_t* src = src0 + o;
-                                const uint64_t len = std::min(slice, n - o);
-                                pool->submit(pend, [dst, src, len]() { std::memcpy(dst, src, len); return std::string(); });
-                            }
-                            return std::string();
-                        });
-                    } else {
-                        for (uint64_t o = 0; o < n; o += slice) {
-                            const int fd = sink.fd[e];
-                            const uint8_t* src = s.h_out[e].p + o;
-                            const uint64_t len = std::min(slice, n - o), off = sink.pos[e] + o;
-                            c->writers.submit(&s.writes, [fd, src, len, off]() { return pwrite_all(fd, src, len, off); });
-                        }
-                    }
-                    sink.pos[e] += n;
-                    s.file_end[e] = sink.pos[e];
-                } else if (sink.kind == SINK_FILES) {
-                    // compressed: the writer threads deflate slices of whole members; their output is
-                    // written in order once the batch is done (wait_writes)
-                    const uint64_t unit = zmethod == DEFLATE_BGZF ? 0xff00ull : (1ull << 20);
-                    const uint64_t slice = unit * (zmethod == DEFLATE_BGZF ? 64 : 4);
-                    const size_t n_slices = (size_t)((n + slice - 1) / slice);
-                    s.zout[e].assign(n_slices, std::vector<uint8_t>());
-                    for (size_t k = 0; k < n_slices; k++) {
-                        const uint8_t* src = s.h_out[e].p + k * slice;
-                        const uint64_t len = std::min<uint64_t>(slice, n - k * slice);
-                        std::vector<uint8_t>* dst = &s.zout[e][k];
-                        const int lvl = P->compress;
-                        c->writers.submit(&s.writes, [zmethod, lvl, src, len, dst]() { return deflate_members(zmethod, lvl, src, len, *dst); });
-                    }
-                    z_pending = &s;
-                } else if (sink.kind == SINK_STREAM) {
-                    if (sink.chunk_cb(sink.chunk_user, job_index, e, reinterpret_cast<const char*>(s.h_out[e].p), n))
-                        throw IoErr("the chunk callback reported an error");
-                } else {
-                    if (sink.len[e] + n <= sink.cap[e]) std::memcpy(sink.mem[e] + sink.len[e], s.h_out[e].p, n);
-                    sink.len[e] += n;
-                }
-            }
+            const uint8_t* data[2] = {s.h_out[0].p, s.h_out[1].p};
+            const uint64_t n[2] = {dev_z ? s.ztot[0] : s.tot[0], dev_z ? s.ztot[1] : s.tot[1]};
+            sink.deliver(s.host, data, n, job_index, n_ends);
         }
         if (P->progress_cb) P->progress_cb(P->cb_user, (uint64_t)s.pairs * n_ends);
         s.busy = false;
@@ -942,18 +727,12 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
         const uint64_t lo = ranges[jk].first, hi = ranges[jk].second;
         if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();   // src/hts.h:536
         if (X.ranges && hi <= lo) { job_index++; continue; }             // a multi-GPU device with no part in this job's files
-        if (sink.kind == SINK_FILES && !sizes_only) {
-            for (Slot& s : c->slot) wait_writes(s);
-            sink.close_files();
-            for (int e = 0; e < n_ends; e++) {
-                sink.names[e] = file_name(job, e, want_gz, P) + (X.job_suffix ? (*X.job_suffix)[jk] : X.part_suffix);
-                sink.pos[e] = sink.done[e] = X.base ? (*X.base)[jk][e] : 0;
-                sink.own_size[e] = !X.shared_files;
-                sink.fd[e] = ::open(sink.names[e].c_str(), X.shared_files ? O_RDWR : (O_RDWR | O_CREAT | O_TRUNC), 0644);
-                if (sink.fd[e] < 0) throw IoErr("Unable to open file " + sink.names[e] + ".\n");  // src/io.h:288-290
-            }
+        if (!sizes_only) {
+            std::string names[2];
+            for (int e = 0; e < n_ends; e++)
+                names[e] = file_name(job, e, Z.want_gz, P) + (X.job_suffix ? (*X.job_suffix)[jk] : "");
+            sink.open_job(names, n_ends, X.base ? (*X.base)[jk].data() : nullptr, X.shared_files);
         }
-        if (sink.kind == SINK_MEMORY && X.base) for (int e = 0; e < n_ends; e++) sink.len[e] = (*X.base)[jk][e];
         if (sizes_only) {
             // size pass: placement and scan only; the totals come back batch by batch (a few hundred microseconds each)
             for (uint64_t b0 = lo; b0 < hi; b0 += B) {
@@ -1029,25 +808,9 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
             if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();   // Quiesce settles what is in flight
         }
         while (!computing.empty() || !copying.empty()) drain_one();
-        if (z_pending) { wait_writes(*z_pending); z_pending = nullptr; }
-        for (Slot& s : c->slot) wait_writes(s);
-        const bool eof_block = !X.shared_files && X.part_suffix.empty() && !X.no_eof;      // a multi-GPU run appends it once, after joining the parts
-        if (sink.kind == SINK_FILES && (zmethod == DEFLATE_BGZF || dev_z) && eof_block)
-            for (int e = 0; e < n_ends; e++) {   // bgzf_close appends the empty end-of-file block
-                std::string w = pwrite_all(sink.fd[e], kBgzfEof, sizeof kBgzfEof, sink.pos[e]);
-                if (!w.empty()) throw IoErr("Error writing to file " + sink.names[e] + ": " + w);
-                sink.pos[e] += sizeof kBgzfEof;
-                sink.done[e] = sink.pos[e];
-            }
-        if (dev_z && sink.kind == SINK_STREAM)
-            for (int e = 0; e < n_ends; e++)
-                if (sink.chunk_cb(sink.chunk_user, job_index, e, reinterpret_cast<const char*>(kBgzfEof), sizeof kBgzfEof))
-                    throw IoErr("the chunk callback reported an error");
-        if (dev_z && sink.kind == SINK_MEMORY)
-            for (int e = 0; e < n_ends; e++) {
-                if (sink.len[e] + sizeof kBgzfEof <= sink.cap[e]) std::memcpy(sink.mem[e] + sink.len[e], kBgzfEof, sizeof kBgzfEof);
-                sink.len[e] += sizeof kBgzfEof;
-            }
+        for (Slot& s : c->slot) sink.settle(s.host);
+        // a multi-GPU run appends the end-of-file block once, after joining the parts
+        sink.end_job(job_index, n_ends, !X.shared_files && !X.job_suffix);
         job_index++;
     }
     CK(cudaEventRecord(c->ev_run[1], c->s_compute));
@@ -1057,7 +820,6 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jl
         CK(cudaEventElapsedTime(&ms, c->ev_run[0], c->ev_run[1]));
         st.run_ms = ms;
     }
-    sink.close_files();
     if (c->upload_pending) {
         // the copies this run issued are done before the caller gets control back; chromosomes no
         // shard of this run touched remain on the host (upload_src must stay valid, see the header)
@@ -1102,41 +864,16 @@ struct MultiShared {
 int multi_abort_cb(void* u) { return static_cast<MultiShared*>(u)->abort.load(std::memory_order_relaxed); }
 void multi_progress_cb(void* u, uint64_t reads) { static_cast<MultiShared*>(u)->progress.fetch_add(reads, std::memory_order_relaxed); }
 
-// n bytes from in_fd at in_off to out_fd at out_off (both files on any file system)
-std::string copy_range(int out_fd, uint64_t out_off, int in_fd, uint64_t in_off, uint64_t n) {
-    std::vector<uint8_t> buf;
-    bool use_cfr = true;
-    while (n) {
-        if (use_cfr) {
-            off_t oi = (off_t)in_off, oo = (off_t)out_off;
-            const ssize_t w = ::copy_file_range(in_fd, &oi, out_fd, &oo, (size_t)std::min<uint64_t>(n, 1ull << 30), 0);
-            if (w > 0) { n -= (uint64_t)w; in_off += (uint64_t)w; out_off += (uint64_t)w; continue; }
-            if (w < 0 && errno == EINTR) continue;
-            if (w == 0) return "unexpected end of a part file";
-            if (errno != EXDEV && errno != EINVAL && errno != ENOSYS && errno != EOPNOTSUPP) return std::strerror(errno);
-            use_cfr = false;                                  // file systems without copy_file_range: read + write
-        }
-        buf.resize(8u << 20);
-        const ssize_t r = ::pread(in_fd, buf.data(), (size_t)std::min<uint64_t>(n, buf.size()), (off_t)in_off);
-        if (r < 0) { if (errno == EINTR) continue; return std::strerror(errno); }
-        if (r == 0) return "unexpected end of a part file";
-        const std::string w = pwrite_all(out_fd, buf.data(), (uint64_t)r, out_off);
-        if (!w.empty()) return w;
-        n -= (uint64_t)r; in_off += (uint64_t)r; out_off += (uint64_t)r;
-    }
-    return std::string();
-}
-
-void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& sink, jlp_run_stats* stats) {
+void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, jlp_run_stats* stats) {
     check_params(c, use_haps, P, sink.kind);
     if (sink.kind == SINK_STREAM)
         throw Unsupported("jlp_illumina_stream on a multi-GPU context: batches of several devices have no single order; "
                           "use files / memory, or one context per device with shard_index / shard_count");
     if (P->shard_count > 1) throw ArgErr("shard_index / shard_count do not combine with a multi-GPU context");
     const size_t N = c->kids.size();
-    const Layout Y = make_layout(c, use_haps, P);
+    const Layout Y = make_layout(c, illumina_spec(c, use_haps, P));
     const size_t nj = Y.jobs.size();
-    const int n_ends = Y.n_ends;
+    const int n_ends = P->paired || P->matepair ? 2 : 1;
     const Compression Z = compression_of(P, sink.kind);
     if (Z.want_gz && Z.dev_z && sink.kind == SINK_MEMORY)
         throw Unsupported("compressed output into memory on a multi-GPU context");
@@ -1204,14 +941,20 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
         }
     };
 
-    // a shared output file gets its final size at once (no pages yet); a file system that cannot hold everything the
-    // run will write is reported here rather than half-way through
+    // a shared output file is created with its final size at once (no pages yet; pages are reserved slice by slice by the
+    // devices' writer threads, see Output::deliver), its last `tail` bytes written now; a file system that cannot hold
+    // everything the run will write is reported here rather than half-way through
     uint64_t need_bytes = 0;
-    auto presize = [](int fd, uint64_t size, uint64_t& need) -> int {
-        need += size;
+    auto create_sized = [&](const std::string& name, uint64_t size, const uint8_t* tail, uint64_t tail_len) {
+        const int fd = ::open(name.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
+        if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");      // src/io.h:288-290
+        need_bytes += size;
         struct statvfs vfs;
-        if (::fstatvfs(fd, &vfs) == 0 && (uint64_t)vfs.f_bavail * vfs.f_frsize < need) return ENOSPC;
-        return ::ftruncate(fd, (off_t)size) == 0 ? 0 : errno;
+        const int rc = ::fstatvfs(fd, &vfs) == 0 && (uint64_t)vfs.f_bavail * vfs.f_frsize < need_bytes ? ENOSPC
+                       : ::ftruncate(fd, (off_t)size) == 0 ? 0 : errno;
+        const std::string w = rc ? std::strerror(rc) : pwrite_all(fd, tail, tail_len, size - tail_len);
+        ::close(fd);
+        if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
     };
 
     // --- size pass
@@ -1220,7 +963,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
     uint64_t launches = 0;
     if (sized) {
         on_devices([&](size_t r) {
-            Sink none;
+            Output none;
             RunExtras X;
             X.ranges = &ranges[r]; X.sizes_out = &sizes[r];
             run(c->kids[r], use_haps, &Pk, none, &st[r], X);
@@ -1236,15 +979,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
         for (size_t r = 0; r < N; r++) launches += st[r].kernel_launches;
         if (sink.kind == SINK_FILES)
             for (size_t k = 0; k < nj; k++)
-                for (int e = 0; e < n_ends; e++) {
-                    const std::string name = file_name(Y.jobs[k], e, false, P);
-                    const int fd = ::open(name.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
-                    if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");      // src/io.h:288-290
-                    // sized now, pages reserved slice by slice by the devices' writer threads (see deliver() in run())
-                    const int rc = presize(fd, job_total[k][e], need_bytes);
-                    ::close(fd);
-                    if (rc != 0) throw IoErr("Error writing to file " + name + ": " + std::strerror(rc));
-                }
+                for (int e = 0; e < n_ends; e++) create_sized(file_name(Y.jobs[k], e, false, P), job_total[k][e], nullptr, 0);
         if (sink.kind == SINK_MEMORY) { sink.len[0] = mem_off[0]; sink.len[1] = mem_off[1]; }
     }
 
@@ -1254,7 +989,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
         jlp_illumina_params Pdry = Pk;
         Pdry.progress_cb = nullptr;
         on_devices([&](size_t r) {
-            Sink none;
+            Output none;
             RunExtras X;
             X.ranges = &ranges[r]; X.zsizes_out = &zsizes[r]; X.dry_files = true;
             run(c->kids[r], use_haps, &Pdry, none, &st[r], X);
@@ -1265,16 +1000,8 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
                 uint64_t o = 0;
                 for (size_t r = 0; r < N; r++) { base[r][k][e] = o; o += zsizes[r][k][e]; }
                 job_total[k][e] = o;
-                const std::string name = file_name(Y.jobs[k], e, true, P);
-                const int fd = ::open(name.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
-                if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");      // src/io.h:288-290
-                const uint64_t size = o + sizeof kBgzfEof;                            // bgzf_close: one empty block ends the file
-                const int rc = presize(fd, size, need_bytes);
-                std::string w;
-                if (rc == 0) w = pwrite_all(fd, kBgzfEof, sizeof kBgzfEof, o);
-                ::close(fd);
-                if (rc != 0) throw IoErr("Error writing to file " + name + ": " + std::strerror(rc));
-                if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
+                // bgzf_close: one empty block ends the file
+                create_sized(file_name(Y.jobs[k], e, true, P), o + sizeof kBgzfEof, kBgzfEof, sizeof kBgzfEof);
             }
     }
 
@@ -1293,8 +1020,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
                 if (ranges[r][k].second > ranges[r][k].first && r != first_dev[k])
                     for (int e = 0; e < n_ends; e++) cleanup.names.push_back(file_name(Y.jobs[k], e, true, P) + ".part" + std::to_string(r));
     on_devices([&](size_t r) {
-        Sink sk;
-        sk.kind = sink.kind;
+        Output sk(sink.kind);
         for (int e = 0; e < 2; e++) { sk.mem[e] = sink.mem[e]; sk.cap[e] = sink.cap[e]; }
         RunExtras X;
         X.ranges = &ranges[r];
@@ -1303,7 +1029,6 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
         std::vector<std::string> suffix;
         if (parts) {
             // per job: the job's first device writes <name> itself (no EOF block yet), every other one <name>.part<r>
-            X.no_eof = true;
             X.job_suffix = &suffix;
             for (size_t k = 0; k < nj; k++) suffix.push_back(r == first_dev[k] ? std::string() : ".part" + std::to_string(r));
         }
@@ -1349,34 +1074,25 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Sink& si
                     if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
                 }
             }
-        std::atomic<size_t> next{0};
-        std::mutex em;
-        std::string first_err;
         // a slice is copied through mappings of both files where that works (threads writing one file through
-        // write() / copy_file_range queue on its inode lock; page-cache pages filled through a mapping do not), else by copy_range
-        auto worker = [&]() {
-            static const uint64_t page = (uint64_t)sysconf(_SC_PAGESIZE);
-            for (size_t i = next.fetch_add(1); i < tasks.size(); i = next.fetch_add(1)) {
-                const CopyTask& t = tasks[i];
+        // write() / copy_file_range queue on its inode lock; page-cache pages filled through a mapping do not), else by
+        // copy_range; the writer threads of this (multi-GPU) context do the copying
+        std::atomic<int> pending{0};
+        c->writers.start(std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32)));
+        for (const CopyTask& t : tasks)
+            c->writers.submit(&pending, [t]() {
+                Mapping mo, mi;
                 std::string w;
-                const uint64_t o0 = t.out_off / page * page, i0 = t.in_off / page * page;
-                void* mo = ::mmap(nullptr, (size_t)(t.out_off + t.len - o0), PROT_READ | PROT_WRITE, MAP_SHARED, t.out_fd, (off_t)o0);
-                void* mi = mo == MAP_FAILED ? MAP_FAILED : ::mmap(nullptr, (size_t)(t.in_off + t.len - i0), PROT_READ, MAP_SHARED, t.in_fd, (off_t)i0);
-                if (mo != MAP_FAILED && mi != MAP_FAILED)
-                    std::memcpy(static_cast<uint8_t*>(mo) + (t.out_off - o0), static_cast<const uint8_t*>(mi) + (t.in_off - i0), t.len);
+                if (map_range(t.out_fd, t.out_off, t.len, mo) && map_range(t.in_fd, t.in_off, t.len, mi, true))
+                    std::memcpy(mo.at, mi.at, t.len);
                 else
                     w = copy_range(t.out_fd, t.out_off, t.in_fd, t.in_off, t.len);
-                if (mi != MAP_FAILED) ::munmap(mi, (size_t)(t.in_off + t.len - i0));
-                if (mo != MAP_FAILED) ::munmap(mo, (size_t)(t.out_off + t.len - o0));
-                if (!w.empty()) { std::lock_guard<std::mutex> l(em); if (first_err.empty()) first_err = w; }
-            }
-        };
-        const size_t nth = std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32));
-        std::vector<std::thread> th;
-        for (size_t i = 1; i < nth; i++) th.emplace_back(worker);
-        worker();
-        for (std::thread& t : th) t.join();
-        if (!first_err.empty()) throw IoErr("Error joining the devices' parts: " + first_err);
+                mi.unmap();
+                mo.unmap();
+                return w;
+            });
+        const std::string w = c->writers.wait(pending);
+        if (!w.empty()) { c->writers.clear_error(); throw IoErr("Error joining the devices' parts: " + w); }
     }
 
     jlp_run_stats tot;
@@ -2006,26 +1722,25 @@ int jlp_set_profile(jlp_ctx* c, int end, uint64_t read_length, const uint32_t* n
     });
 }
 
-static void run_any(jlp_ctx* c, bool use_haps, const jlp_illumina_params* p, Sink& s, jlp_run_stats* stats) {
+static void run_any(jlp_ctx* c, bool use_haps, const jlp_illumina_params* p, Output& s, jlp_run_stats* stats) {
     if (c->kids.empty()) run(c, use_haps, p, s, stats);
     else run_multi(c, use_haps, p, s, stats);
 }
 
 int jlp_illumina_ref(jlp_ctx* c, const jlp_illumina_params* p, jlp_run_stats* stats) {
     if (!c) return JLP_ERR_ARG;
-    return guarded(c, [&]() { Sink s; s.kind = SINK_FILES; run_any(c, false, p, s, stats); });
+    return guarded(c, [&]() { Output s(SINK_FILES); run_any(c, false, p, s, stats); });
 }
 int jlp_illumina_hap(jlp_ctx* c, const jlp_illumina_params* p, jlp_run_stats* stats) {
     if (!c) return JLP_ERR_ARG;
-    return guarded(c, [&]() { Sink s; s.kind = SINK_FILES; run_any(c, true, p, s, stats); });
+    return guarded(c, [&]() { Output s(SINK_FILES); run_any(c, true, p, s, stats); });
 }
 
 int jlp_illumina_to_memory(jlp_ctx* c, int use_haplotypes, const jlp_illumina_params* p, char* out1, uint64_t cap1,
                            uint64_t* len1, char* out2, uint64_t cap2, uint64_t* len2, jlp_run_stats* stats) {
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
-        Sink s;
-        s.kind = SINK_MEMORY;
+        Output s(SINK_MEMORY);
         s.mem[0] = out1; s.cap[0] = out1 ? cap1 : 0;
         s.mem[1] = out2; s.cap[1] = out2 ? cap2 : 0;
         run_any(c, use_haplotypes != 0, p, s, stats);
@@ -2040,15 +1755,15 @@ int jlp_illumina_stream(jlp_ctx* c, int use_haplotypes, const jlp_illumina_param
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
         if (!cb) throw ArgErr("chunk callback is NULL");
-        Sink s;
-        s.kind = SINK_STREAM; s.chunk_cb = cb; s.chunk_user = user;
+        Output s(SINK_STREAM);
+        s.chunk_cb = cb; s.chunk_user = user;
         run_any(c, use_haplotypes != 0, p, s, stats);
     });
 }
 
 int jlp_illumina_device_only(jlp_ctx* c, int use_haplotypes, const jlp_illumina_params* p, jlp_run_stats* stats) {
     if (!c) return JLP_ERR_ARG;
-    return guarded(c, [&]() { Sink s; s.kind = SINK_NONE; run_any(c, use_haplotypes != 0, p, s, stats); });
+    return guarded(c, [&]() { Output s; run_any(c, use_haplotypes != 0, p, s, stats); });
 }
 
 int jlp_illumina_group_counts(jlp_ctx* c, int use_haplotypes, const jlp_illumina_params* p, uint64_t* counts,
@@ -2056,10 +1771,7 @@ int jlp_illumina_group_counts(jlp_ctx* c, int use_haplotypes, const jlp_illumina
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
         if (!p) throw ArgErr("params is NULL");
-        if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
-        if (use_haplotypes && c->haps.empty()) throw ArgErr("no haplotypes have been added");
-        const int n_ends = p->paired || p->matepair ? 2 : 1;
-        std::vector<std::vector<uint64_t>> cnt = apportion(c, use_haplotypes != 0, p, p->n_reads / n_ends);
+        std::vector<std::vector<uint64_t>> cnt = apportion(c, illumina_spec(c, use_haplotypes != 0, p));
         uint64_t n = 0;
         for (const auto& v : cnt) n += v.size();
         if (n_groups) *n_groups = n;
@@ -2091,65 +1803,22 @@ void pb_model_from(const jlp_pacbio_params* P, PbModel& m) {
     try { pb_prepare(m); } catch (const std::exception& e) { throw ArgErr(e.what()); }
 }
 
-struct PbGroups {
-    std::vector<uint64_t> group_off;      // read-index prefix offsets
-    std::vector<GroupDev> groups;
-    std::vector<uint8_t> strpool;
-    std::vector<Job> jobs;
-};
-
-// reads -> haplotypes -> chromosomes, as for Illumina with one "end" (PacBioOneGenome::add_n_reads, src/hts_pacbio.h)
-PbGroups pb_groups(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P) {
-    if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
-    if (use_haps && c->haps.empty()) throw ArgErr("no haplotypes have been added");
-    if (use_haps) finish_upload(c);
-    const uint64_t n_chroms = c->chrom_off.size() - 1, n_haps = c->haps.size();
-    std::vector<uint64_t> sizes;
-    std::vector<std::vector<uint64_t>> counts;
-    if (!use_haps) {
-        for (uint64_t i = 0; i < n_chroms; i++) sizes.push_back(c->chrom_off[i + 1] - c->chrom_off[i]);
-        counts = apportion_sizes(P->seed, P->n_reads, 1, n_chroms, nullptr, sizes.data());
-    } else {
-        if (!P->haplotype_probs) throw ArgErr("haplotype_probs is NULL");
-        for (const HapDev& h : c->haps) sizes.insert(sizes.end(), h.len.begin(), h.len.end());
-        counts = apportion_sizes(P->seed, P->n_reads, n_haps, n_chroms, P->haplotype_probs, sizes.data());
-    }
-    PbGroups G;
-    G.group_off.push_back(0);
-    const std::string prefix = P->out_prefix ? P->out_prefix : "";
-    auto add = [&](const std::string& gname, uint64_t chrom, const uint8_t* seq, uint64_t len, uint64_t count) {
-        GroupDev g;
-        const std::string pre = "@" + gname + "-" + c->chrom_names[chrom] + "-";
-        g.seq = seq; g.len = len;
-        g.prefix_off = (uint32_t)G.strpool.size(); g.prefix_len = (uint32_t)pre.size();
-        G.strpool.insert(G.strpool.end(), pre.begin(), pre.end());
-        g.bc_off = 0; g.bc_len = 0;
-        G.groups.push_back(g);
-        G.group_off.push_back(G.group_off.back() + count);
-        if (count > 0 && len == 0) throw ArgErr("a chromosome of length 0 was given reads");
-    };
-    if (!use_haps) {
-        for (uint64_t i = 0; i < n_chroms; i++) add(c->genome_name, i, c->genome.p + kPad + c->chrom_off[i], sizes[i], counts[0][i]);
-        G.jobs.push_back(Job{0, P->n_reads, prefix});
-    } else {
-        for (uint64_t h = 0; h < n_haps; h++) {
-            const uint64_t lo = G.group_off.back();
-            for (uint64_t i = 0; i < n_chroms; i++) {
-                if (counts[h][i]) ensure_hap_chrom(c, h, i);        // materialised when first read from
-                add(c->haps[h].name(), i, c->haps[h].seq[i], c->haps[h].len[i], counts[h][i]);
-            }
-            if (P->sep_files) G.jobs.push_back(Job{lo, G.group_off.back(), prefix + "_" + c->haps[h].name()});
-        }
-        if (!P->sep_files) G.jobs.push_back(Job{0, G.group_off.back(), prefix});
-    }
-    return G;
+// PacBio's own compression rule: unlike compression_of(), AUTO takes the device coder at levels 1..6 whatever the method
+// and thread count; compressed output goes to files only.
+Compression pacbio_compression(const jlp_pacbio_params* P, SinkKind kind) {
+    Compression z;
+    if (P->compress <= 0) return z;
+    z.want_gz = true;
+    if (kind != SINK_FILES) return z;
+    z.dev_z = P->comp_engine == JLP_COMP_DEVICE || (P->comp_engine == JLP_COMP_AUTO && P->compress <= 6);
+    if (!z.dev_z) z.zmethod = P->n_threads > 1 || std::string(P->comp_method) == "bgzip" ? DEFLATE_BGZF : DEFLATE_GZIP;
+    return z;
 }
 
 // The driver: per batch the per-read quantities are prepared on the host (batch k + 1 on a helper thread while batch k
 // is on the device), then plan upload, k_pb_plan, scan, k_pb_reads, optional BGZF, copy, and the write of batch k
 // overlaps the next batch.  Callbacks are called on the calling thread between batches.
-void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, int sink_kind, char* mem, uint64_t cap, uint64_t* mem_len,
-                jlp_run_stats* stats) {
+void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& sink, jlp_run_stats* stats) {
     PbModel model;
     pb_model_from(P, model);
     // the quantiles computed by earlier calls with the same pass-sampler parameters are kept (each costs a bisection on
@@ -2171,30 +1840,27 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, int sink_
         if (m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");
     }
     finish_upload(c);
-    const PbGroups G = pb_groups(c, use_haps, P);
-    const bool dev_z = P->compress > 0 && sink_kind == SINK_FILES &&
-                       (P->comp_engine == JLP_COMP_DEVICE || (P->comp_engine == JLP_COMP_AUTO && P->compress <= 6));
-    const int zmethod = P->compress <= 0 || dev_z || sink_kind != SINK_FILES ? -1
-                        : (P->n_threads > 1 || std::string(P->comp_method) == "bgzip") ? DEFLATE_BGZF : DEFLATE_GZIP;
-    // every buffer belongs to the context: pinning (and unpinning) a gigabyte of host memory on every call cost more than
-    // generating the reads, and a dozen device allocations and frees per call several milliseconds
-    DevBuf<GroupDev>& d_groups = c->pb_groups;
-    DevBuf<uint8_t>&d_strpool = c->pb_strpool, &d_out = c->pb_out, &d_zslots = c->pb_zslots, &d_zout = c->pb_zout, &d_zcode = c->pb_zcode;
-    DevBuf<PbRead>& d_reads = c->pb_reads;
-    DevBuf<uint32_t>&d_rec_len = c->pb_rec_len, &d_rec_local = c->pb_rec_local, &d_zlen = c->pb_zlen;
-    DevBuf<uint64_t>&d_block_tot = c->pb_block_tot, &d_block_base = c->pb_block_base, &d_totals = c->pb_totals, &d_zoff = c->pb_zoff;
-    // two host buffers: the writer threads copy batch k into the file while batch k + 1 is prepared, generated and copied
-    PinBuf<uint8_t>* h_buf = c->pb_h_buf;
-    Mapping h_map[2];
-    std::atomic<int> h_pending[2];
-    h_pending[0] = 0; h_pending[1] = 0;
+    Layout G = make_layout(c, LayoutSpec(use_haps, P, P->n_reads));
+    for (size_t g = 0; g < G.groups.size(); g++) {
+        const uint32_t h = G.group_hap[g], ci = G.group_chrom[g];
+        if (use_haps && G.group_off[g + 1] > G.group_off[g]) ensure_hap_chrom(c, h, ci);   // materialised when first read from
+        G.groups[g].seq = use_haps ? c->haps[h].seq[ci] : c->genome.p + kPad + c->chrom_off[ci];
+    }
+    const Compression Z = pacbio_compression(P, sink.kind);
+    const bool dev_z = Z.dev_z;
+    // the slots' buffers (pinning a gigabyte of host memory on every call cost more than generating the reads, and a dozen
+    // device allocations and frees per call several milliseconds): the device arrays of slot 0, and the pinned buffers of
+    // slots 0 and 1, between which batches alternate so that batch k is written while batch k + 1 is on its way
+    Slot& S0 = c->slot[0];
+    cudaEvent_t* ev = S0.ev;
+    for (cudaEvent_t& e : S0.ev) if (!e) CK(cudaEventCreate(&e));
     uint64_t n_batch = 0;
-    auto settle = [&](int k) { c->writers.wait(h_pending[k]); h_map[k].unmap(); };
-    struct Settle { decltype(settle)& f; ~Settle() { f(0); f(1); } } settle_all{settle};       // also on error paths, before fd closes
-    d_groups.upload(G.groups, c->s_compute);
-    d_strpool.upload(G.strpool, c->s_compute);
-    d_totals.ensure(4);
-    CK(cudaMemsetAsync(d_totals.p, 0, 4 * sizeof(uint64_t), c->s_compute));
+    sink.begin(Z, P->compress, P->n_threads, c->writers);
+    Quiesce quiesce{c, &sink};
+    c->d_groups.upload(G.groups, c->s_compute);
+    c->d_strpool.upload(G.strpool, c->s_compute);
+    S0.totals.ensure(4);
+    CK(cudaMemsetAsync(S0.totals.p, 0, 4 * sizeof(uint64_t), c->s_compute));
     uint64_t B = P->batch_reads ? P->batch_reads : 32768;
     // a chain of duplicates never leaves its pool (src/hts.h:266-267): batches are whole pools, so a duplicate's leader is in
     // its batch
@@ -2204,234 +1870,184 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, int sink_
     const uint64_t c_rev = thr_ld_lt(0.5).thr;
     jlp_run_stats st;
     std::memset(&st, 0, sizeof st);
-    uint64_t mem_used = 0;
-    cudaEvent_t ev[3];
-    for (cudaEvent_t& e : ev) CK(cudaEventCreate(&e));
-    for (const Job& job : G.jobs) {
-        int fd = -1;
-        uint64_t fpos = 0;
-        std::string fname;
-        if (sink_kind == SINK_FILES) {
-            fname = job.file_prefix + "_R1.fq" + (P->compress > 0 ? ".gz" : "");        // write_reads_one_filetype_, src/hts.h:344
-            fd = ::open(fname.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
-            if (fd < 0) throw IoErr("Unable to open file " + fname + ".\n");
+    for (size_t jk = 0; jk < G.jobs.size(); jk++) {
+        const Job& job = G.jobs[jk];
+        const std::string names[2] = {file_name(job, 0, Z.want_gz, nullptr)};     // PacBio's files have no shard suffix
+        sink.open_job(names, 1, nullptr, false);
+        // this shard's part of the job: whole pools, so that chains of duplicates stay inside it
+        uint64_t s_lo = job.lo, s_hi = job.hi;
+        if (P->shard_count > 1) {
+            if (P->shard_index >= P->shard_count) throw ArgErr("shard_index >= shard_count");
+            const uint64_t pool = std::max<uint64_t>(P->read_pool_size, 1), n_pools = (job.hi - job.lo + pool - 1) / pool;
+            uint64_t p_lo, p_hi;
+            shard_range(0, n_pools, P->shard_index, P->shard_count, p_lo, p_hi);
+            s_lo = std::min(job.hi, job.lo + p_lo * pool);
+            s_hi = std::min(job.hi, job.lo + p_hi * pool);
         }
-        try {
-            // this shard's part of the job: whole pools, so that chains of duplicates stay inside it
-            uint64_t s_lo = job.lo, s_hi = job.hi;
-            if (P->shard_count > 1) {
-                if (P->shard_index >= P->shard_count) throw ArgErr("shard_index >= shard_count");
-                const uint64_t pool = std::max<uint64_t>(P->read_pool_size, 1), n_pools = (job.hi - job.lo + pool - 1) / pool;
-                uint64_t p_lo, p_hi;
-                shard_range(0, n_pools, P->shard_index, P->shard_count, p_lo, p_hi);
-                s_lo = std::min(job.hi, job.lo + p_lo * pool);
-                s_hi = std::min(job.hi, job.lo + p_hi * pool);
-            }
-            // ---- per-read quantities on the host (read length, passes, error probabilities, thresholds): batch k + 1 is
-            //      prepared by a helper thread (which spreads the reads over n_threads workers) while the device
-            //      generates batch k and the sink takes it
-            struct Prepared { std::vector<PbRead> plan; uint64_t bound = 0; std::string err; };
-            auto prepare = [&](uint64_t b0, uint32_t n, Prepared& out) {
-                try {
-                    std::vector<PbRead>& plan = out.plan;
-                    plan.resize(n);
-                    // chains of duplicates: read i re-reads iff the draw made after read i - 1 says so and i does not open a pool
-                    std::vector<uint32_t> lead(n, kPbNoLeader);
-                    if (dups)
-                        for (uint32_t i = 1; i < n; i++)
-                            if ((b0 + i - job.lo) % P->read_pool_size != 0 && (t_dup.all || pb_dup_draw(P->seed, b0 + i - 1) < t_dup.thr))
-                                lead[i] = lead[i - 1] == kPbNoLeader ? i - 1 : lead[i - 1];
-                    // the reads are independent given their leaders: split over the host threads (n_threads, at most 64),
-                    // first the leaders, then the duplicates (which take their leader's chromosome and length)
-                    const uint32_t nt = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 1), 64);
-                    std::vector<uint64_t> part(nt, 0);
-                    std::vector<std::string> errs(nt);
-                    for (int pass = 0; pass < (dups ? 2 : 1); pass++) {
-                        auto work = [&](uint32_t k) {
-                            try {
-                                for (uint32_t i = k; i < n; i += nt) {
-                                    if ((lead[i] != kPbNoLeader) != (pass == 1)) continue;
-                                    const uint64_t j = b0 + i;
-                                    PbSample smp;
-                                    size_t g;
-                                    if (pass == 0) {
-                                        g = (size_t)(std::upper_bound(G.group_off.begin(), G.group_off.end(), j) - G.group_off.begin()) - 1;
-                                        smp = pb_sample(model, P->seed, j, G.groups[g].len);
-                                    } else {
-                                        g = plan[lead[i]].group;
-                                        smp = pb_sample_passes(model, P->seed, j, plan[lead[i]].read_length);
-                                    }
-                                    std::memset(&plan[i], 0, sizeof(PbRead));
-                                    pb_read_model(model, P->seed, j, smp, plan[i]);
-                                    plan[i].group = (uint32_t)g;
-                                    plan[i].leader = lead[i];
-                                    part[k] += max_prefix + 24 + 2 * smp.read_length + 5;
+        // ---- per-read quantities on the host (read length, passes, error probabilities, thresholds): batch k + 1 is
+        //      prepared by a helper thread (which spreads the reads over n_threads workers) while the device
+        //      generates batch k and the sink takes it
+        struct Prepared { std::vector<PbRead> plan; uint64_t bound = 0; std::string err; };
+        auto prepare = [&](uint64_t b0, uint32_t n, Prepared& out) {
+            try {
+                std::vector<PbRead>& plan = out.plan;
+                plan.resize(n);
+                // chains of duplicates: read i re-reads iff the draw made after read i - 1 says so and i does not open a pool
+                std::vector<uint32_t> lead(n, kPbNoLeader);
+                if (dups)
+                    for (uint32_t i = 1; i < n; i++)
+                        if ((b0 + i - job.lo) % P->read_pool_size != 0 && (t_dup.all || pb_dup_draw(P->seed, b0 + i - 1) < t_dup.thr))
+                            lead[i] = lead[i - 1] == kPbNoLeader ? i - 1 : lead[i - 1];
+                // the reads are independent given their leaders: split over the host threads (n_threads, at most 64),
+                // first the leaders, then the duplicates (which take their leader's chromosome and length)
+                const uint32_t nt = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 1), 64);
+                std::vector<uint64_t> part(nt, 0);
+                std::vector<std::string> errs(nt);
+                for (int pass = 0; pass < (dups ? 2 : 1); pass++) {
+                    auto work = [&](uint32_t k) {
+                        try {
+                            for (uint32_t i = k; i < n; i += nt) {
+                                if ((lead[i] != kPbNoLeader) != (pass == 1)) continue;
+                                const uint64_t j = b0 + i;
+                                PbSample smp;
+                                size_t g;
+                                if (pass == 0) {
+                                    g = (size_t)(std::upper_bound(G.group_off.begin(), G.group_off.end(), j) - G.group_off.begin()) - 1;
+                                    smp = pb_sample(model, P->seed, j, G.groups[g].len);
+                                } else {
+                                    g = plan[lead[i]].group;
+                                    smp = pb_sample_passes(model, P->seed, j, plan[lead[i]].read_length);
                                 }
-                            } catch (const std::exception& e) { errs[k] = e.what(); }
-                        };
-                        std::vector<std::thread> th;
-                        for (uint32_t k = 1; k < nt; k++) th.emplace_back(work, k);
-                        work(0);
-                        for (std::thread& t : th) t.join();
-                    }
-                    for (const std::string& e : errs) if (!e.empty()) { out.err = e; return; }
-                    out.bound = 0;
-                    for (uint64_t v : part) out.bound += v;
-                } catch (const std::exception& e) { out.err = e.what(); }
-            };
-            Prepared prep[2];
-            std::thread prep_thread;
-            struct JoinPrep { std::thread& t; ~JoinPrep() { if (t.joinable()) t.join(); } } join_prep{prep_thread};
-            // JLP_TRACE=1: where the host side of the call spends its time (stderr, one line per job)
-            const bool trace = std::getenv("JLP_TRACE") != nullptr;
-            double t_first = 0, t_join = 0, t_alloc = 0, t_sync = 0;
-            auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-            const double t_job = now();
-            // with the default batch size the first batches are small (8192 reads, doubling): the first preparation is the
-            // one nothing overlaps, so the device should not wait for a full batch of it
-            auto batch_size = [&](uint64_t k) -> uint64_t {
-                if (P->batch_reads) return B;
-                uint64_t b = std::min<uint64_t>(B, 8192ull << std::min<uint64_t>(k, 8));
-                if (dups) b = std::max<uint64_t>(P->read_pool_size, b / P->read_pool_size * P->read_pool_size);
-                return b;
-            };
-            {   // the per-read device arrays once, for the largest batch of the job (growing them batch by batch would
-                // free and allocate -- and synchronise -- at every step of the ramp)
-                const uint64_t n_max = std::min<uint64_t>(B, s_hi - s_lo);
-                d_reads.ensure(n_max); d_rec_len.ensure(n_max); d_rec_local.ensure(n_max);
-                const uint64_t nsb_max = (n_max + kScanBlock - 1) / kScanBlock;
-                d_block_tot.ensure(nsb_max); d_block_base.ensure(nsb_max);
-            }
-            uint64_t n_next = std::min<uint64_t>(batch_size(0), s_hi - s_lo), b0_next = s_lo;
-            if (s_lo < s_hi) prepare(s_lo, (uint32_t)n_next, prep[0]);
-            t_first = now() - t_job;
-            uint64_t bk = 0;
-            for (uint64_t b0 = s_lo; b0 < s_hi; b0 = b0_next, bk++) {
-                const uint32_t n = (uint32_t)n_next;
-                double t0 = now();
-                if (prep_thread.joinable()) prep_thread.join();
-                t_join += now() - t0;
-                Prepared& cur = prep[bk & 1];
-                if (!cur.err.empty()) throw ArgErr(cur.err);
-                if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();      // Progress::check_abort, src/hts.h:396-399
-                b0_next = b0 + n;
-                if (b0_next < s_hi) {
-                    Prepared* nxt = &prep[(bk + 1) & 1];
-                    const uint64_t nb0 = b0_next;
-                    n_next = std::min<uint64_t>(batch_size(bk + 1), s_hi - nb0);
-                    const uint32_t nn = (uint32_t)n_next;
-                    prep_thread = std::thread([&prepare, nb0, nn, nxt]() { prepare(nb0, nn, *nxt); });
+                                std::memset(&plan[i], 0, sizeof(PbRead));
+                                pb_read_model(model, P->seed, j, smp, plan[i]);
+                                plan[i].group = (uint32_t)g;
+                                plan[i].leader = lead[i];
+                                part[k] += max_prefix + 24 + 2 * smp.read_length + 5;
+                            }
+                        } catch (const std::exception& e) { errs[k] = e.what(); }
+                    };
+                    std::vector<std::thread> th;
+                    for (uint32_t k = 1; k < nt; k++) th.emplace_back(work, k);
+                    work(0);
+                    for (std::thread& t : th) t.join();
                 }
-                std::vector<PbRead>& plan = cur.plan;
-                const uint64_t bound = cur.bound;
-                t0 = now();
-                d_reads.ensure(n);
-                d_rec_len.ensure(n); d_rec_local.ensure(n);
-                const uint32_t nsb = (n + kScanBlock - 1) / kScanBlock;
-                d_block_tot.ensure(nsb); d_block_base.ensure(nsb);
-                if (bound + 64 > d_out.n) {      // batches differ in size: grow with slack, and at once to what a full batch will need
-                    const uint64_t full = n ? bound / n * std::min<uint64_t>(B, s_hi - s_lo) : bound;
-                    const uint64_t want = std::max(bound, full);
-                    d_out.ensure(want + want / 4 + 64);
-                }
-                t_alloc += now() - t0;
-                CK(cudaMemcpyAsync(d_reads.p, plan.data(), n * sizeof(PbRead), cudaMemcpyHostToDevice, c->s_compute));
-                st.h2d_bytes += n * sizeof(PbRead);
-                CK(cudaEventRecord(ev[0], c->s_compute));
-                CK(launch_pb_plan(d_reads.p, n, b0, P->seed, d_groups.p, c_rev, d_rec_len.p, c->s_compute));
-                if (dups) { CK(launch_pb_dups(d_reads.p, n, b0, P->seed, d_groups.p, d_rec_len.p, c->s_compute)); st.kernel_launches++; }
-                CK(launch_scan(d_rec_len.p, n, 1, d_rec_local.p, d_block_tot.p, d_block_base.p, d_totals.p, c->s_compute));
-                CK(launch_pb_reads(d_reads.p, n, b0, P->seed, d_groups.p, d_strpool.p, d_rec_local.p, d_block_base.p, d_out.p,
-                                   c->s_compute));
-                CK(cudaEventRecord(ev[1], c->s_compute));
-                st.kernel_launches += 4;
-                const uint32_t nblk = (uint32_t)((bound + kBgzfIn - 1) / kBgzfIn) + 1;
-                if (dev_z) {
-                    d_zslots.ensure((size_t)nblk * kBgzfSlot); d_zout.ensure((size_t)nblk * kBgzfSlot);
-                    d_zlen.ensure(2 * nblk); d_zoff.ensure(2 * nblk); d_zcode.ensure(kBgzfCodeBytes);
-                    CK(launch_bgzf(d_out.p, d_out.p, d_totals.p, nblk, P->compress >= 4, d_zslots.p, d_zslots.p, d_zlen.p, d_zlen.p + nblk,
-                                   d_zoff.p, d_zoff.p + nblk, d_zout.p, d_zout.p, d_zcode.p, c->s_compute));
-                    st.kernel_launches += kBgzfLaunches;
-                }
-                CK(cudaEventRecord(ev[2], c->s_compute));
-                uint64_t tot[4];
-                CK(cudaMemcpyAsync(tot, d_totals.p, sizeof tot, cudaMemcpyDeviceToHost, c->s_compute));
-                t0 = now();
-                CK(cudaStreamSynchronize(c->s_compute));
-                t_sync += now() - t0;
-                if (tot[0] > bound) throw std::runtime_error("internal: PacBio batch larger than its bound");
-                float ms = 0;
-                CK(cudaEventElapsedTime(&ms, ev[0], ev[1])); st.reads_ms += ms; st.device_ms += ms;
-                CK(cudaEventElapsedTime(&ms, ev[1], ev[2])); if (dev_z) { st.bgzf_ms += ms; st.device_ms += ms; }
-                st.pairs += n; st.batches++; st.bytes_out[0] += tot[0];
-                if (dev_z) st.z_bytes[0] += tot[2];
-                if (sink_kind == SINK_NONE) { if (P->progress_cb) P->progress_cb(P->cb_user, n); continue; }
-                const uint64_t nb = dev_z ? tot[2] : tot[0];
-                const int hk = (int)(n_batch++ & 1);
-                settle(hk);                                     // the slices of the batch before last are in the file
-                PinBuf<uint8_t>& h_out = h_buf[hk];
-                if (nb + 64 > h_out.n) {          // like d_out: at once to what a full batch will need (pinning is slow)
-                    const uint64_t full = n ? nb / n * std::min<uint64_t>(B, s_hi - s_lo) : nb;
-                    const uint64_t want = std::max(nb, full);
-                    h_out.ensure(want + want / 4 + 64);
-                }
-                CK(cudaMemcpy(h_out.p, dev_z ? d_zout.p : d_out.p, nb, cudaMemcpyDeviceToHost));
-                st.d2h_bytes += nb;
-                if (sink_kind == SINK_MEMORY) {
-                    if (mem && mem_used + nb <= cap) std::memcpy(mem + mem_used, h_out.p, nb);
-                    mem_used += nb;
-                } else {
-                    const uint8_t* src = h_out.p;
-                    uint64_t len = nb;
-                    std::vector<uint8_t> z;
-                    if (zmethod >= 0) {
-                        const std::string e = deflate_members(zmethod, P->compress, h_out.p, nb, z);
-                        if (!e.empty()) throw IoErr(e);
-                        src = z.data(); len = z.size();
-                    }
-                    // several writer threads: the file is extended and the batch copied into a mapping of the new range
-                    // in parallel (see Mapping) while the next batch is on its way; otherwise one pwrite
-                    struct statvfs vfs;
-                    if (zmethod < 0 && P->n_threads > 1 && len > (8u << 20) && ::fstatvfs(fd, &vfs) == 0 &&
-                        (uint64_t)vfs.f_bavail * vfs.f_frsize > 2 * len + (64ull << 20) && ::ftruncate(fd, (off_t)(fpos + len)) == 0 &&
-                        map_range(fd, fpos, len, h_map[hk])) {
-                        c->writers.start((size_t)std::min<uint64_t>(P->n_threads, 64));
-                        const uint64_t slice = 8ull << 20;
-                        for (uint64_t o = 0; o < len; o += slice) {
-                            uint8_t* dst = h_map[hk].at + o;
-                            const uint8_t* from = src + o;
-                            const uint64_t nb2 = std::min(slice, len - o);
-                            c->writers.submit(&h_pending[hk], [dst, from, nb2]() { std::memcpy(dst, from, nb2); return std::string(); });
-                        }
-                    } else {
-                        const std::string w = pwrite_all(fd, src, len, fpos);
-                        if (!w.empty()) throw IoErr("Error writing to file " + fname + ": " + w);
-                    }
-                    fpos += len;
-                }
-                if (P->progress_cb) P->progress_cb(P->cb_user, n);                  // Progress::increment, src/hts.h:414
-            }
-            if (prep_thread.joinable()) prep_thread.join();
-            settle(0); settle(1);
-            if (trace)
-                std::fprintf(stderr, "[jlp trace] pacbio job %llu reads: %.4f s (first prepare %.4f, waiting for later ones %.4f, "
-                             "device allocations %.4f, waiting for the device %.4f)\n", (unsigned long long)(s_hi - s_lo), now() - t_job,
-                             t_first, t_join, t_alloc, t_sync);
-            if (fd >= 0 && (dev_z || zmethod == DEFLATE_BGZF)) {
-                const std::string w = pwrite_all(fd, kBgzfEof, sizeof kBgzfEof, fpos);
-                if (!w.empty()) throw IoErr("Error writing to file " + fname + ": " + w);
-            }
-        } catch (...) {
-            settle(0); settle(1);
-            if (fd >= 0) ::close(fd);
-            for (cudaEvent_t& e : ev) cudaEventDestroy(e);
-            throw;
+                for (const std::string& e : errs) if (!e.empty()) { out.err = e; return; }
+                out.bound = 0;
+                for (uint64_t v : part) out.bound += v;
+            } catch (const std::exception& e) { out.err = e.what(); }
+        };
+        Prepared prep[2];
+        std::thread prep_thread;
+        struct JoinPrep { std::thread& t; ~JoinPrep() { if (t.joinable()) t.join(); } } join_prep{prep_thread};
+        // JLP_TRACE=1: where the host side of the call spends its time (stderr, one line per job)
+        const bool trace = std::getenv("JLP_TRACE") != nullptr;
+        double t_first = 0, t_join = 0, t_alloc = 0, t_sync = 0;
+        auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+        const double t_job = now();
+        // with the default batch size the first batches are small (8192 reads, doubling): the first preparation is the
+        // one nothing overlaps, so the device should not wait for a full batch of it
+        auto batch_size = [&](uint64_t k) -> uint64_t {
+            if (P->batch_reads) return B;
+            uint64_t b = std::min<uint64_t>(B, 8192ull << std::min<uint64_t>(k, 8));
+            if (dups) b = std::max<uint64_t>(P->read_pool_size, b / P->read_pool_size * P->read_pool_size);
+            return b;
+        };
+        {   // the per-read device arrays once, for the largest batch of the job (growing them batch by batch would
+            // free and allocate -- and synchronise -- at every step of the ramp)
+            const uint64_t n_max = std::min<uint64_t>(B, s_hi - s_lo);
+            c->pb_reads.ensure(n_max); S0.rec_len.ensure(n_max); S0.rec_local.ensure(n_max);
+            const uint64_t nsb_max = (n_max + kScanBlock - 1) / kScanBlock;
+            S0.block_tot.ensure(nsb_max); S0.block_base.ensure(nsb_max);
         }
-        if (fd >= 0) ::close(fd);
+        // batches differ in size: the output buffers grow with slack, and at once to what a full batch will need (pinning
+        // is slow)
+        auto grow = [&](auto& buf, uint64_t need, uint32_t n) {
+            if (need + 64 <= buf.n) return;
+            const uint64_t want = std::max(need, n ? need / n * std::min<uint64_t>(B, s_hi - s_lo) : need);
+            buf.ensure(want + want / 4 + 64);
+        };
+        uint64_t n_next = std::min<uint64_t>(batch_size(0), s_hi - s_lo), b0_next = s_lo;
+        if (s_lo < s_hi) prepare(s_lo, (uint32_t)n_next, prep[0]);
+        t_first = now() - t_job;
+        uint64_t bk = 0;
+        for (uint64_t b0 = s_lo; b0 < s_hi; b0 = b0_next, bk++) {
+            const uint32_t n = (uint32_t)n_next;
+            double t0 = now();
+            if (prep_thread.joinable()) prep_thread.join();
+            t_join += now() - t0;
+            Prepared& cur = prep[bk & 1];
+            if (!cur.err.empty()) throw ArgErr(cur.err);
+            if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();      // Progress::check_abort, src/hts.h:396-399
+            b0_next = b0 + n;
+            if (b0_next < s_hi) {
+                Prepared* nxt = &prep[(bk + 1) & 1];
+                const uint64_t nb0 = b0_next;
+                n_next = std::min<uint64_t>(batch_size(bk + 1), s_hi - nb0);
+                const uint32_t nn = (uint32_t)n_next;
+                prep_thread = std::thread([&prepare, nb0, nn, nxt]() { prepare(nb0, nn, *nxt); });
+            }
+            std::vector<PbRead>& plan = cur.plan;
+            const uint64_t bound = cur.bound;
+            t0 = now();
+            c->pb_reads.ensure(n);
+            S0.rec_len.ensure(n); S0.rec_local.ensure(n);
+            const uint32_t nsb = (n + kScanBlock - 1) / kScanBlock;
+            S0.block_tot.ensure(nsb); S0.block_base.ensure(nsb);
+            grow(S0.out[0], bound, n);
+            t_alloc += now() - t0;
+            CK(cudaMemcpyAsync(c->pb_reads.p, plan.data(), n * sizeof(PbRead), cudaMemcpyHostToDevice, c->s_compute));
+            st.h2d_bytes += n * sizeof(PbRead);
+            CK(cudaEventRecord(ev[0], c->s_compute));
+            CK(launch_pb_plan(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, c_rev, S0.rec_len.p, c->s_compute));
+            if (dups) { CK(launch_pb_dups(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, S0.rec_len.p, c->s_compute)); st.kernel_launches++; }
+            CK(launch_scan(S0.rec_len.p, n, 1, S0.rec_local.p, S0.block_tot.p, S0.block_base.p, S0.totals.p, c->s_compute));
+            CK(launch_pb_reads(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, c->d_strpool.p, S0.rec_local.p, S0.block_base.p, S0.out[0].p,
+                               c->s_compute));
+            CK(cudaEventRecord(ev[1], c->s_compute));
+            st.kernel_launches += 4;
+            const uint32_t nblk = (uint32_t)((bound + kBgzfIn - 1) / kBgzfIn) + 1;
+            if (dev_z) {
+                S0.zslots[0].ensure((size_t)nblk * kBgzfSlot); S0.zdev[0].ensure((size_t)nblk * kBgzfSlot);
+                S0.zlen[0].ensure(2 * nblk); S0.zoff[0].ensure(2 * nblk); S0.zcode.ensure(kBgzfCodeBytes);
+                CK(launch_bgzf(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress >= 4, S0.zslots[0].p, S0.zslots[0].p, S0.zlen[0].p, S0.zlen[0].p + nblk,
+                               S0.zoff[0].p, S0.zoff[0].p + nblk, S0.zdev[0].p, S0.zdev[0].p, S0.zcode.p, c->s_compute));
+                st.kernel_launches += kBgzfLaunches;
+            }
+            CK(cudaEventRecord(ev[2], c->s_compute));
+            uint64_t tot[4];
+            CK(cudaMemcpyAsync(tot, S0.totals.p, sizeof tot, cudaMemcpyDeviceToHost, c->s_compute));
+            t0 = now();
+            CK(cudaStreamSynchronize(c->s_compute));
+            t_sync += now() - t0;
+            if (tot[0] > bound) throw std::runtime_error("internal: PacBio batch larger than its bound");
+            float ms = 0;
+            CK(cudaEventElapsedTime(&ms, ev[0], ev[1])); st.reads_ms += ms; st.device_ms += ms;
+            CK(cudaEventElapsedTime(&ms, ev[1], ev[2])); if (dev_z) { st.bgzf_ms += ms; st.device_ms += ms; }
+            st.pairs += n; st.batches++; st.bytes_out[0] += tot[0];
+            if (dev_z) st.z_bytes[0] += tot[2];
+            if (sink.kind == SINK_NONE) { if (P->progress_cb) P->progress_cb(P->cb_user, n); continue; }
+            const uint64_t nb = dev_z ? tot[2] : tot[0];
+            Slot& hs = c->slot[n_batch++ & 1];
+            sink.settle(hs.host);                            // the batch before last is in the file
+            PinBuf<uint8_t>& h_out = hs.h_out[0];
+            grow(h_out, nb, n);
+            CK(cudaMemcpy(h_out.p, dev_z ? S0.zdev[0].p : S0.out[0].p, nb, cudaMemcpyDeviceToHost));
+            st.d2h_bytes += nb;
+            const uint8_t* data[2] = {h_out.p, nullptr};
+            const uint64_t len[2] = {nb, 0};
+            sink.deliver(hs.host, data, len, jk, 1);
+            if (P->progress_cb) P->progress_cb(P->cb_user, n);                  // Progress::increment, src/hts.h:414
+        }
+        if (prep_thread.joinable()) prep_thread.join();
+        sink.settle(c->slot[0].host); sink.settle(c->slot[1].host);
+        if (trace)
+            std::fprintf(stderr, "[jlp trace] pacbio job %llu reads: %.4f s (first prepare %.4f, waiting for later ones %.4f, "
+                         "device allocations %.4f, waiting for the device %.4f)\n", (unsigned long long)(s_hi - s_lo), now() - t_job,
+                         t_first, t_join, t_alloc, t_sync);
+        sink.end_job(jk, 1, true);
     }
-    for (cudaEvent_t& e : ev) cudaEventDestroy(e);
-    if (mem_len) *mem_len = mem_used;
     if (stats) *stats = st;
+    quiesce.armed = false;
 }
 
 }  // namespace
@@ -2440,8 +2056,8 @@ int jlp_pacbio(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params* p, jlp_r
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
         if (!p || !p->out_prefix || !*p->out_prefix) throw ArgErr("out_prefix is empty");
-        jlp_ctx* d = first_device(c);
-        run_pacbio(d, use_haplotypes != 0, p, SINK_FILES, nullptr, 0, nullptr, stats);
+        Output out(SINK_FILES);
+        run_pacbio(first_device(c), use_haplotypes != 0, p, out, stats);
     });
 }
 
@@ -2449,11 +2065,11 @@ int jlp_pacbio_to_memory(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params
                          jlp_run_stats* stats) {
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
-        uint64_t need = 0;
-        jlp_ctx* d = first_device(c);
-        run_pacbio(d, use_haplotypes != 0, p, out ? SINK_MEMORY : SINK_NONE, out, cap, &need, stats);
-        if (len) *len = need;
-        if (out && need > cap) throw ArgErr("output buffer too small");
+        Output sink(out ? SINK_MEMORY : SINK_NONE);
+        sink.mem[0] = out; sink.cap[0] = out ? cap : 0;
+        run_pacbio(first_device(c), use_haplotypes != 0, p, sink, stats);
+        if (len) *len = sink.len[0];
+        if (out && sink.len[0] > cap) throw ArgErr("output buffer too small");
     });
 }
 
@@ -2463,11 +2079,10 @@ int jlp_pacbio_read_plan(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params
     return guarded(c, [&]() {
         PbModel model;
         pb_model_from(p, model);
-        const PbGroups G = pb_groups(first_device(c), use_haplotypes != 0, p);
+        const Layout G = make_layout(c, LayoutSpec(use_haplotypes != 0, p, p->n_reads));
         const Thr t_dup = thr_double_lt(p->prob_dup);
         const bool dups = t_dup.thr != 0 || t_dup.all;
         for (const Job& job : G.jobs) {
-            uint64_t leader = job.lo;
             PbSample ls{};
             size_t lg = 0;
             for (uint64_t j = job.lo; j < job.hi; j++) {
@@ -2475,13 +2090,11 @@ int jlp_pacbio_read_plan(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params
                                  (t_dup.all || pb_dup_draw(p->seed, j - 1) < t_dup.thr);
                 PbSample s;
                 if (!dup) {
-                    leader = j;
                     lg = (size_t)(std::upper_bound(G.group_off.begin(), G.group_off.end(), j) - G.group_off.begin()) - 1;
                     s = ls = pb_sample(model, p->seed, j, G.groups[lg].len);
                 } else {
                     s = pb_sample_passes(model, p->seed, j, ls.read_length);
                 }
-                (void)leader;
                 if (group) group[j] = lg;
                 if (read_len) read_len[j] = s.read_length;
                 if (split_pos) split_pos[j] = s.split_pos;

@@ -81,13 +81,16 @@ def test_pacbio_haplotypes_pooled_and_sep_files(ctx, tmp_path):
     haps = J.random_haplotypes(g, 3, sub_rate=0.01, indel_rate=0.002, seed=6)
     kw = dict(haplotype_probs=[1, 2, 3], custom_read_lengths=[[800, 1], [3000, 1]])
     fq, _, _ = check(ctx, haps, 300, seed=16, **kw)
-    pre = str(tmp_path / "pb")
-    J.pacbio(haps, pre, 300, seed=16, ctx=ctx, sep_files=True, **kw)
-    assert b"".join(open("%s_%s_R1.fq" % (pre, h), "rb").read() for h in haps.hap_names) == fq
-    J.pacbio(haps, pre + "z", 300, seed=16, ctx=ctx, compress=True, **kw)                # BGZF written by the GPU
-    assert gzip.decompress(open(pre + "z_R1.fq.gz", "rb").read()) == fq
-    J.pacbio(haps, pre + "h", 300, seed=16, ctx=ctx, compress=9, **kw)                   # zlib on the host
-    assert gzip.decompress(open(pre + "h_R1.fq.gz", "rb").read()) == fq
+    # one writer thread and the default batches; four writer threads (mapped files, zlib in slices) and small batches
+    for i, files_kw in enumerate([{}, dict(n_threads=4, batch_reads=64)]):
+        pre = str(tmp_path / ("pb%d" % i))
+        J.pacbio(haps, pre, 300, seed=16, ctx=ctx, sep_files=True, **kw, **files_kw)
+        assert b"".join(open("%s_%s_R1.fq" % (pre, h), "rb").read() for h in haps.hap_names) == fq
+        J.pacbio(haps, pre + "z", 300, seed=16, ctx=ctx, compress=True, **kw, **files_kw)      # BGZF written by the GPU
+        assert gzip.decompress(open(pre + "z_R1.fq.gz", "rb").read()) == fq
+        J.pacbio(haps, pre + "h", 300, seed=16, ctx=ctx, compress=9, **kw, **files_kw)         # zlib on the host
+        assert gzip.decompress(open(pre + "h_R1.fq.gz", "rb").read()) == fq
+    pre = str(tmp_path / "pb0")
     with pytest.raises(J.JackalopeError, match="already exists"):
         J.pacbio(haps, pre, 300, seed=16, ctx=ctx, sep_files=True, **kw)
 
