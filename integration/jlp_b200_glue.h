@@ -25,9 +25,7 @@ struct Ctx {                       // destroys the context on every exit path, R
     // every GPU the process can see (CUDA_VISIBLE_DEVICES selects them): one call, one ordered set of files,
     // as the reference's n_threads share one set (src/hts.h:334-353); no CPU fallback
     Ctx() {
-        int rc = jlp_ctx_create_multi(0, nullptr, &p);
-        if (rc == JLP_OK && jlp_ctx_n_devices(p) == 1) { jlp_ctx_destroy(p); p = nullptr; rc = jlp_ctx_create(0, &p); }
-        if (rc != JLP_OK) stop(jlp_last_error(nullptr));
+        if (jlp_ctx_create_multi(0, nullptr, &p) != JLP_OK) stop(jlp_last_error(nullptr));
     }
     ~Ctx() { jlp_ctx_destroy(p); }
     void check(int rc) { if (rc != JLP_OK) stop(std::string(jlp_last_error(p))); }

@@ -16,6 +16,7 @@
 #include <chrono>
 #include <cmath>
 #include <deque>
+#include <exception>
 #include <functional>
 #include <mutex>
 #include <thread>
@@ -44,11 +45,15 @@ std::string g_create_error;
 // fetches template bases as aligned words and may touch a few bytes outside a chromosome.
 constexpr size_t kPad = 64;
 
+// A failed call is reported once: the thread's last error is reset, so that a failure a caller recovers from (a
+// cudaMalloc too large) is not reported again by the next kernel launch's cudaGetLastError().
 #define CK(call)                                                                          \
     do {                                                                                  \
         cudaError_t e_ = (call);                                                          \
-        if (e_ != cudaSuccess)                                                            \
+        if (e_ != cudaSuccess) {                                                          \
+            cudaGetLastError();                                                           \
             throw CudaErr(std::string(#call) + ": " + cudaGetErrorString(e_));            \
+        }                                                                                 \
     } while (0)
 
 template <typename T> struct DevBuf {
@@ -97,12 +102,6 @@ struct HapStore {
     std::string name;
     std::vector<HapChromHost> chrom;
 };
-struct HapDev {
-    std::shared_ptr<HapStore> store;    // shared by the devices of a multi-GPU context
-    std::vector<const uint8_t*> seq;    // per chromosome; aliases the reference when unmutated; NULL = not materialised yet
-    std::vector<uint64_t> len;
-    const std::string& name() const { return store->name; }
-};
 
 // Device memory of the materialised haplotype chromosomes: carved out of a few large slabs (one cudaMalloc per GiB,
 // not one per chromosome -- 96 haplotypes x 20 chromosomes would be 1920 allocations); freed together.
@@ -134,27 +133,25 @@ struct Slot {
     HostBatch host;               // h_out on its way into the files
 };
 
-}  // namespace
-
-struct jlp_ctx {
-    int device = 0;
-    // a multi-GPU context (jlp_ctx_create_multi) owns one child context per device and no device state of its own:
-    // it keeps the genome / haplotype metadata (names, sizes) and fans every call out to its children
-    std::vector<jlp_ctx*> kids;
-    std::string err;
+// Everything a context keeps on one GPU.  A device listed twice in jlp_ctx_create_multi gets two of these.
+struct Device {
+    int id = 0;
+    int n_sm = 148;
     cudaStream_t s_compute = nullptr, s_copy = nullptr;
+    cudaStream_t s_upload = nullptr;            // genome H2D, chromosome by chromosome
     // genome
     DevBuf<uint8_t> genome;
-    std::vector<uint64_t> chrom_off;
-    std::vector<std::string> chrom_names;
-    std::string genome_name;
-    std::vector<HapDev> haps;
+    std::vector<cudaEvent_t> chrom_ev;          // chromosome c is resident once chrom_ev[c] has fired
+    bool upload_pending = false;                // some chromosome is not resident yet (or its copy not waited for)
+    const char* upload_src = nullptr;           // host bases of a deferred upload (jlp_set_genome_async), else NULL
+    std::vector<char> chrom_resident;           // 1: the chromosome's H2D copy has been issued
+    // haplotypes: hap_seq[h][c] is chromosome c of haplotype h on this device; it aliases the reference when
+    // unmutated; NULL = not materialised yet
+    std::vector<std::vector<const uint8_t*>> hap_seq;
+    HapArena hap_mem;
     // profiles
-    EndTables tab[2];
-    bool have_prof[2] = {false, false};
     DevBuf<uint32_t> d_meta[2];
     DevBuf<uint64_t> d_coin[2], d_mis[2], d_entry64[2];
-    int n_sm = 148;
     // run-scoped device data
     DevBuf<uint64_t> d_frag, d_group_off;
     DevBuf<uint32_t> d_frag_guide;
@@ -163,21 +160,10 @@ struct jlp_ctx {
     DevBuf<uint32_t> d_status;
     Slot slot[3];                               // compute | D2H copy | delivery to the sink, one batch each
     WriterPool writers;
-    cudaStream_t s_upload = nullptr;            // genome H2D, chromosome by chromosome
-    std::vector<cudaEvent_t> chrom_ev;          // chromosome c is resident once chrom_ev[c] has fired
-    bool upload_pending = false;                // some chromosome is not resident yet (or its copy not waited for)
-    const char* upload_src = nullptr;           // host bases of a deferred upload (jlp_set_genome_async), else NULL
-    std::vector<char> chrom_resident;           // 1: the chromosome's H2D copy has been issued
     cudaEvent_t ev_run[2] = {nullptr, nullptr};
     uint64_t h2d_bytes = 0;
-    // scratch of the haplotype materialisation (mutation records of one chromosome)
-    HapArena hap_mem;
     // PacBio driver: the per-read plan of a batch (its other buffers are those of the slots)
     DevBuf<PbRead> pb_reads;
-    // PacBioPassSampler's outlier thresholds (one chi-squared quantile per read length up to chi2_params_n[2]) of the last call
-    std::shared_ptr<std::atomic<double>[]> pb_qcache;
-    double pb_qcache_key[3] = {0, 0, 0};
-    size_t pb_qcache_n = 0;
     // materialisation: the records of the next chromosomes are uploaded (s_upload) while k_materialize works on the
     // ones before (s_compute); kMatBufs scratch buffers in turn
     static constexpr int kMatBufs = 3;
@@ -185,6 +171,44 @@ struct jlp_ctx {
     cudaEvent_t m_up[kMatBufs] = {nullptr, nullptr, nullptr}, m_done[kMatBufs] = {nullptr, nullptr, nullptr};
     bool m_busy[kMatBufs] = {false, false, false};
     uint64_t m_next = 0;
+
+    void free_haps() {
+        hap_seq.clear();
+        hap_mem.release();
+    }
+    ~Device() {
+        cudaSetDevice(id);
+        cudaDeviceSynchronize();
+        free_haps();
+        for (Slot& s : slot) for (cudaEvent_t ev : s.ev) if (ev) cudaEventDestroy(ev);
+        for (cudaEvent_t ev : ev_run) if (ev) cudaEventDestroy(ev);
+        if (s_compute) cudaStreamDestroy(s_compute);
+        if (s_copy) cudaStreamDestroy(s_copy);
+        if (s_upload) cudaStreamDestroy(s_upload);
+        for (int k = 0; k < kMatBufs; k++) { if (m_up[k]) cudaEventDestroy(m_up[k]); if (m_done[k]) cudaEventDestroy(m_done[k]); }
+        for (cudaEvent_t ev : chrom_ev) cudaEventDestroy(ev);
+        writers.stop();
+    }
+};
+
+}  // namespace
+
+// What a context keeps once on the host, and its devices (one, or several for jlp_ctx_create_multi).
+struct jlp_ctx {
+    std::string err;
+    // genome
+    std::vector<uint64_t> chrom_off;
+    std::vector<std::string> chrom_names;
+    std::string genome_name;
+    std::vector<std::shared_ptr<HapStore>> haps;
+    // profiles
+    EndTables tab[2];
+    bool have_prof[2] = {false, false};
+    // PacBioPassSampler's outlier thresholds (one chi-squared quantile per read length up to chi2_params_n[2]) of the last call
+    std::shared_ptr<std::atomic<double>[]> pb_qcache;
+    double pb_qcache_key[3] = {0, 0, 0};
+    size_t pb_qcache_n = 0;
+    std::vector<std::unique_ptr<Device>> dev;
 };
 
 namespace {
@@ -203,11 +227,6 @@ uint8_t* HapArena::alloc(size_t n) {
     return r;
 }
 
-void free_haps(jlp_ctx* c) {
-    c->haps.clear();
-    c->hap_mem.release();
-}
-
 int fail(jlp_ctx* c, int code, const std::string& msg) {
     if (c) c->err = msg; else g_create_error = msg;
     return code;
@@ -215,7 +234,7 @@ int fail(jlp_ctx* c, int code, const std::string& msg) {
 
 template <typename F> int guarded(jlp_ctx* c, F f) {
     try {
-        if (c && c->kids.empty()) CK(cudaSetDevice(c->device));
+        if (c && c->dev.size() == 1) CK(cudaSetDevice(c->dev[0]->id));
         f();
         return JLP_OK;
     } catch (const ArgErr& e) { return fail(c, JLP_ERR_ARG, e.what());
@@ -226,50 +245,104 @@ template <typename F> int guarded(jlp_ctx* c, F f) {
     } catch (const std::exception& e) { return fail(c, JLP_ERR_ARG, e.what()); }
 }
 
-// the context itself, or the first child of a multi-GPU context (made current): calls that do not spread over devices
-jlp_ctx* first_device(jlp_ctx* c) {
-    if (c->kids.empty()) return c;
-    CK(cudaSetDevice(c->kids[0]->device));
-    return c->kids[0];
+// The device of the calls that use only the first one (PacBio, create_haplotypes, ...), made current.
+Device& device0(jlp_ctx* c) {
+    CK(cudaSetDevice(c->dev[0]->id));
+    return *c->dev[0];
 }
-// f(device context) for the context itself, or for every child of a multi-GPU context (current device set)
-template <typename F> void for_each_device(jlp_ctx* c, F f) {
-    if (c->kids.empty()) { f(c); return; }
-    for (jlp_ctx* k : c->kids) { CK(cudaSetDevice(k->device)); f(k); }
-}
-// the same, one host thread per device; the first error (if any) is rethrown as a runtime_error of its text
-template <typename F> void for_each_device_parallel(jlp_ctx* c, F f) {
-    if (c->kids.size() <= 1) { for_each_device(c, f); return; }
-    std::vector<std::string> errs(c->kids.size());
+
+// f(d) for every device d of the context, made current: on the calling thread for one device, else on one host thread
+// per device while the calling thread runs `wait` every 20 ms (if given).  The first error other than Aborted is
+// rethrown with its type (CUDA errors name their device), else Aborted if a device was aborted.
+template <typename F> void on_each_device(jlp_ctx* c, F f, const std::function<void()>& wait = nullptr) {
+    const size_t N = c->dev.size();
+    if (N == 1) {
+        CK(cudaSetDevice(c->dev[0]->id));
+        f(*c->dev[0]);
+        return;
+    }
+    std::vector<std::exception_ptr> errs(N);
+    std::atomic<size_t> left{N};
     std::vector<std::thread> th;
-    for (size_t r = 0; r < c->kids.size(); r++)
+    for (size_t r = 0; r < N; r++)
         th.emplace_back([&, r]() {
-            try { CK(cudaSetDevice(c->kids[r]->device)); f(c->kids[r]); } catch (const std::exception& e) { errs[r] = e.what(); if (errs[r].empty()) errs[r] = "error"; }
+            Device& d = *c->dev[r];
+            try {
+                CK(cudaSetDevice(d.id));
+                f(d);
+            } catch (const CudaErr& e) {
+                errs[r] = std::make_exception_ptr(CudaErr("device " + std::to_string(d.id) + ": " + e.what()));
+            } catch (...) {
+                errs[r] = std::current_exception();
+            }
+            left.fetch_sub(1);
         });
+    while (wait && left.load() != 0) {
+        std::this_thread::sleep_for(std::chrono::milliseconds(20));
+        wait();
+    }
     for (std::thread& t : th) t.join();
-    for (const std::string& e : errs) if (!e.empty()) throw CudaErr(e);
+    for (const std::exception_ptr& e : errs)
+        if (e) try { std::rethrow_exception(e); } catch (const Aborted&) {}
+    for (const std::exception_ptr& e : errs)
+        if (e) std::rethrow_exception(e);
+}
+
+void clear_haps(jlp_ctx* c) {
+    c->haps.clear();
+    on_each_device(c, [](Device& d) { d.free_haps(); });
 }
 
 // Issue the H2D copies of chromosomes [first, last] of a deferred genome upload (those not
 // issued yet); every copy is followed by its chromosome's event.
-void issue_upload(jlp_ctx* c, size_t first, size_t last) {
-    if (!c->upload_src) return;
-    for (size_t i = first; i <= last && i < c->chrom_resident.size(); i++) {
-        if (c->chrom_resident[i]) continue;
+void issue_upload(const jlp_ctx* c, Device& d, size_t first, size_t last) {
+    if (!d.upload_src) return;
+    for (size_t i = first; i <= last && i < d.chrom_resident.size(); i++) {
+        if (d.chrom_resident[i]) continue;
         const uint64_t len = c->chrom_off[i + 1] - c->chrom_off[i];
-        if (len) CK(cudaMemcpyAsync(c->genome.p + kPad + c->chrom_off[i], c->upload_src + c->chrom_off[i], len, cudaMemcpyHostToDevice, c->s_upload));
-        CK(cudaEventRecord(c->chrom_ev[i], c->s_upload));
-        c->chrom_resident[i] = 1;
-        c->h2d_bytes += len;
+        if (len) CK(cudaMemcpyAsync(d.genome.p + kPad + c->chrom_off[i], d.upload_src + c->chrom_off[i], len, cudaMemcpyHostToDevice, d.s_upload));
+        CK(cudaEventRecord(d.chrom_ev[i], d.s_upload));
+        d.chrom_resident[i] = 1;
+        d.h2d_bytes += len;
     }
 }
 // Make the whole genome resident and wait for it.
-void finish_upload(jlp_ctx* c) {
-    if (!c->upload_pending) return;
-    if (!c->chrom_resident.empty()) issue_upload(c, 0, c->chrom_resident.size() - 1);
-    CK(cudaStreamSynchronize(c->s_upload));
-    c->upload_pending = false;
-    c->upload_src = nullptr;
+void finish_upload(const jlp_ctx* c, Device& d) {
+    if (!d.upload_pending) return;
+    if (!d.chrom_resident.empty()) issue_upload(c, d, 0, d.chrom_resident.size() - 1);
+    CK(cudaStreamSynchronize(d.s_upload));
+    d.upload_pending = false;
+    d.upload_src = nullptr;
+}
+
+// What the genome setters share: drop the genome and the haplotypes, give every device a buffer for the new genome,
+// record its chromosomes once all devices have one, then fill(d) on every device.  If any of it fails, the context
+// is left without a genome, as a fresh context is.
+template <typename F> void replace_genome(jlp_ctx* c, const std::vector<uint64_t>& off, const std::vector<std::string>& names,
+                                          const char* genome_name, F fill) {
+    try {
+        c->chrom_off.clear();
+        c->chrom_names.clear();
+        c->haps.clear();
+        on_each_device(c, [&](Device& d) {
+            d.free_haps();
+            if (d.upload_pending) {      // a deferred upload that never ran is simply dropped
+                d.upload_pending = false;
+                d.upload_src = nullptr;
+                CK(cudaStreamSynchronize(d.s_upload));
+            }
+            d.genome.ensure(off.back() + 2 * kPad);
+        });
+        c->chrom_off = off;
+        c->chrom_names = names;
+        c->genome_name = genome_name ? genome_name : "REF";
+        on_each_device(c, fill);
+    } catch (...) {
+        c->chrom_off.clear();
+        c->chrom_names.clear();
+        for (auto& d : c->dev) { d->upload_pending = false; d->upload_src = nullptr; }    // the caller's bases are not read again
+        throw;
+    }
 }
 
 // ---------------------------------------------------------------- the run ---
@@ -334,7 +407,6 @@ struct LayoutSpec {
           prefix(P->out_prefix) {}
 };
 
-// needs only the sizes: works on a multi-GPU parent context (metadata, no device state) as well
 std::vector<std::vector<uint64_t>> apportion(const jlp_ctx* c, const LayoutSpec& S) {
     if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
     if (S.use_haps && c->haps.empty()) throw ArgErr("no haplotypes have been added");
@@ -345,7 +417,8 @@ std::vector<std::vector<uint64_t>> apportion(const jlp_ctx* c, const LayoutSpec&
         return apportion_sizes(S.seed, S.n_units, 1, n_chroms, nullptr, sizes.data());
     }
     if (!S.hap_probs) throw ArgErr("haplotype_probs is NULL");
-    for (const HapDev& h : c->haps) sizes.insert(sizes.end(), h.len.begin(), h.len.end());
+    for (const auto& h : c->haps)
+        for (const HapChromHost& M : h->chrom) sizes.push_back(M.size);
     return apportion_sizes(S.seed, S.n_units, c->haps.size(), n_chroms, S.hap_probs, sizes.data());
 }
 
@@ -403,8 +476,8 @@ void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P,
 
 // The (haplotype, chromosome) groups of a run in the order the reference exhausts them (hap-major, chrom-major:
 // src/hts_illumina.cpp:199-201, :505-528), their pair-index prefix offsets, ID-line prefixes and barcodes, and the
-// jobs (= sets of output files).  A pure function of the parameters and of the sizes the context knows, so every
-// device of a multi-GPU run builds the same one.
+// jobs (= sets of output files).  A pure function of the parameters and of the sizes the context knows: a multi-GPU
+// run builds it once for all its devices.
 struct Layout {
     uint64_t n_pairs = 0;
     std::vector<uint64_t> group_off;      // [n_groups + 1]
@@ -453,10 +526,10 @@ Layout make_layout(const jlp_ctx* c, const LayoutSpec& S) {
         Y.jobs.push_back(Job{0, Y.n_pairs, prefix});
     } else {
         for (uint64_t h = 0; h < n_haps; h++) {
-            const HapDev& H = c->haps[h];
+            const HapStore& H = *c->haps[h];
             uint64_t lo = Y.group_off.back();
-            for (uint64_t i = 0; i < n_chroms; i++) add_group(H.name(), (uint32_t)h, i, H.len[i], barcodes[h], counts[h][i]);
-            if (sep) Y.jobs.push_back(Job{lo, Y.group_off.back(), prefix + "_" + H.name()});
+            for (uint64_t i = 0; i < n_chroms; i++) add_group(H.name, (uint32_t)h, i, H.chrom[i].size, barcodes[h], counts[h][i]);
+            if (sep) Y.jobs.push_back(Job{lo, Y.group_off.back(), prefix + "_" + H.name});
         }
         if (!sep) Y.jobs.push_back(Job{0, Y.group_off.back(), prefix});
     }
@@ -481,33 +554,33 @@ std::string file_name(const Job& job, int e, bool gz, const jlp_illumina_params*
     return n;
 }
 
-// Materialise haplotype chromosome (h, ci) on this context's device if it is not resident yet
+// Materialise haplotype chromosome (h, ci) on device d if it is not resident yet
 // (HapChrom::get_chrom_full, src/hap_classes.cpp:80-116).
-void ensure_hap_chrom(jlp_ctx* c, size_t h, size_t ci) {
-    HapDev& H = c->haps[h];
-    if (H.seq[ci]) return;
-    const HapChromHost& M = H.store->chrom[ci];
+void ensure_hap_chrom(const jlp_ctx* c, Device& d, size_t h, size_t ci) {
+    const uint8_t*& seq = d.hap_seq[h][ci];
+    if (seq) return;
+    const HapChromHost& M = c->haps[h]->chrom[ci];
     const uint64_t ref_size = c->chrom_off[ci + 1] - c->chrom_off[ci];
-    const uint8_t* ref = c->genome.p + kPad + c->chrom_off[ci];
-    const int k = (int)(c->m_next++ % jlp_ctx::kMatBufs);
-    if (!c->m_up[k]) {
-        CK(cudaEventCreateWithFlags(&c->m_up[k], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&c->m_done[k], cudaEventDisableTiming));
+    const uint8_t* ref = d.genome.p + kPad + c->chrom_off[ci];
+    const int k = (int)(d.m_next++ % Device::kMatBufs);
+    if (!d.m_up[k]) {
+        CK(cudaEventCreateWithFlags(&d.m_up[k], cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&d.m_done[k], cudaEventDisableTiming));
     }
     // the kernel that read this buffer last must be done before the buffer can grow (cudaFree) or be written again
-    if (c->m_busy[k]) CK(cudaEventSynchronize(c->m_done[k]));
-    c->m_pack[k].upload(M.packed, c->s_upload);
-    CK(cudaEventRecord(c->m_up[k], c->s_upload));
-    c->h2d_bytes += M.n_muts * 32 + M.pool_bytes;
-    uint8_t* out = c->hap_mem.alloc(M.size + 2 * kPad);
-    const uint64_t* w = c->m_pack[k].p;
+    if (d.m_busy[k]) CK(cudaEventSynchronize(d.m_done[k]));
+    d.m_pack[k].upload(M.packed, d.s_upload);
+    CK(cudaEventRecord(d.m_up[k], d.s_upload));
+    d.h2d_bytes += M.n_muts * 32 + M.pool_bytes;
+    uint8_t* out = d.hap_mem.alloc(M.size + 2 * kPad);
+    const uint64_t* w = d.m_pack[k].p;
     const uint64_t n = M.n_muts;
-    CK(cudaStreamWaitEvent(c->s_compute, c->m_up[k], 0));
+    CK(cudaStreamWaitEvent(d.s_compute, d.m_up[k], 0));
     CK(launch_materialize(ref, ref_size, n, w, w + n, reinterpret_cast<const int64_t*>(w + 3 * n), w + 2 * n,
-                          reinterpret_cast<const uint8_t*>(w + 4 * n), M.size, out + kPad, c->s_compute));
-    CK(cudaEventRecord(c->m_done[k], c->s_compute));
-    c->m_busy[k] = true;
-    H.seq[ci] = out + kPad;       // valid in stream order: everything that reads it runs on s_compute
+                          reinterpret_cast<const uint8_t*>(w + 4 * n), M.size, out + kPad, d.s_compute));
+    CK(cudaEventRecord(d.m_done[k], d.s_compute));
+    d.m_busy[k] = true;
+    seq = out + kPad;       // valid in stream order: everything that reads it runs on s_compute
 }
 
 typedef std::vector<std::pair<uint64_t, uint64_t>> Ranges;
@@ -530,25 +603,26 @@ struct RunExtras {
 // tasks still hold the file descriptors the caller's Output is about to close.  Files the run extends itself are cut
 // back to the last completely written batch (an extended, never filled tail would otherwise stay behind as zero bytes).
 struct Quiesce {
-    jlp_ctx* c;
+    Device& d;
     Output* out;
     bool armed = true;
     ~Quiesce() {
         if (!armed) return;
-        cudaStreamSynchronize(c->s_compute);
-        cudaStreamSynchronize(c->s_copy);
+        cudaStreamSynchronize(d.s_compute);
+        cudaStreamSynchronize(d.s_copy);
         HostBatch* b[3];
-        for (int k = 0; k < 3; k++) { c->slot[k].busy = false; b[k] = &c->slot[k].host; }
+        for (int k = 0; k < 3; k++) { d.slot[k].busy = false; b[k] = &d.slot[k].host; }
         out->abandon(b, 3);
     }
 };
 
-void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, jlp_run_stats* stats, const RunExtras& X = RunExtras()) {
-    check_params(c, use_haps, P, sink.kind);
+// One Illumina run on device d, with the run's Layout (make_layout) and parameters checked (check_params) by the caller.
+void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* P, Layout Y, Output& sink, jlp_run_stats* stats,
+         const RunExtras& X = RunExtras()) {
     const int n_ends = P->paired || P->matepair ? 2 : 1;
     const bool matepair = P->matepair != 0;
-    if (use_haps) finish_upload(c);
-    const uint64_t h2d_before = c->h2d_bytes;
+    if (use_haps) finish_upload(c, d);
+    const uint64_t h2d_before = d.h2d_bytes;
     const Compression Z = compression_of(P, X.dry_files ? SINK_FILES : sink.kind);
     const bool dev_z = Z.dev_z;
     const bool sizes_only = X.sizes_out != nullptr;
@@ -556,7 +630,6 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
     const double insp[2] = {P->ins_prob1, P->ins_prob2}, delp[2] = {P->del_prob1, P->del_prob2};
     const uint32_t L = (uint32_t)c->tab[0].L;
 
-    Layout Y = make_layout(c, illumina_spec(c, use_haps, P));
     const std::vector<uint64_t>& group_off = Y.group_off;
     std::vector<GroupDev>& groups = Y.groups;
     const std::vector<Job>& jobs = Y.jobs;
@@ -581,15 +654,15 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
     };
     // --- sequences: the reference's chromosomes, or the haplotype chromosomes the ranges touch (materialised now)
     if (!use_haps) {
-        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = c->genome.p + kPad + c->chrom_off[g];
+        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = d.genome.p + kPad + c->chrom_off[g];
     } else {
         for (size_t k = 0; k < jobs.size(); k++) {
             if (ranges[k].second <= ranges[k].first) continue;
             size_t g_lo, g_hi;
             groups_of(jobs[k], ranges[k].first, ranges[k].second, g_lo, g_hi);
-            for (size_t g = g_lo; g <= g_hi; g++) ensure_hap_chrom(c, Y.group_hap[g], Y.group_chrom[g]);
+            for (size_t g = g_lo; g <= g_hi; g++) ensure_hap_chrom(c, d, Y.group_hap[g], Y.group_chrom[g]);
         }
-        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = c->haps[Y.group_hap[g]].seq[Y.group_chrom[g]];
+        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = d.hap_seq[Y.group_hap[g]][Y.group_chrom[g]];
     }
 
     // --- thresholds
@@ -604,29 +677,29 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
     gp.c_rev = thr_ld_lt(0.5).thr;
     for (int e = 0; e < n_ends; e++) {
         EndDev& E = gp.end[e];
-        E.meta = c->d_meta[e].p; E.entry64 = c->d_entry64[e].p; E.coin = c->d_coin[e].p;
-        E.mis = c->d_mis[e].p;
+        E.meta = d.d_meta[e].p; E.entry64 = d.d_entry64[e].p; E.coin = d.d_coin[e].p;
+        E.mis = d.d_mis[e].p;
         E.entry_n = (uint32_t)c->tab[e].entry64.size();
         Thr ta = thr_double_le(insp[e] + delp[e]);   // u > ins + del  <=>  x >= tA
         Thr ti = thr_double_le(insp[e]);             // u > ins        <=>  x >= tI
         E.tA = ta.thr; E.tA_all = ta.all; E.tI = ti.thr; E.tI_all = ti.all;
         E.hA = ta.all ? 0x10000u : (uint32_t)(ta.thr >> 48);
     }
-    for (cudaEvent_t& ev : c->ev_run) if (!ev) CK(cudaEventCreate(&ev));
-    CK(cudaEventRecord(c->ev_run[0], c->s_compute));
+    for (cudaEvent_t& ev : d.ev_run) if (!ev) CK(cudaEventCreate(&ev));
+    CK(cudaEventRecord(d.ev_run[0], d.s_compute));
     std::vector<uint64_t> frag = frag_table(P->frag_len_shape, P->frag_len_scale, P->frag_len_min, P->frag_len_max);
     std::vector<uint32_t> guide = frag_guide(frag);
-    c->d_frag.upload(frag, c->s_compute);
-    c->d_frag_guide.upload(guide, c->s_compute);
-    c->d_group_off.upload(group_off, c->s_compute);
-    c->d_groups.upload(groups, c->s_compute);
-    c->d_strpool.upload(Y.strpool, c->s_compute);
-    c->d_status.ensure(1);
-    CK(cudaMemsetAsync(c->d_status.p, 0, sizeof(uint32_t), c->s_compute));
-    c->h2d_bytes += frag.size() * 8 + group_off.size() * 8 + groups.size() * sizeof(GroupDev) + Y.strpool.size();
-    gp.frag_cdf = c->d_frag.p; gp.frag_guide = c->d_frag_guide.p; gp.frag_n = (uint32_t)frag.size(); gp.frag_min = P->frag_len_min;
-    gp.group_off = c->d_group_off.p; gp.n_groups = (uint32_t)groups.size();
-    gp.groups = c->d_groups.p; gp.strpool = c->d_strpool.p; gp.status = c->d_status.p;
+    d.d_frag.upload(frag, d.s_compute);
+    d.d_frag_guide.upload(guide, d.s_compute);
+    d.d_group_off.upload(group_off, d.s_compute);
+    d.d_groups.upload(groups, d.s_compute);
+    d.d_strpool.upload(Y.strpool, d.s_compute);
+    d.d_status.ensure(1);
+    CK(cudaMemsetAsync(d.d_status.p, 0, sizeof(uint32_t), d.s_compute));
+    d.h2d_bytes += frag.size() * 8 + group_off.size() * 8 + groups.size() * sizeof(GroupDev) + Y.strpool.size();
+    gp.frag_cdf = d.d_frag.p; gp.frag_guide = d.d_frag_guide.p; gp.frag_n = (uint32_t)frag.size(); gp.frag_min = P->frag_len_min;
+    gp.group_off = d.d_group_off.p; gp.n_groups = (uint32_t)groups.size();
+    gp.groups = d.d_groups.p; gp.strpool = d.d_strpool.p; gp.status = d.d_status.p;
 
     // --- batch buffers
     uint64_t max_range = 0;
@@ -647,7 +720,7 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
     const bool need_host = sink.kind != SINK_NONE && !sizes_only;
     const uint32_t nblk_all = (uint32_t)((B * max_rec + kBgzfIn - 1) / kBgzfIn) + 1;
     const uint32_t nblk_max = dev_z && !sizes_only ? nblk_all : 0;
-    for (Slot& s : c->slot) {
+    for (Slot& s : d.slot) {
         s.plan.ensure(n_rec_max);
         s.rec_len.ensure(n_rec_max);
         s.rec_local.ensure(n_rec_max);
@@ -655,7 +728,7 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
         s.block_base.ensure((size_t)nsb_max * 2);
         s.totals.ensure(4);
         s.h_totals.ensure(4);
-        CK(cudaMemsetAsync(s.totals.p, 0, 4 * sizeof(uint64_t), c->s_compute));
+        CK(cudaMemsetAsync(s.totals.p, 0, 4 * sizeof(uint64_t), d.s_compute));
         for (int e = 0; e < n_ends && !sizes_only; e++) {
             s.out[e].ensure(B * max_rec + 64);
             // compressed bytes of a batch never exceed its FASTQ bytes plus the members' framing (an incompressible block is stored)
@@ -677,8 +750,8 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
     jlp_run_stats st;
     std::memset(&st, 0, sizeof st);
 
-    sink.begin(Z, P->compress, P->n_threads, c->writers);
-    Quiesce quiesce{c, &sink};
+    sink.begin(Z, P->compress, P->n_threads, d.writers);
+    Quiesce quiesce{d, &sink};
     uint64_t job_index = 0;
     // stage 2 of a batch: its kernels are done -> statistics, then its FASTQ starts its way to the host
     // (queued right behind the previous batch's copy, so the bus never idles)
@@ -702,10 +775,10 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
         sink.settle(s.host);                    // the pinned buffers of this slot are free again
         for (int e = 0; e < n_ends; e++) {
             const uint64_t nb = dev_z ? s.ztot[e] : s.tot[e];
-            CK(cudaMemcpyAsync(s.h_out[e].p, dev_z ? s.zdev[e].p : s.out[e].p, nb, cudaMemcpyDeviceToHost, c->s_copy));
+            CK(cudaMemcpyAsync(s.h_out[e].p, dev_z ? s.zdev[e].p : s.out[e].p, nb, cudaMemcpyDeviceToHost, d.s_copy));
             st.d2h_bytes += nb;
         }
-        CK(cudaEventRecord(s.ev[4], c->s_copy));
+        CK(cudaEventRecord(s.ev[4], d.s_copy));
     };
     // stage 3: the copy has landed -> hand the batch to the sink
     auto deliver = [&](Slot& s) {
@@ -719,7 +792,7 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
         s.busy = false;
     };
 
-    std::vector<char> chrom_waited(c->chrom_ev.size(), 0);
+    std::vector<char> chrom_waited(d.chrom_ev.size(), 0);
     if (sizes_only) X.sizes_out->assign(jobs.size(), std::array<uint64_t, 2>{0, 0});
 
     for (size_t jk = 0; jk < jobs.size(); jk++) {
@@ -736,15 +809,15 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
         if (sizes_only) {
             // size pass: placement and scan only; the totals come back batch by batch (a few hundred microseconds each)
             for (uint64_t b0 = lo; b0 < hi; b0 += B) {
-                Slot& s = c->slot[0];
+                Slot& s = d.slot[0];
                 const uint32_t np = (uint32_t)std::min<uint64_t>(B, hi - b0);
                 gp.job_lo = job.lo; gp.job_hi = job.hi; gp.batch_lo = b0; gp.batch_pairs = np;
                 gp.plan = s.plan.p; gp.rec_len = s.rec_len.p; gp.rec_local = s.rec_local.p; gp.block_base = s.block_base.p;
                 gp.n_scan_blocks = (np + kScanBlock - 1) / kScanBlock;
-                CK(launch_place(gp, c->s_compute));
-                CK(launch_scan(s.rec_len.p, np * n_ends, n_ends, s.rec_local.p, s.block_tot.p, s.block_base.p, s.totals.p, c->s_compute));
-                CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->s_compute));
-                CK(cudaStreamSynchronize(c->s_compute));
+                CK(launch_place(gp, d.s_compute));
+                CK(launch_scan(s.rec_len.p, np * n_ends, n_ends, s.rec_local.p, s.block_tot.p, s.block_base.p, s.totals.p, d.s_compute));
+                CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
+                CK(cudaStreamSynchronize(d.s_compute));
                 for (int e = 0; e < n_ends; e++) (*X.sizes_out)[jk][e] += s.h_totals.p[e];
                 st.kernel_launches += 3; st.pairs += np; st.batches++;
             }
@@ -759,46 +832,46 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
         };
         uint64_t bi = 0;
         for (uint64_t b0 = lo; b0 < hi; b0 += B, bi++) {
-            Slot& s = c->slot[bi % 3];
+            Slot& s = d.slot[bi % 3];
             while (s.busy) drain_one();
             const uint32_t np = (uint32_t)std::min<uint64_t>(B, hi - b0);
-            if (c->upload_pending && !use_haps) {
+            if (d.upload_pending && !use_haps) {
                 // make the compute stream wait for exactly the uploads of the chromosomes this batch reads
                 size_t g_lo, g_hi;
                 groups_of(job, b0, b0 + np, g_lo, g_hi);
-                g_hi = std::min(g_hi, c->chrom_ev.size() - 1);
+                g_hi = std::min(g_hi, d.chrom_ev.size() - 1);
                 g_lo = std::min(g_lo, g_hi);
                 if (b0 == lo) {
                     // first batch of this call's part of the job: a deferred upload copies, in the order the part
                     // will read them, all the chromosomes it reads and nothing else (with N GPUs each needs about
                     // 1/N of the genome); the rest stays on the host until some run asks for it
                     size_t g_end = (size_t)(std::upper_bound(group_off.begin(), group_off.end(), hi - 1) - group_off.begin()) - 1;
-                    issue_upload(c, g_lo, std::min(g_end, c->chrom_ev.size() - 1));
+                    issue_upload(c, d, g_lo, std::min(g_end, d.chrom_ev.size() - 1));
                 }
-                issue_upload(c, g_lo, g_hi);
+                issue_upload(c, d, g_lo, g_hi);
                 for (size_t g = g_lo; g <= g_hi; g++)
-                    if (!chrom_waited[g]) { CK(cudaStreamWaitEvent(c->s_compute, c->chrom_ev[g], 0)); chrom_waited[g] = 1; }
+                    if (!chrom_waited[g]) { CK(cudaStreamWaitEvent(d.s_compute, d.chrom_ev[g], 0)); chrom_waited[g] = 1; }
             }
             gp.job_lo = job.lo; gp.job_hi = job.hi; gp.batch_lo = b0; gp.batch_pairs = np;
             const uint32_t n_rec = np * n_ends;
             const uint32_t nsb = (np + kScanBlock - 1) / kScanBlock;
             gp.plan = s.plan.p; gp.rec_len = s.rec_len.p; gp.rec_local = s.rec_local.p; gp.block_base = s.block_base.p;
             gp.n_scan_blocks = nsb; gp.out[0] = s.out[0].p; gp.out[1] = s.out[1].p;
-            CK(cudaEventRecord(s.ev[0], c->s_compute));
-            CK(launch_place(gp, c->s_compute));
-            CK(cudaEventRecord(s.ev[1], c->s_compute));
+            CK(cudaEventRecord(s.ev[0], d.s_compute));
+            CK(launch_place(gp, d.s_compute));
+            CK(cudaEventRecord(s.ev[1], d.s_compute));
             CK(launch_scan(s.rec_len.p, n_rec, n_ends, s.rec_local.p, s.block_tot.p, s.block_base.p, s.totals.p,
-                           c->s_compute));
-            CK(cudaEventRecord(s.ev[2], c->s_compute));
-            CK(launch_reads(gp, c->n_sm, c->s_compute));
-            CK(cudaEventRecord(s.ev[3], c->s_compute));
+                           d.s_compute));
+            CK(cudaEventRecord(s.ev[2], d.s_compute));
+            CK(launch_reads(gp, d.n_sm, d.s_compute));
+            CK(cudaEventRecord(s.ev[3], d.s_compute));
             if (dev_z) {
                 CK(launch_bgzf(s.out[0].p, s.out[1].p, s.totals.p, nblk_max, P->compress >= 4, s.zslots[0].p, s.zslots[1].p, s.zlen[0].p,
-                               s.zlen[1].p, s.zoff[0].p, s.zoff[1].p, s.zdev[0].p, s.zdev[1].p, s.zcode.p, c->s_compute));
+                               s.zlen[1].p, s.zoff[0].p, s.zoff[1].p, s.zdev[0].p, s.zdev[1].p, s.zcode.p, d.s_compute));
                 st.kernel_launches += kBgzfLaunches;
             }
-            CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->s_compute));
-            CK(cudaEventRecord(s.ev[5], c->s_compute));
+            CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
+            CK(cudaEventRecord(s.ev[5], d.s_compute));
             st.kernel_launches += 4;
             s.pairs = np; s.busy = true;
             computing.push_back(&s);
@@ -808,31 +881,31 @@ void run(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, 
             if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();   // Quiesce settles what is in flight
         }
         while (!computing.empty() || !copying.empty()) drain_one();
-        for (Slot& s : c->slot) sink.settle(s.host);
+        for (Slot& s : d.slot) sink.settle(s.host);
         // a multi-GPU run appends the end-of-file block once, after joining the parts
         sink.end_job(job_index, n_ends, !X.shared_files && !X.job_suffix);
         job_index++;
     }
-    CK(cudaEventRecord(c->ev_run[1], c->s_compute));
-    CK(cudaEventSynchronize(c->ev_run[1]));
+    CK(cudaEventRecord(d.ev_run[1], d.s_compute));
+    CK(cudaEventSynchronize(d.ev_run[1]));
     {
         float ms = 0;
-        CK(cudaEventElapsedTime(&ms, c->ev_run[0], c->ev_run[1]));
+        CK(cudaEventElapsedTime(&ms, d.ev_run[0], d.ev_run[1]));
         st.run_ms = ms;
     }
-    if (c->upload_pending) {
+    if (d.upload_pending) {
         // the copies this run issued are done before the caller gets control back; chromosomes no
         // shard of this run touched remain on the host (upload_src must stay valid, see the header)
-        CK(cudaStreamSynchronize(c->s_upload));
-        if (std::find(c->chrom_resident.begin(), c->chrom_resident.end(), 0) == c->chrom_resident.end()) {
-            c->upload_pending = false;
-            c->upload_src = nullptr;
+        CK(cudaStreamSynchronize(d.s_upload));
+        if (std::find(d.chrom_resident.begin(), d.chrom_resident.end(), 0) == d.chrom_resident.end()) {
+            d.upload_pending = false;
+            d.upload_src = nullptr;
         }
     }
     uint32_t status = 0;
-    CK(cudaMemcpy(&status, c->d_status.p, sizeof status, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&status, d.d_status.p, sizeof status, cudaMemcpyDeviceToHost));
     if (status & 1u) throw ArgErr("a barcode is at least as long as a read's template (fragment or chromosome too short)");
-    st.h2d_bytes = c->h2d_bytes - h2d_before;      // of this call (a deferred genome upload it performed included)
+    st.h2d_bytes = d.h2d_bytes - h2d_before;      // of this call (a deferred genome upload it performed included)
     if (stats) *stats = st;
     quiesce.armed = false;
 }
@@ -865,12 +938,11 @@ int multi_abort_cb(void* u) { return static_cast<MultiShared*>(u)->abort.load(st
 void multi_progress_cb(void* u, uint64_t reads) { static_cast<MultiShared*>(u)->progress.fetch_add(reads, std::memory_order_relaxed); }
 
 void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, jlp_run_stats* stats) {
-    check_params(c, use_haps, P, sink.kind);
     if (sink.kind == SINK_STREAM)
         throw Unsupported("jlp_illumina_stream on a multi-GPU context: batches of several devices have no single order; "
                           "use files / memory, or one context per device with shard_index / shard_count");
     if (P->shard_count > 1) throw ArgErr("shard_index / shard_count do not combine with a multi-GPU context");
-    const size_t N = c->kids.size();
+    const size_t N = c->dev.size();
     const Layout Y = make_layout(c, illumina_spec(c, use_haps, P));
     const size_t nj = Y.jobs.size();
     const int n_ends = P->paired || P->matepair ? 2 : 1;
@@ -901,44 +973,28 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
     Pk.abort_cb = multi_abort_cb; Pk.progress_cb = multi_progress_cb; Pk.cb_user = &shared;
     Pk.n_threads = P->n_threads <= 1 ? 1 : std::max<uint64_t>(2, (P->n_threads + N - 1) / N);   // host writer threads per device
 
-    std::vector<std::string> errs(N);
-    std::vector<int> codes(N, JLP_OK);
     std::vector<jlp_run_stats> st(N);
-    // run f(r) for every device on its own thread; the calling thread serves the callbacks meanwhile
-    auto on_devices = [&](const std::function<void(size_t)>& f, bool with_callbacks) {
-        std::atomic<size_t> left{N};
-        std::vector<std::thread> th;
-        for (size_t r = 0; r < N; r++)
-            th.emplace_back([&, r]() {
-                codes[r] = guarded(c->kids[r], [&]() { f(r); });
-                if (codes[r] != JLP_OK) {                     // the others stop at their next batch
-                    errs[r] = c->kids[r]->err;
-                    int none = 0;
-                    shared.abort.compare_exchange_strong(none, 1);
-                }
-                left.fetch_sub(1);
-            });
-        while (left.load() != 0) {
-            std::this_thread::sleep_for(std::chrono::milliseconds(with_callbacks ? 20 : 2));
-            if (!with_callbacks) continue;
-            const uint64_t d = shared.progress.exchange(0);
-            if (d && P->progress_cb) P->progress_cb(P->cb_user, d);
-            if (P->abort_cb && !shared.abort.load() && P->abort_cb(P->cb_user)) shared.abort.store(2);
-        }
-        for (std::thread& t : th) t.join();
-        const uint64_t d = shared.progress.exchange(0);
-        if (d && P->progress_cb && with_callbacks) P->progress_cb(P->cb_user, d);
-        if (shared.abort.load() == 2) throw Aborted();
-        for (size_t r = 0; r < N; r++) {
-            if (codes[r] == JLP_OK || codes[r] == JLP_ERR_ABORTED) continue;      // a device aborted because another failed
-            const std::string m = "device " + std::to_string(c->kids[r]->device) + ": " + errs[r];
-            switch (codes[r]) {
-            case JLP_ERR_ARG: throw ArgErr(errs[r]);
-            case JLP_ERR_IO: throw IoErr(errs[r]);
-            case JLP_ERR_UNSUPPORTED: throw Unsupported(errs[r]);
-            default: throw CudaErr(m);
+    auto serve_callbacks = [&]() {
+        const uint64_t n = shared.progress.exchange(0);
+        if (n && P->progress_cb) P->progress_cb(P->cb_user, n);
+        if (P->abort_cb && !shared.abort.load() && P->abort_cb(P->cb_user)) shared.abort.store(2);
+    };
+    // run f(d, r) for every device d (the r-th); the calling thread serves the callbacks meanwhile
+    auto on_devices = [&](const std::function<void(Device&, size_t)>& f, bool with_callbacks) {
+        on_each_device(c, [&](Device& d) {
+            size_t r = 0;
+            while (c->dev[r].get() != &d) r++;
+            try {
+                f(d, r);
+            } catch (...) {                   // the others stop at their next batch
+                int none = 0;
+                shared.abort.compare_exchange_strong(none, 1);
+                throw;
             }
-        }
+        }, with_callbacks ? std::function<void()>(serve_callbacks) : nullptr);
+        const uint64_t n = shared.progress.exchange(0);
+        if (n && P->progress_cb && with_callbacks) P->progress_cb(P->cb_user, n);
+        if (shared.abort.load() == 2) throw Aborted();
     };
 
     // a shared output file is created with its final size at once (no pages yet; pages are reserved slice by slice by the
@@ -962,11 +1018,11 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
     std::vector<std::array<uint64_t, 2>> job_total(nj, std::array<uint64_t, 2>{0, 0});
     uint64_t launches = 0;
     if (sized) {
-        on_devices([&](size_t r) {
+        on_devices([&](Device& d, size_t r) {
             Output none;
             RunExtras X;
             X.ranges = &ranges[r]; X.sizes_out = &sizes[r];
-            run(c->kids[r], use_haps, &Pk, none, &st[r], X);
+            run(c, d, use_haps, &Pk, Y, none, &st[r], X);
         }, false);
         uint64_t mem_off[2] = {0, 0};
         for (size_t k = 0; k < nj; k++)
@@ -988,11 +1044,11 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
     if (zsized) {
         jlp_illumina_params Pdry = Pk;
         Pdry.progress_cb = nullptr;
-        on_devices([&](size_t r) {
+        on_devices([&](Device& d, size_t r) {
             Output none;
             RunExtras X;
             X.ranges = &ranges[r]; X.zsizes_out = &zsizes[r]; X.dry_files = true;
-            run(c->kids[r], use_haps, &Pdry, none, &st[r], X);
+            run(c, d, use_haps, &Pdry, Y, none, &st[r], X);
         }, true);
         for (size_t r = 0; r < N; r++) launches += st[r].kernel_launches;
         for (size_t k = 0; k < nj; k++)
@@ -1019,7 +1075,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
             for (size_t k = 0; k < nj; k++)
                 if (ranges[r][k].second > ranges[r][k].first && r != first_dev[k])
                     for (int e = 0; e < n_ends; e++) cleanup.names.push_back(file_name(Y.jobs[k], e, true, P) + ".part" + std::to_string(r));
-    on_devices([&](size_t r) {
+    on_devices([&](Device& d, size_t r) {
         Output sk(sink.kind);
         for (int e = 0; e < 2; e++) { sk.mem[e] = sink.mem[e]; sk.cap[e] = sink.cap[e]; }
         RunExtras X;
@@ -1032,7 +1088,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
             X.job_suffix = &suffix;
             for (size_t k = 0; k < nj; k++) suffix.push_back(r == first_dev[k] ? std::string() : ".part" + std::to_string(r));
         }
-        run(c->kids[r], use_haps, &Pk, sk, &st[r], X);
+        run(c, d, use_haps, &Pk, Y, sk, &st[r], X);
     }, true);
 
     if (zsized)         // the coder is deterministic; a difference between the two passes would have put members in the wrong place
@@ -1076,11 +1132,12 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
             }
         // a slice is copied through mappings of both files where that works (threads writing one file through
         // write() / copy_file_range queue on its inode lock; page-cache pages filled through a mapping do not), else by
-        // copy_range; the writer threads of this (multi-GPU) context do the copying
+        // copy_range; the writer threads of the first device do the copying
+        WriterPool& writers = c->dev[0]->writers;
         std::atomic<int> pending{0};
-        c->writers.start(std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32)));
+        writers.start(std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32)));
         for (const CopyTask& t : tasks)
-            c->writers.submit(&pending, [t]() {
+            writers.submit(&pending, [t]() {
                 Mapping mo, mi;
                 std::string w;
                 if (map_range(t.out_fd, t.out_off, t.len, mo) && map_range(t.in_fd, t.in_off, t.len, mi, true))
@@ -1091,8 +1148,8 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
                 mo.unmap();
                 return w;
             });
-        const std::string w = c->writers.wait(pending);
-        if (!w.empty()) { c->writers.clear_error(); throw IoErr("Error joining the devices' parts: " + w); }
+        const std::string w = writers.wait(pending);
+        if (!w.empty()) { writers.clear_error(); throw IoErr("Error joining the devices' parts: " + w); }
     }
 
     jlp_run_stats tot;
@@ -1116,7 +1173,8 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
 
 extern "C" {
 
-int jlp_ctx_create(int device, jlp_ctx** out) {
+// A context over devices[0..n_devices) (NULL: devices 0..n_devices-1; n_devices == 0: every visible device).
+static int create_ctx(int n_devices, const int* devices, jlp_ctx** out) {
     if (!out) return fail(nullptr, JLP_ERR_ARG, "out is NULL");
     *out = nullptr;
     int n = 0;
@@ -1125,115 +1183,64 @@ int jlp_ctx_create(int device, jlp_ctx** out) {
         return fail(nullptr, JLP_ERR_NO_DEVICE,
                     std::string("no CUDA device available (") + cudaGetErrorString(e) +
                         "); this library has no CPU fallback");
-    if (device < 0 || device >= n) return fail(nullptr, JLP_ERR_ARG, "device index out of range");
+    if (n_devices < 0 || n_devices > 64) return fail(nullptr, JLP_ERR_ARG, "n_devices must be 0 (all visible devices) .. 64");
+    if (n_devices == 0) { n_devices = n; devices = nullptr; }
     std::unique_ptr<jlp_ctx> c(new jlp_ctx);
-    c->device = device;
     int rc = guarded(c.get(), [&]() {
-        CK(cudaDeviceGetAttribute(&c->n_sm, cudaDevAttrMultiProcessorCount, device));
-        CK(cudaStreamCreateWithFlags(&c->s_compute, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&c->s_copy, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&c->s_upload, cudaStreamNonBlocking));
-        CK(bgzf_init());
+        for (int i = 0; i < n_devices; i++) {
+            const int id = devices ? devices[i] : i;
+            if (id < 0 || id >= n) throw ArgErr("device index out of range");
+            c->dev.emplace_back(new Device);
+            Device& d = *c->dev.back();
+            d.id = id;
+            CK(cudaSetDevice(id));
+            CK(cudaDeviceGetAttribute(&d.n_sm, cudaDevAttrMultiProcessorCount, id));
+            CK(cudaStreamCreateWithFlags(&d.s_compute, cudaStreamNonBlocking));
+            CK(cudaStreamCreateWithFlags(&d.s_copy, cudaStreamNonBlocking));
+            CK(cudaStreamCreateWithFlags(&d.s_upload, cudaStreamNonBlocking));
+            CK(bgzf_init());
+        }
     });
     if (rc != JLP_OK) { g_create_error = c->err; return rc; }
     *out = c.release();
     return JLP_OK;
 }
 
-int jlp_ctx_create_multi(int n_devices, const int* devices, jlp_ctx** out) {
-    if (!out) return fail(nullptr, JLP_ERR_ARG, "out is NULL");
-    *out = nullptr;
-    int n = 0;
-    cudaError_t e = cudaGetDeviceCount(&n);
-    if (e != cudaSuccess || n == 0)
-        return fail(nullptr, JLP_ERR_NO_DEVICE, std::string("no CUDA device available (") + cudaGetErrorString(e) +
-                                                    "); this library has no CPU fallback");
-    if (n_devices < 0 || n_devices > 64) return fail(nullptr, JLP_ERR_ARG, "n_devices must be 0 (all visible devices) .. 64");
-    if (n_devices == 0) { n_devices = n; devices = nullptr; }
-    std::unique_ptr<jlp_ctx> c(new jlp_ctx);
-    c->device = -1;
-    for (int i = 0; i < n_devices; i++) {
-        const int d = devices ? devices[i] : i;
-        jlp_ctx* k = nullptr;
-        const int rc = jlp_ctx_create(d, &k);
-        if (rc != JLP_OK) { for (jlp_ctx* q : c->kids) jlp_ctx_destroy(q); return rc; }
-        c->kids.push_back(k);
-    }
-    *out = c.release();
-    return JLP_OK;
-}
+int jlp_ctx_create(int device, jlp_ctx** out) { return create_ctx(1, &device, out); }
 
-int jlp_ctx_n_devices(const jlp_ctx* c) { return c ? (c->kids.empty() ? 1 : (int)c->kids.size()) : 0; }
+int jlp_ctx_create_multi(int n_devices, const int* devices, jlp_ctx** out) { return create_ctx(n_devices, devices, out); }
 
-void jlp_ctx_destroy(jlp_ctx* c) {
-    if (!c) return;
-    if (!c->kids.empty()) {
-        for (jlp_ctx* k : c->kids) jlp_ctx_destroy(k);
-        delete c;
-        return;
-    }
-    cudaSetDevice(c->device);
-    cudaDeviceSynchronize();
-    free_haps(c);
-    for (Slot& s : c->slot) for (cudaEvent_t ev : s.ev) if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : c->ev_run) if (ev) cudaEventDestroy(ev);
-    if (c->s_compute) cudaStreamDestroy(c->s_compute);
-    if (c->s_copy) cudaStreamDestroy(c->s_copy);
-    if (c->s_upload) cudaStreamDestroy(c->s_upload);
-    for (int k = 0; k < jlp_ctx::kMatBufs; k++) { if (c->m_up[k]) cudaEventDestroy(c->m_up[k]); if (c->m_done[k]) cudaEventDestroy(c->m_done[k]); }
-    for (cudaEvent_t ev : c->chrom_ev) cudaEventDestroy(ev);
-    c->writers.stop();
-    delete c;
-}
+int jlp_ctx_n_devices(const jlp_ctx* c) { return c ? (int)c->dev.size() : 0; }
+
+void jlp_ctx_destroy(jlp_ctx* c) { delete c; }
 
 const char* jlp_last_error(const jlp_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
 static int set_genome_impl(jlp_ctx* c, const char* bases, const uint64_t* chrom_off, uint64_t n_chroms,
                            const char* const* chrom_names, const char* genome_name, bool wait) {
     if (!c) return JLP_ERR_ARG;
-    if (!c->kids.empty()) {
-        // every device gets a deferred upload (a run copies only the chromosomes the device's piece reads); the
-        // synchronous form then makes the whole genome resident everywhere, one host thread per device
-        return guarded(c, [&]() {
-            for (jlp_ctx* k : c->kids) {
-                const int rc = set_genome_impl(k, bases, chrom_off, n_chroms, chrom_names, genome_name, false);
-                if (rc != JLP_OK) throw ArgErr(k->err);
-            }
-            c->haps.clear();
-            c->chrom_off = c->kids[0]->chrom_off; c->chrom_names = c->kids[0]->chrom_names; c->genome_name = c->kids[0]->genome_name;
-            if (wait) for_each_device_parallel(c, [](jlp_ctx* d) { finish_upload(d); });
-        });
-    }
     return guarded(c, [&]() {
         if (!bases || !chrom_off || !chrom_names || n_chroms == 0) throw ArgErr("empty genome");
         for (uint64_t i = 0; i < n_chroms; i++)
             if (chrom_off[i + 1] < chrom_off[i]) throw ArgErr("chrom_off must be non-decreasing");
         if (chrom_off[0] != 0) throw ArgErr("chrom_off[0] must be 0");
-        if (c->upload_pending) {      // a deferred upload that never ran is simply dropped
-            c->upload_src = nullptr;
-            CK(cudaStreamSynchronize(c->s_upload));
-            c->upload_pending = false;
-        }
-        free_haps(c);
-        c->chrom_off.assign(chrom_off, chrom_off + n_chroms + 1);
-        c->chrom_names.clear();
-        for (uint64_t i = 0; i < n_chroms; i++) c->chrom_names.push_back(chrom_names[i] ? chrom_names[i] : "");
-        c->genome_name = genome_name ? genome_name : "REF";
-        uint64_t total = chrom_off[n_chroms];
-        c->genome.ensure(total + 2 * kPad);
-        while (c->chrom_ev.size() < n_chroms) {
-            cudaEvent_t ev;
-            CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            c->chrom_ev.push_back(ev);
-        }
+        std::vector<std::string> names;
+        for (uint64_t i = 0; i < n_chroms; i++) names.push_back(chrom_names[i] ? chrom_names[i] : "");
         // one copy and one event per chromosome: generation starts as soon as the chromosomes a batch
         // reads are resident, the rest of the genome follows underneath (PCIe is full duplex, the
         // FASTQ flows the other way).  The asynchronous form defers the copies to the next run, which
-        // starts them at the first chromosome its shard reads.
-        c->upload_src = bases;
-        c->upload_pending = true;
-        c->chrom_resident.assign(n_chroms, 0);
-        if (wait) finish_upload(c);
+        // starts them at the first chromosome its shard reads (with several devices: each device's piece).
+        replace_genome(c, std::vector<uint64_t>(chrom_off, chrom_off + n_chroms + 1), names, genome_name, [&](Device& d) {
+            while (d.chrom_ev.size() < n_chroms) {
+                cudaEvent_t ev;
+                CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+                d.chrom_ev.push_back(ev);
+            }
+            d.upload_src = bases;
+            d.upload_pending = true;
+            d.chrom_resident.assign(n_chroms, 0);
+            if (wait) finish_upload(c, d);
+        });
     });
 }
 
@@ -1249,40 +1256,24 @@ int jlp_set_genome_async(jlp_ctx* c, const char* bases, const uint64_t* chrom_of
 
 int jlp_genome_sync(jlp_ctx* c) {
     if (!c) return JLP_ERR_ARG;
-    return guarded(c, [&]() {
-        for_each_device_parallel(c, [](jlp_ctx* d) { finish_upload(d); });
-    });
+    return guarded(c, [&]() { on_each_device(c, [&](Device& d) { finish_upload(c, d); }); });
 }
 
 int jlp_create_genome(jlp_ctx* c, uint64_t n_chroms, const uint64_t* lens, const double* pi_tcag, uint64_t seed,
                       const char* const* chrom_names, const char* genome_name) {
     if (!c) return JLP_ERR_ARG;
-    if (!c->kids.empty())        // the same seed gives every device the same genome: generated in place everywhere, nothing copied
-        return guarded(c, [&]() {
-            for (jlp_ctx* k : c->kids) {
-                const int rc = jlp_create_genome(k, n_chroms, lens, pi_tcag, seed, chrom_names, genome_name);
-                if (rc != JLP_OK) throw ArgErr(k->err);
-            }
-            c->haps.clear();
-            c->chrom_off = c->kids[0]->chrom_off; c->chrom_names = c->kids[0]->chrom_names; c->genome_name = c->kids[0]->genome_name;
-        });
     return guarded(c, [&]() {
         if (!lens || !pi_tcag || n_chroms == 0) throw ArgErr("empty genome");
         double tot = 0;
         for (int k = 0; k < 4; k++) { if (!(pi_tcag[k] >= 0)) throw ArgErr("pi_tcag must be >= 0"); tot += pi_tcag[k]; }
         if (!(tot > 0)) throw ArgErr("pi_tcag must have at least one value > 0");
-        if (c->upload_pending) { c->upload_src = nullptr; CK(cudaStreamSynchronize(c->s_upload)); c->upload_pending = false; }
-        free_haps(c);
-        c->chrom_off.assign(1, 0);
-        c->chrom_names.clear();
+        std::vector<uint64_t> off(1, 0);
+        std::vector<std::string> names;
         for (uint64_t i = 0; i < n_chroms; i++) {
             if (lens[i] == 0) throw ArgErr("chromosome lengths must be >= 1");       // "never returns empty chromosomes"
-            c->chrom_off.push_back(c->chrom_off.back() + lens[i]);
-            c->chrom_names.push_back(chrom_names && chrom_names[i] ? chrom_names[i] : "chrom" + std::to_string(i));   // src/create_sequences.cpp:178-181
+            off.push_back(off.back() + lens[i]);
+            names.push_back(chrom_names && chrom_names[i] ? chrom_names[i] : "chrom" + std::to_string(i));   // src/create_sequences.cpp:178-181
         }
-        c->genome_name = genome_name ? genome_name : "REF";
-        c->chrom_resident.assign(n_chroms, 1);
-        c->genome.ensure(c->chrom_off.back() + 2 * kPad);
         // AliasSampler(pi_tcag), src/alias_sampler.h:68-106
         double Prob[4];
         uint64_t Alias[4];
@@ -1292,36 +1283,33 @@ int jlp_create_genome(jlp_ctx* c, uint64_t n_chroms, const uint64_t* lens, const
             Thr th = thr_double_lt(Prob[k]);
             t.thr[k] = th.thr; t.thr16[k] = (uint32_t)(th.thr >> 48); t.alias[k] = (uint32_t)Alias[k];
         }
-        for (uint64_t i = 0; i < n_chroms; i++)
-            CK(launch_create_chrom(c->genome.p + kPad + c->chrom_off[i], lens[i], (uint32_t)i, seed, t, c->s_compute));
-        CK(cudaStreamSynchronize(c->s_compute));
+        // the same seed gives every device the same genome: generated in place everywhere, nothing copied
+        replace_genome(c, off, names, genome_name, [&](Device& d) {
+            d.chrom_resident.assign(n_chroms, 1);
+            for (uint64_t i = 0; i < n_chroms; i++)
+                CK(launch_create_chrom(d.genome.p + kPad + off[i], lens[i], (uint32_t)i, seed, t, d.s_compute));
+            CK(cudaStreamSynchronize(d.s_compute));
+        });
     });
 }
 
 int jlp_get_genome(jlp_ctx* c, char* out, uint64_t cap, uint64_t* len) {
     if (!c) return JLP_ERR_ARG;
-    if (!c->kids.empty()) {
-        const int rc = jlp_get_genome(c->kids[0], out, cap, len);
-        if (rc != JLP_OK) c->err = c->kids[0]->err;
-        return rc;
-    }
     return guarded(c, [&]() {
         if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
-        finish_upload(c);
+        Device& d = device0(c);
+        finish_upload(c, d);
         const uint64_t n = c->chrom_off.back();
         if (len) *len = n;
         if (!out) return;
         if (n > cap) throw ArgErr("output buffer too small");
-        CK(cudaMemcpy(out, c->genome.p + kPad, n, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(out, d.genome.p + kPad, n, cudaMemcpyDeviceToHost));
     });
 }
 
 int jlp_clear_haplotypes(jlp_ctx* c) {
     if (!c) return JLP_ERR_ARG;
-    return guarded(c, [&]() {
-        for_each_device(c, [](jlp_ctx* d) { free_haps(d); });
-        c->haps.clear();
-    });
+    return guarded(c, [&]() { clear_haps(c); });
 }
 
 // the host-side store of one haplotype: a copy of the caller's AllMutations arrays + size_modifier per record, one packed
@@ -1382,15 +1370,13 @@ static std::shared_ptr<HapStore> make_hap_store(const jlp_ctx* c, const char* na
 
 // attach a haplotype to a context: unmutated chromosomes alias the reference, the others wait for a run to touch them
 static void attach_hap(jlp_ctx* c, const std::shared_ptr<HapStore>& S) {
-    HapDev H;
-    H.store = S;
-    const bool device = c->kids.empty();
-    for (size_t ci = 0; ci < S->chrom.size(); ci++) {
-        const HapChromHost& M = S->chrom[ci];
-        H.len.push_back(M.size);
-        H.seq.push_back(device && M.n_muts == 0 ? c->genome.p + kPad + c->chrom_off[ci] : nullptr);
+    c->haps.push_back(S);
+    for (auto& d : c->dev) {
+        std::vector<const uint8_t*> seq;
+        for (size_t ci = 0; ci < S->chrom.size(); ci++)
+            seq.push_back(S->chrom[ci].n_muts == 0 ? d->genome.p + kPad + c->chrom_off[ci] : nullptr);
+        d->hap_seq.push_back(std::move(seq));
     }
-    c->haps.push_back(std::move(H));
 }
 
 int jlp_add_haplotype(jlp_ctx* c, const char* name, const uint64_t* n_muts, const uint64_t* const* old_pos,
@@ -1402,18 +1388,17 @@ int jlp_add_haplotype(jlp_ctx* c, const char* name, const uint64_t* n_muts, cons
         std::shared_ptr<HapStore> S = make_hap_store(c, name, n_muts, old_pos, new_pos, nuc_off, nuc_pool, nuc_pool_len, chrom_sizes);
         if (hap_index) *hap_index = c->haps.size();
         attach_hap(c, S);
-        for (jlp_ctx* k : c->kids) attach_hap(k, S);
     });
 }
 
 int jlp_materialize_haplotypes(jlp_ctx* c) {
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
-        for_each_device(c, [&](jlp_ctx* d) {
-            finish_upload(d);
-            for (size_t h = 0; h < d->haps.size(); h++)
-                for (size_t ci = 0; ci < d->haps[h].seq.size(); ci++) ensure_hap_chrom(d, h, ci);
-            CK(cudaStreamSynchronize(d->s_compute));
+        on_each_device(c, [&](Device& d) {
+            finish_upload(c, d);
+            for (size_t h = 0; h < d.hap_seq.size(); h++)
+                for (size_t ci = 0; ci < d.hap_seq[h].size(); ci++) ensure_hap_chrom(c, d, h, ci);
+            CK(cudaStreamSynchronize(d.s_compute));
         });
     });
 }
@@ -1421,16 +1406,15 @@ int jlp_materialize_haplotypes(jlp_ctx* c) {
 int jlp_get_haplotype_chrom(jlp_ctx* c, uint64_t hap, uint64_t chrom, char* out, uint64_t cap, uint64_t* len) {
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
-        jlp_ctx* d = c->kids.empty() ? c : c->kids[0];
-        if (!c->kids.empty()) CK(cudaSetDevice(d->device));
-        if (hap >= d->haps.size() || chrom >= d->haps[hap].seq.size()) throw ArgErr("haplotype / chromosome index out of range");
-        uint64_t n = d->haps[hap].len[chrom];
+        if (hap >= c->haps.size() || chrom >= c->haps[hap]->chrom.size()) throw ArgErr("haplotype / chromosome index out of range");
+        uint64_t n = c->haps[hap]->chrom[chrom].size;
         if (len) *len = n;
         if (n > cap) throw ArgErr("output buffer too small");
-        finish_upload(d);
-        ensure_hap_chrom(d, hap, chrom);
-        CK(cudaStreamSynchronize(d->s_compute));
-        if (n) CK(cudaMemcpy(out, d->haps[hap].seq[chrom], n, cudaMemcpyDeviceToHost));
+        Device& d = device0(c);
+        finish_upload(c, d);
+        ensure_hap_chrom(c, d, hap, chrom);
+        CK(cudaStreamSynchronize(d.s_compute));
+        if (n) CK(cudaMemcpy(out, d.hap_seq[hap][chrom], n, cudaMemcpyDeviceToHost));
     });
 }
 
@@ -1439,8 +1423,8 @@ int jlp_get_haplotype_muts(jlp_ctx* c, uint64_t hap, uint64_t chrom, uint64_t* o
                            uint64_t* pool_len, uint64_t* chrom_size) {
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
-        if (hap >= c->haps.size() || chrom >= c->haps[hap].store->chrom.size()) throw ArgErr("haplotype / chromosome index out of range");
-        const HapChromHost& H = c->haps[hap].store->chrom[chrom];
+        if (hap >= c->haps.size() || chrom >= c->haps[hap]->chrom.size()) throw ArgErr("haplotype / chromosome index out of range");
+        const HapChromHost& H = c->haps[hap]->chrom[chrom];
         const uint64_t M = H.n_muts;
         if (n_muts) *n_muts = M;
         if (pool_len) *pool_len = H.pool_bytes;
@@ -1579,14 +1563,14 @@ int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation
         cat_thr[0] = prob_threshold(p->invariant);
         for (uint32_t j = 1; j < K; j++) cat_thr[j] = prob_threshold(p->invariant + j * (1 - p->invariant) / K);
 
-        jlp_ctx* d = first_device(c);
-        finish_upload(d);
-        cudaStream_t s = d->s_compute;
+        Device& d = device0(c);
+        finish_upload(c, d);
+        cudaStream_t s = d.s_compute;
         DevBuf<uint64_t> d_off, d_cat, d_region, d_region_n, d_out;
         DevBuf<uint32_t> d_tile0, d_cnt;
         DevBuf<MutNode> d_sched;
         DevBuf<uint4> d_hi, d_lo;
-        d_off.upload(d->chrom_off, s);
+        d_off.upload(c->chrom_off, s);
         d_tile0.upload(tile0, s);
         d_sched.upload(sched, s);
         d_cat.upload(cat_thr, s);
@@ -1598,7 +1582,7 @@ int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation
         d_region_n.ensure((size_t)n_tips * nc);
         MutParams mp{};
         mp.seed = p->seed;
-        mp.genome = d->genome.p + kPad;
+        mp.genome = d.genome.p + kPad;
         mp.chrom_off = d_off.p;
         mp.tile0 = d_tile0.p;
         mp.n_chroms = (uint32_t)nc; mp.n_tiles = n_tiles; mp.n_tips = n_tips; mp.n_sched = (uint32_t)sched.size();
@@ -1648,7 +1632,7 @@ int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation
         std::atomic<size_t> next{0};
         std::mutex err_mu;
         std::string err;
-        const int dev = d->device;
+        const int dev = d.id;
         auto work = [&]() {
             try {
                 CK(cudaSetDevice(dev));
@@ -1673,12 +1657,8 @@ int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation
         if (!err.empty()) throw CudaErr(err);
         CK(cudaSetDevice(dev));
 
-        for_each_device(c, [](jlp_ctx* k) { free_haps(k); });
-        c->haps.clear();
-        for (const auto& S : stores) {
-            attach_hap(c, S);
-            for (jlp_ctx* k : c->kids) attach_hap(k, S);
-        }
+        clear_haps(c);
+        for (const auto& S : stores) attach_hap(c, S);
         if (stats) {
             const auto t1 = std::chrono::steady_clock::now();
             stats->count_ms = count_ms;
@@ -1703,27 +1683,22 @@ int jlp_set_profile(jlp_ctx* c, int end, uint64_t read_length, const uint32_t* n
         if (!nq || !probs || !quals) throw ArgErr("profile arrays are NULL");
         if (read_length >= 65536) throw ArgErr("read_length too large");
         build_end_tables(read_length, nq, probs, quals, c->tab[end]);
-        if (!c->kids.empty()) {        // the parent keeps the host tables (read length, checks); every device gets its copy
-            for (jlp_ctx* k : c->kids) {
-                const int rc = jlp_set_profile(k, end, read_length, nq, probs, quals);
-                if (rc != JLP_OK) throw ArgErr(k->err);
-            }
-            c->have_prof[end] = true;
-            return;
-        }
         const EndTables& t = c->tab[end];
-        c->d_meta[end].upload(t.meta, c->s_compute);
-        c->d_entry64[end].upload(t.entry64, c->s_compute);
-        c->d_coin[end].upload(t.coin, c->s_compute);
-        c->d_mis[end].upload(t.mis, c->s_compute);
-        CK(cudaStreamSynchronize(c->s_compute));
-        c->h2d_bytes += t.meta.size() * 4 + t.entry64.size() * 16 + 256 * 8;
+        on_each_device(c, [&](Device& d) {
+            d.d_meta[end].upload(t.meta, d.s_compute);
+            d.d_entry64[end].upload(t.entry64, d.s_compute);
+            d.d_coin[end].upload(t.coin, d.s_compute);
+            d.d_mis[end].upload(t.mis, d.s_compute);
+            CK(cudaStreamSynchronize(d.s_compute));
+            d.h2d_bytes += t.meta.size() * 4 + t.entry64.size() * 16 + 256 * 8;
+        });
         c->have_prof[end] = true;
     });
 }
 
 static void run_any(jlp_ctx* c, bool use_haps, const jlp_illumina_params* p, Output& s, jlp_run_stats* stats) {
-    if (c->kids.empty()) run(c, use_haps, p, s, stats);
+    check_params(c, use_haps, p, s.kind);
+    if (c->dev.size() == 1) run(c, *c->dev[0], use_haps, p, make_layout(c, illumina_spec(c, use_haps, p)), s, stats);
     else run_multi(c, use_haps, p, s, stats);
 }
 
@@ -1818,7 +1793,7 @@ Compression pacbio_compression(const jlp_pacbio_params* P, SinkKind kind) {
 // The driver: per batch the per-read quantities are prepared on the host (batch k + 1 on a helper thread while batch k
 // is on the device), then plan upload, k_pb_plan, scan, k_pb_reads, optional BGZF, copy, and the write of batch k
 // overlaps the next batch.  Callbacks are called on the calling thread between batches.
-void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& sink, jlp_run_stats* stats) {
+void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P, Output& sink, jlp_run_stats* stats) {
     PbModel model;
     pb_model_from(P, model);
     // the quantiles computed by earlier calls with the same pass-sampler parameters are kept (each costs a bisection on
@@ -1839,28 +1814,28 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& s
         const std::string m = P->comp_method ? P->comp_method : "";
         if (m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");
     }
-    finish_upload(c);
+    finish_upload(c, d);
     Layout G = make_layout(c, LayoutSpec(use_haps, P, P->n_reads));
     for (size_t g = 0; g < G.groups.size(); g++) {
         const uint32_t h = G.group_hap[g], ci = G.group_chrom[g];
-        if (use_haps && G.group_off[g + 1] > G.group_off[g]) ensure_hap_chrom(c, h, ci);   // materialised when first read from
-        G.groups[g].seq = use_haps ? c->haps[h].seq[ci] : c->genome.p + kPad + c->chrom_off[ci];
+        if (use_haps && G.group_off[g + 1] > G.group_off[g]) ensure_hap_chrom(c, d, h, ci);   // materialised when first read from
+        G.groups[g].seq = use_haps ? d.hap_seq[h][ci] : d.genome.p + kPad + c->chrom_off[ci];
     }
     const Compression Z = pacbio_compression(P, sink.kind);
     const bool dev_z = Z.dev_z;
     // the slots' buffers (pinning a gigabyte of host memory on every call cost more than generating the reads, and a dozen
     // device allocations and frees per call several milliseconds): the device arrays of slot 0, and the pinned buffers of
     // slots 0 and 1, between which batches alternate so that batch k is written while batch k + 1 is on its way
-    Slot& S0 = c->slot[0];
+    Slot& S0 = d.slot[0];
     cudaEvent_t* ev = S0.ev;
     for (cudaEvent_t& e : S0.ev) if (!e) CK(cudaEventCreate(&e));
     uint64_t n_batch = 0;
-    sink.begin(Z, P->compress, P->n_threads, c->writers);
-    Quiesce quiesce{c, &sink};
-    c->d_groups.upload(G.groups, c->s_compute);
-    c->d_strpool.upload(G.strpool, c->s_compute);
+    sink.begin(Z, P->compress, P->n_threads, d.writers);
+    Quiesce quiesce{d, &sink};
+    d.d_groups.upload(G.groups, d.s_compute);
+    d.d_strpool.upload(G.strpool, d.s_compute);
     S0.totals.ensure(4);
-    CK(cudaMemsetAsync(S0.totals.p, 0, 4 * sizeof(uint64_t), c->s_compute));
+    CK(cudaMemsetAsync(S0.totals.p, 0, 4 * sizeof(uint64_t), d.s_compute));
     uint64_t B = P->batch_reads ? P->batch_reads : 32768;
     // a chain of duplicates never leaves its pool (src/hts.h:266-267): batches are whole pools, so a duplicate's leader is in
     // its batch
@@ -1955,7 +1930,7 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& s
         {   // the per-read device arrays once, for the largest batch of the job (growing them batch by batch would
             // free and allocate -- and synchronise -- at every step of the ramp)
             const uint64_t n_max = std::min<uint64_t>(B, s_hi - s_lo);
-            c->pb_reads.ensure(n_max); S0.rec_len.ensure(n_max); S0.rec_local.ensure(n_max);
+            d.pb_reads.ensure(n_max); S0.rec_len.ensure(n_max); S0.rec_local.ensure(n_max);
             const uint64_t nsb_max = (n_max + kScanBlock - 1) / kScanBlock;
             S0.block_tot.ensure(nsb_max); S0.block_base.ensure(nsb_max);
         }
@@ -1989,35 +1964,35 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& s
             std::vector<PbRead>& plan = cur.plan;
             const uint64_t bound = cur.bound;
             t0 = now();
-            c->pb_reads.ensure(n);
+            d.pb_reads.ensure(n);
             S0.rec_len.ensure(n); S0.rec_local.ensure(n);
             const uint32_t nsb = (n + kScanBlock - 1) / kScanBlock;
             S0.block_tot.ensure(nsb); S0.block_base.ensure(nsb);
             grow(S0.out[0], bound, n);
             t_alloc += now() - t0;
-            CK(cudaMemcpyAsync(c->pb_reads.p, plan.data(), n * sizeof(PbRead), cudaMemcpyHostToDevice, c->s_compute));
+            CK(cudaMemcpyAsync(d.pb_reads.p, plan.data(), n * sizeof(PbRead), cudaMemcpyHostToDevice, d.s_compute));
             st.h2d_bytes += n * sizeof(PbRead);
-            CK(cudaEventRecord(ev[0], c->s_compute));
-            CK(launch_pb_plan(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, c_rev, S0.rec_len.p, c->s_compute));
-            if (dups) { CK(launch_pb_dups(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, S0.rec_len.p, c->s_compute)); st.kernel_launches++; }
-            CK(launch_scan(S0.rec_len.p, n, 1, S0.rec_local.p, S0.block_tot.p, S0.block_base.p, S0.totals.p, c->s_compute));
-            CK(launch_pb_reads(c->pb_reads.p, n, b0, P->seed, c->d_groups.p, c->d_strpool.p, S0.rec_local.p, S0.block_base.p, S0.out[0].p,
-                               c->s_compute));
-            CK(cudaEventRecord(ev[1], c->s_compute));
+            CK(cudaEventRecord(ev[0], d.s_compute));
+            CK(launch_pb_plan(d.pb_reads.p, n, b0, P->seed, d.d_groups.p, c_rev, S0.rec_len.p, d.s_compute));
+            if (dups) { CK(launch_pb_dups(d.pb_reads.p, n, b0, P->seed, d.d_groups.p, S0.rec_len.p, d.s_compute)); st.kernel_launches++; }
+            CK(launch_scan(S0.rec_len.p, n, 1, S0.rec_local.p, S0.block_tot.p, S0.block_base.p, S0.totals.p, d.s_compute));
+            CK(launch_pb_reads(d.pb_reads.p, n, b0, P->seed, d.d_groups.p, d.d_strpool.p, S0.rec_local.p, S0.block_base.p, S0.out[0].p,
+                               d.s_compute));
+            CK(cudaEventRecord(ev[1], d.s_compute));
             st.kernel_launches += 4;
             const uint32_t nblk = (uint32_t)((bound + kBgzfIn - 1) / kBgzfIn) + 1;
             if (dev_z) {
                 S0.zslots[0].ensure((size_t)nblk * kBgzfSlot); S0.zdev[0].ensure((size_t)nblk * kBgzfSlot);
                 S0.zlen[0].ensure(2 * nblk); S0.zoff[0].ensure(2 * nblk); S0.zcode.ensure(kBgzfCodeBytes);
                 CK(launch_bgzf(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress >= 4, S0.zslots[0].p, S0.zslots[0].p, S0.zlen[0].p, S0.zlen[0].p + nblk,
-                               S0.zoff[0].p, S0.zoff[0].p + nblk, S0.zdev[0].p, S0.zdev[0].p, S0.zcode.p, c->s_compute));
+                               S0.zoff[0].p, S0.zoff[0].p + nblk, S0.zdev[0].p, S0.zdev[0].p, S0.zcode.p, d.s_compute));
                 st.kernel_launches += kBgzfLaunches;
             }
-            CK(cudaEventRecord(ev[2], c->s_compute));
+            CK(cudaEventRecord(ev[2], d.s_compute));
             uint64_t tot[4];
-            CK(cudaMemcpyAsync(tot, S0.totals.p, sizeof tot, cudaMemcpyDeviceToHost, c->s_compute));
+            CK(cudaMemcpyAsync(tot, S0.totals.p, sizeof tot, cudaMemcpyDeviceToHost, d.s_compute));
             t0 = now();
-            CK(cudaStreamSynchronize(c->s_compute));
+            CK(cudaStreamSynchronize(d.s_compute));
             t_sync += now() - t0;
             if (tot[0] > bound) throw std::runtime_error("internal: PacBio batch larger than its bound");
             float ms = 0;
@@ -2027,7 +2002,7 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& s
             if (dev_z) st.z_bytes[0] += tot[2];
             if (sink.kind == SINK_NONE) { if (P->progress_cb) P->progress_cb(P->cb_user, n); continue; }
             const uint64_t nb = dev_z ? tot[2] : tot[0];
-            Slot& hs = c->slot[n_batch++ & 1];
+            Slot& hs = d.slot[n_batch++ & 1];
             sink.settle(hs.host);                            // the batch before last is in the file
             PinBuf<uint8_t>& h_out = hs.h_out[0];
             grow(h_out, nb, n);
@@ -2039,7 +2014,7 @@ void run_pacbio(jlp_ctx* c, bool use_haps, const jlp_pacbio_params* P, Output& s
             if (P->progress_cb) P->progress_cb(P->cb_user, n);                  // Progress::increment, src/hts.h:414
         }
         if (prep_thread.joinable()) prep_thread.join();
-        sink.settle(c->slot[0].host); sink.settle(c->slot[1].host);
+        sink.settle(d.slot[0].host); sink.settle(d.slot[1].host);
         if (trace)
             std::fprintf(stderr, "[jlp trace] pacbio job %llu reads: %.4f s (first prepare %.4f, waiting for later ones %.4f, "
                          "device allocations %.4f, waiting for the device %.4f)\n", (unsigned long long)(s_hi - s_lo), now() - t_job,
@@ -2057,7 +2032,7 @@ int jlp_pacbio(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params* p, jlp_r
     return guarded(c, [&]() {
         if (!p || !p->out_prefix || !*p->out_prefix) throw ArgErr("out_prefix is empty");
         Output out(SINK_FILES);
-        run_pacbio(first_device(c), use_haplotypes != 0, p, out, stats);
+        run_pacbio(c, device0(c), use_haplotypes != 0, p, out, stats);
     });
 }
 
@@ -2067,7 +2042,7 @@ int jlp_pacbio_to_memory(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params
     return guarded(c, [&]() {
         Output sink(out ? SINK_MEMORY : SINK_NONE);
         sink.mem[0] = out; sink.cap[0] = out ? cap : 0;
-        run_pacbio(first_device(c), use_haplotypes != 0, p, sink, stats);
+        run_pacbio(c, device0(c), use_haplotypes != 0, p, sink, stats);
         if (len) *len = sink.len[0];
         if (out && sink.len[0] > cap) throw ArgErr("output buffer too small");
     });
@@ -2140,7 +2115,7 @@ int jlp_bgzf_device(jlp_ctx* c, int level, const void* in, uint64_t n, void* out
     if (!c) return JLP_ERR_ARG;
     return guarded(c, [&]() {
         if ((n && !in) || !len) throw ArgErr("NULL argument");
-        c = first_device(c);
+        Device& d = device0(c);
         const uint32_t nblk = (uint32_t)((n + kBgzfIn - 1) / kBgzfIn);
         DevBuf<uint8_t> d_in, d_slots, d_out, d_code;
         DevBuf<uint32_t> d_zlen;
@@ -2148,13 +2123,13 @@ int jlp_bgzf_device(jlp_ctx* c, int level, const void* in, uint64_t n, void* out
         d_in.ensure(n + 64); d_slots.ensure((size_t)nblk * kBgzfSlot); d_out.ensure((size_t)nblk * kBgzfSlot);
         d_zlen.ensure(nblk); d_zoff.ensure(nblk); d_tot.ensure(4); d_code.ensure(kBgzfCodeBytes);
         const uint64_t tot[4] = {n, 0, 0, 0};
-        if (n) CK(cudaMemcpyAsync(d_in.p, in, n, cudaMemcpyHostToDevice, c->s_compute));
-        CK(cudaMemcpyAsync(d_tot.p, tot, sizeof tot, cudaMemcpyHostToDevice, c->s_compute));
+        if (n) CK(cudaMemcpyAsync(d_in.p, in, n, cudaMemcpyHostToDevice, d.s_compute));
+        CK(cudaMemcpyAsync(d_tot.p, tot, sizeof tot, cudaMemcpyHostToDevice, d.s_compute));
         CK(launch_bgzf(d_in.p, d_in.p, d_tot.p, nblk, level >= 4, d_slots.p, d_slots.p, d_zlen.p, d_zlen.p, d_zoff.p, d_zoff.p, d_out.p,
-                       d_out.p, d_code.p, c->s_compute));
+                       d_out.p, d_code.p, d.s_compute));
         uint64_t back[4];
-        CK(cudaMemcpyAsync(back, d_tot.p, sizeof back, cudaMemcpyDeviceToHost, c->s_compute));
-        CK(cudaStreamSynchronize(c->s_compute));
+        CK(cudaMemcpyAsync(back, d_tot.p, sizeof back, cudaMemcpyDeviceToHost, d.s_compute));
+        CK(cudaStreamSynchronize(d.s_compute));
         *len = back[2] + sizeof kBgzfEof;
         if (!out) return;
         if (cap < *len) throw ArgErr("output buffer too small");
