@@ -81,10 +81,27 @@ class MutationStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class IndelParams(C.Structure):
+    _fields_ = [
+        ("rate_ins", C.c_double), ("rate_del", C.c_double), ("n_ins", C.c_uint32), ("n_del", C.c_uint32),
+        ("w_ins", f64p), ("w_del", f64p), ("epsilon", C.c_double), ("pi", C.c_double * 4),
+    ]
+
+
+class IndelStats(C.Structure):
+    _fields_ = [
+        ("insertions", C.c_uint64), ("deletions", C.c_uint64), ("inserted_bases", C.c_uint64),
+        ("indel_records", C.c_uint64), ("steps", C.c_uint64), ("event_ms", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/jlp_b200.h declares
 SYMBOLS = [
     "jlp_ctx_create", "jlp_ctx_create_multi", "jlp_ctx_n_devices", "jlp_materialize_haplotypes", "jlp_ctx_destroy", "jlp_last_error", "jlp_set_genome", "jlp_set_genome_async", "jlp_genome_sync", "jlp_create_genome", "jlp_get_genome", "jlp_genome_draw", "jlp_clear_haplotypes",
-    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_get_haplotype_muts", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
+    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_get_haplotype_muts", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
     "jlp_illumina_to_memory", "jlp_illumina_stream", "jlp_illumina_device_only", "jlp_illumina_group_counts", "jlp_apportion", "jlp_shard_range", "jlp_deflate", "jlp_bgzf_device", "jlp_pacbio", "jlp_pacbio_to_memory", "jlp_pacbio_read_plan", "jlp_pacbio_sample", "jlp_reads_per_group", "jlp_alias_build",
     "jlp_threshold", "jlp_unif_expr", "jlp_frag_table", "jlp_philox4x32_10", "jlp_draw_pos", "jlp_draw_pair",
     "jlp_version",
@@ -123,6 +140,8 @@ def lib():
                                     C.POINTER(u64p), C.POINTER(C.c_void_p), u64p, u64p, u64p]
     L.jlp_get_haplotype_chrom.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint64, u64p]
     L.jlp_create_haplotypes.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(MutationStats)]
+    L.jlp_create_haplotypes_indels.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(IndelParams),
+                                               C.POINTER(MutationStats), C.POINTER(IndelStats)]
     L.jlp_get_haplotype_muts.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, u64p, u64p, u64p, C.c_void_p, C.c_uint64,
                                          C.c_uint64, u64p, u64p, u64p]
     L.jlp_transition_matrix.argtypes = [f64p, C.c_double, f64p]

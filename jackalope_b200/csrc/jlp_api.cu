@@ -1500,178 +1500,367 @@ struct EventSet {
 
 }  // namespace
 
-int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation_stats* stats) {
-    if (!c || !p) return JLP_ERR_ARG;
-    return guarded(c, [&]() {
-        const auto t0 = std::chrono::steady_clock::now();
-        if (c->chrom_off.size() < 2) throw ArgErr("set the reference genome first");
-        for (int i = 0; i < 16; i++)
-            if (i % 5 && !(std::isfinite(p->Q[i]) && p->Q[i] >= 0)) throw ArgErr("the off-diagonal rates of Q must be finite and >= 0");
-        if (!(p->invariant >= 0 && p->invariant < 1)) throw ArgErr("invariant must be >= 0 and < 1");
-        if (p->n_rates < 1 || p->n_rates > 255 || !p->rates) throw ArgErr("n_rates must be 1..255 (rates not NULL)");
-        for (uint32_t k = 0; k < p->n_rates; k++)
-            if (!(std::isfinite(p->rates[k]) && p->rates[k] >= 0)) throw ArgErr("category rates must be finite and >= 0");
-        const uint32_t n = p->n_nodes;
-        if (n < 2 || n > kMutMaxNodes || !p->parent || !p->branch_len)
-            throw ArgErr("the tree needs 2 to " + std::to_string(kMutMaxNodes) + " nodes (parent / branch_len not NULL)");
-        if (p->parent[0] != -1) throw ArgErr("parent[0] must be -1 (the root comes first)");
-        std::vector<char> has_kid(n, 0);
-        for (uint32_t i = 1; i < n; i++) {
-            if (p->parent[i] < 0 || (uint32_t)p->parent[i] >= i) throw ArgErr("the tree must be in preorder: 0 <= parent[i] < i");
-            if (!(std::isfinite(p->branch_len[i]) && p->branch_len[i] >= 0)) throw ArgErr("branch lengths must be finite and >= 0");
-            has_kid[p->parent[i]] = 1;
-        }
-        if (p->n_tips < 1 || p->n_tips > kMutMaxTips)
-            throw ArgErr("a tree of " + std::to_string(p->n_tips) + " tips: 1 to " + std::to_string(kMutMaxTips) + " tips are supported");
-        if (!p->tip_node || !p->tip_names) throw ArgErr("tip_node / tip_names is NULL");
-        std::vector<int32_t> tip_of(n, -1);
-        for (uint32_t t = 0; t < p->n_tips; t++) {
-            const uint32_t v = p->tip_node[t];
-            if (v >= n || has_kid[v] || tip_of[v] >= 0) throw ArgErr("tip_node must list distinct childless nodes");
-            if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
-            tip_of[v] = (int32_t)t;
-        }
-        const uint64_t nc = c->chrom_off.size() - 1;
-        std::vector<uint32_t> tile0(nc + 1, 0);
-        for (uint64_t ci = 0; ci < nc; ci++) {
-            const uint64_t len = c->chrom_off[ci + 1] - c->chrom_off[ci];
-            if (len >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
-            const uint64_t t = tile0[ci] + (len + kMutTile - 1) / kMutTile;
-            if (t >> 32) throw ArgErr("genome too large");
-            tile0[ci + 1] = (uint32_t)t;
-        }
-        const uint32_t K = p->n_rates, n_tips = p->n_tips, n_tiles = tile0[nc];
+// The whole call; im == nullptr: substitutions only, otherwise the indel model (ins_pi: the inserted columns' birth
+// distribution) and its stats.
+static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelModel* im, const double* ins_pi,
+                        jlp_mutation_stats* stats, jlp_indel_stats* istats) {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (c->chrom_off.size() < 2) throw ArgErr("set the reference genome first");
+    for (int i = 0; i < 16; i++)
+        if (i % 5 && !(std::isfinite(p->Q[i]) && p->Q[i] >= 0)) throw ArgErr("the off-diagonal rates of Q must be finite and >= 0");
+    if (!(p->invariant >= 0 && p->invariant < 1)) throw ArgErr("invariant must be >= 0 and < 1");
+    if (p->n_rates < 1 || p->n_rates > 255 || !p->rates) throw ArgErr("n_rates must be 1..255 (rates not NULL)");
+    for (uint32_t k = 0; k < p->n_rates; k++)
+        if (!(std::isfinite(p->rates[k]) && p->rates[k] >= 0)) throw ArgErr("category rates must be finite and >= 0");
+    const uint32_t n = p->n_nodes;
+    if (n < 2 || n > kMutMaxNodes || !p->parent || !p->branch_len)
+        throw ArgErr("the tree needs 2 to " + std::to_string(kMutMaxNodes) + " nodes (parent / branch_len not NULL)");
+    if (p->parent[0] != -1) throw ArgErr("parent[0] must be -1 (the root comes first)");
+    std::vector<char> has_kid(n, 0);
+    for (uint32_t i = 1; i < n; i++) {
+        if (p->parent[i] < 0 || (uint32_t)p->parent[i] >= i) throw ArgErr("the tree must be in preorder: 0 <= parent[i] < i");
+        if (!(std::isfinite(p->branch_len[i]) && p->branch_len[i] >= 0)) throw ArgErr("branch lengths must be finite and >= 0");
+        has_kid[p->parent[i]] = 1;
+    }
+    if (p->n_tips < 1 || p->n_tips > kMutMaxTips)
+        throw ArgErr("a tree of " + std::to_string(p->n_tips) + " tips: 1 to " + std::to_string(kMutMaxTips) + " tips are supported");
+    if (!p->tip_node || !p->tip_names) throw ArgErr("tip_node / tip_names is NULL");
+    std::vector<int32_t> tip_of(n, -1);
+    for (uint32_t t = 0; t < p->n_tips; t++) {
+        const uint32_t v = p->tip_node[t];
+        if (v >= n || has_kid[v] || tip_of[v] >= 0) throw ArgErr("tip_node must list distinct childless nodes");
+        if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
+        tip_of[v] = (int32_t)t;
+    }
+    const uint64_t nc = c->chrom_off.size() - 1;
+    std::vector<uint32_t> tile0(nc + 1, 0);
+    for (uint64_t ci = 0; ci < nc; ci++) {
+        const uint64_t len = c->chrom_off[ci + 1] - c->chrom_off[ci];
+        if (len >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
+        const uint64_t t = tile0[ci] + (len + kMutTile - 1) / kMutTile;
+        if (t >> 32) throw ArgErr("genome too large");
+        tile0[ci + 1] = (uint32_t)t;
+    }
+    const uint32_t K = p->n_rates, n_tips = p->n_tips, n_tiles = tile0[nc];
+    const size_t n_items = (size_t)n_tips * nc;
 
-        // host tables: the schedule, per (node, category, parent state) the row thresholds, the category thresholds
-        uint32_t max_slots = 0;
-        const std::vector<MutNode> sched = mut_schedule(p, tip_of, K, max_slots);
-        const uint64_t rows = (uint64_t)n * K * 4;
-        std::vector<uint4> thr_hi(rows, make_uint4(0, 0, 0, 0)), thr_lo(rows, make_uint4(0, 0, 0, 0));
-        for (const MutNode& m : sched)
-            for (uint32_t k = 0; k < K; k++) {
-                double P[16];
-                transition_matrix(p->Q, p->rates[k] * p->branch_len[m.node], P);
-                for (uint32_t a = 0; a < 4; a++) {
-                    uint64_t t[3];
-                    row_thresholds(P + 4 * a, t);
-                    const uint64_t r = m.tab + 4ull * k + a;
-                    thr_hi[r] = make_uint4((uint32_t)(t[0] >> 32), (uint32_t)(t[1] >> 32), (uint32_t)(t[2] >> 32), 0);
-                    thr_lo[r] = make_uint4((uint32_t)t[0], (uint32_t)t[1], (uint32_t)t[2], 0);
-                }
-            }
-        std::vector<uint64_t> cat_thr(K);
-        cat_thr[0] = prob_threshold(p->invariant);
-        for (uint32_t j = 1; j < K; j++) cat_thr[j] = prob_threshold(p->invariant + j * (1 - p->invariant) / K);
-
-        Device& d = device0(c);
-        finish_upload(c, d);
-        cudaStream_t s = d.s_compute;
-        DevBuf<uint64_t> d_off, d_cat, d_region, d_region_n, d_out;
-        DevBuf<uint32_t> d_tile0, d_cnt;
-        DevBuf<MutNode> d_sched;
-        DevBuf<uint4> d_hi, d_lo;
-        d_off.upload(c->chrom_off, s);
-        d_tile0.upload(tile0, s);
-        d_sched.upload(sched, s);
-        d_cat.upload(cat_thr, s);
-        d_hi.upload(thr_hi, s);
-        d_lo.upload(thr_lo, s);
-        const size_t n_cnt = (size_t)n_tips * n_tiles;
-        d_cnt.ensure(n_cnt);
-        if (n_cnt) CK(cudaMemsetAsync(d_cnt.p, 0, n_cnt * 4, s));
-        d_region_n.ensure((size_t)n_tips * nc);
-        MutParams mp{};
-        mp.seed = p->seed;
-        mp.genome = d.genome.p + kPad;
-        mp.chrom_off = d_off.p;
-        mp.tile0 = d_tile0.p;
-        mp.n_chroms = (uint32_t)nc; mp.n_tiles = n_tiles; mp.n_tips = n_tips; mp.n_sched = (uint32_t)sched.size();
-        mp.sched = d_sched.p;
-        mp.n_cat = K;
-        mp.cat_thr = d_cat.p;
-        mp.thr_hi = d_hi.p; mp.thr_lo = d_lo.p;
-        mp.tab_rows = (uint32_t)rows;
-        mp.tab_smem = mut_smem_bytes((uint32_t)rows) <= (64u << 10);
-        mp.cnt = d_cnt.p;
-        EventSet ev;
-        CK(cudaEventRecord(ev.e[0], s));
-        CK(launch_mutate(mp, false, s));
-        CK(cudaEventRecord(ev.e[1], s));
-        CK(launch_mut_scan(mp, d_region_n.p, s));
-        CK(cudaEventRecord(ev.e[2], s));
-        std::vector<uint64_t> region_n((size_t)n_tips * nc), region((size_t)n_tips * nc);
-        CK(cudaMemcpyAsync(region_n.data(), d_region_n.p, region_n.size() * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        uint64_t words = 0, records = 0;
-        for (size_t r = 0; r < region.size(); r++) {
-            region[r] = words;
-            words += 4 * region_n[r] + (region_n[r] + 7) / 8;
-            records += region_n[r];
-        }
-        d_region.upload(region, s);
-        mp.region = d_region.p;
-        mp.region_n = d_region_n.p;              // k_mut_scan left the totals there
-        d_out.ensure(words);
-        if (words) CK(cudaMemsetAsync(d_out.p, 0, words * 8, s));
-        mp.out = d_out.p;
-        CK(cudaEventRecord(ev.e[3], s));
-        if (records) CK(launch_mutate(mp, true, s));
-        CK(cudaEventRecord(ev.e[4], s));
-        CK(cudaStreamSynchronize(s));
-        const float count_ms = ev.ms(0, 1), scan_ms = ev.ms(1, 2), write_ms = ev.ms(3, 4);
-        const auto t_gen = std::chrono::steady_clock::now();
-
-        // the records into one HapStore per tip, copied straight into the packed arrays by a few host threads
-        std::vector<std::shared_ptr<HapStore>> stores(n_tips);
-        for (uint32_t t = 0; t < n_tips; t++) {
-            stores[t] = std::make_shared<HapStore>();
-            stores[t]->name = p->tip_names[t];
-            stores[t]->chrom.resize(nc);
-        }
-        const size_t n_items = (size_t)n_tips * nc;
-        std::atomic<size_t> next{0};
+    // indels: the event pass, chromosomes on up to 16 host threads; then the tips' records in one array (region
+    // tip * nc + chromosome), each tile's first record, and the inserted columns with their places in the pools
+    std::vector<IndelChrom> ich(im ? nc : 0);
+    std::vector<IndelRec> irec;
+    std::vector<uint64_t> ir_start;
+    std::vector<uint32_t> icur;
+    double event_ms = 0;
+    if (im) {
+        const auto te = std::chrono::steady_clock::now();
+        std::atomic<uint64_t> next{0};
         std::mutex err_mu;
         std::string err;
-        const int dev = d.id;
         auto work = [&]() {
             try {
-                CK(cudaSetDevice(dev));
-                for (size_t r; (r = next.fetch_add(1)) < n_items;) {
-                    HapChromHost& H = stores[r / nc]->chrom[r % nc];
-                    const uint64_t M = region_n[r];
-                    H.size = c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
-                    H.n_muts = M;
-                    H.pool_bytes = M;
-                    if (!M) continue;
-                    H.packed.resize(4 * M + (M + 7) / 8);
-                    CK(cudaMemcpy(H.packed.data(), d_out.p + region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
-                }
+                for (uint64_t ci; (ci = next.fetch_add(1)) < nc;)
+                    indel_events(p->seed, (uint32_t)ci, c->chrom_off[ci + 1] - c->chrom_off[ci], n, p->parent,
+                                 p->branch_len, tip_of.data(), n_tips, *im, ich[ci]);
             } catch (const std::exception& e) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = e.what(); }
         };
-        const unsigned nt = records < (1u << 16) ? 1u
-                            : (unsigned)std::min<uint64_t>(std::min<uint64_t>(n_items, 16), std::max(1u, std::thread::hardware_concurrency()));
+        const unsigned nt = (unsigned)std::min<uint64_t>(std::min<uint64_t>(nc, 16), std::max(1u, std::thread::hardware_concurrency()));
         std::vector<std::thread> th;
         for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
         work();
         for (std::thread& t : th) t.join();
-        if (!err.empty()) throw CudaErr(err);
-        CK(cudaSetDevice(dev));
-
-        clear_haps(c);
-        for (const auto& S : stores) attach_hap(c, S);
-        if (stats) {
-            const auto t1 = std::chrono::steady_clock::now();
-            stats->count_ms = count_ms;
-            stats->scan_ms = scan_ms;
-            stats->write_ms = write_ms;
-            stats->store_ms = std::chrono::duration<double, std::milli>(t1 - t_gen).count();
-            stats->total_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
-            stats->records = records;
-            stats->d2h_bytes = words * 8;
-            stats->table_bytes = rows * 2 * sizeof(uint4);
-            stats->table_in_smem = (int)mp.tab_smem;
-            stats->max_slots = max_slots;
+        if (!err.empty()) throw ArgErr(err);
+        ir_start.resize(n_items + 1);
+        for (size_t r = 0; r < n_items; r++) {
+            ir_start[r] = irec.size();
+            const std::vector<IndelRec>& v = ich[r % nc].tip[r / nc].recs;
+            irec.insert(irec.end(), v.begin(), v.end());
         }
+        ir_start[n_items] = irec.size();
+        if (irec.size() >> 32) throw ArgErr("2^32 or more insertion and deletion records are not supported");
+        icur.resize((size_t)n_tips * n_tiles);
+        for (size_t r = 0; r < n_items; r++) {
+            const uint64_t ci = r % nc;
+            uint64_t j = ir_start[r];
+            for (uint32_t tl = tile0[ci]; tl < tile0[ci + 1]; tl++) {
+                const uint64_t start = (uint64_t)(tl - tile0[ci]) * kMutTile;
+                while (j < ir_start[r + 1] && irec[j].old_pos < start) j++;
+                icur[(r / nc) * n_tiles + tl] = (uint32_t)j;
+            }
+        }
+        event_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - te).count();
+    }
+
+    // host tables: the schedule, per (node, category, parent state) the row thresholds, the category thresholds
+    uint32_t max_slots = 0;
+    const std::vector<MutNode> sched = mut_schedule(p, tip_of, K, max_slots);
+    // the inserted columns: birth node -> its schedule index and the end of its subtree's interval; per column the
+    // (tip, record, byte) it fills, tips in schedule order
+    std::vector<InsCol> cols;
+    std::vector<InsEnt> ents;
+    if (im) {
+        std::vector<int64_t> spos(n, -1);
+        std::vector<uint32_t> scount(n, 0);
+        for (size_t i = 0; i < sched.size(); i++) spos[sched[i].node] = (int64_t)i;
+        for (uint32_t i = n; i-- > 1;) {
+            scount[i] += spos[i] >= 0;
+            scount[p->parent[i]] += scount[i];
+        }
+        std::vector<uint64_t> col_base(nc + 1, 0);
+        for (uint64_t ci = 0; ci < nc; ci++) col_base[ci + 1] = col_base[ci] + ich[ci].birth.size();
+        if (col_base[nc] >> 32) throw ArgErr("2^32 or more inserted columns are not supported");
+        cols.resize(col_base[nc]);
+        std::vector<uint64_t> ecount(cols.size() + 1, 0);
+        for (int pass = 0; pass < 2; pass++) {
+            for (size_t si = 0; si < sched.size(); si++) {
+                if (sched[si].tip < 0) continue;
+                const uint32_t t = (uint32_t)sched[si].tip;
+                for (uint64_t ci = 0; ci < nc; ci++) {
+                    const IndelTip& T = ich[ci].tip[t];
+                    const size_t r = (size_t)t * nc + ci;
+                    for (size_t j = 0; j < T.recs.size(); j++)
+                        for (uint64_t q = T.ids_off[j]; q < T.ids_off[j + 1]; q++) {
+                            const uint64_t g = col_base[ci] + T.ids[q];
+                            if (pass == 0) { ecount[g + 1]++; continue; }
+                            const uint32_t k = (uint32_t)(q - T.ids_off[j]) + (T.recs[j].kind == kAnchorRec);
+                            ents[cols[g].e1++] = InsEnt{(uint32_t)si, k, r, ir_start[r] + j};
+                        }
+                }
+            }
+            if (pass == 0) {
+                for (size_t g = 0; g < cols.size(); g++) ecount[g + 1] += ecount[g];
+                ents.resize(ecount.back());
+                for (uint64_t ci = 0; ci < nc; ci++)
+                    for (uint32_t id = 0; id < ich[ci].birth.size(); id++) {
+                        const uint64_t g = col_base[ci] + id;
+                        const uint32_t u = ich[ci].birth[id];
+                        InsCol& col = cols[g];
+                        col.chrom = (uint32_t)ci; col.id = id;
+                        col.n0 = spos[u] >= 0 ? (uint32_t)spos[u] : 0;
+                        col.n1 = spos[u] >= 0 ? (uint32_t)spos[u] + scount[u] : 0;
+                        col.e0 = col.e1 = ecount[g];
+                    }
+            }
+        }
+    }
+    const uint64_t rows = (uint64_t)n * K * 4;
+    std::vector<uint4> thr_hi(rows, make_uint4(0, 0, 0, 0)), thr_lo(rows, make_uint4(0, 0, 0, 0));
+    for (const MutNode& m : sched)
+        for (uint32_t k = 0; k < K; k++) {
+            double P[16];
+            transition_matrix(p->Q, p->rates[k] * p->branch_len[m.node], P);
+            for (uint32_t a = 0; a < 4; a++) {
+                uint64_t t[3];
+                row_thresholds(P + 4 * a, t);
+                const uint64_t r = m.tab + 4ull * k + a;
+                thr_hi[r] = make_uint4((uint32_t)(t[0] >> 32), (uint32_t)(t[1] >> 32), (uint32_t)(t[2] >> 32), 0);
+                thr_lo[r] = make_uint4((uint32_t)t[0], (uint32_t)t[1], (uint32_t)t[2], 0);
+            }
+        }
+    std::vector<uint64_t> cat_thr(K);
+    cat_thr[0] = prob_threshold(p->invariant);
+    for (uint32_t j = 1; j < K; j++) cat_thr[j] = prob_threshold(p->invariant + j * (1 - p->invariant) / K);
+
+    Device& d = device0(c);
+    finish_upload(c, d);
+    cudaStream_t s = d.s_compute;
+    DevBuf<uint64_t> d_off, d_cat, d_region, d_region_n, d_out, d_ir_start, d_ir_nuc;
+    DevBuf<uint32_t> d_tile0, d_cnt, d_icur;
+    DevBuf<IndelRec> d_irec;
+    DevBuf<InsCol> d_cols;
+    DevBuf<InsEnt> d_ents;
+    DevBuf<MutNode> d_sched;
+    DevBuf<uint4> d_hi, d_lo;
+    d_off.upload(c->chrom_off, s);
+    d_tile0.upload(tile0, s);
+    d_sched.upload(sched, s);
+    d_cat.upload(cat_thr, s);
+    d_hi.upload(thr_hi, s);
+    d_lo.upload(thr_lo, s);
+    const size_t n_cnt = (size_t)n_tips * n_tiles;
+    d_cnt.ensure(n_cnt);
+    if (n_cnt) CK(cudaMemsetAsync(d_cnt.p, 0, n_cnt * 4, s));
+    d_region_n.ensure((size_t)n_tips * nc);
+    MutParams mp{};
+    mp.seed = p->seed;
+    mp.genome = d.genome.p + kPad;
+    mp.chrom_off = d_off.p;
+    mp.tile0 = d_tile0.p;
+    mp.n_chroms = (uint32_t)nc; mp.n_tiles = n_tiles; mp.n_tips = n_tips; mp.n_sched = (uint32_t)sched.size();
+    mp.sched = d_sched.p;
+    mp.n_cat = K;
+    mp.cat_thr = d_cat.p;
+    mp.thr_hi = d_hi.p; mp.thr_lo = d_lo.p;
+    mp.tab_rows = (uint32_t)rows;
+    mp.tab_smem = mut_smem_bytes((uint32_t)rows) <= (64u << 10);
+    mp.cnt = d_cnt.p;
+    if (im) {
+        d_irec.upload(irec, s);
+        d_ir_start.upload(ir_start, s);
+        d_icur.upload(icur, s);
+        d_ir_nuc.ensure(irec.size());
+        mp.irec = d_irec.p; mp.ir_start = d_ir_start.p; mp.icur = d_icur.p; mp.ir_nuc = d_ir_nuc.p;
+    }
+    EventSet ev;
+    CK(cudaEventRecord(ev.e[0], s));
+    CK(launch_mutate(mp, false, im != nullptr, s));
+    CK(cudaEventRecord(ev.e[1], s));
+    CK(launch_mut_scan(mp, d_region_n.p, s));
+    CK(cudaEventRecord(ev.e[2], s));
+    std::vector<uint64_t> region_n((size_t)n_tips * nc), region((size_t)n_tips * nc);
+    CK(cudaMemcpyAsync(region_n.data(), d_region_n.p, region_n.size() * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    // with indels region_n becomes substitution + indel records, pool the substitutions' bytes + the indel records'
+    std::vector<uint64_t> pool(region_n);
+    if (im)
+        for (size_t r = 0; r < region.size(); r++) {
+            const uint64_t a = ir_start[r], b = ir_start[r + 1];
+            region_n[r] += b - a;
+            if (b > a) pool[r] += irec[b - 1].pool_before + indel_pool_len(irec[b - 1]);
+        }
+    uint64_t words = 0, records = 0;
+    for (size_t r = 0; r < region.size(); r++) {
+        region[r] = words;
+        words += 4 * region_n[r] + (pool[r] + 7) / 8;
+        records += region_n[r];
+    }
+    d_region.upload(region, s);
+    if (im) {
+        d_region_n.upload(region_n, s);
+        d_icur.upload(icur, s);
+    }
+    mp.region = d_region.p;
+    mp.region_n = d_region_n.p;              // k_mut_scan left the totals there
+    d_out.ensure(words);
+    if (words) CK(cudaMemsetAsync(d_out.p, 0, words * 8, s));
+    mp.out = d_out.p;
+    CK(cudaEventRecord(ev.e[3], s));
+    if (records) CK(launch_mutate(mp, true, im != nullptr, s));
+    if (im && !cols.empty()) {
+        d_cols.upload(cols, s);
+        d_ents.upload(ents, s);
+        InsParams ip{};
+        ip.seed = p->seed;
+        if (cols.size() >> 32) throw ArgErr("2^32 or more inserted columns are not supported");
+        ip.n_cols = (uint32_t)cols.size();
+        ip.n_cat = K;
+        ip.cols = d_cols.p; ip.ent = d_ents.p; ip.sched = d_sched.p; ip.cat_thr = d_cat.p;
+        row_thresholds(ins_pi, ip.pi_thr);
+        ip.thr_hi = d_hi.p; ip.thr_lo = d_lo.p;
+        ip.out = d_out.p; ip.region = d_region.p; ip.region_n = d_region_n.p; ip.ir_nuc = d_ir_nuc.p;
+        CK(launch_ins_walk(ip, s));
+    }
+    CK(cudaEventRecord(ev.e[4], s));
+    CK(cudaStreamSynchronize(s));
+    const float count_ms = ev.ms(0, 1), scan_ms = ev.ms(1, 2), write_ms = ev.ms(3, 4);
+    const auto t_gen = std::chrono::steady_clock::now();
+
+    // the records into one HapStore per tip, copied straight into the packed arrays by a few host threads
+    std::vector<std::shared_ptr<HapStore>> stores(n_tips);
+    for (uint32_t t = 0; t < n_tips; t++) {
+        stores[t] = std::make_shared<HapStore>();
+        stores[t]->name = p->tip_names[t];
+        stores[t]->chrom.resize(nc);
+    }
+    std::atomic<size_t> next{0};
+    std::mutex err_mu;
+    std::string err;
+    const int dev = d.id;
+    auto work = [&]() {
+        try {
+            CK(cudaSetDevice(dev));
+            for (size_t r; (r = next.fetch_add(1)) < n_items;) {
+                HapChromHost& H = stores[r / nc]->chrom[r % nc];
+                const uint64_t M = region_n[r];
+                H.size = im ? ich[r % nc].tip[r / nc].size : c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
+                H.n_muts = M;
+                H.pool_bytes = pool[r];
+                if (!M) continue;
+                H.packed.resize(4 * M + (pool[r] + 7) / 8);
+                CK(cudaMemcpy(H.packed.data(), d_out.p + region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
+            }
+        } catch (const std::exception& e) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = e.what(); }
+    };
+    const unsigned nt = records < (1u << 16) ? 1u
+                        : (unsigned)std::min<uint64_t>(std::min<uint64_t>(n_items, 16), std::max(1u, std::thread::hardware_concurrency()));
+    std::vector<std::thread> th;
+    for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
+    work();
+    for (std::thread& t : th) t.join();
+    if (!err.empty()) throw CudaErr(err);
+    CK(cudaSetDevice(dev));
+
+    clear_haps(c);
+    for (const auto& S : stores) attach_hap(c, S);
+    if (stats) {
+        const auto t1 = std::chrono::steady_clock::now();
+        stats->count_ms = count_ms;
+        stats->scan_ms = scan_ms;
+        stats->write_ms = write_ms;
+        stats->store_ms = std::chrono::duration<double, std::milli>(t1 - t_gen).count();
+        stats->total_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
+        stats->records = records;
+        stats->d2h_bytes = words * 8;
+        stats->table_bytes = rows * 2 * sizeof(uint4);
+        stats->table_in_smem = (int)mp.tab_smem;
+        stats->max_slots = max_slots;
+    }
+    if (istats) {
+        *istats = jlp_indel_stats{};
+        for (const IndelChrom& x : ich) {
+            istats->insertions += x.insertions;
+            istats->deletions += x.deletions;
+            istats->inserted_bases += x.inserted_bases;
+            istats->steps += x.steps;
+        }
+        istats->indel_records = irec.size();
+        istats->event_ms = event_ms;
+    }
+}
+
+int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation_stats* stats) {
+    if (!c || !p) return JLP_ERR_ARG;
+    return guarded(c, [&]() { create_haps(c, p, nullptr, nullptr, stats, nullptr); });
+}
+
+int jlp_create_haplotypes_indels(jlp_ctx* c, const jlp_mutation_params* p, const jlp_indel_params* ip,
+                                 jlp_mutation_stats* stats, jlp_indel_stats* istats) {
+    if (!c || !p || !ip) return JLP_ERR_ARG;
+    return guarded(c, [&]() {
+        auto rate_ok = [](double x) { return std::isfinite(x) && x >= 0; };
+        if (!rate_ok(ip->rate_ins) || !rate_ok(ip->rate_del)) throw ArgErr("indel rates must be finite and >= 0");
+        const double R = ip->rate_ins + ip->rate_del;
+        if (R == 0) {
+            create_haps(c, p, nullptr, nullptr, stats, nullptr);
+            if (istats) *istats = jlp_indel_stats{};
+            return;
+        }
+        if (!(std::isfinite(ip->epsilon) && ip->epsilon > 0))
+            throw ArgErr("epsilon must be > 0 when an indel rate is > 0");
+        auto weights_ok = [&](double rate, uint32_t nw, const double* w) {
+            if (rate == 0) return;
+            if (nw < 1 || !w) throw ArgErr("an indel kind with a rate > 0 needs length weights (n >= 1, not NULL)");
+            double sum = 0;
+            for (uint32_t u = 0; u < nw; u++) {
+                if (!rate_ok(w[u])) throw ArgErr("indel length weights must be finite and >= 0");
+                sum += w[u];
+            }
+            if (!(sum > 0)) throw ArgErr("indel length weights need one weight > 0");
+        };
+        weights_ok(ip->rate_ins, ip->n_ins, ip->w_ins);
+        weights_ok(ip->rate_del, ip->n_del, ip->w_del);
+        double pis = 0;
+        for (double x : ip->pi) {
+            if (!rate_ok(x)) throw ArgErr("pi must be finite and >= 0");
+            pis += x;
+        }
+        if (!(pis > 0)) throw ArgErr("pi needs one value > 0");
+        // a kind of rate 0 has no lengths
+        const uint32_t n_ins = ip->rate_ins > 0 ? ip->n_ins : 0, n_del = ip->rate_del > 0 ? ip->n_del : 0;
+        IndelModel im;
+        im.rate_ins = ip->rate_ins; im.rate_del = ip->rate_del; im.epsilon = ip->epsilon;
+        im.n_ins = n_ins;
+        im.kl_thr = indel_thresholds(ip->rate_ins, ip->w_ins, n_ins, ip->rate_del, ip->w_del, n_del);
+        create_haps(c, p, &im, ip->pi, stats, istats);
     });
 }
 

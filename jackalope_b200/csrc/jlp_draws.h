@@ -39,7 +39,8 @@
 namespace jlp {
 
 // plane 6 is the oracle's PacBio plane
-enum Plane : uint32_t { PL_PAIR = 0, PL_INDEL = 1, PL_QUAL = 2, PL_SLOW = 3, PL_GENOME = 4, PL_GSLOW = 5, PL_MUT = 7, PL_MSLOW = 8 };
+enum Plane : uint32_t { PL_PAIR = 0, PL_INDEL = 1, PL_QUAL = 2, PL_SLOW = 3, PL_GENOME = 4, PL_GSLOW = 5, PL_MUT = 7, PL_MSLOW = 8,
+                        PL_IEV = 9, PL_ICOL = 10, PL_IMUT = 11, PL_IMSLOW = 12 };
 enum Purpose : uint32_t { PU_INDEL = 0, PU_DIE = 1, PU_COIN = 2, PU_MIS = 3, PU_SUB = 4, PU_INS = 5 };
 
 struct U4 { uint32_t w0, w1, w2, w3; };
@@ -175,6 +176,27 @@ JLP_HD uint32_t mut_low(uint64_t seed, uint32_t chrom, uint64_t b, uint32_t node
 JLP_HD uint64_t mut_draw(uint64_t seed, uint32_t chrom, uint64_t b, uint32_t node) {
     const uint32_t h = genome_word(mut_block(seed, chrom, b >> 2, node), (uint32_t)b & 3u);
     return ((uint64_t)h << 32) | mut_low(seed, chrom, b, node);
+}
+
+// ---- draws of insertions and deletions along the tree (create_haplotypes with indels) ----
+//   plane IEV  : counter (k, step, c, PL_IEV | v<<8): event k of step `step` on the branch above node v;
+//                w1:w0 = the gap draw (the k-th event is 1 + floor(log(U) / log1p(-p)) positions after the one before,
+//                U = ((X >> 11) + 1) 2^-53), w3:w2 = the (kind, length) draw
+//   plane ICOL : counter (id, 0, c, PL_ICOL): inserted column `id` of chromosome c; w1:w0 = its rate-category draw,
+//                w3:w2 = its state at the end of the branch where it was born (against the thresholds of pi)
+//   plane IMUT / IMSLOW: the transition draws of inserted column `id` at node v, laid out as MUT / MSLOW with id in
+//                place of the site
+JLP_HD U4 indel_event_block(uint64_t seed, uint32_t chrom, uint32_t node, uint32_t step, uint32_t k) {
+    return philox4x32_10(k, step, chrom, PL_IEV | (node << 8), (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+JLP_HD U4 ins_col_block(uint64_t seed, uint32_t chrom, uint32_t id) {
+    return philox4x32_10(id, 0u, chrom, PL_ICOL, (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+JLP_HD U4 imut_block(uint64_t seed, uint32_t chrom, uint64_t id4, uint32_t node) {
+    return philox4x32_10((uint32_t)id4, (uint32_t)(id4 >> 32), chrom, PL_IMUT | (node << 8), (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+JLP_HD uint32_t imut_low(uint64_t seed, uint32_t chrom, uint64_t id, uint32_t node) {
+    return philox4x32_10((uint32_t)id, (uint32_t)(id >> 32), chrom, PL_IMSLOW | (node << 8), (uint32_t)seed, (uint32_t)(seed >> 32)).w0;
 }
 
 // ---- exact restatements of the reference's uses of u = runif_01(x) ----

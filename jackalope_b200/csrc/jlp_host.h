@@ -76,5 +76,49 @@ uint64_t prob_threshold(double c);
 // and renormalised, thr[j] = prob_threshold(p[0] + ... + p[j])
 void row_thresholds(const double* row, uint64_t thr[3]);
 
+// --- insertions and deletions along the tree (create_haplotypes, jlp_indel.cpp) --------
+// One insertion or deletion record of a (tip, chromosome) in HapChromHost::packed terms (DESIGN.md section 10).
+struct IndelRec {
+    uint32_t old_pos, new_pos;
+    uint32_t kind;          // kDelRec, kAnchorRec (pool = the tip base at old_pos, then the inserted bases), kLeadRec
+    uint32_t pad;
+    int64_t size_mod;       // -(deleted columns), or the inserted bases (kLeadRec: minus one)
+    uint64_t pool_before;   // pool bytes of the indel records before this one in its (tip, chromosome)
+};
+constexpr uint32_t kDelRec = 0, kAnchorRec = 1, kLeadRec = 2;
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+inline uint64_t indel_pool_len(const IndelRec& r) { return r.kind == kDelRec ? 0 : (uint64_t)(r.size_mod + 1); }
+
+struct IndelModel {
+    double rate_ins = 0, rate_del = 0, epsilon = 0;
+    uint32_t n_ins = 0;                 // (kind, length) index < n_ins: insertion of index + 1 columns, else deletion
+    std::vector<uint64_t> kl_thr;       // the (kind, length) draw's cumulative thresholds (see indel_thresholds)
+};
+// (kind, length) probabilities (rate_ins / R) (w_ins[u] / sum w_ins) for u = 1..n_ins, then the deletions alike, summed
+// in that order into prob_threshold()s (all but the last)
+std::vector<uint64_t> indel_thresholds(double rate_ins, const double* w_ins, uint32_t n_ins, double rate_del,
+                                       const double* w_del, uint32_t n_del);
+// the steps of a branch: max(1, ceil(R t / epsilon)); throws past 2^31
+uint32_t indel_steps(double R, double t, double epsilon);
+
+struct IndelTip {                       // one (tip, chromosome)
+    std::vector<IndelRec> recs;         // by old_pos
+    std::vector<uint32_t> ids;          // the inserted columns of the insertion records, in pool order
+    std::vector<uint64_t> ids_off;      // [recs.size() + 1]: record j's columns are ids[ids_off[j] .. ids_off[j + 1])
+    uint64_t size = 0;                  // the tip's chromosome length
+};
+struct IndelChrom {
+    std::vector<uint32_t> birth;        // per inserted column (its id): the node at the end of the branch it was born on
+    std::vector<IndelTip> tip;          // per tip
+    uint64_t insertions = 0, deletions = 0, inserted_bases = 0, steps = 0;
+};
+// The event pass of one chromosome of `len` reference columns: nodes in preorder (parent[v] < v), each branch cut into
+// indel_steps() steps, the events of a step drawn from plane IEV and applied at once.  tip_of[v] = tip index or -1.
+// Throws std::runtime_error past the limits (a tip chromosome or the inserted columns at 2^32).
+void indel_events(uint64_t seed, uint32_t chrom, uint64_t len, uint32_t n_nodes, const int32_t* parent,
+                  const double* branch_len, const int32_t* tip_of, uint32_t n_tips, const IndelModel& m, IndelChrom& out);
+
 }  // namespace jlp
 #endif

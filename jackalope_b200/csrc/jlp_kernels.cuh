@@ -106,6 +106,8 @@ constexpr uint32_t kMutSlots = 32;                 // node-state slots per lane
 constexpr uint32_t kMutMaxTips = 4096;
 constexpr uint32_t kMutMaxNodes = 65536;
 
+struct IndelRec;          // jlp_host.h
+
 struct MutNode {          // a non-root node in visiting order
     uint32_t node;        // index in the caller's preorder: addresses the draws
     uint32_t tab;         // its first threshold row: row = tab + 4 * category + parent state
@@ -131,9 +133,45 @@ struct MutParams {
     uint64_t* out;               // pass 2: the packed regions (HapChromHost::packed layout)
     const uint64_t* region;      // [n_tips][n_chroms] word offset of the region in `out`
     const uint64_t* region_n;    // [n_tips][n_chroms] records of the region
+    // with indels only: cnt then counts the substitution records alone
+    const IndelRec* irec;        // the indel records of every (tip, chromosome), by old_pos
+    const uint64_t* ir_start;    // [n_tips * n_chroms + 1] first record of each (tip, chromosome)
+    uint32_t* icur;              // [n_tips][n_tiles] the first record not yet passed by the tile's warp
+    uint64_t* ir_nuc;            // pass 2: each indel record's nuc_off (where k_ins_walk puts its inserted bases)
 };
-// pass 1 (write = false): records per (tip, tile) added into cnt; pass 2 (write = true): records written
-cudaError_t launch_mutate(const MutParams& p, bool write, cudaStream_t s);
+// pass 1 (write = false): records per (tip, tile) added into cnt; pass 2 (write = true): records written.
+// indels: the tips' records follow p.irec (substitutions at live, non-anchor columns; the indel records themselves)
+cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, cudaStream_t s);
+
+// The inserted columns' walk: one thread per column from its birth node through the schedule interval of its subtree
+// (state at birth drawn from pi, then the same P rows as a reference site); its tip states go into the insertion
+// records' pools.
+struct InsCol {
+    uint32_t chrom, id;
+    uint32_t n0, n1;             // schedule index of the birth node, end of its subtree's interval (n0 == n1: no tip below)
+    uint64_t e0, e1;             // its entries
+};
+struct InsEnt {                  // the column is live at the tip of schedule entry `sched`, byte k of indel record ir
+    uint32_t sched, k;
+    uint64_t region;             // tip * n_chroms + chromosome
+    uint64_t ir;
+};
+struct InsParams {
+    uint64_t seed;
+    uint32_t n_cols, n_cat;
+    const InsCol* cols;
+    const InsEnt* ent;
+    const MutNode* sched;
+    const uint64_t* cat_thr;
+    uint64_t pi_thr[3];
+    const uint4* thr_hi;
+    const uint4* thr_lo;
+    uint64_t* out;
+    const uint64_t* region;
+    const uint64_t* region_n;
+    const uint64_t* ir_nuc;
+};
+cudaError_t launch_ins_walk(const InsParams& p, cudaStream_t s);
 // exclusive scan of every (tip, chromosome) run of cnt in place; region_n receives the totals
 cudaError_t launch_mut_scan(const MutParams& p, uint64_t* region_n, cudaStream_t s);
 size_t mut_smem_bytes(uint32_t tab_rows);

@@ -15,6 +15,7 @@
 #include <stdint.h>
 
 #include "jlp_draws.h"
+#include "jlp_host.h"
 #include "jlp_kernels.cuh"
 
 namespace jlp {
@@ -38,7 +39,103 @@ __device__ __forceinline__ uint32_t decide(uint32_t H, const uint4& th, const ui
     return b;
 }
 
+__device__ __forceinline__ uint8_t base_char(uint32_t states, uint32_t k) {
+    return (uint8_t)(__byte_perm(0x47414354u, 0u, (states >> (2 * k)) & 3u) & 0xffu);
+}
+
+// At tip `tip`, the indel instantiation: the step's sites against the tip's indel records.  A site is dead (covered by a
+// deletion, or column 0 under a leading insertion) or an anchor (its base is pool[0] of an insertion record): neither
+// gives a substitution record.  A substitution record at site b goes to index (substitutions before b) + (indel records
+// before b), new_pos = b + the shift after those records; an indel record of the step goes to index j + (substitutions
+// before its old_pos), written by the lane that owns that site.
 template <bool WRITE>
+__device__ __forceinline__ void indel_tip(const MutParams& p, uint32_t tip, uint32_t c, uint32_t tile, uint64_t step0,
+                                          uint64_t s0, const uint8_t* seq, uint32_t ev, uint32_t ref, uint32_t ns,
+                                          uint32_t lane) {
+    const size_t r = (size_t)tip * p.n_chroms + c;
+    const uint64_t rs = p.ir_start[r], re = p.ir_start[r + 1];
+    uint32_t* cur = p.icur + (size_t)tip * p.n_tiles + tile;
+    uint32_t* cp = p.cnt + (size_t)tip * p.n_tiles + tile;
+    const uint32_t j0 = *cur;
+    uint32_t j1 = j0;
+    while (j1 < re && p.irec[j1].old_pos < step0 + 128) j1++;
+    int64_t sh = 0;                                      // new_pos - old_pos after the records passed
+    uint64_t ix = 0, pb = 0, dend = 0;                   // records passed, their pool bytes, end of the dead run
+    auto pass = [&](uint32_t j) {
+        const IndelRec q = p.irec[j];
+        sh = (int64_t)q.new_pos - (int64_t)q.old_pos + q.size_mod;
+        ix = j - rs + 1;
+        pb = q.pool_before + indel_pool_len(q);
+        dend = q.kind == kDelRec ? q.old_pos - q.size_mod : q.kind == kLeadRec ? 1 : 0;
+    };
+    if (j0 > rs) pass(j0 - 1);
+    uint32_t skip = 0, jj = j0;
+    int64_t shk[4];
+    uint64_t ixk[4], pbk[4];
+#pragma unroll
+    for (uint32_t k = 0; k < 4; k++) {
+        const uint64_t b = s0 + k;
+        while (jj < j1 && p.irec[jj].old_pos <= b) {
+            if (p.irec[jj].old_pos == b && p.irec[jj].kind == kAnchorRec) skip |= 1u << k;
+            pass(jj++);
+        }
+        if (b < dend) skip |= 1u << k;
+        shk[k] = sh; ixk[k] = ix; pbk[k] = pb;
+    }
+    uint32_t dm = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < 4; k++)
+        if (((ev >> k) & 1u) && (((ns ^ ref) >> (2 * k)) & 3u) && !((skip >> k) & 1u)) dm |= 1u << k;
+    if (!WRITE) {
+        const uint32_t tot = __reduce_add_sync(~0u, (uint32_t)__popc(dm));
+        if (lane == 0) { if (tot) *cp += tot; if (j1 != j0) *cur = j1; }
+        return;
+    }
+    if (j1 == j0 && __ballot_sync(~0u, dm) == 0) return;
+    const uint32_t mine = (uint32_t)__popc(dm);
+    uint32_t incl = mine;
+#pragma unroll
+    for (uint32_t d = 1; d < 32; d <<= 1) {
+        const uint32_t v = __shfl_up_sync(~0u, incl, d);
+        if (lane >= d) incl += v;
+    }
+    uint32_t base = lane == 0 ? *cp : 0u;
+    base = __shfl_sync(~0u, base, 0);
+    const uint32_t tot = __shfl_sync(~0u, incl, 31);
+    const uint32_t excl = base + incl - mine;            // substitution records before the lane's first site
+    uint64_t* R = p.out + p.region[r];
+    const uint64_t N = p.region_n[r];
+    uint8_t* pool = reinterpret_cast<uint8_t*>(R + 4 * N);
+    uint64_t before = excl;
+#pragma unroll
+    for (uint32_t k = 0; k < 4; k++) {
+        if (!((dm >> k) & 1u)) continue;
+        const uint64_t b = s0 + k, i = before + ixk[k], off = before + pbk[k];
+        R[i] = b;
+        R[N + i] = (uint64_t)((int64_t)b + shk[k]);
+        R[2 * N + i] = off;                              // size_modifier, R[3N + i], stays 0
+        pool[off] = base_char(ns, k);
+        before++;
+    }
+    for (uint32_t j = j0; j < j1; j++) {
+        const IndelRec q = p.irec[j];
+        const uint32_t l = (uint32_t)((q.old_pos - step0) >> 2), kk = q.old_pos & 3u;
+        const uint32_t sb = __shfl_sync(~0u, excl + (uint32_t)__popc(dm & ((1u << kk) - 1u)), l);
+        if (lane == l) {
+            const uint64_t i = sb + (j - rs), off = sb + q.pool_before;
+            R[i] = q.old_pos;
+            R[N + i] = q.new_pos;
+            R[2 * N + i] = off;
+            R[3 * N + i] = (uint64_t)q.size_mod;
+            p.ir_nuc[j] = off;
+            if (q.kind == kAnchorRec) pool[off] = ((ev >> kk) & 1u) ? base_char(ns, kk) : seq[q.old_pos];
+        }
+    }
+    __syncwarp();
+    if (lane == 0) { *cp = base + tot; *cur = j1; }
+}
+
+template <bool WRITE, bool INDEL>
 __global__ void __launch_bounds__(kMutWarps * 32)
 k_mutate(const __grid_constant__ MutParams p) {
     __shared__ uint8_t st[kMutSlots][kMutWarps * 32];     // node states: 2 bits per site, one byte per (slot, thread)
@@ -95,7 +192,7 @@ k_mutate(const __grid_constant__ MutParams p) {
                 if (idx) { ev |= 1u << k; cats |= (idx - 1) << (8 * k); }
             }
         }
-        if (__ballot_sync(~0u, ev) == 0) continue;
+        if (!INDEL && __ballot_sync(~0u, ev) == 0) continue;      // with indels the tips' records still need the step
         st[0][tid] = (uint8_t)ref;
         for (uint32_t n = 0; n < p.n_sched; n++) {
             const MutNode nd = p.sched[n];
@@ -112,6 +209,10 @@ k_mutate(const __grid_constant__ MutParams p) {
                 }
             }
             if (nd.tip < 0) { st[nd.slot][tid] = (uint8_t)ns; continue; }
+            if (INDEL) {
+                indel_tip<WRITE>(p, (uint32_t)nd.tip, c, tile, first + step * 128u, s0, seq, ev, ref, ns, lane);
+                continue;
+            }
             uint32_t dm = 0;                                 // sites where the tip differs from the reference
 #pragma unroll
             for (uint32_t k = 0; k < 4; k++)
@@ -147,7 +248,7 @@ k_mutate(const __grid_constant__ MutParams p) {
                 R[i] = pos;
                 R[N + i] = pos;
                 R[2 * N + i] = i;                        // size_modifier, R[3N + i], stays 0
-                pool[i] = (uint8_t)(__byte_perm(0x47414354u, 0u, (ns >> (2 * k)) & 3u) & 0xffu);
+                pool[i] = base_char(ns, k);
                 i++;
             }
         }
@@ -190,23 +291,76 @@ __global__ void __launch_bounds__(1024) k_mut_scan(const __grid_constant__ MutPa
     if (threadIdx.x == 0) region_n[r] = carry;
 }
 
+// one thread per inserted column: its category and birth state (plane ICOL), then the nodes of its birth node's subtree
+// in schedule order (planes IMUT / IMSLOW), node states in shared memory as in k_mutate; at a tip the state goes to
+// every entry of that tip (the column's byte in an insertion record's pool)
+__global__ void __launch_bounds__(256) k_ins_walk(const __grid_constant__ InsParams p) {
+    __shared__ uint8_t st[kMutSlots][256];
+    const uint32_t tid = threadIdx.x, g = blockIdx.x * 256u + tid;
+    if (g >= p.n_cols) return;
+    const InsCol col = p.cols[g];
+    if (col.e0 == col.e1) return;
+    const U4 w = ins_col_block(p.seed, col.chrom, col.id);
+    const uint64_t xc = lo64(w), xs = hi64(w);
+    uint32_t idx = 0;
+    for (uint32_t j = 0; j < p.n_cat; j++) idx += (uint32_t)(xc >= p.cat_thr[j]);
+    uint32_t s = (uint32_t)(xs >= p.pi_thr[0]) + (uint32_t)(xs >= p.pi_thr[1]) + (uint32_t)(xs >= p.pi_thr[2]);
+    uint64_t e = col.e0;
+    auto put = [&](uint32_t sched, uint32_t state) {
+        for (; e < col.e1 && p.ent[e].sched == sched; e++) {
+            const InsEnt E = p.ent[e];
+            uint64_t* R = p.out + p.region[E.region];
+            uint8_t* pool = reinterpret_cast<uint8_t*>(R + 4 * p.region_n[E.region]);
+            pool[p.ir_nuc[E.ir] + E.k] = base_char(state, 0);
+        }
+    };
+    put(col.n0, s);
+    if (col.n0 + 1 >= col.n1) return;
+    st[p.sched[col.n0].slot][tid] = (uint8_t)s;
+    for (uint32_t n = col.n0 + 1; n < col.n1 && e < col.e1; n++) {
+        const MutNode nd = p.sched[n];
+        uint32_t ns = st[nd.pslot][tid];
+        if (idx) {
+            const uint32_t row = nd.tab + 4u * (idx - 1) + ns;
+            const uint32_t H = genome_word(imut_block(p.seed, col.chrom, col.id >> 2, nd.node), col.id & 3u);
+            const uint4 th = p.thr_hi[row];
+            if (H == th.x || H == th.y || H == th.z) {
+                const uint4 tl = p.thr_lo[row];
+                const uint32_t L = imut_low(p.seed, col.chrom, col.id, nd.node);
+                ns = (uint32_t)(H > th.x || (H == th.x && L >= tl.x)) + (uint32_t)(H > th.y || (H == th.y && L >= tl.y)) +
+                     (uint32_t)(H > th.z || (H == th.z && L >= tl.z));
+            } else {
+                ns = (uint32_t)(H > th.x) + (uint32_t)(H > th.y) + (uint32_t)(H > th.z);
+            }
+        }
+        if (nd.tip < 0) st[nd.slot][tid] = (uint8_t)ns;
+        else put(n, ns);
+    }
+}
+
 }  // namespace
 
 size_t mut_smem_bytes(uint32_t tab_rows) { return (size_t)tab_rows * sizeof(uint4); }
 
-cudaError_t launch_mutate(const MutParams& p, bool write, cudaStream_t s) {
-    if (p.n_tiles == 0) return cudaSuccess;
+template <bool WRITE, bool INDEL>
+cudaError_t launch_mutate_t(const MutParams& p, cudaStream_t s) {
     const size_t smem = p.tab_smem ? mut_smem_bytes(p.tab_rows) : 0;
     const unsigned grid = (p.n_tiles + kMutWarps - 1) / kMutWarps;
-    if (write) {
-        cudaError_t e = cudaFuncSetAttribute(k_mutate<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        k_mutate<true><<<grid, kMutWarps * 32, smem, s>>>(p);
-    } else {
-        cudaError_t e = cudaFuncSetAttribute(k_mutate<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        k_mutate<false><<<grid, kMutWarps * 32, smem, s>>>(p);
-    }
+    cudaError_t e = cudaFuncSetAttribute(k_mutate<WRITE, INDEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    k_mutate<WRITE, INDEL><<<grid, kMutWarps * 32, smem, s>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, cudaStream_t s) {
+    if (p.n_tiles == 0) return cudaSuccess;
+    if (indels) return write ? launch_mutate_t<true, true>(p, s) : launch_mutate_t<false, true>(p, s);
+    return write ? launch_mutate_t<true, false>(p, s) : launch_mutate_t<false, false>(p, s);
+}
+
+cudaError_t launch_ins_walk(const InsParams& p, cudaStream_t s) {
+    if (p.n_cols == 0) return cudaSuccess;
+    k_ins_walk<<<(p.n_cols + 255) / 256, 256, 0, s>>>(p);
     return cudaGetLastError();
 }
 

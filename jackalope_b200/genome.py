@@ -8,8 +8,8 @@ size, src/hap_classes.h:100-104,287-296,540).  The objects only *hold* data;
 they are flattened into plain arrays before crossing into the library.
 
 ``create_genome`` below makes a reference on the GPU; ``create_haplotypes``
-(mutate.py) evolves haplotypes from it along a tree under a substitution model,
-also on the GPU (substitutions only; indels along a tree are not built yet).
+(mutate.py) evolves haplotypes from it along a tree under a substitution model
+and optional insertion / deletion models, also on the GPU.
 ``random_genome`` and ``random_haplotypes`` below exist so that tests and the
 benchmark have inputs of the named shapes; they are input generators, not
 restatements: their mutations are scattered uniformly and the haplotypes share

@@ -1,4 +1,4 @@
-"""``create_haplotypes()`` -- haplotypes evolved from the reference along a tree, substitutions only.
+"""``create_haplotypes()`` -- haplotypes evolved from the reference along a tree: substitutions, insertions, deletions.
 
 jackalope's middle step (reference -> haplotypes -> reads) with the per-site work on the GPU
 (``jlp_create_haplotypes``, ``csrc/jlp_mutate.cu``).  The definitions this module implements are the
@@ -12,6 +12,9 @@ project's own (DESIGN.md section 10):
 * The root state is the reference base; a child's state is drawn from row ``parent state`` of
   ``expm(Q * rate * branch_length)``.  Only T/C/A/G sites evolve.  A haplotype's records are the sites where its
   tip differs from the reference.
+* Insertions and deletions (``ins`` / ``del_``, models from ``indels()``) happen along each branch in steps of at most
+  ``epsilon`` expected events per site; inserted columns start from ``sub.pi`` and evolve below like any site.  A
+  haplotype's records then follow one canonical encoding of its tip sequence (DESIGN.md section 10).
 """
 from __future__ import annotations
 
@@ -223,6 +226,53 @@ def transition_matrix(Q, t):
     if _lib.lib().jlp_transition_matrix(q.ctypes.data_as(_lib.f64p), float(t), P.ctypes.data_as(_lib.f64p)) != 0:
         raise JackalopeError("jlp_transition_matrix: invalid arguments")
     return P.reshape(4, 4)
+
+
+# ---------------------------------------------------------------------------- indel models ---
+
+class IndelModel:
+    """An insertion or deletion model: ``rate`` per site per unit branch length (summed over the lengths) and the
+    relative weights ``rel_rates[u - 1]`` of the lengths u = 1..``max_length``."""
+
+    def __init__(self, rate, rel_rates):
+        self.rate = float(rate)
+        self.rel_rates = np.ascontiguousarray(rel_rates, dtype=np.float64)
+
+    @property
+    def max_length(self):
+        return int(self.rel_rates.size)
+
+    def probs(self):
+        return self.rel_rates / self.rel_rates.sum()
+
+    def __repr__(self):
+        return "<indel_info rate %g, lengths 1..%d>" % (self.rate, self.max_length)
+
+
+def indels(rate, max_length=10, a=None, rel_rates=None):
+    """An indel model for ``create_haplotypes(ins=..., del_=...)``.  Lengths 1..L have the relative weights
+    ``rel_rates`` when given (L = its length; ``max_length`` and ``a`` are then ignored), otherwise Lavalette's
+    ``(u L / (L - u + 1))^-a`` when ``a`` is given, otherwise ``exp(-u)``, with L = ``max_length``."""
+    f = "indels"
+    if not (_is_number(rate) and rate >= 0):
+        _bad(f, "rate", "a single number >= 0")
+    if rel_rates is not None:
+        try:
+            w = np.asarray(rel_rates, dtype=np.float64)
+        except (TypeError, ValueError):
+            w = None
+        if w is None or w.ndim != 1 or w.size == 0 or not np.all(np.isfinite(w)) or np.any(w < 0) or not np.any(w > 0):
+            _bad(f, "rel_rates", "NULL or a numeric vector, where no number can be < 0 and at least one must be > 0")
+        return IndelModel(rate, w)
+    if not (_is_int(max_length) and max_length >= 1):
+        _bad(f, "max_length", "a single integer >= 1")
+    L = int(max_length)
+    u = np.arange(1, L + 1, dtype=np.float64)
+    if a is not None:
+        if not (_is_number(a) and a > 0):
+            _bad(f, "a", "NULL or a single number > 0")
+        return IndelModel(rate, (u * L / (L - u + 1)) ** (-float(a)))
+    return IndelModel(rate, np.exp(-u))
 
 
 # ------------------------------------------------------------------------------- trees ---
@@ -496,12 +546,14 @@ def haps_theta(theta, n_haps):
 
 def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.03, n_threads=1,
                       show_progress=False, *, seed=None, ctx=None, device=0):
-    """Haplotypes evolved from ``reference`` along the tree of ``haps_info`` under the substitution model ``sub``,
-    generated on the GPU.  Returns a ``Haplotypes`` object (substitution records only; the tree as Newick text in
-    ``.tree``, the call's figures in ``.stats``) and leaves it resident in the context, so a following
-    ``illumina()`` / ``pacbio()`` on it uploads nothing.  ``epsilon`` (validated, unused: substitutions are drawn
-    exactly from P(t)), ``n_threads`` and ``show_progress`` are accepted for compatibility.  ``seed`` (keyword-only)
-    addresses every draw; None draws one from numpy's global RNG."""
+    """Haplotypes evolved from ``reference`` along the tree of ``haps_info`` under the substitution model ``sub`` and
+    the indel models ``ins`` / ``del_`` (``indels()`` or None), generated on the GPU.  Returns a ``Haplotypes`` object
+    (substitution, insertion and deletion records; the tree as Newick text in ``.tree``, the call's figures in
+    ``.stats``) and leaves it resident in the context, so a following ``illumina()`` / ``pacbio()`` on it uploads
+    nothing.  ``epsilon`` bounds the expected indel events per site of one step of a branch; it must be > 0 once an
+    indel rate is > 0 (jackalope's exact Gillespie sampling at 0 is not offered) and is otherwise unused
+    (substitutions are drawn exactly from P(t)).  ``n_threads`` and ``show_progress`` are accepted for compatibility.
+    ``seed`` (keyword-only) addresses every draw; None draws one from numpy's global RNG."""
     from . import _lib
     from .illumina import default_context
 
@@ -512,11 +564,16 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
         _bad(f, "haps_info", "a \"haps_info\" object (from `haps_phylo` or `haps_theta`)")
     if not isinstance(sub, SubModel):
         _bad(f, "sub", "a \"sub_info\" object (from one of the `sub_*` functions)")
-    if ins is not None or del_ is not None:
-        raise JackalopeError("\nFor the `create_haplotypes` function in jackalope, insertions and deletions along a "
-                             "tree are not built yet: arguments `ins` and `del_` must be NULL.")
+    for par, x in (("ins", ins), ("del_", del_)):
+        if x is not None and not isinstance(x, IndelModel):
+            _bad(f, par, "NULL or an \"indel_info\" object (from `indels`); a bare rate is not built yet, "
+                 "use `indels(rate)`")
     if not (_is_number(epsilon) and 0 <= epsilon < 1):
         _bad(f, "epsilon", "a single number >= 0 and < 1")
+    with_indels = ins is not None or del_ is not None
+    if sum(m.rate for m in (ins, del_) if m is not None) > 0 and epsilon == 0:
+        _bad(f, "epsilon", "a single number > 0 and < 1 when `ins` or `del_` has a rate > 0 (exact Gillespie "
+             "sampling, epsilon = 0, is not implemented)")
     if not (_is_int(n_threads) and n_threads >= 1):
         _bad(f, "n_threads", "a single integer >= 1")
     if not isinstance(show_progress, (bool, np.bool_)):
@@ -542,14 +599,39 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     p.seed = int(seed) & (2 ** 64 - 1)
     st = _lib.MutationStats()
     ctx._haps = None
-    ctx._check(ctx.lib.jlp_create_haplotypes(ctx.h, C.byref(p), C.byref(st)), "jlp_create_haplotypes")
+    if with_indels:
+        ip, ist = indel_params(ins, del_, epsilon, sub.pi), _lib.IndelStats()
+        ctx._check(ctx.lib.jlp_create_haplotypes_indels(ctx.h, C.byref(p), C.byref(ip), C.byref(st), C.byref(ist)),
+                   "jlp_create_haplotypes_indels")
+    else:
+        ctx._check(ctx.lib.jlp_create_haplotypes(ctx.h, C.byref(p), C.byref(st)), "jlp_create_haplotypes")
 
     muts = [[haplotype_muts(ctx, h, c) for c in range(reference.n_chroms())] for h in range(len(tree.tip_names))]
     haps = Haplotypes(reference, tree.tip_names, muts)
     haps.tree = tree.newick()
     haps.stats = st.as_dict()
+    if with_indels:
+        haps.stats.update(ist.as_dict())
     ctx._haps = haps
     return haps
+
+
+def indel_params(ins, del_, epsilon, pi):
+    """The jlp_indel_params of (ins, del_) (None: rate 0); the weight arrays are kept alive on the struct."""
+    from . import _lib
+    ip = _lib.IndelParams()
+    ip.epsilon = float(epsilon)
+    ip.pi[:] = [float(x) for x in pi]
+    ip._keep = []
+    for m, rate, n, w in ((ins, "rate_ins", "n_ins", "w_ins"), (del_, "rate_del", "n_del", "w_del")):
+        if m is None:
+            continue
+        arr = np.ascontiguousarray(m.rel_rates, dtype=np.float64)
+        ip._keep.append(arr)
+        setattr(ip, rate, m.rate)
+        setattr(ip, n, arr.size)
+        setattr(ip, w, arr.ctypes.data_as(_lib.f64p))
+    return ip
 
 
 def haplotype_muts(ctx, hap, chrom) -> HapChromMuts:

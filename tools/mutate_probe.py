@@ -1,8 +1,11 @@
 """create_haplotypes at two benchmark shapes: kernel time per pass (CUDA events inside jlp_create_haplotypes, after a
 warm-up call), records and bytes copied to the host, wall time of the call, table sizes, and the wall time of
-random_haplotypes for the same shape on the same host (the input generator the benchmark used so far).
+random_haplotypes for the same shape on the same host (the input generator the benchmark used so far).  Each shape runs
+substitutions only and then with insertions and deletions (ins = del_ = indels(0.1 mu_bar)); the indel rows add the
+host event pass (event_ms) to the kernel passes (count_ms, scan_ms, write_ms: pass 2 and the inserted columns' walk)
+and the store copy (store_ms).
 
-    python tools/mutate_probe.py [--out profiles/r03_mutate_probe.json] [--reps 3] [--small]
+    python tools/mutate_probe.py [--out profiles/r04_mutate_probe.json] [--reps 3] [--small]
 """
 import argparse
 import json
@@ -32,17 +35,7 @@ def shape(ctx, name, n_chroms, chrom_len, n_haps, theta, reps, sub_rate):
     g = J.create_genome(n_chroms, chrom_len, seed=1, ctx=ctx)
     sub = J.sub_TN93((0.25, 0.25, 0.25, 0.25), 2.0, 2.0, 1.0, gamma_shape=0.5, gamma_k=5)
     info = J.haps_theta(theta, n_haps)
-    J.create_haplotypes(g, info, sub, seed=100, ctx=ctx)              # warm-up
-    runs = []
-    for r in range(reps):
-        t0 = time.perf_counter()
-        haps = J.create_haplotypes(g, info, sub, seed=101 + r, ctx=ctx)
-        wall = time.perf_counter() - t0
-        st = dict(haps.stats)
-        st["wall_s"] = wall
-        st["records_per_hap_mean"] = st["records"] / n_haps
-        runs.append(st)
-        del haps
+    out = [one(ctx, g, sub, info, n_haps, reps, {}), one(ctx, g, sub, info, n_haps, reps, indel_kw(sub))]
     t0 = time.perf_counter()
     rh = J.random_haplotypes(g, n_haps, sub_rate=sub_rate, indel_rate=0.0, seed=5)
     rh_wall = time.perf_counter() - t0
@@ -50,12 +43,33 @@ def shape(ctx, name, n_chroms, chrom_len, n_haps, theta, reps, sub_rate):
     del rh
     return dict(shape=name, n_chroms=n_chroms, chrom_len=chrom_len, n_haps=n_haps, theta=theta,
                 model="TN93 (alpha_1 = alpha_2 = 2, beta = 1, uniform pi), gamma_shape 0.5, gamma_k 5",
-                runs=runs, random_haplotypes=dict(sub_rate=sub_rate, indel_rate=0.0, wall_s=rh_wall, records=rh_records))
+                substitutions_only=out[0], indels=dict(ins_del="indels(0.1 * mu_bar) each", **out[1]),
+                random_haplotypes=dict(sub_rate=sub_rate, indel_rate=0.0, wall_s=rh_wall, records=rh_records))
+
+
+def indel_kw(sub):
+    m = J.indels(0.1 * sub.mu_bar())
+    return dict(ins=m, del_=m, epsilon=0.03)
+
+
+def one(ctx, g, sub, info, n_haps, reps, kw):
+    J.create_haplotypes(g, info, sub, seed=100, ctx=ctx, **kw)              # warm-up
+    runs = []
+    for r in range(reps):
+        t0 = time.perf_counter()
+        haps = J.create_haplotypes(g, info, sub, seed=101 + r, ctx=ctx, **kw)
+        wall = time.perf_counter() - t0
+        st = dict(haps.stats)
+        st["wall_s"] = wall
+        st["records_per_hap_mean"] = st["records"] / n_haps
+        runs.append(st)
+        del haps
+    return dict(runs=runs)
 
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_mutate_probe.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r04_mutate_probe.json"))
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--small", action="store_true", help="tiny shapes (rehearsal)")
     a = ap.parse_args()
