@@ -18,7 +18,6 @@
 #include <deque>
 #include <exception>
 #include <functional>
-#include <mutex>
 #include <thread>
 #include <cstdio>
 #include <cstdlib>
@@ -1323,48 +1322,36 @@ static std::shared_ptr<HapStore> make_hap_store(const jlp_ctx* c, const char* na
     auto S = std::make_shared<HapStore>();
     S->name = name ? name : "";
     S->chrom.resize(nc);
-    std::atomic<uint64_t> next{0};
-    std::mutex err_mu;
-    std::string err;
-    auto work = [&]() {
-        for (uint64_t ci; (ci = next.fetch_add(1)) < nc;) {
-            const char* bad = nullptr;
-            const uint64_t M = n_muts[ci];
-            const uint64_t ref_size = c->chrom_off[ci + 1] - c->chrom_off[ci];
-            HapChromHost& H = S->chrom[ci];
-            H.size = chrom_sizes[ci];
-            if (M == 0) {   // get_chrom_full returns the reference string (src/hap_classes.cpp:82)
-                if (chrom_sizes[ci] != ref_size) bad = "chromosome without mutations must keep the reference size";
-            } else if (!old_pos || !new_pos || !nuc_off || !nuc_pool || !nuc_pool_len || !old_pos[ci] || !new_pos[ci] || !nuc_off[ci]) {
-                bad = "mutation arrays are NULL";
-            } else {
-                const uint64_t pb = nuc_pool_len[ci];
-                H.n_muts = M; H.pool_bytes = pb;
-                H.packed.resize(4 * M + (pb + 7) / 8);
-                uint64_t* w = H.packed.data();
-                std::memcpy(w, old_pos[ci], M * 8);
-                std::memcpy(w + M, new_pos[ci], M * 8);
-                std::memcpy(w + 2 * M, nuc_off[ci], M * 8);
-                // size_modifier per record, src/hap_classes.h:314-333
-                int64_t* sm = reinterpret_cast<int64_t*>(w + 3 * M);
-                for (uint64_t i = 0; i < M; i++) {
-                    if (i && new_pos[ci][i] < new_pos[ci][i - 1]) { bad = "mutations must be sorted by new_pos"; break; }
-                    const int64_t s = (i + 1 < M) ? (int64_t)(new_pos[ci][i + 1] - old_pos[ci][i + 1]) : (int64_t)(chrom_sizes[ci] - ref_size);
-                    sm[i] = s + (int64_t)(old_pos[ci][i] - new_pos[ci][i]);
-                }
-                if (pb) std::memcpy(w + 4 * M, nuc_pool[ci], pb);
-            }
-            if (bad) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = bad; }
-        }
-    };
     uint64_t total = 0;
     for (uint64_t ci = 0; ci < nc; ci++) total += n_muts[ci];
     const unsigned nt = total < (1u << 16) ? 1u : (unsigned)std::min<uint64_t>(std::min<uint64_t>(nc, 16), std::max(1u, std::thread::hardware_concurrency()));
-    std::vector<std::thread> th;
-    for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
-    work();
-    for (std::thread& t : th) t.join();
-    if (!err.empty()) throw ArgErr(err);
+    parallel_for(nc, nt, [&](uint64_t ci) {
+        const uint64_t M = n_muts[ci];
+        const uint64_t ref_size = c->chrom_off[ci + 1] - c->chrom_off[ci];
+        HapChromHost& H = S->chrom[ci];
+        H.size = chrom_sizes[ci];
+        if (M == 0) {   // get_chrom_full returns the reference string (src/hap_classes.cpp:82)
+            if (chrom_sizes[ci] != ref_size) throw ArgErr("chromosome without mutations must keep the reference size");
+            return;
+        }
+        if (!old_pos || !new_pos || !nuc_off || !nuc_pool || !nuc_pool_len || !old_pos[ci] || !new_pos[ci] || !nuc_off[ci])
+            throw ArgErr("mutation arrays are NULL");
+        const uint64_t pb = nuc_pool_len[ci];
+        H.n_muts = M; H.pool_bytes = pb;
+        H.packed.resize(4 * M + (pb + 7) / 8);
+        uint64_t* w = H.packed.data();
+        std::memcpy(w, old_pos[ci], M * 8);
+        std::memcpy(w + M, new_pos[ci], M * 8);
+        std::memcpy(w + 2 * M, nuc_off[ci], M * 8);
+        // size_modifier per record, src/hap_classes.h:314-333
+        int64_t* sm = reinterpret_cast<int64_t*>(w + 3 * M);
+        for (uint64_t i = 0; i < M; i++) {
+            if (i && new_pos[ci][i] < new_pos[ci][i - 1]) throw ArgErr("mutations must be sorted by new_pos");
+            const int64_t s = (i + 1 < M) ? (int64_t)(new_pos[ci][i + 1] - old_pos[ci][i + 1]) : (int64_t)(chrom_sizes[ci] - ref_size);
+            sm[i] = s + (int64_t)(old_pos[ci][i] - new_pos[ci][i]);
+        }
+        if (pb) std::memcpy(w + 4 * M, nuc_pool[ci], pb);
+    });
     return S;
 }
 
@@ -1553,22 +1540,11 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     double event_ms = 0;
     if (im) {
         const auto te = std::chrono::steady_clock::now();
-        std::atomic<uint64_t> next{0};
-        std::mutex err_mu;
-        std::string err;
-        auto work = [&]() {
-            try {
-                for (uint64_t ci; (ci = next.fetch_add(1)) < nc;)
-                    indel_events(p->seed, (uint32_t)ci, c->chrom_off[ci + 1] - c->chrom_off[ci], n, p->parent,
-                                 p->branch_len, tip_of.data(), n_tips, *im, ich[ci]);
-            } catch (const std::exception& e) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = e.what(); }
-        };
         const unsigned nt = (unsigned)std::min<uint64_t>(std::min<uint64_t>(nc, 16), std::max(1u, std::thread::hardware_concurrency()));
-        std::vector<std::thread> th;
-        for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
-        work();
-        for (std::thread& t : th) t.join();
-        if (!err.empty()) throw ArgErr(err);
+        parallel_for(nc, nt, [&](uint64_t ci) {
+            indel_events(p->seed, (uint32_t)ci, c->chrom_off[ci + 1] - c->chrom_off[ci], n, p->parent, p->branch_len,
+                         tip_of.data(), n_tips, *im, ich[ci]);
+        });
         ir_start.resize(n_items + 1);
         for (size_t r = 0; r < n_items; r++) {
             ir_start[r] = irec.size();
@@ -1761,33 +1737,19 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         stores[t]->name = p->tip_names[t];
         stores[t]->chrom.resize(nc);
     }
-    std::atomic<size_t> next{0};
-    std::mutex err_mu;
-    std::string err;
-    const int dev = d.id;
-    auto work = [&]() {
-        try {
-            CK(cudaSetDevice(dev));
-            for (size_t r; (r = next.fetch_add(1)) < n_items;) {
-                HapChromHost& H = stores[r / nc]->chrom[r % nc];
-                const uint64_t M = region_n[r];
-                H.size = im ? ich[r % nc].tip[r / nc].size : c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
-                H.n_muts = M;
-                H.pool_bytes = pool[r];
-                if (!M) continue;
-                H.packed.resize(4 * M + (pool[r] + 7) / 8);
-                CK(cudaMemcpy(H.packed.data(), d_out.p + region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
-            }
-        } catch (const std::exception& e) { std::lock_guard<std::mutex> g(err_mu); if (err.empty()) err = e.what(); }
-    };
     const unsigned nt = records < (1u << 16) ? 1u
                         : (unsigned)std::min<uint64_t>(std::min<uint64_t>(n_items, 16), std::max(1u, std::thread::hardware_concurrency()));
-    std::vector<std::thread> th;
-    for (unsigned i = 1; i < nt; i++) th.emplace_back(work);
-    work();
-    for (std::thread& t : th) t.join();
-    if (!err.empty()) throw CudaErr(err);
-    CK(cudaSetDevice(dev));
+    parallel_for(n_items, nt, [&](uint64_t r) {
+        HapChromHost& H = stores[r / nc]->chrom[r % nc];
+        const uint64_t M = region_n[r];
+        H.size = im ? ich[r % nc].tip[r / nc].size : c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
+        H.n_muts = M;
+        H.pool_bytes = pool[r];
+        if (!M) return;
+        H.packed.resize(4 * M + (pool[r] + 7) / 8);
+        CK(cudaSetDevice(d.id));
+        CK(cudaMemcpy(H.packed.data(), d_out.p + region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
+    });
 
     clear_haps(c);
     for (const auto& S : stores) attach_hap(c, S);
@@ -2050,55 +2012,15 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
         }
         // ---- per-read quantities on the host (read length, passes, error probabilities, thresholds): batch k + 1 is
         //      prepared by a helper thread (which spreads the reads over n_threads workers) while the device
-        //      generates batch k and the sink takes it
-        struct Prepared { std::vector<PbRead> plan; uint64_t bound = 0; std::string err; };
+        //      generates batch k and the sink takes it; bound: the FASTQ bytes of the batch at most
+        struct Prepared { std::vector<PbRead> plan; uint64_t bound = 0; std::exception_ptr err; };
         auto prepare = [&](uint64_t b0, uint32_t n, Prepared& out) {
             try {
-                std::vector<PbRead>& plan = out.plan;
-                plan.resize(n);
-                // chains of duplicates: read i re-reads iff the draw made after read i - 1 says so and i does not open a pool
-                std::vector<uint32_t> lead(n, kPbNoLeader);
-                if (dups)
-                    for (uint32_t i = 1; i < n; i++)
-                        if ((b0 + i - job.lo) % P->read_pool_size != 0 && (t_dup.all || pb_dup_draw(P->seed, b0 + i - 1) < t_dup.thr))
-                            lead[i] = lead[i - 1] == kPbNoLeader ? i - 1 : lead[i - 1];
-                // the reads are independent given their leaders: split over the host threads (n_threads, at most 64),
-                // first the leaders, then the duplicates (which take their leader's chromosome and length)
-                const uint32_t nt = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 1), 64);
-                std::vector<uint64_t> part(nt, 0);
-                std::vector<std::string> errs(nt);
-                for (int pass = 0; pass < (dups ? 2 : 1); pass++) {
-                    auto work = [&](uint32_t k) {
-                        try {
-                            for (uint32_t i = k; i < n; i += nt) {
-                                if ((lead[i] != kPbNoLeader) != (pass == 1)) continue;
-                                const uint64_t j = b0 + i;
-                                PbSample smp;
-                                size_t g;
-                                if (pass == 0) {
-                                    g = (size_t)(std::upper_bound(G.group_off.begin(), G.group_off.end(), j) - G.group_off.begin()) - 1;
-                                    smp = pb_sample(model, P->seed, j, G.groups[g].len);
-                                } else {
-                                    g = plan[lead[i]].group;
-                                    smp = pb_sample_passes(model, P->seed, j, plan[lead[i]].read_length);
-                                }
-                                std::memset(&plan[i], 0, sizeof(PbRead));
-                                pb_read_model(model, P->seed, j, smp, plan[i]);
-                                plan[i].group = (uint32_t)g;
-                                plan[i].leader = lead[i];
-                                part[k] += max_prefix + 24 + 2 * smp.read_length + 5;
-                            }
-                        } catch (const std::exception& e) { errs[k] = e.what(); }
-                    };
-                    std::vector<std::thread> th;
-                    for (uint32_t k = 1; k < nt; k++) th.emplace_back(work, k);
-                    work(0);
-                    for (std::thread& t : th) t.join();
-                }
-                for (const std::string& e : errs) if (!e.empty()) { out.err = e; return; }
-                out.bound = 0;
-                for (uint64_t v : part) out.bound += v;
-            } catch (const std::exception& e) { out.err = e.what(); }
+                out.plan.resize(n);
+                const uint64_t len = pb_plan(model, P->seed, b0, n, job.lo, P->read_pool_size, t_dup, G.group_off, G.groups.data(),
+                                             P->n_threads, out.plan.data(), nullptr);
+                out.bound = (uint64_t)n * (max_prefix + 24 + 5) + 2 * len;
+            } catch (...) { out.err = std::current_exception(); }
         };
         Prepared prep[2];
         std::thread prep_thread;
@@ -2140,7 +2062,7 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
             if (prep_thread.joinable()) prep_thread.join();
             t_join += now() - t0;
             Prepared& cur = prep[bk & 1];
-            if (!cur.err.empty()) throw ArgErr(cur.err);
+            if (cur.err) std::rethrow_exception(cur.err);
             if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();      // Progress::check_abort, src/hts.h:396-399
             b0_next = b0 + n;
             if (b0_next < s_hi) {
@@ -2245,27 +2167,25 @@ int jlp_pacbio_read_plan(jlp_ctx* c, int use_haplotypes, const jlp_pacbio_params
         pb_model_from(p, model);
         const Layout G = make_layout(c, LayoutSpec(use_haplotypes != 0, p, p->n_reads));
         const Thr t_dup = thr_double_lt(p->prob_dup);
-        const bool dups = t_dup.thr != 0 || t_dup.all;
-        for (const Job& job : G.jobs) {
-            PbSample ls{};
-            size_t lg = 0;
-            for (uint64_t j = job.lo; j < job.hi; j++) {
-                const bool dup = dups && j > job.lo && (j - job.lo) % std::max<uint64_t>(p->read_pool_size, 1) != 0 &&
-                                 (t_dup.all || pb_dup_draw(p->seed, j - 1) < t_dup.thr);
-                PbSample s;
-                if (!dup) {
-                    lg = (size_t)(std::upper_bound(G.group_off.begin(), G.group_off.end(), j) - G.group_off.begin()) - 1;
-                    s = ls = pb_sample(model, p->seed, j, G.groups[lg].len);
-                } else {
-                    s = pb_sample_passes(model, p->seed, j, ls.read_length);
+        // chunks of whole pools, as the driver's batches
+        const uint64_t pool = std::max<uint64_t>(p->read_pool_size, 1), B = std::max<uint64_t>(pool, 32768 / pool * pool);
+        std::vector<PbRead> plan;
+        std::vector<PbSample> smp;
+        for (const Job& job : G.jobs)
+            for (uint64_t b0 = job.lo; b0 < job.hi; b0 += B) {
+                const uint32_t n = (uint32_t)std::min(B, job.hi - b0);
+                plan.resize(n);
+                smp.resize(n);
+                pb_plan(model, p->seed, b0, n, job.lo, pool, t_dup, G.group_off, G.groups.data(), p->n_threads, plan.data(), smp.data());
+                for (uint32_t i = 0; i < n; i++) {
+                    const uint64_t j = b0 + i;
+                    if (group) group[j] = plan[i].group;
+                    if (read_len) read_len[j] = smp[i].read_length;
+                    if (split_pos) split_pos[j] = smp[i].split_pos;
+                    if (passes_left) passes_left[j] = smp[i].passes_left;
+                    if (passes_right) passes_right[j] = smp[i].passes_right;
                 }
-                if (group) group[j] = lg;
-                if (read_len) read_len[j] = s.read_length;
-                if (split_pos) split_pos[j] = s.split_pos;
-                if (passes_left) passes_left[j] = s.passes_left;
-                if (passes_right) passes_right[j] = s.passes_right;
             }
-        }
     });
 }
 

@@ -1,15 +1,48 @@
 // Host-side model preparation for the Illumina kernels: alias tables, integer
-// thresholds, fragment-length table, read apportioning.  Plain C++ (g++), no
+// thresholds, fragment-length table, read apportioning; the loop that spreads host
+// work over a few threads.  Plain C++ (g++), no
 // CUDA.  Each function cites the reference code it stands in for
 // (paths relative to /root/reference).
 #ifndef JLP_HOST_H
 #define JLP_HOST_H
 
+#include <atomic>
 #include <cstdint>
+#include <exception>
+#include <mutex>
 #include <string>
+#include <thread>
 #include <vector>
 
 namespace jlp {
+
+// --- host work over a few threads --------------------------------------------------
+// f(i) for every i in [0, n) on n_threads threads, the calling thread one of them; items are handed out one at a time.
+// Every item runs even when others throw; then the exception of the lowest failing i is rethrown, as a serial loop would
+// report it.  Every thread started is joined before this returns or throws; a thread that cannot be started is reported
+// after the items have run on the others.
+template <typename F> void parallel_for(uint64_t n, unsigned n_threads, F f) {
+    std::atomic<uint64_t> next{0};
+    std::mutex mu;
+    uint64_t first_bad = n;
+    std::exception_ptr err, start_err;
+    auto work = [&]() {
+        for (uint64_t i; (i = next.fetch_add(1)) < n;) {
+            try { f(i); } catch (...) {
+                std::lock_guard<std::mutex> g(mu);
+                if (i < first_bad) { first_bad = i; err = std::current_exception(); }
+            }
+        }
+    };
+    std::vector<std::thread> th;
+    try {
+        for (unsigned k = 1; k < n_threads; k++) th.emplace_back(work);
+    } catch (...) { start_err = std::current_exception(); }
+    work();
+    for (std::thread& t : th) t.join();
+    if (err) std::rethrow_exception(err);
+    if (start_err) std::rethrow_exception(start_err);
+}
 
 // --- comparison thresholds -------------------------------------------------
 // A comparison of u = runif_01(x) against a constant is monotone in x, so it

@@ -1,8 +1,10 @@
 // Host side of the PacBio read generator: see jlp_pacbio.h.
 #include "jlp_pacbio.h"
 
+#include <algorithm>
 #include <atomic>
 #include <cmath>
+#include <cstring>
 #include <stdexcept>
 
 #include "jlp_draws.h"
@@ -286,6 +288,45 @@ void pb_read_model(const PbModel& m, uint64_t seed, uint64_t j, const PbSample& 
     out.read_length = (uint32_t)s.read_length;
     out.split_pos = (uint32_t)s.split_pos;
     out.flags = flags;
+}
+
+uint64_t pb_plan(const PbModel& m, uint64_t seed, uint64_t b0, uint32_t n, uint64_t job_lo, uint64_t pool, Thr t_dup,
+                 const std::vector<uint64_t>& group_off, const GroupDev* groups, uint64_t n_threads, PbRead* out,
+                 PbSample* samples) {
+    const bool dups = t_dup.thr != 0 || t_dup.all;
+    std::vector<uint32_t> lead(n, kPbNoLeader);
+    if (dups)
+        for (uint32_t i = 1; i < n; i++)
+            if ((b0 + i - job_lo) % pool != 0 && (t_dup.all || pb_dup_draw(seed, b0 + i - 1) < t_dup.thr))
+                lead[i] = lead[i - 1] == kPbNoLeader ? i - 1 : lead[i - 1];
+    // the reads are independent given their leaders
+    const uint32_t nt = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(n_threads, 1), 64);
+    std::vector<uint64_t> len(nt, 0);
+    for (int pass = 0; pass < (dups ? 2 : 1); pass++)
+        parallel_for(nt, nt, [&](uint64_t k) {
+            for (uint32_t i = (uint32_t)k; i < n; i += nt) {
+                if ((lead[i] != kPbNoLeader) != (pass == 1)) continue;
+                const uint64_t j = b0 + i;
+                PbSample s;
+                size_t g;
+                if (pass == 0) {
+                    g = (size_t)(std::upper_bound(group_off.begin(), group_off.end(), j) - group_off.begin()) - 1;
+                    s = pb_sample(m, seed, j, groups[g].len);
+                } else {
+                    g = out[lead[i]].group;
+                    s = pb_sample_passes(m, seed, j, out[lead[i]].read_length);
+                }
+                std::memset(&out[i], 0, sizeof(PbRead));
+                pb_read_model(m, seed, j, s, out[i]);
+                out[i].group = (uint32_t)g;
+                out[i].leader = lead[i];
+                if (samples) samples[i] = s;
+                len[k] += s.read_length;
+            }
+        });
+    uint64_t total = 0;
+    for (uint64_t v : len) total += v;
+    return total;
 }
 
 }  // namespace jlp

@@ -12,6 +12,7 @@
 #include <memory>
 #include <vector>
 
+#include "jlp_host.h"
 #include "jlp_kernels.cuh"
 
 namespace jlp {
@@ -74,6 +75,17 @@ static_assert(sizeof(PbRead) == 104, "PbRead layout");
 constexpr uint32_t kPbNoLeader = 0xffffffffu;
 constexpr uint32_t kPbSerial = 1u << 24;      // PbRead::flags: the read is walked by one lane throughout
 void pb_read_model(const PbModel& m, uint64_t seed, uint64_t j, const PbSample& s, PbRead& out);
+
+// The plan of reads [b0, b0 + n) of a job whose reads start at job_lo (b0 - job_lo a whole number of pools of `pool`
+// reads).  Chains of duplicates (ReadWriterOneThread::create_reads, src/hts.h:264-277): read j re-reads its chain's first
+// read iff pb_dup_draw(seed, j - 1) passes t_dup and j does not open a pool.  A chain's first read takes the group of
+// group_off (reads per group, cumulative) that j falls in and a pb_sample of its chromosome; a duplicate takes its
+// leader's group and read length and a pb_sample_passes.  out[i] is filled by pb_read_model, with group and leader.
+// Worker k of min(max(n_threads, 1), 64) takes reads k, k + nt, ...: first the leaders, then the duplicates.
+// samples (may be NULL) receives what was drawn per read.  Returns the sum of the read lengths.
+uint64_t pb_plan(const PbModel& m, uint64_t seed, uint64_t b0, uint32_t n, uint64_t job_lo, uint64_t pool, Thr t_dup,
+                 const std::vector<uint64_t>& group_off, const GroupDev* groups, uint64_t n_threads, PbRead* out,
+                 PbSample* samples);
 
 // plan: walk -> counts -> template span, start, strand, record length; reads: the record itself
 cudaError_t launch_pb_plan(PbRead* reads, uint32_t n, uint64_t first_read, uint64_t seed, const GroupDev* groups,
