@@ -98,10 +98,29 @@ class IndelStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class VcfParams(C.Structure):
+    _fields_ = [
+        ("path", C.c_char_p), ("n_samples", C.c_uint64), ("ploidy", C.c_uint32), ("sample_haps", u64p),
+        ("sample_names", C.POINTER(C.c_char_p)), ("file_date", C.c_char_p), ("compress", C.c_int), ("comp_method", C.c_char_p),
+        ("comp_engine", C.c_int), ("n_threads", C.c_uint64), ("batch_bytes", C.c_uint64),
+    ]
+
+
+class VcfStats(C.Structure):
+    _fields_ = [
+        ("lines", C.c_uint64), ("records", C.c_uint64), ("text_bytes", C.c_uint64), ("file_bytes", C.c_uint64),
+        ("batches", C.c_uint64), ("span_ms", C.c_double), ("text_ms", C.c_double), ("bgzf_ms", C.c_double),
+        ("total_ms", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/jlp_b200.h declares
 SYMBOLS = [
     "jlp_ctx_create", "jlp_ctx_create_multi", "jlp_ctx_n_devices", "jlp_materialize_haplotypes", "jlp_ctx_destroy", "jlp_last_error", "jlp_set_genome", "jlp_set_genome_async", "jlp_genome_sync", "jlp_create_genome", "jlp_get_genome", "jlp_genome_draw", "jlp_clear_haplotypes",
-    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_get_haplotype_muts", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
+    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_get_haplotype_muts", "jlp_write_vcf", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
     "jlp_illumina_to_memory", "jlp_illumina_stream", "jlp_illumina_device_only", "jlp_illumina_group_counts", "jlp_apportion", "jlp_shard_range", "jlp_deflate", "jlp_bgzf_device", "jlp_pacbio", "jlp_pacbio_to_memory", "jlp_pacbio_read_plan", "jlp_pacbio_sample", "jlp_reads_per_group", "jlp_alias_build",
     "jlp_threshold", "jlp_unif_expr", "jlp_frag_table", "jlp_philox4x32_10", "jlp_draw_pos", "jlp_draw_pair",
     "jlp_version",
@@ -144,6 +163,7 @@ def lib():
                                                C.POINTER(MutationStats), C.POINTER(IndelStats)]
     L.jlp_get_haplotype_muts.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, u64p, u64p, u64p, C.c_void_p, C.c_uint64,
                                          C.c_uint64, u64p, u64p, u64p]
+    L.jlp_write_vcf.argtypes = [C.c_void_p, C.POINTER(VcfParams), C.POINTER(VcfStats)]
     L.jlp_transition_matrix.argtypes = [f64p, C.c_double, f64p]
     L.jlp_set_profile.argtypes = [C.c_void_p, C.c_int, C.c_uint64, u32p, f64p, u8p]
     L.jlp_illumina_ref.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(RunStats)]

@@ -193,6 +193,53 @@ bool reads_fits(const GenParams& p);
 
 constexpr uint32_t kScanBlock = 1024;
 
+// write_vcf (jlp_vcf.cu, DESIGN.md section 11), one chromosome at a time.  The records of the included haplotypes are
+// numbered haplotype-major; their packed arrays (HapChromHost::packed layout) sit in `recs`.
+struct VcfHap {
+    uint64_t woff;               // word offset of the haplotype's packed records in recs
+    uint32_t n, rec0;            // its records, and the number of its first one
+};
+struct VcfCar {                  // a haplotype with records in a line (a carrier)
+    uint64_t new_s, len;         // where its allele starts in the haplotype, and its length
+    uint64_t key;                // the allele's first min(len, 8) bytes
+    uint32_t u, i0, i1;          // included haplotype; its first and last record of the line
+    uint32_t idx;                // its allele index (0: REF)
+};
+struct VcfChrom {
+    const uint64_t* recs;
+    const VcfHap* hap;           // [n_hap + 1] included haplotypes (rec0 of the last entry = n_rec)
+    uint32_t n_hap, n_rec;
+    const uint8_t* ref;          // the chromosome's reference bases
+    uint64_t L;
+    const uint8_t* name;         // the chromosome's name
+    uint32_t name_len;
+    uint32_t ploidy, n_samples;
+    const uint32_t* slot_hap;    // [n_samples * ploidy] included haplotype of each slot of the sample matrix
+    const uint32_t* first_slot;  // [n_hap] its first slot
+    const uint32_t* n_slots;     // [n_hap] the slots it fills
+    // [n_rec] per record, in record order and in sorted order
+    uint64_t *start, *end, *start_sorted, *end_sorted, *maxend, *key2, *key2_sorted;
+    uint32_t *rec_hap, *val, *order, *flag, *lid;
+    // [n_rec] per position of the line-sorted order: the line's carriers, alleles classes and ALTs start at line_first
+    VcfCar* car;
+    uint32_t *car_pos, *cls_car, *cls_slot, *cls_rank, *alt_car;
+    // [n_rec + 1] per line
+    uint32_t *line_first, *n_car, *n_alt;
+    uint64_t *line_s, *line_e, *line_len, *line_end;   // line_end: inclusive prefix of line_len
+    uint32_t* hidx;              // [warps of the line kernels][n_hap], zero between lines
+    uint8_t* cub_tmp;
+    size_t cub_bytes;
+};
+size_t vcf_cub_bytes(uint32_t n_rec);
+unsigned vcf_line_blocks(uint64_t n_lines, int n_sm);     // CTAs of 8 warps of the line kernels
+// spans, sort by start, running maximum of the ends, line flags and their inclusive prefix (lid[n_rec - 1] = lines)
+cudaError_t launch_vcf_spans(const VcfChrom& v, cudaStream_t s);
+// line extents, the line-major sort, k_vcf_lines<false> (carriers, alleles, text lengths) and line_end
+cudaError_t launch_vcf_size(const VcfChrom& v, uint32_t n_lines, int n_sm, cudaStream_t s);
+// the text of lines [l0, l1) into out + out_skip
+cudaError_t launch_vcf_text(const VcfChrom& v, uint32_t l0, uint32_t l1, uint8_t* out, uint64_t out_skip, int n_sm,
+                            cudaStream_t s);
+
 // BGZF on the device (jlp_bgzf.cu).  totals[0..1] hold the FASTQ bytes of the two files of a batch (device
 // memory, as launch_scan leaves them); the compressed sizes come back in totals[2..3].  Block b of a file is
 // compressed into slots + b * kBgzfSlot, then gathered to out + (sum of the sizes before it).  nblk_max sizes
