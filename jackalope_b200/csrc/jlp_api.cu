@@ -113,6 +113,34 @@ struct HapArena {
     ~HapArena() { release(); }
 };
 
+// The device BGZF coder's buffers for one or two files: per file one 64 KiB slot per block, the members' sizes and
+// offsets, and the contiguous compressed image (`out`, what the D2H copy moves); the codes of the batch.
+struct Bgzf {
+    DevBuf<uint8_t> slots[2], out[2], code;
+    DevBuf<uint32_t> zlen[2];
+    DevBuf<uint64_t> zoff[2];
+    int files = 1;
+    // room per file for nblk blocks holding in_bytes: a member never exceeds its input plus 64 bytes (a block that does
+    // not compress is stored)
+    void ensure(uint32_t nblk, uint64_t in_bytes, int n_files) {
+        files = n_files;
+        for (int e = 0; e < n_files; e++) {
+            slots[e].ensure((size_t)nblk * kBgzfSlot);
+            out[e].ensure(in_bytes + (size_t)nblk * 64 + 64);
+            zlen[e].ensure(nblk);
+            zoff[e].ensure(nblk);
+        }
+        code.ensure(kBgzfCodeBytes);
+    }
+    // launch_bgzf on the files of the last ensure(); with one file, totals[1] must be 0: the second file's buffers alias
+    // the first's.  Levels 4 and above also search for matches.
+    cudaError_t launch(const uint8_t* in0, const uint8_t* in1, uint64_t* totals, uint32_t nblk, int level, cudaStream_t s) {
+        const int f = files - 1;
+        return launch_bgzf(in0, in1, totals, nblk, level >= 4, slots[0].p, slots[f].p, zlen[0].p, zlen[f].p, zoff[0].p, zoff[f].p,
+                           out[0].p, out[f].p, code.p, s);
+    }
+};
+
 struct Slot {
     DevBuf<uint8_t> out[2];
     DevBuf<EndPlan> plan;
@@ -120,11 +148,7 @@ struct Slot {
     DevBuf<uint64_t> block_tot, block_base, totals;
     PinBuf<uint8_t> h_out[2];
     PinBuf<uint64_t> h_totals;
-    // device BGZF: one 64 KiB slot per block, the members' sizes and offsets, the contiguous compressed batch
-    DevBuf<uint8_t> zslots[2], zdev[2];
-    DevBuf<uint32_t> zlen[2];
-    DevBuf<uint64_t> zoff[2];
-    DevBuf<uint8_t> zcode;        // launch_bgzf's scratch (the codes of the batch)
+    Bgzf z;                       // device BGZF
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // start, placed, scanned, reads done, copied, all kernels done
     uint32_t pairs = 0;
     uint64_t tot[2] = {0, 0};     // FASTQ bytes of the batch per file (read back from the device)
@@ -169,7 +193,6 @@ struct Device {
     static constexpr int kMatBufs = 3;
     DevBuf<uint64_t> m_pack[kMatBufs];
     cudaEvent_t m_up[kMatBufs] = {nullptr, nullptr, nullptr}, m_done[kMatBufs] = {nullptr, nullptr, nullptr};
-    bool m_busy[kMatBufs] = {false, false, false};
     uint64_t m_next = 0;
 
     void free_haps() {
@@ -441,6 +464,15 @@ Compression compression_of(const jlp_illumina_params* P, SinkKind kind) {
     return z;
 }
 
+// The compression arguments of every driver.  A level <= 0 is no compression, and the method is then not looked at.
+void check_compression(int compress, const char* comp_method, int comp_engine) {
+    const std::string m = comp_method ? comp_method : "";
+    if (compress > 0 && m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");  // src/hts.h:470
+    if (compress > 9) throw ArgErr("\nInvalid bgzip compress level of " + std::to_string(compress) +
+                                   ". It must be in range [0,9].");                                      // src/io.h:113-117
+    if (comp_engine < JLP_COMP_AUTO || comp_engine > JLP_COMP_DEVICE) throw ArgErr("comp_engine must be 0 (auto), 1 (host) or 2 (device)");
+}
+
 // the argument checks the C++ layer of the reference performs, plus the ranges of the additions
 void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, SinkKind kind) {
     if (!P) throw ArgErr("params is NULL");
@@ -453,13 +485,7 @@ void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P,
         if (c->tab[0].L != c->tab[1].L)   // src/hts_illumina.h:348-352
             throw ArgErr("In IlluminaOneGenome constr., read lengths for R1 and R2 don't match.");
     }
-    if (P->compress > 0) {
-        std::string m = P->comp_method ? P->comp_method : "";
-        if (m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");  // src/hts.h:470
-        if (P->compress > 9) throw ArgErr("\nInvalid bgzip compress level of " + std::to_string(P->compress) +
-                                          ". It must be in range [0,9].");                   // src/io.h:113-117
-    }
-    if (P->comp_engine < JLP_COMP_AUTO || P->comp_engine > JLP_COMP_DEVICE) throw ArgErr("comp_engine must be 0 (auto), 1 (host) or 2 (device)");
+    check_compression(P->compress, P->comp_method, P->comp_engine);
     if (!(P->prob_dup >= 0 && P->prob_dup <= 1)) throw ArgErr("prob_dup must be in [0,1]");
     const double insp[2] = {P->ins_prob1, P->ins_prob2}, delp[2] = {P->del_prob1, P->del_prob2};
     for (int e = 0; e < n_ends; e++)
@@ -554,6 +580,14 @@ std::string file_name(const Job& job, int e, bool gz, const jlp_illumina_params*
     return n;
 }
 
+// The next of materialisation's buffers, free: the kernels that read it last, whose end the caller records in m_done,
+// must be done before the buffer can grow (cudaFree) or be written again.  An event never recorded is complete.
+int claim_mat_buf(Device& d) {
+    const int k = (int)(d.m_next++ % Device::kMatBufs);
+    CK(cudaEventSynchronize(d.m_done[k]));
+    return k;
+}
+
 // Materialise haplotype chromosome (h, ci) on device d if it is not resident yet
 // (HapChrom::get_chrom_full, src/hap_classes.cpp:80-116).
 void ensure_hap_chrom(const jlp_ctx* c, Device& d, size_t h, size_t ci) {
@@ -562,13 +596,7 @@ void ensure_hap_chrom(const jlp_ctx* c, Device& d, size_t h, size_t ci) {
     const HapChromHost& M = c->haps[h]->chrom[ci];
     const uint64_t ref_size = c->chrom_off[ci + 1] - c->chrom_off[ci];
     const uint8_t* ref = d.genome.p + kPad + c->chrom_off[ci];
-    const int k = (int)(d.m_next++ % Device::kMatBufs);
-    if (!d.m_up[k]) {
-        CK(cudaEventCreateWithFlags(&d.m_up[k], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&d.m_done[k], cudaEventDisableTiming));
-    }
-    // the kernel that read this buffer last must be done before the buffer can grow (cudaFree) or be written again
-    if (d.m_busy[k]) CK(cudaEventSynchronize(d.m_done[k]));
+    const int k = claim_mat_buf(d);
     d.m_pack[k].upload(M.packed, d.s_upload);
     CK(cudaEventRecord(d.m_up[k], d.s_upload));
     d.h2d_bytes += M.n_muts * 32 + M.pool_bytes;
@@ -579,7 +607,6 @@ void ensure_hap_chrom(const jlp_ctx* c, Device& d, size_t h, size_t ci) {
     CK(launch_materialize(ref, ref_size, n, w, w + n, reinterpret_cast<const int64_t*>(w + 3 * n), w + 2 * n,
                           reinterpret_cast<const uint8_t*>(w + 4 * n), M.size, out + kPad, d.s_compute));
     CK(cudaEventRecord(d.m_done[k], d.s_compute));
-    d.m_busy[k] = true;
     seq = out + kPad;       // valid in stream order: everything that reads it runs on s_compute
 }
 
@@ -685,7 +712,6 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
         E.tA = ta.thr; E.tA_all = ta.all; E.tI = ti.thr; E.tI_all = ti.all;
         E.hA = ta.all ? 0x10000u : (uint32_t)(ta.thr >> 48);
     }
-    for (cudaEvent_t& ev : d.ev_run) if (!ev) CK(cudaEventCreate(&ev));
     CK(cudaEventRecord(d.ev_run[0], d.s_compute));
     std::vector<uint64_t> frag = frag_table(P->frag_len_shape, P->frag_len_scale, P->frag_len_min, P->frag_len_max);
     std::vector<uint32_t> guide = frag_guide(frag);
@@ -718,8 +744,7 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
     const uint64_t n_rec_max = B * n_ends;
     const uint32_t nsb_max = (uint32_t)((B + kScanBlock - 1) / kScanBlock);
     const bool need_host = sink.kind != SINK_NONE && !sizes_only;
-    const uint32_t nblk_all = (uint32_t)((B * max_rec + kBgzfIn - 1) / kBgzfIn) + 1;
-    const uint32_t nblk_max = dev_z && !sizes_only ? nblk_all : 0;
+    const uint32_t nblk = (uint32_t)((B * max_rec + kBgzfIn - 1) / kBgzfIn) + 1;
     for (Slot& s : d.slot) {
         s.plan.ensure(n_rec_max);
         s.rec_len.ensure(n_rec_max);
@@ -733,17 +758,9 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
             s.out[e].ensure(B * max_rec + 64);
             // compressed bytes of a batch never exceed its FASTQ bytes plus the members' framing (an incompressible block is stored)
             // (the same size with and without compression: pinning a gigabyte again for the first compressed call took seconds)
-            if (need_host) s.h_out[e].ensure(B * max_rec + (size_t)nblk_all * 64 + 64);
+            if (need_host) s.h_out[e].ensure(B * max_rec + (size_t)nblk * 64 + 64);
         }
-        if (dev_z && !sizes_only)
-            for (int e = 0; e < 2; e++) {
-                s.zslots[e].ensure((size_t)nblk_max * kBgzfSlot);
-                s.zdev[e].ensure(B * max_rec + (size_t)nblk_max * 64 + 64);
-                s.zlen[e].ensure(nblk_max);
-                s.zoff[e].ensure(nblk_max);
-                s.zcode.ensure(kBgzfCodeBytes);
-            }
-        for (cudaEvent_t& ev : s.ev) if (!ev) CK(cudaEventCreate(&ev));
+        if (dev_z && !sizes_only) s.z.ensure(nblk, B * max_rec, n_ends);
         s.busy = false;
     }
 
@@ -775,7 +792,7 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
         sink.settle(s.host);                    // the pinned buffers of this slot are free again
         for (int e = 0; e < n_ends; e++) {
             const uint64_t nb = dev_z ? s.ztot[e] : s.tot[e];
-            CK(cudaMemcpyAsync(s.h_out[e].p, dev_z ? s.zdev[e].p : s.out[e].p, nb, cudaMemcpyDeviceToHost, d.s_copy));
+            CK(cudaMemcpyAsync(s.h_out[e].p, dev_z ? s.z.out[e].p : s.out[e].p, nb, cudaMemcpyDeviceToHost, d.s_copy));
             st.d2h_bytes += nb;
         }
         CK(cudaEventRecord(s.ev[4], d.s_copy));
@@ -866,8 +883,7 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
             CK(launch_reads(gp, d.n_sm, d.s_compute));
             CK(cudaEventRecord(s.ev[3], d.s_compute));
             if (dev_z) {
-                CK(launch_bgzf(s.out[0].p, s.out[1].p, s.totals.p, nblk_max, P->compress >= 4, s.zslots[0].p, s.zslots[1].p, s.zlen[0].p,
-                               s.zlen[1].p, s.zoff[0].p, s.zoff[1].p, s.zdev[0].p, s.zdev[1].p, s.zcode.p, d.s_compute));
+                CK(s.z.launch(s.out[0].p, s.out[1].p, s.totals.p, nblk, P->compress, d.s_compute));
                 st.kernel_launches += kBgzfLaunches;
             }
             CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
@@ -1198,6 +1214,12 @@ static int create_ctx(int n_devices, const int* devices, jlp_ctx** out) {
             CK(cudaStreamCreateWithFlags(&d.s_compute, cudaStreamNonBlocking));
             CK(cudaStreamCreateWithFlags(&d.s_copy, cudaStreamNonBlocking));
             CK(cudaStreamCreateWithFlags(&d.s_upload, cudaStreamNonBlocking));
+            for (Slot& s : d.slot) for (cudaEvent_t& ev : s.ev) CK(cudaEventCreate(&ev));
+            for (cudaEvent_t& ev : d.ev_run) CK(cudaEventCreate(&ev));
+            for (int k = 0; k < Device::kMatBufs; k++) {
+                CK(cudaEventCreateWithFlags(&d.m_up[k], cudaEventDisableTiming));
+                CK(cudaEventCreateWithFlags(&d.m_done[k], cudaEventDisableTiming));
+            }
             CK(bgzf_init());
         }
     });
@@ -1942,6 +1964,20 @@ Compression file_compression(int compress, const char* comp_method, uint64_t n_t
     return z;
 }
 
+// One batch of the drivers that write one file per job (PacBio, VCF), its stream synchronised: nb bytes at src on the
+// device go through the pinned buffer of slot n_batch & 1 (free once the batch before last is settled; grown to
+// max(nb, cap) + 64 bytes when it holds less than nb + 64) to the sink, which writes them while the next batch is made.
+void hand_over(Device& d, Output& sink, uint64_t& n_batch, const uint8_t* src, uint64_t nb, uint64_t job, uint64_t cap) {
+    Slot& hs = d.slot[n_batch++ & 1];
+    sink.settle(hs.host);
+    PinBuf<uint8_t>& h = hs.h_out[0];
+    if (h.n < nb + 64) h.ensure(std::max(nb, cap) + 64);
+    CK(cudaMemcpy(h.p, src, nb, cudaMemcpyDeviceToHost));
+    const uint8_t* data[2] = {h.p, nullptr};
+    const uint64_t len[2] = {nb, 0};
+    sink.deliver(hs.host, data, len, job, 1);
+}
+
 // The driver: per batch the per-read quantities are prepared on the host (batch k + 1 on a helper thread while batch k
 // is on the device), then plan upload, k_pb_plan, scan, k_pb_reads, optional BGZF, copy, and the write of batch k
 // overlaps the next batch.  Callbacks are called on the calling thread between batches.
@@ -1961,11 +1997,9 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
     const Thr t_dup = thr_double_lt(P->prob_dup);
     const bool dups = t_dup.thr != 0 || t_dup.all;
     if (dups && P->read_pool_size > 65536) throw Unsupported("prob_dup > 0 with read_pool_size > 65536");
-    if (P->compress < 0 || P->compress > 9) throw ArgErr("\nInvalid bgzip compress level. It must be in range [0,9].");
-    if (P->compress > 0) {
-        const std::string m = P->comp_method ? P->comp_method : "";
-        if (m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");
-    }
+    if (P->compress < 0) throw ArgErr("\nInvalid bgzip compress level. It must be in range [0,9].");
+    check_compression(P->compress, P->comp_method, P->comp_engine);
+    if (P->shard_count > 1 && P->shard_index >= P->shard_count) throw ArgErr("shard_index >= shard_count");
     finish_upload(c, d);
     Layout G = make_layout(c, LayoutSpec(use_haps, P, P->n_reads));
     for (size_t g = 0; g < G.groups.size(); g++) {
@@ -1976,11 +2010,9 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
     const Compression Z = file_compression(P->compress, P->comp_method, P->n_threads, P->comp_engine, sink.kind);
     const bool dev_z = Z.dev_z;
     // the slots' buffers (pinning a gigabyte of host memory on every call cost more than generating the reads, and a dozen
-    // device allocations and frees per call several milliseconds): the device arrays of slot 0, and the pinned buffers of
-    // slots 0 and 1, between which batches alternate so that batch k is written while batch k + 1 is on its way
+    // device allocations and frees per call several milliseconds): the device arrays of slot 0; hand_over's pinned buffers
     Slot& S0 = d.slot[0];
     cudaEvent_t* ev = S0.ev;
-    for (cudaEvent_t& e : S0.ev) if (!e) CK(cudaEventCreate(&e));
     uint64_t n_batch = 0;
     sink.begin(Z, P->compress, P->n_threads, d.writers);
     Quiesce quiesce{d, &sink};
@@ -2004,7 +2036,6 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
         // this shard's part of the job: whole pools, so that chains of duplicates stay inside it
         uint64_t s_lo = job.lo, s_hi = job.hi;
         if (P->shard_count > 1) {
-            if (P->shard_index >= P->shard_count) throw ArgErr("shard_index >= shard_count");
             const uint64_t pool = std::max<uint64_t>(P->read_pool_size, 1), n_pools = (job.hi - job.lo + pool - 1) / pool;
             uint64_t p_lo, p_hi;
             shard_range(0, n_pools, P->shard_index, P->shard_count, p_lo, p_hi);
@@ -2048,10 +2079,9 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
         }
         // batches differ in size: the output buffers grow with slack, and at once to what a full batch will need (pinning
         // is slow)
-        auto grow = [&](auto& buf, uint64_t need, uint32_t n) {
-            if (need + 64 <= buf.n) return;
+        auto grow_to = [&](uint64_t need, uint32_t n) {
             const uint64_t want = std::max(need, n ? need / n * std::min<uint64_t>(B, s_hi - s_lo) : need);
-            buf.ensure(want + want / 4 + 64);
+            return want + want / 4;
         };
         uint64_t n_next = std::min<uint64_t>(batch_size(0), s_hi - s_lo), b0_next = s_lo;
         if (s_lo < s_hi) prepare(s_lo, (uint32_t)n_next, prep[0]);
@@ -2080,7 +2110,7 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
             S0.rec_len.ensure(n); S0.rec_local.ensure(n);
             const uint32_t nsb = (n + kScanBlock - 1) / kScanBlock;
             S0.block_tot.ensure(nsb); S0.block_base.ensure(nsb);
-            grow(S0.out[0], bound, n);
+            if (S0.out[0].n < bound + 64) S0.out[0].ensure(grow_to(bound, n) + 64);
             t_alloc += now() - t0;
             CK(cudaMemcpyAsync(d.pb_reads.p, plan.data(), n * sizeof(PbRead), cudaMemcpyHostToDevice, d.s_compute));
             st.h2d_bytes += n * sizeof(PbRead);
@@ -2094,10 +2124,8 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
             st.kernel_launches += 4;
             const uint32_t nblk = (uint32_t)((bound + kBgzfIn - 1) / kBgzfIn) + 1;
             if (dev_z) {
-                S0.zslots[0].ensure((size_t)nblk * kBgzfSlot); S0.zdev[0].ensure((size_t)nblk * kBgzfSlot);
-                S0.zlen[0].ensure(2 * nblk); S0.zoff[0].ensure(2 * nblk); S0.zcode.ensure(kBgzfCodeBytes);
-                CK(launch_bgzf(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress >= 4, S0.zslots[0].p, S0.zslots[0].p, S0.zlen[0].p, S0.zlen[0].p + nblk,
-                               S0.zoff[0].p, S0.zoff[0].p + nblk, S0.zdev[0].p, S0.zdev[0].p, S0.zcode.p, d.s_compute));
+                S0.z.ensure(nblk, bound, 1);
+                CK(S0.z.launch(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress, d.s_compute));
                 st.kernel_launches += kBgzfLaunches;
             }
             CK(cudaEventRecord(ev[2], d.s_compute));
@@ -2114,15 +2142,8 @@ void run_pacbio(jlp_ctx* c, Device& d, bool use_haps, const jlp_pacbio_params* P
             if (dev_z) st.z_bytes[0] += tot[2];
             if (sink.kind == SINK_NONE) { if (P->progress_cb) P->progress_cb(P->cb_user, n); continue; }
             const uint64_t nb = dev_z ? tot[2] : tot[0];
-            Slot& hs = d.slot[n_batch++ & 1];
-            sink.settle(hs.host);                            // the batch before last is in the file
-            PinBuf<uint8_t>& h_out = hs.h_out[0];
-            grow(h_out, nb, n);
-            CK(cudaMemcpy(h_out.p, dev_z ? S0.zdev[0].p : S0.out[0].p, nb, cudaMemcpyDeviceToHost));
+            hand_over(d, sink, n_batch, dev_z ? S0.z.out[0].p : S0.out[0].p, nb, jk, grow_to(nb, n));
             st.d2h_bytes += nb;
-            const uint8_t* data[2] = {h_out.p, nullptr};
-            const uint64_t len[2] = {nb, 0};
-            sink.deliver(hs.host, data, len, jk, 1);
             if (P->progress_cb) P->progress_cb(P->cb_user, n);                  // Progress::increment, src/hts.h:414
         }
         if (prep_thread.joinable()) prep_thread.join();
@@ -2152,12 +2173,8 @@ void write_vcf(jlp_ctx* c, Device& d, const jlp_vcf_params* P, jlp_vcf_stats* st
     if (P->n_samples < 1 || P->ploidy < 1 || !P->sample_haps) throw ArgErr("the sample matrix is empty");
     if (P->n_samples * P->ploidy >= 0xffffffffull) throw ArgErr("the sample matrix has 2^32 slots or more");
     if (!P->sample_names || !P->file_date) throw ArgErr("sample_names / file_date is NULL");
-    if (P->compress < 0 || P->compress > 9) throw ArgErr("\nInvalid bgzip compress level. It must be in range [0,9].");
-    if (P->compress > 0) {
-        const std::string m = P->comp_method ? P->comp_method : "";
-        if (m != "gzip" && m != "bgzip") throw ArgErr("\nUnrecognized compression method.");
-    }
-    if (P->comp_engine < JLP_COMP_AUTO || P->comp_engine > JLP_COMP_DEVICE) throw ArgErr("comp_engine must be 0 (auto), 1 (host) or 2 (device)");
+    if (P->compress < 0) throw ArgErr("\nInvalid bgzip compress level. It must be in range [0,9].");
+    check_compression(P->compress, P->comp_method, P->comp_engine);
     if (P->n_threads < 1 || P->n_threads > 64) throw ArgErr("n_threads must be in 1..64");
     const uint64_t n_haps = c->haps.size(), n_chroms = c->chrom_off.size() - 1, n_slots = P->n_samples * P->ploidy;
     for (const std::string& n : c->chrom_names)
@@ -2214,7 +2231,6 @@ void write_vcf(jlp_ctx* c, Device& d, const jlp_vcf_params* P, jlp_vcf_stats* st
     Quiesce quiesce{d, &sink};
     Slot& S0 = d.slot[0];
     cudaEvent_t* ev = S0.ev;
-    for (cudaEvent_t& e : S0.ev) if (!e) CK(cudaEventCreate(&e));
     // device scratch for the largest chromosome
     DevBuf<uint64_t> b_start, b_end, b_start_s, b_end_s, b_maxend, b_key2, b_key2_s, b_line_s, b_line_e, b_line_len, b_line_end;
     DevBuf<uint32_t> b_rec_hap, b_val, b_order, b_flag, b_lid, b_car_pos, b_cls_car, b_cls_slot, b_cls_rank, b_alt_car, b_line_first,
@@ -2257,26 +2273,17 @@ void write_vcf(jlp_ctx* c, Device& d, const jlp_vcf_params* P, jlp_vcf_stats* st
         CK(cudaEventRecord(ev[1], s));
         if (dev_z) {
             const uint32_t nblk = (uint32_t)(total / kBgzfIn) + 1;
-            S0.zslots[0].ensure((size_t)nblk * kBgzfSlot); S0.zdev[0].ensure((size_t)nblk * kBgzfSlot);
-            S0.zlen[0].ensure(2 * nblk); S0.zoff[0].ensure(2 * nblk); S0.zcode.ensure(kBgzfCodeBytes); S0.totals.ensure(4);
+            S0.z.ensure(nblk, total, 1); S0.totals.ensure(4);
             h_small.p[0] = total; h_small.p[1] = 0;
             CK(cudaMemcpyAsync(S0.totals.p, h_small.p, 2 * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-            CK(launch_bgzf(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress >= 4, S0.zslots[0].p, S0.zslots[0].p, S0.zlen[0].p,
-                           S0.zlen[0].p + nblk, S0.zoff[0].p, S0.zoff[0].p + nblk, S0.zdev[0].p, S0.zdev[0].p, S0.zcode.p, s));
+            CK(S0.z.launch(S0.out[0].p, S0.out[0].p, S0.totals.p, nblk, P->compress, s));
             CK(cudaMemcpyAsync(h_small.p, S0.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
         }
         CK(cudaEventRecord(ev[2], s));
         CK(cudaStreamSynchronize(s));
         st.text_ms += elapsed(ev[0], ev[1]);
         if (dev_z) st.bgzf_ms += elapsed(ev[1], ev[2]);
-        const uint64_t nb = dev_z ? h_small.p[2] : total;
-        Slot& hs = d.slot[n_batch++ & 1];
-        sink.settle(hs.host);                            // the batch before last is in the file
-        if (hs.h_out[0].n < nb + 64) hs.h_out[0].ensure(std::max(nb, B) + 64);
-        CK(cudaMemcpy(hs.h_out[0].p, dev_z ? S0.zdev[0].p : S0.out[0].p, nb, cudaMemcpyDeviceToHost));
-        const uint8_t* data[2] = {hs.h_out[0].p, nullptr};
-        const uint64_t len[2] = {nb, 0};
-        sink.deliver(hs.host, data, len, 0, 1);
+        hand_over(d, sink, n_batch, dev_z ? S0.z.out[0].p : S0.out[0].p, dev_z ? h_small.p[2] : total, 0, B);
         st.batches++;
         st.text_bytes += total;
         hdr_done = true;
@@ -2285,12 +2292,7 @@ void write_vcf(jlp_ctx* c, Device& d, const jlp_vcf_params* P, jlp_vcf_stats* st
     // materialisation's buffers
     std::vector<VcfHap> hap_tab;
     auto upload = [&](uint64_t ci) {
-        const int k = (int)(d.m_next++ % Device::kMatBufs);
-        if (!d.m_up[k]) {
-            CK(cudaEventCreateWithFlags(&d.m_up[k], cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&d.m_done[k], cudaEventDisableTiming));
-        }
-        if (d.m_busy[k]) CK(cudaEventSynchronize(d.m_done[k]));
+        const int k = claim_mat_buf(d);
         uint64_t words = 0;
         for (uint32_t h : inc) words += c->haps[h]->chrom[ci].packed.size();
         d.m_pack[k].ensure(words);
@@ -2361,7 +2363,6 @@ void write_vcf(jlp_ctx* c, Device& d, const jlp_vcf_params* P, jlp_vcf_stats* st
             l0 = l1;
         }
         CK(cudaEventRecord(d.m_done[k], s));
-        d.m_busy[k] = true;
     }
     if (!hdr_done) emit(nullptr, 0, 0, 0);
     sink.settle(d.slot[0].host); sink.settle(d.slot[1].host);
@@ -2468,23 +2469,21 @@ int jlp_bgzf_device(jlp_ctx* c, int level, const void* in, uint64_t n, void* out
         if ((n && !in) || !len) throw ArgErr("NULL argument");
         Device& d = device0(c);
         const uint32_t nblk = (uint32_t)((n + kBgzfIn - 1) / kBgzfIn);
-        DevBuf<uint8_t> d_in, d_slots, d_out, d_code;
-        DevBuf<uint32_t> d_zlen;
-        DevBuf<uint64_t> d_zoff, d_tot;
-        d_in.ensure(n + 64); d_slots.ensure((size_t)nblk * kBgzfSlot); d_out.ensure((size_t)nblk * kBgzfSlot);
-        d_zlen.ensure(nblk); d_zoff.ensure(nblk); d_tot.ensure(4); d_code.ensure(kBgzfCodeBytes);
+        DevBuf<uint8_t> d_in;
+        DevBuf<uint64_t> d_tot;
+        Bgzf z;
+        d_in.ensure(n + 64); d_tot.ensure(4); z.ensure(nblk, n, 1);
         const uint64_t tot[4] = {n, 0, 0, 0};
         if (n) CK(cudaMemcpyAsync(d_in.p, in, n, cudaMemcpyHostToDevice, d.s_compute));
         CK(cudaMemcpyAsync(d_tot.p, tot, sizeof tot, cudaMemcpyHostToDevice, d.s_compute));
-        CK(launch_bgzf(d_in.p, d_in.p, d_tot.p, nblk, level >= 4, d_slots.p, d_slots.p, d_zlen.p, d_zlen.p, d_zoff.p, d_zoff.p, d_out.p,
-                       d_out.p, d_code.p, d.s_compute));
+        CK(z.launch(d_in.p, d_in.p, d_tot.p, nblk, level, d.s_compute));
         uint64_t back[4];
         CK(cudaMemcpyAsync(back, d_tot.p, sizeof back, cudaMemcpyDeviceToHost, d.s_compute));
         CK(cudaStreamSynchronize(d.s_compute));
         *len = back[2] + sizeof kBgzfEof;
         if (!out) return;
         if (cap < *len) throw ArgErr("output buffer too small");
-        if (back[2]) CK(cudaMemcpy(out, d_out.p, back[2], cudaMemcpyDeviceToHost));
+        if (back[2]) CK(cudaMemcpy(out, z.out[0].p, back[2], cudaMemcpyDeviceToHost));
         std::memcpy(static_cast<uint8_t*>(out) + back[2], kBgzfEof, sizeof kBgzfEof);
     });
 }

@@ -1,5 +1,5 @@
 // Delivery of generated batches to their sink: plain or zlib-compressed files, the caller's memory, or a chunk
-// callback.  Host code only (no CUDA), shared by the Illumina and PacBio drivers.
+// callback.  Host code only (no CUDA), shared by the Illumina, PacBio and VCF drivers.
 #ifndef JLP_OUTPUT_H
 #define JLP_OUTPUT_H
 

@@ -229,3 +229,39 @@ def test_pacbio_callbacks(ctx):
     p.abort_cb = _lib.ABORT_CB(abort)
     assert ctx.lib.jlp_pacbio_to_memory(ctx.h, 0, C.byref(p), None, 0, C.byref(n), C.byref(st)) == _lib.JLP_ERR_ABORTED
     assert seen[0] == 900 + 2 * 200
+
+
+def _c_params(ctx, out_prefix):
+    """jlp_pacbio_params of a small reference run, set up as test_pacbio_callbacks sets them up."""
+    from jackalope_b200.pacbio import _params
+    from oracle.harness_pacbio import DEFAULTS as D
+    g = J.random_genome(2, 40_000, seed=51)
+    ctx.set_genome(g)
+    return _params(g, out_prefix, 900, D["chi2_params_s"], D["chi2_params_n"], D["max_passes"], D["sqrt_params"], D["norm_params"],
+                   D["prob_thresh"], D["ins_prob"], D["del_prob"], D["sub_prob"], D["min_read_length"], D["lognorm_read_length"],
+                   None, 0.0, None, False, 0, "bgzip", 2, 100, 77, 200, "auto")
+
+
+def test_pacbio_rejects_an_unknown_comp_engine(ctx, tmp_path):
+    """comp_engine is checked as for Illumina and VCF: 7 is an argument error, not zlib output."""
+    import ctypes as C
+    from jackalope_b200 import _lib
+    p, keep = _c_params(ctx, str(tmp_path / "pb"))
+    p.compress, p.comp_engine = 6, 7
+    assert ctx.lib.jlp_pacbio(ctx.h, 0, C.byref(p), C.byref(_lib.RunStats())) == _lib.JLP_ERR_ARG
+    assert b"comp_engine" in ctx.lib.jlp_last_error(ctx.h)
+    assert not (tmp_path / "pb_R1.fq.gz").exists()
+
+
+def test_pacbio_bad_shard_leaves_existing_file(ctx, tmp_path):
+    """shard_index >= shard_count is rejected before the job's file is opened (and truncated)."""
+    import ctypes as C
+    from jackalope_b200 import _lib
+    prefix = tmp_path / "pb"
+    p, keep = _c_params(ctx, str(prefix))
+    p.shard_index, p.shard_count = 2, 2
+    old = tmp_path / "pb_R1.fq"
+    old.write_bytes(b"@earlier run\nACGT\n+\nIIII\n")
+    assert ctx.lib.jlp_pacbio(ctx.h, 0, C.byref(p), C.byref(_lib.RunStats())) == _lib.JLP_ERR_ARG
+    assert b"shard_index" in ctx.lib.jlp_last_error(ctx.h)
+    assert old.read_bytes() == b"@earlier run\nACGT\n+\nIIII\n"
