@@ -77,7 +77,7 @@ def oracle_jobs(obj, n_reads, read_length, paired, seed, **kw):
 def oracle_run(obj, n_reads, read_length, paired, seed, lo=None, hi=None, want_ledger=False, hap_seqs=None,
                only_job=None, _jobs_only=False, **kw):
     """Oracle output for the run illumina(obj, ..., seed=seed) performs.
-    Returns dict(r1, r2[, plan, ledger, ledger_cnt, groups]); with sep_files the
+    Returns dict(r1, r2, fallback[, plan, ledger, ledger_cnt, groups]); with sep_files the
     jobs' outputs are concatenated in haplotype order (as sink="memory" does).
     hap_seqs: materialised haplotype chromosomes [h][c], or a callable (h, c) -> bytes asked only for the groups
     the pair range [lo, hi) can touch (runs at sizes where materialising everything on the CPU is out of reach)."""
@@ -140,7 +140,8 @@ def oracle_run(obj, n_reads, read_length, paired, seed, lo=None, hi=None, want_l
         bcs = [p.barcodes[0].decode()] * nc
     groups = H.Groups(counts, seqs, gnames, cnames, bcs, lens=lens)
     cdf = frag_table(p.frag_len_shape, p.frag_len_scale, p.frag_len_min, p.frag_len_max)
-    res = dict(r1=b"", r2=b"", groups=groups, jobs=jobs, params=p, profiles=(prof1, prof2), n_chroms=nc)
+    res = dict(r1=b"", r2=b"", groups=groups, jobs=jobs, params=p, profiles=(prof1, prof2), n_chroms=nc,
+               fallback=dict.fromkeys(H.FALLBACK_KINDS, 0))
     for (jl, jh) in jobs:
         if only_job is not None and (jl, jh) != tuple(only_job):
             continue
@@ -154,6 +155,8 @@ def oracle_run(obj, n_reads, read_length, paired, seed, lo=None, hi=None, want_l
                        lo=a_lo, hi=a_hi, job_lo=jl, job_hi=jh, want_ledger=want_ledger, want_plan=want_ledger)
         res["r1"] += r["r1"]
         res["r2"] += r["r2"]
+        for k, v in r["fallback"].items():
+            res["fallback"][k] += v
         if want_ledger:
             for k in ("plan", "ledger", "ledger_cnt"):
                 res.setdefault(k, []).append(r[k])

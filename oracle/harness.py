@@ -49,10 +49,14 @@ class OrcJob(C.Structure):
         ("group_genome_name", C.POINTER(C.c_char_p)),
         ("group_chrom_name", C.POINTER(C.c_char_p)),
         ("group_barcode", C.POINTER(C.c_char_p)),
+        ("fallback", u64p),
     ]
 
 
 _orc = None
+
+# OrcJob.fallback, in its order: (slot, N quality, substitution index) x (ambiguous, flipped)
+FALLBACK_KINDS = ("slot_ambiguous", "slot_flipped", "nqual_ambiguous", "nqual_flipped", "sub_ambiguous", "sub_flipped")
 
 
 def oracle():
@@ -157,7 +161,8 @@ def generate(*, seed, paired, matepair, groups: Groups, prof1, prof2, ins_prob, 
              prob_dup, pool_pairs, frag_cdf, frag_min, lo=None, hi=None, job_lo=0, job_hi=None,
              want_ledger=False, want_plan=False):
     """Run the oracle for pair instances [lo, hi) of job [job_lo, job_hi).
-    prof1/prof2 are flattened profiles (L, nq, probs, quals)."""
+    prof1/prof2 are flattened profiles (L, nq, probs, quals).  res["fallback"]: the counts of draws that k_reads
+    decides with its exact-draw fallbacks (FALLBACK_KINDS; OrcJob.fallback in jlp_oracle.c)."""
     lib = oracle()
     n_total = int(groups.off[-1])
     job_hi = n_total if job_hi is None else job_hi
@@ -182,6 +187,8 @@ def generate(*, seed, paired, matepair, groups: Groups, prof1, prof2, ins_prob, 
     gn, cn, bc = _strs(groups.genome_names), _strs(groups.chrom_names), _strs(groups.barcodes)
     J.group_seq, J.group_len = seqs, _ptr(glen, u64p)
     J.group_genome_name, J.group_chrom_name, J.group_barcode = gn, cn, bc
+    fallback = np.zeros(len(FALLBACK_KINDS), dtype=np.uint64)
+    J.fallback = _ptr(fallback, u64p)
     max_name = max(len(a) + len(b) for a, b in zip(groups.genome_names, groups.chrom_names)) if ng else 0
     cap = n * (max_name + 32 + 2 * L + 8) + 64
     o1, o2 = C.create_string_buffer(cap), C.create_string_buffer(cap if paired else 1)
@@ -195,7 +202,8 @@ def generate(*, seed, paired, matepair, groups: Groups, prof1, prof2, ins_prob, 
                           _ptr(plan, u64p), _ptr(ledger, u64p), led_cap, C.byref(led_n), _ptr(led_cnt, u64p))
     if rc != 0:
         raise RuntimeError("orc_generate failed rc=%d" % rc)
-    res = dict(r1=o1.raw[:l1.value], r2=o2.raw[:l2.value] if paired else b"")
+    res = dict(r1=o1.raw[:l1.value], r2=o2.raw[:l2.value] if paired else b"",
+               fallback=dict(zip(FALLBACK_KINDS, (int(x) for x in fallback))))
     if want_plan:
         res["plan"] = plan.reshape(-1, 4)[:n]
     if want_ledger:

@@ -302,6 +302,11 @@ typedef struct {
     const char* const* group_genome_name;
     const char* const* group_chrom_name;
     const char* const* group_barcode;
+    /* optional out (NULL: not counted), added to: the draws whose high bits alone leave the answer open in k_reads
+     * (base_fast / base_rare, jackalope_b200/csrc/jlp_kernels.cu), and those where the exact answer differs from the
+     * one the high bits give -- coverage accounting of the kernels' exact-draw fallbacks, never part of the output.
+     * [0] ambiguous / [1] flipped alias slot, [2] / [3] N quality, [4] / [5] substitution index. */
+    uint64_t* fallback;
 } OrcJob;
 
 static uint64_t find_group(const OrcJob* J, uint64_t k) {
@@ -437,6 +442,13 @@ int orc_generate(const OrcJob* J, uint64_t lo, uint64_t hi,
                     uint64_t x = orc_draw_pos(J->seed, j, (uint32_t)i, PU_DIE, (uint32_t)pos);
                     led(&lg, x);
                     qint = (uint8_t)(runif_01(x) * 10 + (uint8_t)'!');
+                    if (J->fallback) {          /* base_rare: u * 10 + 33 on the draw's high 24 bits */
+                        const uint32_t dn = (uint32_t)(x >> 40) << 8;
+                        if (dn * 10u + 2560u < 2560u) {
+                            J->fallback[2]++;
+                            J->fallback[3] += (uint8_t)((uint32_t)(((uint64_t)dn * 10u) >> 32) + 33u) != qint;
+                        }
+                    }
                     qual[pos] = (char)qint;
                     read[pos] = 'N';
                     continue;
@@ -449,6 +461,13 @@ int orc_generate(const OrcJob* J, uint64_t lo, uint64_t hi,
                 led(&lg, xd);
                 uint64_t ii = (uint64_t)(runif_01(xd) * n);
                 if (ii >= n) ii = n - 1;   /* u == 1.0 (x = 2^64-1) reads past the table in the reference: clamp (DESIGN.md) */
+                if (J->fallback) {          /* base_fast / base_rare: the slot from the draw's high 24 bits */
+                    const uint32_t dc = (uint32_t)(xd >> 40) << 8, n32 = (uint32_t)n;
+                    if (dc * n32 + (n32 << 8) < (n32 << 8)) {
+                        J->fallback[0]++;
+                        J->fallback[1] += (uint32_t)(((uint64_t)dc * n32) >> 32) != ii;
+                    }
+                }
                 uint64_t xc = orc_draw_pos(J->seed, j, (uint32_t)i, PU_COIN, (uint32_t)pos);
                 led(&lg, xc);
                 double u = (double)runif_01(xc);
@@ -465,6 +484,13 @@ int orc_generate(const OrcJob* J, uint64_t lo, uint64_t hi,
                     led(&lg, xsub);
                     uint64_t si = (uint64_t)(runif_01(xsub) * 3.0);
                     if (si > 2) si = 2;    /* same 2^-64 edge as above */
+                    if (J->fallback) {      /* base_rare: u * 3 on the draw's high 8 bits */
+                        const uint32_t p3 = (uint32_t)(xsub >> 56) * 3u;
+                        if ((p3 & 0xffu) + 3u > 0xffu) {
+                            J->fallback[4]++;
+                            J->fallback[5] += (p3 >> 8) != si;
+                        }
+                    }
                     read[pos] = MM[nt_ind][si];
                 }
             }
