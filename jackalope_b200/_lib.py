@@ -98,6 +98,20 @@ class IndelStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class GtreeParams(C.Structure):
+    _fields_ = [("text", C.c_char_p), ("text_len", C.c_uint64), ("table_budget", C.c_uint64)]
+
+
+class GtreeStats(C.Structure):
+    _fields_ = [
+        ("n_trees", C.c_uint64), ("n_regions", C.c_uint64), ("windows", C.c_uint64), ("parse_ms", C.c_double),
+        ("table_ms", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 class VcfParams(C.Structure):
     _fields_ = [
         ("path", C.c_char_p), ("n_samples", C.c_uint64), ("ploidy", C.c_uint32), ("sample_haps", u64p),
@@ -120,7 +134,7 @@ class VcfStats(C.Structure):
 # every symbol include/jlp_b200.h declares
 SYMBOLS = [
     "jlp_ctx_create", "jlp_ctx_create_multi", "jlp_ctx_n_devices", "jlp_materialize_haplotypes", "jlp_ctx_destroy", "jlp_last_error", "jlp_set_genome", "jlp_set_genome_async", "jlp_genome_sync", "jlp_create_genome", "jlp_get_genome", "jlp_genome_draw", "jlp_clear_haplotypes",
-    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_get_haplotype_muts", "jlp_write_vcf", "jlp_transition_matrix", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
+    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_create_haplotypes_gtrees", "jlp_get_haplotype_muts", "jlp_write_vcf", "jlp_transition_matrix", "jlp_transition_tables", "jlp_ms_regions", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
     "jlp_illumina_to_memory", "jlp_illumina_stream", "jlp_illumina_device_only", "jlp_illumina_group_counts", "jlp_apportion", "jlp_shard_range", "jlp_deflate", "jlp_bgzf_device", "jlp_pacbio", "jlp_pacbio_to_memory", "jlp_pacbio_read_plan", "jlp_pacbio_sample", "jlp_reads_per_group", "jlp_alias_build",
     "jlp_threshold", "jlp_unif_expr", "jlp_frag_table", "jlp_philox4x32_10", "jlp_draw_pos", "jlp_draw_pair",
     "jlp_version",
@@ -161,6 +175,11 @@ def lib():
     L.jlp_create_haplotypes.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(MutationStats)]
     L.jlp_create_haplotypes_indels.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(IndelParams),
                                                C.POINTER(MutationStats), C.POINTER(IndelStats)]
+    L.jlp_create_haplotypes_gtrees.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(GtreeParams),
+                                               C.POINTER(MutationStats), C.POINTER(GtreeStats)]
+    L.jlp_ms_regions.argtypes = [C.c_char_p, C.c_uint64, u64p, C.c_uint64, pp, C.c_uint32, u64p, C.c_uint64, u64p, u64p,
+                                 C.c_char_p, C.c_uint64]
+    L.jlp_transition_tables.argtypes = [C.c_void_p, f64p, f64p, C.c_uint64, f64p, u64p, u64p]
     L.jlp_get_haplotype_muts.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, u64p, u64p, u64p, C.c_void_p, C.c_uint64,
                                          C.c_uint64, u64p, u64p, u64p]
     L.jlp_write_vcf.argtypes = [C.c_void_p, C.POINTER(VcfParams), C.POINTER(VcfStats)]

@@ -1457,18 +1457,19 @@ int jlp_get_haplotype_muts(jlp_ctx* c, uint64_t hap, uint64_t chrom, uint64_t* o
 
 namespace {
 
-// The visiting order of the tree and the node-state slots (k_mutate): preorder with the child of fewer tips first, a
+// The visiting order of one tree and the node-state slots (k_mutate): preorder with the child of fewer tips first, a
 // parent's slot freed when its last child is visited (before that child takes one), so at most about log2(tips) + 2
-// slots are live.  Childless nodes that are not tips are left out.
-std::vector<MutNode> mut_schedule(const jlp_mutation_params* p, const std::vector<int32_t>& tip_of, uint32_t n_cat,
-                                  uint32_t& max_slots) {
-    const uint32_t n = p->n_nodes;
+// slots are live.  Childless nodes that are not tips are left out.  tab: the node's first row after the tree's.
+std::vector<MutNode> mut_schedule(const GeneTree& T, uint32_t n_cat, uint32_t& max_slots) {
+    const uint32_t n = (uint32_t)T.parent.size();
+    std::vector<int32_t> tip_of(n, -1);
+    for (uint32_t t = 0; t < T.tip_node.size(); t++) tip_of[T.tip_node[t]] = (int32_t)t;
     std::vector<std::vector<uint32_t>> kids(n);
-    for (uint32_t i = 1; i < n; i++) kids[p->parent[i]].push_back(i);
+    for (uint32_t i = 1; i < n; i++) kids[T.parent[i]].push_back(i);
     std::vector<uint64_t> tips(n, 0);
     for (uint32_t i = n; i-- > 0;) {
         if (kids[i].empty()) tips[i] = tip_of[i] >= 0 ? 1 : 0;
-        if (i) tips[p->parent[i]] += tips[i];
+        if (i) tips[T.parent[i]] += tips[i];
     }
     for (auto& k : kids) std::stable_sort(k.begin(), k.end(), [&](uint32_t a, uint32_t b) { return tips[a] < tips[b]; });
     std::vector<uint32_t> left(n), slot(n, 0), free_slots;
@@ -1480,7 +1481,7 @@ std::vector<MutNode> mut_schedule(const jlp_mutation_params* p, const std::vecto
     while (!stack.empty()) {
         const uint32_t v = stack.back();
         stack.pop_back();
-        const uint32_t par = (uint32_t)p->parent[v];
+        const uint32_t par = (uint32_t)T.parent[v];
         MutNode m;
         m.node = v;
         m.tab = v * n_cat * 4;
@@ -1508,13 +1509,59 @@ struct EventSet {
     float ms(int a, int b) const { float t = 0; cudaEventElapsedTime(&t, e[a], e[b]); return t; }
 };
 
-}  // namespace
+constexpr uint64_t kTableBudget = 1ull << 30;       // default bytes of threshold tables per window
 
-// The whole call; im == nullptr: substitutions only, otherwise the indel model (ins_pi: the inserted columns' birth
-// distribution) and its stats.
-static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelModel* im, const double* ins_pi,
-                        jlp_mutation_stats* stats, jlp_indel_stats* istats) {
-    const auto t0 = std::chrono::steady_clock::now();
+// Device buffers of the threshold tables: the items of a window, the flagged items, the tables.
+struct TableBufs {
+    DevBuf<TabItem> items;
+    DevBuf<uint32_t> flag;
+    std::vector<uint32_t> h_flag;
+    std::vector<uint4> h_rows;
+};
+
+// The tables of `items` built on the device (k_mut_tables); the items it flags are recomputed here with the host's
+// transition_matrix + row_thresholds and copied over theirs (and over P_out's, when given).  Returns their count.
+uint64_t device_tables(cudaStream_t s, const double Q[16], const std::vector<TabItem>& items, TableBufs& B, uint4* hi,
+                       uint4* lo, double* P_out) {
+    if (items.empty()) return 0;
+    if (items.size() >> 32) throw ArgErr("2^32 or more transition matrices in one window");
+    TabQ q;
+    std::memcpy(q.q, Q, sizeof q.q);
+    B.items.upload(items, s);
+    B.flag.ensure(items.size() + 1);
+    CK(cudaMemsetAsync(B.flag.p, 0, 4, s));
+    CK(launch_mut_tables(B.items.p, (uint32_t)items.size(), q, hi, lo, P_out, B.flag.p, B.flag.p + 1, s));
+    uint32_t nf = 0;
+    CK(cudaMemcpyAsync(&nf, B.flag.p, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (nf == 0) return 0;
+    B.h_flag.resize(nf);
+    CK(cudaMemcpyAsync(B.h_flag.data(), B.flag.p + 1, (size_t)nf * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    B.h_rows.resize((size_t)nf * 8);
+    std::vector<double> Ps(P_out ? (size_t)nf * 16 : 0);
+    for (uint32_t f = 0; f < nf; f++) {
+        const TabItem& it = items[B.h_flag[f]];
+        double P[16];
+        transition_matrix(Q, it.t, P);
+        if (P_out) std::memcpy(&Ps[16 * (size_t)f], P, sizeof P);
+        for (uint32_t a = 0; a < 4; a++) {
+            uint64_t t[3];
+            row_thresholds(P + 4 * a, t);
+            B.h_rows[8 * (size_t)f + a] = make_uint4((uint32_t)(t[0] >> 32), (uint32_t)(t[1] >> 32), (uint32_t)(t[2] >> 32), 0);
+            B.h_rows[8 * (size_t)f + 4 + a] = make_uint4((uint32_t)t[0], (uint32_t)t[1], (uint32_t)t[2], 0);
+        }
+        CK(cudaMemcpyAsync(hi + it.row, &B.h_rows[8 * (size_t)f], 4 * sizeof(uint4), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(lo + it.row, &B.h_rows[8 * (size_t)f + 4], 4 * sizeof(uint4), cudaMemcpyHostToDevice, s));
+        if (P_out)
+            CK(cudaMemcpyAsync(P_out + 16 * (size_t)B.h_flag[f], &Ps[16 * (size_t)f], 16 * sizeof(double),
+                               cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaStreamSynchronize(s));
+    return nf;
+}
+
+void check_model(const jlp_ctx* c, const jlp_mutation_params* p) {
     if (c->chrom_off.size() < 2) throw ArgErr("set the reference genome first");
     for (int i = 0; i < 16; i++)
         if (i % 5 && !(std::isfinite(p->Q[i]) && p->Q[i] >= 0)) throw ArgErr("the off-diagonal rates of Q must be finite and >= 0");
@@ -1522,6 +1569,15 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     if (p->n_rates < 1 || p->n_rates > 255 || !p->rates) throw ArgErr("n_rates must be 1..255 (rates not NULL)");
     for (uint32_t k = 0; k < p->n_rates; k++)
         if (!(std::isfinite(p->rates[k]) && p->rates[k] >= 0)) throw ArgErr("category rates must be finite and >= 0");
+    if (p->n_tips < 1 || p->n_tips > kMutMaxTips)
+        throw ArgErr("a tree of " + std::to_string(p->n_tips) + " tips: 1 to " + std::to_string(kMutMaxTips) + " tips are supported");
+    if (!p->tip_names) throw ArgErr("tip_node / tip_names is NULL");
+    for (uint32_t t = 0; t < p->n_tips; t++)
+        if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
+}
+
+// the tree of p as the one tree of the genome: one region per (non-empty) chromosome
+GeneTrees one_tree(const jlp_ctx* c, const jlp_mutation_params* p) {
     const uint32_t n = p->n_nodes;
     if (n < 2 || n > kMutMaxNodes || !p->parent || !p->branch_len)
         throw ArgErr("the tree needs 2 to " + std::to_string(kMutMaxNodes) + " nodes (parent / branch_len not NULL)");
@@ -1532,27 +1588,109 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         if (!(std::isfinite(p->branch_len[i]) && p->branch_len[i] >= 0)) throw ArgErr("branch lengths must be finite and >= 0");
         has_kid[p->parent[i]] = 1;
     }
-    if (p->n_tips < 1 || p->n_tips > kMutMaxTips)
-        throw ArgErr("a tree of " + std::to_string(p->n_tips) + " tips: 1 to " + std::to_string(kMutMaxTips) + " tips are supported");
-    if (!p->tip_node || !p->tip_names) throw ArgErr("tip_node / tip_names is NULL");
-    std::vector<int32_t> tip_of(n, -1);
+    if (!p->tip_node) throw ArgErr("tip_node / tip_names is NULL");
+    std::vector<char> is_tip(n, 0);
     for (uint32_t t = 0; t < p->n_tips; t++) {
         const uint32_t v = p->tip_node[t];
-        if (v >= n || has_kid[v] || tip_of[v] >= 0) throw ArgErr("tip_node must list distinct childless nodes");
-        if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
-        tip_of[v] = (int32_t)t;
+        if (v >= n || has_kid[v] || is_tip[v]) throw ArgErr("tip_node must list distinct childless nodes");
+        is_tip[v] = 1;
     }
+    GeneTrees g;
+    g.trees.resize(1);
+    g.trees[0].parent.assign(p->parent, p->parent + n);
+    g.trees[0].branch_len.assign(p->branch_len, p->branch_len + n);
+    g.trees[0].tip_node.assign(p->tip_node, p->tip_node + p->n_tips);
     const uint64_t nc = c->chrom_off.size() - 1;
-    std::vector<uint32_t> tile0(nc + 1, 0);
+    g.regions.resize(nc);
     for (uint64_t ci = 0; ci < nc; ci++) {
         const uint64_t len = c->chrom_off[ci + 1] - c->chrom_off[ci];
         if (len >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
-        const uint64_t t = tile0[ci] + (len + kMutTile - 1) / kMutTile;
-        if (t >> 32) throw ArgErr("genome too large");
-        tile0[ci + 1] = (uint32_t)t;
+        if (len) g.regions[ci].push_back(TreeRegion{0, (uint32_t)len, 0});
     }
-    const uint32_t K = p->n_rates, n_tips = p->n_tips, n_tiles = tile0[nc];
+    return g;
+}
+
+unsigned host_threads(uint64_t items) {
+    return (unsigned)std::min<uint64_t>(std::min<uint64_t>(items, 16), std::max(1u, std::thread::hardware_concurrency()));
+}
+
+}  // namespace
+
+// The whole call: the trees and every chromosome's regions (one tree for the genome: one region per chromosome);
+// im == nullptr: substitutions only, otherwise the indel model (ins_pi: the inserted columns' birth distribution) and
+// its stats (one tree only).  table_budget: bytes of threshold tables per window (0: the default).
+static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const GeneTrees& G, uint64_t table_budget,
+                        const IndelModel* im, const double* ins_pi, jlp_mutation_stats* stats, jlp_indel_stats* istats,
+                        jlp_gtree_stats* gstats) {
+    const auto t0 = std::chrono::steady_clock::now();
+    const uint32_t n = p->n_nodes;           // the one tree's nodes (indels only)
+    const uint64_t nc = c->chrom_off.size() - 1;
+    const uint32_t K = p->n_rates, n_tips = p->n_tips;
     const size_t n_items = (size_t)n_tips * nc;
+    const uint64_t n_trees = G.trees.size();
+
+    // the trees' schedules, one after the other (trees no region uses get none)
+    std::vector<char> used(n_trees, 0);
+    for (const auto& rs : G.regions)
+        for (const TreeRegion& r : rs) used[r.tree] = 1;
+    std::vector<std::vector<MutNode>> scheds(n_trees);
+    std::vector<uint32_t> slots(n_trees, 0);
+    parallel_for(n_trees, host_threads(n_trees / 64 + 1), [&](uint64_t i) {
+        if (used[i]) scheds[i] = mut_schedule(G.trees[i], K, slots[i]);
+    });
+    std::vector<uint64_t> sched0(n_trees + 1, 0);
+    for (uint64_t i = 0; i < n_trees; i++) sched0[i + 1] = sched0[i] + scheds[i].size();
+    if (sched0[n_trees] >> 32) throw ArgErr("2^32 or more tree nodes in all");
+    std::vector<MutNode> sched(sched0[n_trees]);
+    for (uint64_t i = 0; i < n_trees; i++) std::copy(scheds[i].begin(), scheds[i].end(), sched.begin() + sched0[i]);
+    const uint32_t max_slots = n_trees ? *std::max_element(slots.begin(), slots.end()) : 0;
+
+    // tiles: per region from its start rounded down to a multiple of 4, kMutTile sites apart
+    std::vector<uint32_t> tile0(nc + 1, 0);
+    std::vector<MutTile> tiles;
+    std::vector<uint32_t> tile_tree;
+    for (uint64_t ci = 0; ci < nc; ci++) {
+        tile0[ci] = (uint32_t)tiles.size();
+        for (const TreeRegion& r : G.regions[ci])
+            for (uint64_t f = r.start & ~3u; f < r.end; f += kMutTile) {
+                tiles.push_back(MutTile{(uint32_t)ci, (uint32_t)f, r.start, r.end, (uint32_t)sched0[r.tree],
+                                        (uint32_t)(sched0[r.tree + 1] - sched0[r.tree]), 0, 0});
+                tile_tree.push_back(r.tree);
+            }
+        if (tiles.size() >> 32) throw ArgErr("genome too large");
+    }
+    tile0[nc] = (uint32_t)tiles.size();
+    const uint32_t n_tiles = tile0[nc];
+
+    // windows: contiguous tile ranges whose trees' tables fit the budget (a window holds at least one tree)
+    struct Window { uint32_t t0, t1; uint64_t rows; std::vector<uint32_t> trees; };
+    std::vector<Window> win;
+    {
+        const uint64_t budget = table_budget ? table_budget : kTableBudget;
+        const uint64_t max_rows = std::min<uint64_t>(budget / (2 * sizeof(uint4)), 1ull << 31);
+        std::vector<uint64_t> stamp(n_trees, UINT64_MAX), base(n_trees, 0);
+        for (uint32_t tl = 0; tl < n_tiles; tl++) {
+            const uint32_t tr = tile_tree[tl];
+            if (win.empty() || stamp[tr] != win.size() - 1) {
+                const uint64_t rows = (uint64_t)G.trees[tr].parent.size() * K * 4;
+                if (win.empty() || (win.back().rows && win.back().rows + rows > max_rows)) {
+                    if (!win.empty()) win.back().t1 = tl;
+                    win.push_back(Window{tl, tl, 0, {}});
+                }
+                stamp[tr] = win.size() - 1;
+                base[tr] = win.back().rows;
+                win.back().rows += rows;
+                win.back().trees.push_back(tr);
+            }
+            tiles[tl].tab0 = (uint32_t)base[tr];
+        }
+        if (!win.empty()) win.back().t1 = n_tiles;
+    }
+    uint64_t max_win_rows = 0, table_bytes = 0;
+    for (const Window& w : win) {
+        max_win_rows = std::max(max_win_rows, w.rows);
+        table_bytes += w.rows * 2 * sizeof(uint4);
+    }
 
     // indels: the event pass, chromosomes on up to 16 host threads; then the tips' records in one array (region
     // tip * nc + chromosome), each tile's first record, and the inserted columns with their places in the pools
@@ -1560,11 +1698,12 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     std::vector<IndelRec> irec;
     std::vector<uint64_t> ir_start;
     std::vector<uint32_t> icur;
+    std::vector<int32_t> tip_of(im ? n : 0, -1);
     double event_ms = 0;
     if (im) {
+        for (uint32_t t = 0; t < n_tips; t++) tip_of[p->tip_node[t]] = (int32_t)t;
         const auto te = std::chrono::steady_clock::now();
-        const unsigned nt = (unsigned)std::min<uint64_t>(std::min<uint64_t>(nc, 16), std::max(1u, std::thread::hardware_concurrency()));
-        parallel_for(nc, nt, [&](uint64_t ci) {
+        parallel_for(nc, host_threads(nc), [&](uint64_t ci) {
             indel_events(p->seed, (uint32_t)ci, c->chrom_off[ci + 1] - c->chrom_off[ci], n, p->parent, p->branch_len,
                          tip_of.data(), n_tips, *im, ich[ci]);
         });
@@ -1581,17 +1720,13 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
             const uint64_t ci = r % nc;
             uint64_t j = ir_start[r];
             for (uint32_t tl = tile0[ci]; tl < tile0[ci + 1]; tl++) {
-                const uint64_t start = (uint64_t)(tl - tile0[ci]) * kMutTile;
-                while (j < ir_start[r + 1] && irec[j].old_pos < start) j++;
+                while (j < ir_start[r + 1] && irec[j].old_pos < tiles[tl].first) j++;
                 icur[(r / nc) * n_tiles + tl] = (uint32_t)j;
             }
         }
         event_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - te).count();
     }
 
-    // host tables: the schedule, per (node, category, parent state) the row thresholds, the category thresholds
-    uint32_t max_slots = 0;
-    const std::vector<MutNode> sched = mut_schedule(p, tip_of, K, max_slots);
     // the inserted columns: birth node -> its schedule index and the end of its subtree's interval; per column the
     // (tip, record, byte) it fills, tips in schedule order
     std::vector<InsCol> cols;
@@ -1641,20 +1776,6 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
             }
         }
     }
-    const uint64_t rows = (uint64_t)n * K * 4;
-    std::vector<uint4> thr_hi(rows, make_uint4(0, 0, 0, 0)), thr_lo(rows, make_uint4(0, 0, 0, 0));
-    for (const MutNode& m : sched)
-        for (uint32_t k = 0; k < K; k++) {
-            double P[16];
-            transition_matrix(p->Q, p->rates[k] * p->branch_len[m.node], P);
-            for (uint32_t a = 0; a < 4; a++) {
-                uint64_t t[3];
-                row_thresholds(P + 4 * a, t);
-                const uint64_t r = m.tab + 4ull * k + a;
-                thr_hi[r] = make_uint4((uint32_t)(t[0] >> 32), (uint32_t)(t[1] >> 32), (uint32_t)(t[2] >> 32), 0);
-                thr_lo[r] = make_uint4((uint32_t)t[0], (uint32_t)t[1], (uint32_t)t[2], 0);
-            }
-        }
     std::vector<uint64_t> cat_thr(K);
     cat_thr[0] = prob_threshold(p->invariant);
     for (uint32_t j = 1; j < K; j++) cat_thr[j] = prob_threshold(p->invariant + j * (1 - p->invariant) / K);
@@ -1664,17 +1785,24 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     cudaStream_t s = d.s_compute;
     DevBuf<uint64_t> d_off, d_cat, d_region, d_region_n, d_out, d_ir_start, d_ir_nuc;
     DevBuf<uint32_t> d_tile0, d_cnt, d_icur;
+    DevBuf<MutTile> d_tiles;
     DevBuf<IndelRec> d_irec;
     DevBuf<InsCol> d_cols;
     DevBuf<InsEnt> d_ents;
     DevBuf<MutNode> d_sched;
     DevBuf<uint4> d_hi, d_lo;
+    TableBufs tb;
     d_off.upload(c->chrom_off, s);
     d_tile0.upload(tile0, s);
+    d_tiles.upload(tiles, s);
     d_sched.upload(sched, s);
     d_cat.upload(cat_thr, s);
-    d_hi.upload(thr_hi, s);
-    d_lo.upload(thr_lo, s);
+    d_hi.ensure(max_win_rows);
+    d_lo.ensure(max_win_rows);
+    if (max_win_rows) {                      // rows no node uses (the root's) are staged too: defined, never read
+        CK(cudaMemsetAsync(d_hi.p, 0, max_win_rows * sizeof(uint4), s));
+        CK(cudaMemsetAsync(d_lo.p, 0, max_win_rows * sizeof(uint4), s));
+    }
     const size_t n_cnt = (size_t)n_tips * n_tiles;
     d_cnt.ensure(n_cnt);
     if (n_cnt) CK(cudaMemsetAsync(d_cnt.p, 0, n_cnt * 4, s));
@@ -1684,13 +1812,12 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     mp.genome = d.genome.p + kPad;
     mp.chrom_off = d_off.p;
     mp.tile0 = d_tile0.p;
+    mp.tiles = d_tiles.p;
     mp.n_chroms = (uint32_t)nc; mp.n_tiles = n_tiles; mp.n_tips = n_tips; mp.n_sched = (uint32_t)sched.size();
     mp.sched = d_sched.p;
     mp.n_cat = K;
     mp.cat_thr = d_cat.p;
     mp.thr_hi = d_hi.p; mp.thr_lo = d_lo.p;
-    mp.tab_rows = (uint32_t)rows;
-    mp.tab_smem = mut_smem_bytes((uint32_t)rows) <= (64u << 10);
     mp.cnt = d_cnt.p;
     if (im) {
         d_irec.upload(irec, s);
@@ -1699,15 +1826,49 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         d_ir_nuc.ensure(irec.size());
         mp.irec = d_irec.p; mp.ir_start = d_ir_start.p; mp.icur = d_icur.p; mp.ir_nuc = d_ir_nuc.p;
     }
+
+    // a window's tables: one item per (tree, scheduled node, category)
+    double table_ms = 0;
+    std::vector<TabItem> titems;
+    auto build_tables = [&](const Window& w) {
+        const auto tt = std::chrono::steady_clock::now();
+        titems.clear();
+        uint64_t base = 0;
+        for (uint32_t tr : w.trees) {
+            const double* bl = G.trees[tr].branch_len.data();
+            for (const MutNode& m : scheds[tr])
+                for (uint32_t k = 0; k < K; k++)
+                    titems.push_back(TabItem{p->rates[k] * bl[m.node], (uint32_t)(base + m.tab + 4ull * k), 0});
+            base += (uint64_t)G.trees[tr].parent.size() * K * 4;
+        }
+        device_tables(s, p->Q, titems, tb, d_hi.p, d_lo.p, nullptr);
+        table_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tt).count();
+    };
+    bool all_smem = true;
+    auto set_window = [&](const Window& w) {
+        mp.tile_begin = w.t0; mp.tile_end = w.t1;
+        mp.tab_rows = (uint32_t)w.rows;
+        mp.tab_smem = w.trees.size() == 1 && mut_smem_bytes((uint32_t)w.rows) <= (64u << 10);
+        all_smem &= mp.tab_smem != 0;
+    };
     EventSet ev;
-    CK(cudaEventRecord(ev.e[0], s));
-    CK(launch_mutate(mp, false, im != nullptr, s));
+    float count_ms = 0, write_ms = 0;
+    for (const Window& w : win) {
+        build_tables(w);
+        set_window(w);
+        CK(cudaEventRecord(ev.e[0], s));
+        CK(launch_mutate(mp, false, im != nullptr, gstats != nullptr, s));
+        CK(cudaEventRecord(ev.e[1], s));
+        CK(cudaEventSynchronize(ev.e[1]));
+        count_ms += ev.ms(0, 1);
+    }
     CK(cudaEventRecord(ev.e[1], s));
     CK(launch_mut_scan(mp, d_region_n.p, s));
     CK(cudaEventRecord(ev.e[2], s));
     std::vector<uint64_t> region_n((size_t)n_tips * nc), region((size_t)n_tips * nc);
     CK(cudaMemcpyAsync(region_n.data(), d_region_n.p, region_n.size() * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
+    const float scan_ms = ev.ms(1, 2);
     // with indels region_n becomes substitution + indel records, pool the substitutions' bytes + the indel records'
     std::vector<uint64_t> pool(region_n);
     if (im)
@@ -1732,9 +1893,17 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
     d_out.ensure(words);
     if (words) CK(cudaMemsetAsync(d_out.p, 0, words * 8, s));
     mp.out = d_out.p;
-    CK(cudaEventRecord(ev.e[3], s));
-    if (records) CK(launch_mutate(mp, true, im != nullptr, s));
-    if (im && !cols.empty()) {
+    if (records)
+        for (const Window& w : win) {
+            if (win.size() > 1) build_tables(w);
+            set_window(w);
+            CK(cudaEventRecord(ev.e[3], s));
+            CK(launch_mutate(mp, true, im != nullptr, gstats != nullptr, s));
+            CK(cudaEventRecord(ev.e[4], s));
+            CK(cudaEventSynchronize(ev.e[4]));
+            write_ms += ev.ms(3, 4);
+        }
+    if (im && !cols.empty()) {               // one tree: one window, whose tables are still in place
         d_cols.upload(cols, s);
         d_ents.upload(ents, s);
         InsParams ip{};
@@ -1746,11 +1915,13 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         row_thresholds(ins_pi, ip.pi_thr);
         ip.thr_hi = d_hi.p; ip.thr_lo = d_lo.p;
         ip.out = d_out.p; ip.region = d_region.p; ip.region_n = d_region_n.p; ip.ir_nuc = d_ir_nuc.p;
+        CK(cudaEventRecord(ev.e[3], s));
         CK(launch_ins_walk(ip, s));
+        CK(cudaEventRecord(ev.e[4], s));
+        CK(cudaEventSynchronize(ev.e[4]));
+        write_ms += ev.ms(3, 4);
     }
-    CK(cudaEventRecord(ev.e[4], s));
     CK(cudaStreamSynchronize(s));
-    const float count_ms = ev.ms(0, 1), scan_ms = ev.ms(1, 2), write_ms = ev.ms(3, 4);
     const auto t_gen = std::chrono::steady_clock::now();
 
     // the records into one HapStore per tip, copied straight into the packed arrays by a few host threads
@@ -1760,8 +1931,7 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         stores[t]->name = p->tip_names[t];
         stores[t]->chrom.resize(nc);
     }
-    const unsigned nt = records < (1u << 16) ? 1u
-                        : (unsigned)std::min<uint64_t>(std::min<uint64_t>(n_items, 16), std::max(1u, std::thread::hardware_concurrency()));
+    const unsigned nt = records < (1u << 16) ? 1u : host_threads(n_items);
     parallel_for(n_items, nt, [&](uint64_t r) {
         HapChromHost& H = stores[r / nc]->chrom[r % nc];
         const uint64_t M = region_n[r];
@@ -1785,8 +1955,8 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         stats->total_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
         stats->records = records;
         stats->d2h_bytes = words * 8;
-        stats->table_bytes = rows * 2 * sizeof(uint4);
-        stats->table_in_smem = (int)mp.tab_smem;
+        stats->table_bytes = table_bytes;
+        stats->table_in_smem = (int)(all_smem && !win.empty());
         stats->max_slots = max_slots;
     }
     if (istats) {
@@ -1800,11 +1970,21 @@ static void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelMod
         istats->indel_records = irec.size();
         istats->event_ms = event_ms;
     }
+    if (gstats) {
+        gstats->n_trees = n_trees;
+        gstats->n_regions = 0;
+        for (const auto& rs : G.regions) gstats->n_regions += rs.size();
+        gstats->windows = win.size();
+        gstats->table_ms = table_ms;
+    }
 }
 
 int jlp_create_haplotypes(jlp_ctx* c, const jlp_mutation_params* p, jlp_mutation_stats* stats) {
     if (!c || !p) return JLP_ERR_ARG;
-    return guarded(c, [&]() { create_haps(c, p, nullptr, nullptr, stats, nullptr); });
+    return guarded(c, [&]() {
+        check_model(c, p);
+        create_haps(c, p, one_tree(c, p), 0, nullptr, nullptr, stats, nullptr, nullptr);
+    });
 }
 
 int jlp_create_haplotypes_indels(jlp_ctx* c, const jlp_mutation_params* p, const jlp_indel_params* ip,
@@ -1815,7 +1995,8 @@ int jlp_create_haplotypes_indels(jlp_ctx* c, const jlp_mutation_params* p, const
         if (!rate_ok(ip->rate_ins) || !rate_ok(ip->rate_del)) throw ArgErr("indel rates must be finite and >= 0");
         const double R = ip->rate_ins + ip->rate_del;
         if (R == 0) {
-            create_haps(c, p, nullptr, nullptr, stats, nullptr);
+            check_model(c, p);
+            create_haps(c, p, one_tree(c, p), 0, nullptr, nullptr, stats, nullptr, nullptr);
             if (istats) *istats = jlp_indel_stats{};
             return;
         }
@@ -1845,7 +2026,88 @@ int jlp_create_haplotypes_indels(jlp_ctx* c, const jlp_mutation_params* p, const
         im.rate_ins = ip->rate_ins; im.rate_del = ip->rate_del; im.epsilon = ip->epsilon;
         im.n_ins = n_ins;
         im.kl_thr = indel_thresholds(ip->rate_ins, ip->w_ins, n_ins, ip->rate_del, ip->w_del, n_del);
-        create_haps(c, p, &im, ip->pi, stats, istats);
+        check_model(c, p);
+        create_haps(c, p, one_tree(c, p), 0, &im, ip->pi, stats, istats, nullptr);
+    });
+}
+
+int jlp_create_haplotypes_gtrees(jlp_ctx* c, const jlp_mutation_params* p, const jlp_gtree_params* g,
+                                 jlp_mutation_stats* stats, jlp_gtree_stats* gstats) {
+    if (!c || !p || !g) return JLP_ERR_ARG;
+    return guarded(c, [&]() {
+        check_model(c, p);
+        if (p->n_nodes || p->parent || p->branch_len || p->tip_node)
+            throw ArgErr("with gene trees the trees come from the ms text: n_nodes, parent, branch_len and tip_node must be 0 / NULL");
+        if (!g->text && g->text_len) throw ArgErr("the ms text is NULL");
+        const uint64_t nc = c->chrom_off.size() - 1;
+        std::vector<uint64_t> len(nc);
+        for (uint64_t ci = 0; ci < nc; ci++) {
+            len[ci] = c->chrom_off[ci + 1] - c->chrom_off[ci];
+            if (len[ci] >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
+        }
+        const auto t0 = std::chrono::steady_clock::now();
+        GeneTrees G;
+        parse_ms(g->text, g->text_len, len, p->tip_names, p->n_tips, kMutMaxNodes,
+                 std::max(1u, std::thread::hardware_concurrency()), G);
+        const double parse_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        jlp_gtree_stats gs{};
+        create_haps(c, p, G, g->table_budget, nullptr, nullptr, stats, nullptr, &gs);
+        gs.parse_ms = parse_ms;
+        if (stats) stats->total_ms += parse_ms;
+        if (gstats) *gstats = gs;
+    });
+}
+
+int jlp_ms_regions(const char* text, uint64_t text_len, const uint64_t* chrom_len, uint64_t n_chroms,
+                   const char* const* tip_names, uint32_t n_tips, uint64_t* reg, uint64_t cap, uint64_t* n_regions,
+                   uint64_t* n_trees, char* err, uint64_t err_cap) {
+    try {
+        if ((!text && text_len) || (!chrom_len && n_chroms) || (!tip_names && n_tips)) throw ArgErr("NULL argument");
+        GeneTrees G;
+        parse_ms(text, text_len, std::vector<uint64_t>(chrom_len, chrom_len + n_chroms), tip_names, n_tips, kMutMaxNodes,
+                 std::max(1u, std::thread::hardware_concurrency()), G);
+        uint64_t k = 0;
+        for (uint64_t ci = 0; ci < n_chroms; ci++)
+            for (const TreeRegion& r : G.regions[ci]) {
+                if (reg && k < cap) { reg[4 * k] = ci; reg[4 * k + 1] = r.start; reg[4 * k + 2] = r.end; reg[4 * k + 3] = r.tree; }
+                k++;
+            }
+        if (n_regions) *n_regions = k;
+        if (n_trees) *n_trees = G.trees.size();
+        return JLP_OK;
+    } catch (const std::exception& e) {
+        if (err && err_cap) { std::strncpy(err, e.what(), err_cap - 1); err[err_cap - 1] = 0; }
+        return JLP_ERR_ARG;
+    }
+}
+
+int jlp_transition_tables(jlp_ctx* c, const double Q[16], const double* t, uint64_t n, double* P, uint64_t* thr,
+                          uint64_t* n_host) {
+    if (!c || !Q || (n && (!t || !P || !thr))) return JLP_ERR_ARG;
+    return guarded(c, [&]() {
+        if (n >> 28) throw ArgErr("n must be below 2^28");
+        std::vector<TabItem> items(n);
+        for (uint64_t i = 0; i < n; i++) items[i] = TabItem{t[i], (uint32_t)(4 * i), 0};
+        Device& d = device0(c);
+        cudaStream_t s = d.s_compute;
+        DevBuf<uint4> hi, lo;
+        DevBuf<double> dP;
+        TableBufs tb;
+        hi.ensure(4 * n); lo.ensure(4 * n); dP.ensure(16 * n);
+        const uint64_t nh = device_tables(s, Q, items, tb, hi.p, lo.p, dP.p);
+        std::vector<uint4> h(4 * n), l(4 * n);
+        if (n) {
+            CK(cudaMemcpyAsync(h.data(), hi.p, 4 * n * sizeof(uint4), cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(l.data(), lo.p, 4 * n * sizeof(uint4), cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(P, dP.p, 16 * n * sizeof(double), cudaMemcpyDeviceToHost, s));
+        }
+        CK(cudaStreamSynchronize(s));
+        for (uint64_t r = 0; r < 4 * n; r++) {
+            thr[3 * r] = (uint64_t)h[r].x << 32 | l[r].x;
+            thr[3 * r + 1] = (uint64_t)h[r].y << 32 | l[r].y;
+            thr[3 * r + 2] = (uint64_t)h[r].z << 32 | l[r].z;
+        }
+        if (n_host) *n_host = nh;
     });
 }
 

@@ -109,6 +109,24 @@ uint64_t prob_threshold(double c);
 // and renormalised, thr[j] = prob_threshold(p[0] + ... + p[j])
 void row_thresholds(const double* row, uint64_t thr[3]);
 
+// --- gene trees (create_haplotypes along ms output, jlp_gtrees.cpp) ---------------------
+struct GeneTree {                       // a tree in preorder, nodes numbered as parse_newick numbers them
+    std::vector<int32_t> parent;        // parent[0] = -1, parent[i] < i
+    std::vector<double> branch_len;
+    std::vector<uint32_t> tip_node;     // [n_tips]: the node of haplotype i
+};
+struct TreeRegion {                     // sites [start, end) of a chromosome follow trees[tree]
+    uint32_t start, end, tree;
+};
+struct GeneTrees {
+    std::vector<GeneTree> trees;
+    std::vector<std::vector<TreeRegion>> regions;   // per chromosome, in position order, none empty
+};
+// ms-format text (DESIGN.md section 10, "Gene trees") -> its trees and each chromosome's regions; tip labels are matched
+// to tip_names.  Trees are parsed on up to n_threads threads.  Throws std::runtime_error naming the problem.
+void parse_ms(const char* text, uint64_t len, const std::vector<uint64_t>& chrom_len, const char* const* tip_names,
+              uint32_t n_tips, uint32_t max_nodes, unsigned n_threads, GeneTrees& out);
+
 // --- insertions and deletions along the tree (create_haplotypes, jlp_indel.cpp) --------
 // One insertion or deletion record of a (tip, chromosome) in HapChromHost::packed terms (DESIGN.md section 10).
 struct IndelRec {

@@ -109,11 +109,22 @@ constexpr uint32_t kMutMaxNodes = 65536;
 struct IndelRec;          // jlp_host.h
 
 struct MutNode {          // a non-root node in visiting order
-    uint32_t node;        // index in the caller's preorder: addresses the draws
-    uint32_t tab;         // its first threshold row: row = tab + 4 * category + parent state
+    uint32_t node;        // index in its tree's preorder: addresses the draws
+    uint32_t tab;         // its first threshold row after the tree's: row = tab0 + tab + 4 * category + parent state
     int32_t tip;          // tip index, or -1 for an internal node
     uint16_t pslot;       // slot holding the parent's states
     uint16_t slot;        // slot receiving this node's states (internal nodes)
+};
+
+// A tile lies in one region (a run of sites that follows one tree): it starts at a multiple of 4 (one Philox block per
+// lane and step) and decides only the sites in [lo, hi), the region.  A chromosome's tiles are contiguous and in
+// position order.
+struct MutTile {
+    uint32_t chrom, first;       // chromosome, first site (a multiple of 4)
+    uint32_t lo, hi;             // the region
+    uint32_t sched0, n_sched;    // the region's tree: its schedule entries
+    uint32_t tab0;               // the tree's first threshold row in its window's tables
+    uint32_t pad;
 };
 
 struct MutParams {
@@ -121,11 +132,14 @@ struct MutParams {
     const uint8_t* genome;       // reference bases; chromosome c at chrom_off[c]
     const uint64_t* chrom_off;   // [n_chroms + 1]
     const uint32_t* tile0;       // [n_chroms + 1] first tile of each chromosome
-    uint32_t n_chroms, n_tiles, n_tips, n_sched;
-    const MutNode* sched;        // [n_sched]
+    const MutTile* tiles;        // [n_tiles] (gene trees)
+    uint32_t n_chroms, n_tiles, n_tips;
+    uint32_t n_sched;            // one tree: its schedule entries
+    uint32_t tile_begin, tile_end;   // the window: the tiles a launch covers
+    const MutNode* sched;        // every tree's schedule, one after the other
     uint32_t n_cat;              // rate categories of the variable sites
     const uint64_t* cat_thr;     // [n_cat]: index = #{j : X_cat >= cat_thr[j]}; 0 = invariant, k = category k - 1
-    const uint4* thr_hi;         // [rows] high words of the three thresholds of a row (.w unused)
+    const uint4* thr_hi;         // [rows] the window's tables: high words of the three thresholds of a row (.w unused)
     const uint4* thr_lo;         // [rows] low words
     uint32_t tab_rows;
     uint32_t tab_smem;           // 1: stage thr_hi in shared memory (thr_lo, read only on ties, stays in global memory)
@@ -141,7 +155,8 @@ struct MutParams {
 };
 // pass 1 (write = false): records per (tip, tile) added into cnt; pass 2 (write = true): records written.
 // indels: the tips' records follow p.irec (substitutions at live, non-anchor columns; the indel records themselves)
-cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, cudaStream_t s);
+// gtrees: each tile's region, schedule and table rows from p.tiles; otherwise one tree, one region per chromosome
+cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, bool gtrees, cudaStream_t s);
 
 // The inserted columns' walk: one thread per column from its birth node through the schedule interval of its subtree
 // (state at birth drawn from pi, then the same P rows as a reference site); its tip states go into the insertion
@@ -175,6 +190,20 @@ cudaError_t launch_ins_walk(const InsParams& p, cudaStream_t s);
 // exclusive scan of every (tip, chromosome) run of cnt in place; region_n receives the totals
 cudaError_t launch_mut_scan(const MutParams& p, uint64_t* region_n, cudaStream_t s);
 size_t mut_smem_bytes(uint32_t tab_rows);
+
+// The threshold tables on the device (k_mut_tables): per item P = expm(Q t) and the thresholds of its four rows into
+// rows row .. row + 3 of hi / lo, bit for bit what transition_matrix + row_thresholds give on the host, except for the
+// items the kernel lists in flag[0 .. *n_flag) (the scaling exponent the host's log2 might round differently, or a
+// norm that is not finite), which the caller recomputes on the host.  P_out (may be NULL): P of item i at 16 i.
+struct TabItem {
+    double t;
+    uint32_t row, pad;
+};
+struct TabQ {
+    double q[16];
+};
+cudaError_t launch_mut_tables(const TabItem* items, uint32_t n, const TabQ& Q, uint4* hi, uint4* lo, double* P_out,
+                              uint32_t* n_flag, uint32_t* flag, cudaStream_t s);
 
 // fragment placement + indel summary + record lengths, one thread per read end
 cudaError_t launch_place(const GenParams& p, cudaStream_t s);

@@ -1,10 +1,15 @@
-// create_haplotypes on the device: substitutions along a tree (DESIGN.md section 10).
+// create_haplotypes on the device: substitutions along a tree, or along gene trees, one per region of a chromosome
+// (DESIGN.md section 10).
 //
-// Every T/C/A/G site of the reference walks down the tree in the schedule the host prepared (preorder, the child
+// Every T/C/A/G site of the reference walks down its region's tree in the schedule the host prepared (preorder, the child
 // with fewer tips first, so at most log2(tips) + 2 internal nodes are live at once).  Per (site, node) it is one
 // decision on a 64-bit draw X(chromosome, site, node) (jlp_draws.h, planes MUT / MSLOW) against the cumulative
 // thresholds of row `parent state` of P(node, category); the decision is taken on the high 32 bits and the low word
 // is fetched only when the high word equals a threshold's, so it always equals the full 64-bit comparison.
+//
+// With gene trees (k_mutate<., ., true>) a tile's chromosome, first site, region and schedule come from its MutTile.
+// The threshold tables are built on the device (k_mut_tables) for a window of tiles at a time; both passes run window
+// by window (one tree: one window).
 //
 // Two passes over the same draws, no atomics:
 //   k_mutate<false>  records per (tip, tile) into cnt (a tile is owned by one warp, its lane 0 adds)
@@ -135,7 +140,10 @@ __device__ __forceinline__ void indel_tip(const MutParams& p, uint32_t tip, uint
     if (lane == 0) { *cp = base + tot; *cur = j1; }
 }
 
-template <bool WRITE, bool INDEL>
+// GT = false: one tree for the genome (jlp_create_haplotypes and _indels); the tile's chromosome from tile0 and the
+// schedule and tables from the parameters, as before gene trees.  GT = true: the tile's region, schedule and table rows from its
+// MutTile.  The two are kept apart so that the one-tree passes keep their speed (DESIGN.md section 10, "Gene trees").
+template <bool WRITE, bool INDEL, bool GT>
 __global__ void __launch_bounds__(kMutWarps * 32)
 k_mutate(const __grid_constant__ MutParams p) {
     __shared__ uint8_t st[kMutSlots][kMutWarps * 32];     // node states: 2 bits per site, one byte per (slot, thread)
@@ -147,27 +155,42 @@ k_mutate(const __grid_constant__ MutParams p) {
         thi = tab_s;
     }
     const uint32_t tid = threadIdx.x, lane = tid & 31u;
-    const uint32_t tile = blockIdx.x * kMutWarps + (tid >> 5);
-    if (tile >= p.n_tiles) return;
-    uint32_t lo = 0, hi = p.n_chroms;                     // the last chromosome whose first tile is <= tile
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (p.tile0[mid] <= tile) lo = mid; else hi = mid;
+    const uint32_t tile = (GT ? p.tile_begin : 0u) + blockIdx.x * kMutWarps + (tid >> 5);
+    if (tile >= (GT ? p.tile_end : p.n_tiles)) return;     // one tree: one window of every tile
+    uint32_t c;
+    const uint8_t* seq;
+    uint64_t first, lo = 0, hi;                           // the tile's first site; the sites it decides, [lo, hi)
+    uint32_t n_begin = 0, n_end = p.n_sched;              // its tree's schedule entries
+    const uint4* tlo = p.thr_lo;
+    if (GT) {
+        const MutTile T = p.tiles[tile];
+        c = T.chrom; first = T.first; lo = T.lo; hi = T.hi;
+        seq = p.genome + p.chrom_off[c];
+        n_begin = T.sched0; n_end = T.sched0 + T.n_sched;
+        thi += T.tab0;                                    // tab0 is 0 when the table is staged (one tree)
+        tlo += T.tab0;
+    } else {
+        uint32_t a = 0, b = p.n_chroms;                   // the last chromosome whose first tile is <= tile
+        while (b - a > 1) {
+            const uint32_t mid = (a + b) >> 1;
+            if (p.tile0[mid] <= tile) a = mid; else b = mid;
+        }
+        c = a;
+        const uint64_t off = p.chrom_off[c];
+        seq = p.genome + off;
+        hi = p.chrom_off[c + 1] - off;
+        first = (uint64_t)(tile - p.tile0[c]) * kMutTile;
     }
-    const uint32_t c = lo;
-    const uint64_t off = p.chrom_off[c], len = p.chrom_off[c + 1] - off;
-    const uint8_t* seq = p.genome + off;
-    const uint64_t first = (uint64_t)(tile - p.tile0[c]) * kMutTile;
     const uint64_t seed = p.seed;
     uint32_t* cnt = p.cnt + tile;
 
     for (uint32_t step = 0; step < kMutSteps; step++) {
         const uint64_t s0 = first + step * 128u + lane * 4u;
-        if (first + step * 128u >= len) break;
+        if (first + step * 128u >= hi) break;
         uint32_t ref = 0, cand = 0, ev = 0, cats = 0;      // 2 bits per site; T/C/A/G sites; evolving sites; 8 bits per site
 #pragma unroll
         for (uint32_t k = 0; k < 4; k++)
-            if (s0 + k < len) {
+            if ((!GT || s0 + k >= lo) && s0 + k < hi) {
                 const uint32_t code = base_code(seq[s0 + k]);
                 if (code < 4) { ref |= code << (2 * k); cand |= 1u << k; }
             }
@@ -194,7 +217,7 @@ k_mutate(const __grid_constant__ MutParams p) {
         }
         if (!INDEL && __ballot_sync(~0u, ev) == 0) continue;      // with indels the tips' records still need the step
         st[0][tid] = (uint8_t)ref;
-        for (uint32_t n = 0; n < p.n_sched; n++) {
+        for (uint32_t n = n_begin; n < (GT ? n_end : p.n_sched); n++) {
             const MutNode nd = p.sched[n];
             const uint32_t ps = st[nd.pslot][tid];
             uint32_t ns = ps;
@@ -204,7 +227,7 @@ k_mutate(const __grid_constant__ MutParams p) {
                 for (uint32_t k = 0; k < 4; k++) {
                     if (!((ev >> k) & 1u)) continue;
                     const uint32_t a = (ps >> (2 * k)) & 3u, row = nd.tab + 4u * ((cats >> (8 * k)) & 0xffu) + a;
-                    const uint32_t b = decide(genome_word(w, k), thi[row], p.thr_lo, row, seed, c, s0 + k, nd.node);
+                    const uint32_t b = decide(genome_word(w, k), thi[row], GT ? tlo : p.thr_lo, row, seed, c, s0 + k, nd.node);
                     ns = (ns & ~(3u << (2 * k))) | (b << (2 * k));
                 }
             }
@@ -338,24 +361,134 @@ __global__ void __launch_bounds__(256) k_ins_walk(const __grid_constant__ InsPar
     }
 }
 
+// One thread per (tree, node, category) item: P = expm(Q t) and its four rows' thresholds, restating
+// transition_matrix + row_thresholds (jlp_host.cpp) operation for operation: every product and sum rounded on its own
+// (__dmul_rn / __dadd_rn, no contraction), IEEE division, in the host's order; fabs, max, ldexp and the truncating
+// conversion are exact on both sides.  The one libm step is the host's s = ceil(log2(norm)).  Here s comes from frexp:
+// norm = m 2^e, m in [0.5, 1), so s = e - 1 when m = 0.5 and e otherwise.  glibc's log2 is within an ulp of the exact
+// value; the result's ulp is at most 2^-42 for norms below 2^1024, and log2(2^(e-1) (1 + d)) exceeds e - 1 by about
+// 1.44 d, so the host's ceil can only differ when 0 < d <= 2^-40, i.e. 0.5 < m <= 0.5 + 2^-41.  Those items, and a
+// norm that is not finite, are listed in `flag` and recomputed on the host by the caller.
+__global__ void __launch_bounds__(128) k_mut_tables(const TabItem* __restrict__ items, uint32_t n, const TabQ Q,
+                                                   uint4* __restrict__ thr_hi, uint4* __restrict__ thr_lo,
+                                                   double* __restrict__ P_out, uint32_t* n_flag, uint32_t* flag) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const TabItem it = items[i];
+    const double t = it.t;
+    double P[16];
+#pragma unroll
+    for (int k = 0; k < 16; k++) P[k] = (k % 5 == 0) ? 1.0 : 0.0;
+    if (t != 0) {
+        double A[16], norm = 0;
+#pragma unroll
+        for (int r = 0; r < 4; r++) {
+            double row = 0;
+#pragma unroll
+            for (int j = 0; j < 4; j++)
+                if (j != r) { A[4 * r + j] = __dmul_rn(Q.q[4 * r + j], t); row = __dadd_rn(row, A[4 * r + j]); }
+            A[5 * r] = -row;
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            double col = 0;
+#pragma unroll
+            for (int r = 0; r < 4; r++) col = __dadd_rn(col, fabs(A[4 * r + j]));
+            norm = norm < col ? col : norm;                 // std::max(norm, col)
+        }
+        int s = 0;
+        if (!isfinite(norm)) {
+            s = 0;
+            flag[atomicAdd(n_flag, 1u)] = i;
+        } else if (norm > 1) {
+            int e;
+            const double m = frexp(norm, &e);
+            s = min(1000, m == 0.5 ? e - 1 : e);
+            if (m > 0.5 && m <= 0.5 + 0x1p-41) flag[atomicAdd(n_flag, 1u)] = i;
+        }
+        const double sc = ldexp(1.0, -s);
+#pragma unroll
+        for (int k = 0; k < 16; k++) A[k] = __dmul_rn(A[k], sc);
+        double term[16];
+#pragma unroll
+        for (int k = 0; k < 16; k++) term[k] = P[k];
+        for (int k = 1; k <= 30; k++) {
+            const double dk = (double)k;
+#pragma unroll
+            for (int r = 0; r < 4; r++) {                    // row r of the next term needs row r of this one only
+                double nx[4];
+#pragma unroll
+                for (int j = 0; j < 4; j++) {
+                    double acc = 0;
+#pragma unroll
+                    for (int m = 0; m < 4; m++) acc = __dadd_rn(acc, __dmul_rn(term[4 * r + m], A[4 * m + j]));
+                    nx[j] = __ddiv_rn(acc, dk);
+                }
+#pragma unroll
+                for (int j = 0; j < 4; j++) { term[4 * r + j] = nx[j]; P[4 * r + j] = __dadd_rn(P[4 * r + j], nx[j]); }
+            }
+        }
+        for (int q = 0; q < s; q++) {
+            double nx[16];
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int j = 0; j < 4; j++) {
+                    double acc = 0;
+#pragma unroll
+                    for (int m = 0; m < 4; m++) acc = __dadd_rn(acc, __dmul_rn(P[4 * r + m], P[4 * m + j]));
+                    nx[4 * r + j] = acc;
+                }
+#pragma unroll
+            for (int k = 0; k < 16; k++) P[k] = nx[k];
+        }
+    }
+    if (P_out) {
+#pragma unroll
+        for (int k = 0; k < 16; k++) P_out[16 * (size_t)i + k] = P[k];
+    }
+#pragma unroll
+    for (int a = 0; a < 4; a++) {
+        double p[4], sum = 0, cum = 0;
+        uint64_t th[3];
+#pragma unroll
+        for (int j = 0; j < 4; j++) { p[j] = P[4 * a + j] > 0 ? P[4 * a + j] : 0.0; sum = __dadd_rn(sum, p[j]); }
+#pragma unroll
+        for (int j = 0; j < 3; j++) {
+            cum = __dadd_rn(cum, __ddiv_rn(p[j], sum));
+            th[j] = !(cum > 0) ? 0ull : cum >= 1 ? ~0ull : __double2ull_rz(ldexp(cum, 64));   // prob_threshold
+        }
+        thr_hi[it.row + a] = make_uint4((uint32_t)(th[0] >> 32), (uint32_t)(th[1] >> 32), (uint32_t)(th[2] >> 32), 0);
+        thr_lo[it.row + a] = make_uint4((uint32_t)th[0], (uint32_t)th[1], (uint32_t)th[2], 0);
+    }
+}
+
 }  // namespace
 
-size_t mut_smem_bytes(uint32_t tab_rows) { return (size_t)tab_rows * sizeof(uint4); }
-
-template <bool WRITE, bool INDEL>
-cudaError_t launch_mutate_t(const MutParams& p, cudaStream_t s) {
-    const size_t smem = p.tab_smem ? mut_smem_bytes(p.tab_rows) : 0;
-    const unsigned grid = (p.n_tiles + kMutWarps - 1) / kMutWarps;
-    cudaError_t e = cudaFuncSetAttribute(k_mutate<WRITE, INDEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    k_mutate<WRITE, INDEL><<<grid, kMutWarps * 32, smem, s>>>(p);
+cudaError_t launch_mut_tables(const TabItem* items, uint32_t n, const TabQ& Q, uint4* hi, uint4* lo, double* P_out,
+                              uint32_t* n_flag, uint32_t* flag, cudaStream_t s) {
+    if (n == 0) return cudaSuccess;
+    k_mut_tables<<<(n + 127) / 128, 128, 0, s>>>(items, n, Q, hi, lo, P_out, n_flag, flag);
     return cudaGetLastError();
 }
 
-cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, cudaStream_t s) {
-    if (p.n_tiles == 0) return cudaSuccess;
-    if (indels) return write ? launch_mutate_t<true, true>(p, s) : launch_mutate_t<false, true>(p, s);
-    return write ? launch_mutate_t<true, false>(p, s) : launch_mutate_t<false, false>(p, s);
+size_t mut_smem_bytes(uint32_t tab_rows) { return (size_t)tab_rows * sizeof(uint4); }
+
+template <bool WRITE, bool INDEL, bool GT>
+cudaError_t launch_mutate_t(const MutParams& p, cudaStream_t s) {
+    const size_t smem = p.tab_smem ? mut_smem_bytes(p.tab_rows) : 0;
+    const unsigned grid = (p.tile_end - p.tile_begin + kMutWarps - 1) / kMutWarps;
+    cudaError_t e = cudaFuncSetAttribute(k_mutate<WRITE, INDEL, GT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    k_mutate<WRITE, INDEL, GT><<<grid, kMutWarps * 32, smem, s>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_mutate(const MutParams& p, bool write, bool indels, bool gtrees, cudaStream_t s) {
+    if (p.tile_end <= p.tile_begin) return cudaSuccess;
+    if (gtrees) return write ? launch_mutate_t<true, false, true>(p, s) : launch_mutate_t<false, false, true>(p, s);
+    if (indels) return write ? launch_mutate_t<true, true, false>(p, s) : launch_mutate_t<false, true, false>(p, s);
+    return write ? launch_mutate_t<true, false, false>(p, s) : launch_mutate_t<false, false, false>(p, s);
 }
 
 cudaError_t launch_ins_walk(const InsParams& p, cudaStream_t s) {

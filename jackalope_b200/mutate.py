@@ -12,6 +12,8 @@ project's own (DESIGN.md section 10):
 * The root state is the reference base; a child's state is drawn from row ``parent state`` of
   ``expm(Q * rate * branch_length)``.  Only T/C/A/G sites evolve.  A haplotype's records are the sites where its
   tip differs from the reference.
+* With ``haps_gtrees`` (ms-format gene trees) each chromosome is cut into regions, each evolving along its own tree
+  (DESIGN.md section 10, "Gene trees").
 * Insertions and deletions (``ins`` / ``del_``, models from ``indels()``) happen along each branch in steps of at most
   ``epsilon`` expected events per site; inserted columns start from ``sub.pi`` and evolve below like any site.  A
   haplotype's records then follow one canonical encoding of its tip sequence (DESIGN.md section 10).
@@ -482,7 +484,7 @@ def kingman(n, rng):
 
 
 class HapsInfo:
-    """Where the haplotypes' tree comes from (``haps_phylo`` or ``haps_theta``)."""
+    """Where the haplotypes' trees come from (``haps_phylo``, ``haps_theta`` or ``haps_gtrees``)."""
 
     def tree(self, sub, seed):
         raise NotImplementedError
@@ -542,10 +544,99 @@ def haps_theta(theta, n_haps):
     return HapsTheta(theta, n_haps)
 
 
+class HapsGtrees(HapsInfo):
+    """Gene trees in ms format: one `//` block per chromosome, each chromosome cut into regions by the trees' [n]
+    prefixes (DESIGN.md section 10, "Gene trees").  The library parses the text; here only the first tree is read, for
+    the haplotypes' names and order."""
+
+    def __init__(self, text, names):
+        self.text, self.names = text, names
+
+    def __repr__(self):
+        return "<haps_info gtrees, %d haplotypes>" % len(self.names)
+
+
+def _first_ms_tree(text):
+    in_block = False
+    for line in text.splitlines():
+        if line.startswith("//"):
+            in_block = True
+        elif in_block and line[:1] in ("[", "("):
+            if line[0] == "[":
+                close = line.find("]")
+                if close > 1 and line[1:close].isdigit() and line[1:close].isascii():
+                    line = line[close + 1:]
+            return line
+    return None
+
+
+def haps_gtrees(obj=None, fn=None):
+    """Gene trees from a coalescent simulator with recombination (ms, scrm, msprime's mspms): ``fn`` an ms-format
+    file, or ``obj`` a list with one entry per chromosome, each a list of tree lines (``[n]`` prefix and Newick tree,
+    the shape of scrm's ``trees``).  Block k of the text is chromosome k; a tree with prefix [n] covers its share n / S
+    of the chromosome (S the block's sum), a block of one tree without a prefix the whole chromosome.  Haplotypes are
+    the tips, ordered numerically when every label is an integer (as ms numbers them), else as in the first tree."""
+    f = "haps_gtrees"
+    if (obj is None) == (fn is None):
+        _bad(f, "obj", "a list of tree lines per chromosome when `fn` is NULL (exactly one of `obj` and `fn` is given)")
+    if fn is not None:
+        if not isinstance(fn, str) or not os.path.isfile(os.path.expanduser(fn)):
+            _bad(f, "fn", "the name of an existing file of ms-format output")
+        with open(os.path.expanduser(fn)) as fh:
+            text = fh.read()
+    else:
+        if (not isinstance(obj, (list, tuple)) or not obj or
+                not all(isinstance(b, (list, tuple)) and all(isinstance(x, str) for x in b) for b in obj)):
+            _bad(f, "obj", "a list with one list of tree lines (strings) per chromosome")
+        text = "".join("//\n" + "".join(x.rstrip("\n") + "\n" for x in b) for b in obj)
+    first = _first_ms_tree(text)
+    if first is None:
+        raise JackalopeError("\nFor `haps_gtrees`, the ms output has no trees (a '//' line followed by tree lines).")
+    names = parse_newick(first).tip_names
+    if all(x.isascii() and x.isdigit() for x in names):
+        names = sorted(names, key=int)
+    return HapsGtrees(text, names)
+
+
+def ms_regions(text, chrom_lens, names):
+    """The library's reading of ms text (jlp_ms_regions): (regions as (chromosome, start, end, tree index), tree
+    count); a JackalopeError with the library's message when it rejects the text."""
+    from . import _lib
+    raw = text.encode() if isinstance(text, str) else bytes(text)
+    lens = np.ascontiguousarray(chrom_lens, dtype=np.uint64)
+    nm = (C.c_char_p * len(names))(*[n.encode() for n in names])
+    nr, ntr, err = C.c_uint64(), C.c_uint64(), C.create_string_buffer(1024)
+    reg = np.zeros((0, 4), dtype=np.uint64)
+    for _ in range(2):                   # the count, then the regions
+        if _lib.lib().jlp_ms_regions(raw, len(raw), lens.ctypes.data_as(_lib.u64p), lens.size, nm, len(names),
+                                     reg.ctypes.data_as(_lib.u64p), reg.shape[0], C.byref(nr), C.byref(ntr), err,
+                                     1024) != 0:
+            raise JackalopeError("\nFor `haps_gtrees`: " + err.value.decode())
+        reg = np.zeros((nr.value, 4), dtype=np.uint64) if reg.shape[0] < nr.value else reg
+    return [tuple(int(x) for x in r) for r in reg[:nr.value]], ntr.value
+
+
+def transition_tables(Q, t, ctx=None, device=0):
+    """P = expm(Q t) and the row thresholds for each t, as create_haplotypes builds them on the device
+    (jlp_transition_tables): (P [n, 4, 4], thresholds [n, 4, 3] uint64, items recomputed on the host)."""
+    from . import _lib
+    from .illumina import default_context
+    ctx = ctx or default_context(device)
+    q = np.ascontiguousarray(np.asarray(Q, dtype=np.float64).reshape(16))
+    t = np.ascontiguousarray(t, dtype=np.float64).reshape(-1)
+    P = np.zeros((t.size, 4, 4))
+    thr = np.zeros((t.size, 4, 3), dtype=np.uint64)
+    nh = C.c_uint64()
+    ctx._check(ctx.lib.jlp_transition_tables(ctx.h, q.ctypes.data_as(_lib.f64p), t.ctypes.data_as(_lib.f64p), t.size,
+                                             P.ctypes.data_as(_lib.f64p), thr.ctypes.data_as(_lib.u64p), C.byref(nh)),
+               "jlp_transition_tables")
+    return P, thr, nh.value
+
+
 # -------------------------------------------------------------------- create_haplotypes ---
 
 def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.03, n_threads=1,
-                      show_progress=False, *, seed=None, ctx=None, device=0):
+                      show_progress=False, *, seed=None, ctx=None, device=0, table_budget=0):
     """Haplotypes evolved from ``reference`` along the tree of ``haps_info`` under the substitution model ``sub`` and
     the indel models ``ins`` / ``del_`` (``indels()`` or None), generated on the GPU.  Returns a ``Haplotypes`` object
     (substitution, insertion and deletion records; the tree as Newick text in ``.tree``, the call's figures in
@@ -553,7 +644,9 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     nothing.  ``epsilon`` bounds the expected indel events per site of one step of a branch; it must be > 0 once an
     indel rate is > 0 (jackalope's exact Gillespie sampling at 0 is not offered) and is otherwise unused
     (substitutions are drawn exactly from P(t)).  ``n_threads`` and ``show_progress`` are accepted for compatibility.
-    ``seed`` (keyword-only) addresses every draw; None draws one from numpy's global RNG."""
+    ``seed`` (keyword-only) addresses every draw; None draws one from numpy's global RNG.  With ``haps_gtrees`` each
+    region follows its own tree (``.tree`` is None); ``table_budget`` (keyword-only) then bounds the bytes of threshold
+    tables built at once (0: the library's default) and does not change the result."""
     from . import _lib
     from .illumina import default_context
 
@@ -561,7 +654,7 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     if not isinstance(reference, RefGenome):
         _bad(f, "reference", "a \"ref_genome\" object")
     if not isinstance(haps_info, HapsInfo):
-        _bad(f, "haps_info", "a \"haps_info\" object (from `haps_phylo` or `haps_theta`)")
+        _bad(f, "haps_info", "a \"haps_info\" object (from `haps_phylo`, `haps_theta` or `haps_gtrees`)")
     if not isinstance(sub, SubModel):
         _bad(f, "sub", "a \"sub_info\" object (from one of the `sub_*` functions)")
     for par, x in (("ins", ins), ("del_", del_)):
@@ -578,9 +671,16 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
         _bad(f, "n_threads", "a single integer >= 1")
     if not isinstance(show_progress, (bool, np.bool_)):
         _bad(f, "show_progress", "a single logical")
+    gtrees = isinstance(haps_info, HapsGtrees)
+    if gtrees and with_indels:
+        raise JackalopeError("\nFor `create_haplotypes`, insertions and deletions (`ins` / `del_`) are not supported "
+                             "with `haps_gtrees` (gene trees); they need one tree for the genome.")
+    if not (_is_int(table_budget) and table_budget >= 0):
+        _bad(f, "table_budget", "a single integer >= 0")
     if seed is None:
         seed = int(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64))
-    tree = haps_info.tree(sub, seed)
+    tree = None if gtrees else haps_info.tree(sub, seed)
+    hap_names = haps_info.names if gtrees else tree.tip_names
     ctx = ctx or default_context(device)
     ctx.set_genome(reference)
 
@@ -589,27 +689,35 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     p.invariant = sub.invariant
     rates = np.ascontiguousarray(sub.rates, dtype=np.float64)
     p.n_rates, p.rates = rates.size, rates.ctypes.data_as(_lib.f64p)
-    p.n_nodes = tree.n_nodes
-    p.parent = tree.parent.ctypes.data_as(C.POINTER(C.c_int32))
-    p.branch_len = tree.branch_len.ctypes.data_as(_lib.f64p)
-    p.n_tips = len(tree.tip_names)
-    p.tip_node = tree.tip_node.ctypes.data_as(_lib.u32p)
-    names = (C.c_char_p * len(tree.tip_names))(*[n.encode() for n in tree.tip_names])
+    if not gtrees:
+        p.n_nodes = tree.n_nodes
+        p.parent = tree.parent.ctypes.data_as(C.POINTER(C.c_int32))
+        p.branch_len = tree.branch_len.ctypes.data_as(_lib.f64p)
+        p.tip_node = tree.tip_node.ctypes.data_as(_lib.u32p)
+    p.n_tips = len(hap_names)
+    names = (C.c_char_p * len(hap_names))(*[n.encode() for n in hap_names])
     p.tip_names = names
     p.seed = int(seed) & (2 ** 64 - 1)
     st = _lib.MutationStats()
     ctx._haps = None
-    if with_indels:
+    if gtrees:
+        text = haps_info.text.encode()
+        g, gst = _lib.GtreeParams(text, len(text), int(table_budget)), _lib.GtreeStats()
+        ctx._check(ctx.lib.jlp_create_haplotypes_gtrees(ctx.h, C.byref(p), C.byref(g), C.byref(st), C.byref(gst)),
+                   "jlp_create_haplotypes_gtrees")
+    elif with_indels:
         ip, ist = indel_params(ins, del_, epsilon, sub.pi), _lib.IndelStats()
         ctx._check(ctx.lib.jlp_create_haplotypes_indels(ctx.h, C.byref(p), C.byref(ip), C.byref(st), C.byref(ist)),
                    "jlp_create_haplotypes_indels")
     else:
         ctx._check(ctx.lib.jlp_create_haplotypes(ctx.h, C.byref(p), C.byref(st)), "jlp_create_haplotypes")
 
-    muts = [[haplotype_muts(ctx, h, c) for c in range(reference.n_chroms())] for h in range(len(tree.tip_names))]
-    haps = Haplotypes(reference, tree.tip_names, muts)
-    haps.tree = tree.newick()
+    muts = [[haplotype_muts(ctx, h, c) for c in range(reference.n_chroms())] for h in range(len(hap_names))]
+    haps = Haplotypes(reference, hap_names, muts)
+    haps.tree = None if gtrees else tree.newick()
     haps.stats = st.as_dict()
+    if gtrees:
+        haps.stats.update(gst.as_dict())
     if with_indels:
         haps.stats.update(ist.as_dict())
     ctx._haps = haps
