@@ -131,10 +131,26 @@ class VcfStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class VcfReadParams(C.Structure):
+    _fields_ = [("path", C.c_char_p), ("n_threads", C.c_uint64), ("batch_bytes", C.c_uint64)]
+
+
+class VcfReadStats(C.Structure):
+    _fields_ = [
+        ("lines", C.c_uint64), ("samples", C.c_uint64), ("haplotypes", C.c_uint64), ("calls", C.c_uint64),
+        ("records", C.c_uint64), ("overlaps_skipped", C.c_uint64), ("symbolic_calls", C.c_uint64),
+        ("missing_calls", C.c_uint64), ("text_bytes", C.c_uint64), ("batches", C.c_uint64), ("inflate_ms", C.c_double),
+        ("parse_ms", C.c_double), ("build_ms", C.c_double), ("store_ms", C.c_double), ("total_ms", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/jlp_b200.h declares
 SYMBOLS = [
     "jlp_ctx_create", "jlp_ctx_create_multi", "jlp_ctx_n_devices", "jlp_materialize_haplotypes", "jlp_ctx_destroy", "jlp_last_error", "jlp_set_genome", "jlp_set_genome_async", "jlp_genome_sync", "jlp_create_genome", "jlp_get_genome", "jlp_genome_draw", "jlp_clear_haplotypes",
-    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_create_haplotypes_gtrees", "jlp_get_haplotype_muts", "jlp_write_vcf", "jlp_transition_matrix", "jlp_transition_tables", "jlp_ms_regions", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
+    "jlp_add_haplotype", "jlp_get_haplotype_chrom", "jlp_create_haplotypes", "jlp_create_haplotypes_indels", "jlp_create_haplotypes_gtrees", "jlp_create_haplotypes_vcf", "jlp_haplotype_name", "jlp_get_haplotype_muts", "jlp_write_vcf", "jlp_transition_matrix", "jlp_transition_tables", "jlp_ms_regions", "jlp_set_profile", "jlp_illumina_ref", "jlp_illumina_hap",
     "jlp_illumina_to_memory", "jlp_illumina_stream", "jlp_illumina_device_only", "jlp_illumina_group_counts", "jlp_apportion", "jlp_shard_range", "jlp_deflate", "jlp_bgzf_device", "jlp_pacbio", "jlp_pacbio_to_memory", "jlp_pacbio_read_plan", "jlp_pacbio_sample", "jlp_reads_per_group", "jlp_alias_build",
     "jlp_threshold", "jlp_unif_expr", "jlp_frag_table", "jlp_philox4x32_10", "jlp_draw_pos", "jlp_draw_pair",
     "jlp_version",
@@ -177,6 +193,8 @@ def lib():
                                                C.POINTER(MutationStats), C.POINTER(IndelStats)]
     L.jlp_create_haplotypes_gtrees.argtypes = [C.c_void_p, C.POINTER(MutationParams), C.POINTER(GtreeParams),
                                                C.POINTER(MutationStats), C.POINTER(GtreeStats)]
+    L.jlp_create_haplotypes_vcf.argtypes = [C.c_void_p, C.POINTER(VcfReadParams), C.POINTER(VcfReadStats)]
+    L.jlp_haplotype_name.argtypes = [C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint64, u64p]
     L.jlp_ms_regions.argtypes = [C.c_char_p, C.c_uint64, u64p, C.c_uint64, pp, C.c_uint32, u64p, C.c_uint64, u64p, u64p,
                                  C.c_char_p, C.c_uint64]
     L.jlp_transition_tables.argtypes = [C.c_void_p, f64p, f64p, C.c_uint64, f64p, u64p, u64p]

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libjlp_b200.so")
-SOURCES = ["jlp_api.cu", "jlp_run_illumina.cu", "jlp_run_pacbio.cu", "jlp_run_vcf.cu", "jlp_run_haps.cu", "jlp_kernels.cu", "jlp_bgzf.cu", "jlp_pacbio.cu", "jlp_mutate.cu", "jlp_vcf.cu", "jlp_pacbio.cpp", "jlp_host.cpp", "jlp_indel.cpp", "jlp_gtrees.cpp", "jlp_deflate.cpp", "jlp_output.cpp"]
+SOURCES = ["jlp_api.cu", "jlp_run_illumina.cu", "jlp_run_pacbio.cu", "jlp_run_vcf.cu", "jlp_run_haps.cu", "jlp_run_vcf_read.cu", "jlp_kernels.cu", "jlp_bgzf.cu", "jlp_pacbio.cu", "jlp_mutate.cu", "jlp_vcf.cu", "jlp_vcf_read.cu", "jlp_pacbio.cpp", "jlp_host.cpp", "jlp_indel.cpp", "jlp_gtrees.cpp", "jlp_deflate.cpp", "jlp_output.cpp"]
 HEADERS = ["jlp_ctx.h", "jlp_draws.h", "jlp_host.h", "jlp_kernels.cuh", "jlp_deflate.h", "jlp_output.h", "jlp_pacbio.h", os.path.join("..", "..", "include", "jlp_b200.h")]
 
 

@@ -1,6 +1,6 @@
 // C ABI (include/jlp_b200.h): the context, genome, haplotype and profile calls, the stateless helpers, and the
-// definitions behind jlp_ctx.h.  The drivers are jlp_run_illumina.cu, jlp_run_pacbio.cu, jlp_run_vcf.cu and
-// jlp_run_haps.cu.
+// definitions behind jlp_ctx.h.  The drivers are jlp_run_illumina.cu, jlp_run_pacbio.cu, jlp_run_vcf.cu,
+// jlp_run_haps.cu and jlp_run_vcf_read.cu.
 #include "jlp_ctx.h"
 
 #include <cmath>
@@ -248,6 +248,46 @@ void attach_hap(jlp_ctx* c, const std::shared_ptr<HapStore>& S) {
             seq.push_back(S->chrom[ci].n_muts == 0 ? d->genome.p + kPad + c->chrom_off[ci] : nullptr);
         d->hap_seq.push_back(std::move(seq));
     }
+}
+
+// the reference's chromosome lengths; positions in a chromosome are 32 bits wide (TreeRegion, MutTile, VrLine)
+std::vector<uint64_t> chrom_lengths(const jlp_ctx* c) {
+    const uint64_t nc = c->chrom_off.size() - 1;
+    std::vector<uint64_t> len(nc);
+    for (uint64_t ci = 0; ci < nc; ci++) {
+        len[ci] = c->chrom_off[ci + 1] - c->chrom_off[ci];
+        if (len[ci] >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
+    }
+    return len;
+}
+
+void store_haps(jlp_ctx* c, const HapRegions& G, unsigned threads) {
+    const uint64_t nc = c->chrom_off.size() - 1;
+    const size_t n_haps = G.names.size(), n_items = n_haps * nc;
+    const int dev = c->dev[0]->id;
+    std::vector<std::shared_ptr<HapStore>> stores(n_haps);
+    uint64_t records = 0;
+    for (size_t h = 0; h < n_haps; h++) {
+        stores[h] = std::make_shared<HapStore>();
+        stores[h]->name = G.names[h];
+        stores[h]->chrom.resize(nc);
+    }
+    for (size_t r = 0; r < n_items; r++) records += G.n[r];
+    const unsigned nt = records < (1u << 16) ? 1u : threads;
+    parallel_for(n_items, nt, [&](uint64_t r) {
+        HapChromHost& H = stores[r / nc]->chrom[r % nc];
+        const uint64_t M = G.n[r];
+        H.size = G.size[r];
+        H.n_muts = M;
+        H.pool_bytes = G.pool[r];
+        if (!M) return;
+        H.packed.resize(4 * M + (G.pool[r] + 7) / 8);
+        CK(cudaSetDevice(dev));
+        CK(cudaMemcpy(H.packed.data(), G.src[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
+    });
+
+    clear_haps(c);
+    for (const auto& S : stores) attach_hap(c, S);
 }
 
 // The compression rule of the drivers that write one file per job (PacBio, VCF): unlike compression_of(), AUTO takes the

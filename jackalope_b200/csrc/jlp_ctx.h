@@ -1,6 +1,6 @@
 // Internal to the library, not installed: the context and device types behind the C ABI (include/jlp_b200.h) and the
 // helpers its drivers share.  jlp_api.cu defines the functions declared here; the drivers are jlp_run_illumina.cu,
-// jlp_run_pacbio.cu, jlp_run_vcf.cu and jlp_run_haps.cu.
+// jlp_run_pacbio.cu, jlp_run_vcf.cu, jlp_run_haps.cu and jlp_run_vcf_read.cu.
 #pragma once
 
 #include "../../include/jlp_b200.h"
@@ -303,6 +303,21 @@ void finish_upload(const jlp_ctx* c, Device& d);
 int claim_mat_buf(Device& d);
 void ensure_hap_chrom(const jlp_ctx* c, Device& d, size_t h, size_t ci);
 void attach_hap(jlp_ctx* c, const std::shared_ptr<HapStore>& S);
+
+// the reference's chromosome lengths, JLP_ERR_ARG if one has 2^32 bases or more
+std::vector<uint64_t> chrom_lengths(const jlp_ctx* c);
+
+// Haplotypes made on the first device, one region per (haplotype, chromosome), r = haplotype * chromosomes + chromosome:
+// its records in the HapChromHost::packed layout at src[r] (device memory; unread when n[r] == 0), their pool bytes and
+// the chromosome's size.
+struct HapRegions {
+    std::vector<std::string> names;
+    std::vector<const uint64_t*> src;
+    std::vector<uint64_t> n, pool, size;
+};
+// the regions copied into one HapStore per haplotype by up to `threads` host threads (one when there are few records);
+// the stores replace the context's haplotypes
+void store_haps(jlp_ctx* c, const HapRegions& G, unsigned threads);
 
 // ------------------------------------------------------------------------------------------------------ layout ---
 

@@ -269,6 +269,86 @@ cudaError_t launch_vcf_size(const VcfChrom& v, uint32_t n_lines, int n_sm, cudaS
 cudaError_t launch_vcf_text(const VcfChrom& v, uint32_t l0, uint32_t l1, uint8_t* out, uint64_t out_skip, int n_sm,
                             cudaStream_t s);
 
+// haps_vcf: haplotypes read from a VCF file (jlp_vcf_read.cu, DESIGN.md section 12).  A batch of whole lines is parsed
+// on the device; its lines' alleles and non-REF calls go to the chromosome they belong to, and once a chromosome's lines
+// are all seen its calls are sorted by haplotype slot (sample * kVrMaxPloidy + copy) and walked into records.
+constexpr uint32_t kVrMaxPloidy = 8;
+constexpr uint32_t kVrNone = 0xffffffffu;
+// the reasons a line is rejected, in the order its checks are made; the status word keeps min(line << 8 | reason)
+enum VrReason : uint32_t {
+    VR_COLUMNS = 1, VR_CHROM, VR_POS, VR_REF_LETTERS, VR_REF_RANGE, VR_REF_DIFF, VR_ALT, VR_FORMAT, VR_GT, VR_PLOIDY,
+    VR_INDEX, VR_CONTIG, VR_ORDER
+};
+enum VrKind : uint32_t { VR_SEQ = 0, VR_STAR = 1, VR_SYM = 2 };
+struct VrLine {
+    uint32_t chrom;              // kVrNone: a fixed column is malformed
+    uint32_t s, m;               // POS - 1, len(REF)
+    uint32_t alt_at, alt_len;    // the ALT field in the batch
+    uint32_t gt_at;              // the first sample field in the batch
+    uint32_t n_alt;
+    uint32_t sv_info;            // INFO has an END or SVLEN key
+};
+struct VrAllele {                // one ALT entry of a line
+    uint32_t s, m, n;            // the span it replaces and its length
+    uint32_t kind;
+    uint64_t text;               // its bytes in the batch's (then the chromosome's) allele text
+    uint32_t nrec, pool;         // records and pool bytes of its encoding
+};
+struct VrSlot {                  // one haplotype slot of a chromosome, from the walk
+    unsigned long long nrec, pool, applied, skipped;
+    long long delta;
+};
+struct VrBatch {
+    const uint8_t* text;
+    uint32_t n_bytes, n_lines;   // the batch ends with '\n'
+    uint64_t line0;              // data-line index of its first line
+    const uint8_t* genome;       // the resident reference and its chromosomes' offsets
+    const uint64_t* chrom_off;
+    const uint8_t* names;        // reference chromosome names, sorted bytewise: name_off[k]..name_off[k+1], index name_idx[k]
+    const uint32_t* name_off;
+    const uint32_t* name_idx;
+    uint32_t n_chroms, n_cols, n_samples;
+    uint32_t prev_chrom, prev_s; // the line before the batch (prev_chrom kVrNone: none)
+    uint32_t* nl;                // [n_lines] newline positions
+    VrLine* line;
+    uint32_t *n_alt, *alt0, *alt_len, *text0, *n_calls, *call0;   // per line, and their exclusive prefixes
+    VrAllele* allele;
+    uint8_t* alt_text;
+    uint32_t *call_slot, *call_allele;
+    uint32_t* ploidy;            // [n_samples] largest allele count of a GT, over the file
+    unsigned long long* counts;  // missing, symbolic calls
+    unsigned long long* status;  // min(data line << 8 | reason)
+    uint8_t* run_flag;
+    uint64_t *run_key, *runs;    // line << 32 | chromosome where a line's chromosome differs from the line's before
+    uint32_t* n_sel;             // DeviceSelect's count
+};
+// CUB scratch for any of the calls below over n items
+size_t vr_cub_bytes(uint64_t n);
+// stage 0: newline positions (n_lines in *n_sel).  1: the fixed columns and the prefixes alt0 / text0 ([n_lines + 1]).
+// 2: the alleles and their text, the GT count pass and call0.  3: the calls, and the runs of lines of one chromosome
+// (their count in *n_sel).  The host sizes the buffers of a stage from the totals of the one before.
+cudaError_t launch_vr_parse(const VrBatch& b, int stage, uint8_t* tmp, size_t tmp_bytes, cudaStream_t s);
+// the alleles [a0, a1) and calls [c0, c1) of a batch (lines [l0, l1) with t0 = text0[l0]) appended to a chromosome that
+// holds n_alleles alleles and text_bytes of allele text; the text itself is copied by the caller
+cudaError_t launch_vr_append(const VrBatch& b, uint32_t a0, uint32_t a1, uint32_t c0, uint32_t c1, uint32_t t0,
+                             uint64_t n_alleles, uint64_t n_calls, uint64_t text_bytes, VrAllele* allele, uint32_t* slot,
+                             uint32_t* val, cudaStream_t s);
+struct VrChrom {
+    const VrAllele* allele;
+    const uint8_t* text;
+    const uint8_t* ref;          // the chromosome's reference bases
+    uint32_t *slot, *val, *slot2, *val2;    // [n_calls] line-major, then sorted by slot
+    uint64_t n_calls;
+    uint32_t n_slots;
+    uint64_t* seg;               // [2 * n_slots] each slot's calls in the sorted order
+    VrSlot* out_slot;
+    const uint64_t* region;      // [n_slots] word offset of each slot's records in out
+    uint64_t* out;
+};
+// the calls sorted by slot (stable: file order within a slot) and each slot's range, then the walk's count pass
+cudaError_t launch_vr_count(const VrChrom& v, uint8_t* tmp, size_t tmp_bytes, cudaStream_t s);
+cudaError_t launch_vr_write(const VrChrom& v, cudaStream_t s);
+
 // BGZF on the device (jlp_bgzf.cu).  totals[0..1] hold the FASTQ bytes of the two files of a batch (device
 // memory, as launch_scan leaves them); the compressed sizes come back in totals[2..3].  Block b of a file is
 // compressed into slots + b * kBgzfSlot, then gathered to out + (sum of the sizes before it).  nblk_max sizes

@@ -127,17 +127,6 @@ void check_model(const jlp_ctx* c, const jlp_mutation_params* p) {
         if (!p->tip_names[t]) throw ArgErr("tip name is NULL");
 }
 
-// the reference's chromosome lengths; positions in a chromosome are 32 bits wide (TreeRegion, MutTile)
-std::vector<uint64_t> chrom_lengths(const jlp_ctx* c) {
-    const uint64_t nc = c->chrom_off.size() - 1;
-    std::vector<uint64_t> len(nc);
-    for (uint64_t ci = 0; ci < nc; ci++) {
-        len[ci] = c->chrom_off[ci + 1] - c->chrom_off[ci];
-        if (len[ci] >> 32) throw ArgErr("chromosomes of 2^32 bases or more are not supported");
-    }
-    return len;
-}
-
 // the tree of p as the one tree of the genome: one region per (non-empty) chromosome
 GeneTrees one_tree(const jlp_ctx* c, const jlp_mutation_params* p) {
     const uint32_t n = p->n_nodes;
@@ -514,34 +503,22 @@ void run_passes(jlp_ctx* c, const jlp_mutation_params* p, const GeneTrees& G, co
     CK(cudaStreamSynchronize(s));
 }
 
-// the records into one HapStore per tip, copied straight into the packed arrays by a few host threads; the stores
-// replace the context's haplotypes
-void store_haps(jlp_ctx* c, const jlp_mutation_params* p, const IndelModel* im, const MutPlan& P, const MutPasses& R) {
+// the tips' records as regions of the passes' output, for store_haps
+HapRegions tip_regions(const jlp_ctx* c, const jlp_mutation_params* p, const IndelModel* im, const MutPlan& P,
+                       const MutPasses& R) {
     const uint64_t nc = c->chrom_off.size() - 1;
-    const uint32_t n_tips = p->n_tips;
-    const size_t n_items = (size_t)n_tips * nc;
-    const int dev = c->dev[0]->id;
-    std::vector<std::shared_ptr<HapStore>> stores(n_tips);
-    for (uint32_t t = 0; t < n_tips; t++) {
-        stores[t] = std::make_shared<HapStore>();
-        stores[t]->name = p->tip_names[t];
-        stores[t]->chrom.resize(nc);
+    const size_t n_items = (size_t)p->n_tips * nc;
+    HapRegions G;
+    G.names.assign(p->tip_names, p->tip_names + p->n_tips);
+    G.src.resize(n_items);
+    G.size.resize(n_items);
+    for (size_t r = 0; r < n_items; r++) {
+        G.src[r] = R.d_out.p + R.region[r];
+        G.size[r] = im ? P.ich[r % nc].tip[r / nc].size : c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
     }
-    const unsigned nt = R.records < (1u << 16) ? 1u : host_threads(n_items);
-    parallel_for(n_items, nt, [&](uint64_t r) {
-        HapChromHost& H = stores[r / nc]->chrom[r % nc];
-        const uint64_t M = R.region_n[r];
-        H.size = im ? P.ich[r % nc].tip[r / nc].size : c->chrom_off[r % nc + 1] - c->chrom_off[r % nc];
-        H.n_muts = M;
-        H.pool_bytes = R.pool[r];
-        if (!M) return;
-        H.packed.resize(4 * M + (R.pool[r] + 7) / 8);
-        CK(cudaSetDevice(dev));
-        CK(cudaMemcpy(H.packed.data(), R.d_out.p + R.region[r], H.packed.size() * 8, cudaMemcpyDeviceToHost));
-    });
-
-    clear_haps(c);
-    for (const auto& S : stores) attach_hap(c, S);
+    G.n = R.region_n;
+    G.pool = R.pool;
+    return G;
 }
 
 // The whole call: the trees and every chromosome's regions (one tree for the genome: one region per chromosome);
@@ -558,7 +535,7 @@ void create_haps(jlp_ctx* c, const jlp_mutation_params* p, const GeneTrees& G, u
     MutPasses R;
     run_passes(c, p, G, P, im, ins_pi, gstats != nullptr, R);
     const auto t_gen = std::chrono::steady_clock::now();
-    store_haps(c, p, im, P, R);
+    store_haps(c, tip_regions(c, p, im, P, R), host_threads((uint64_t)p->n_tips * (c->chrom_off.size() - 1)));
 
     if (stats) {
         const auto t1 = std::chrono::steady_clock::now();

@@ -14,6 +14,7 @@ project's own (DESIGN.md section 10):
   tip differs from the reference.
 * With ``haps_gtrees`` (ms-format gene trees) each chromosome is cut into regions, each evolving along its own tree
   (DESIGN.md section 10, "Gene trees").
+* With ``haps_vcf`` the haplotypes are read from a VCF file instead (DESIGN.md section 12): no model is used.
 * Insertions and deletions (``ins`` / ``del_``, models from ``indels()``) happen along each branch in steps of at most
   ``epsilon`` expected events per site; inserted columns start from ``sub.pi`` and evolve below like any site.  A
   haplotype's records then follow one canonical encoding of its tip sequence (DESIGN.md section 10).
@@ -484,7 +485,8 @@ def kingman(n, rng):
 
 
 class HapsInfo:
-    """Where the haplotypes' trees come from (``haps_phylo``, ``haps_theta`` or ``haps_gtrees``)."""
+    """Where the haplotypes come from: a tree (``haps_phylo``, ``haps_theta``), gene trees (``haps_gtrees``) or a VCF
+    file (``haps_vcf``)."""
 
     def tree(self, sub, seed):
         raise NotImplementedError
@@ -598,6 +600,24 @@ def haps_gtrees(obj=None, fn=None):
     return HapsGtrees(text, names)
 
 
+class HapsVcf(HapsInfo):
+    """Haplotypes read from a VCF file by the library (DESIGN.md section 12)."""
+
+    def __init__(self, path):
+        self.path = path
+
+    def __repr__(self):
+        return "<haps_info vcf %s>" % self.path
+
+
+def haps_vcf(fn):
+    """Haplotypes from the VCF file ``fn`` (plain, gzip or BGZF): one per (sample, copy), named by the sample when it has
+    one copy, else ``<sample>__<k>``; each takes the alleles its GT calls name (DESIGN.md section 12)."""
+    if not isinstance(fn, str) or not os.path.isfile(os.path.expanduser(fn)):
+        _bad("haps_vcf", "fn", "the name of an existing VCF file")
+    return HapsVcf(os.path.expanduser(fn))
+
+
 def ms_regions(text, chrom_lens, names):
     """The library's reading of ms text (jlp_ms_regions): (regions as (chromosome, start, end, tree index), tree
     count); a JackalopeError with the library's message when it rejects the text."""
@@ -635,8 +655,8 @@ def transition_tables(Q, t, ctx=None, device=0):
 
 # -------------------------------------------------------------------- create_haplotypes ---
 
-def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.03, n_threads=1,
-                      show_progress=False, *, seed=None, ctx=None, device=0, table_budget=0):
+def create_haplotypes(reference, haps_info, sub=None, ins=None, del_=None, epsilon=0.03, n_threads=1,
+                      show_progress=False, *, seed=None, ctx=None, device=0, table_budget=0, batch_bytes=0):
     """Haplotypes evolved from ``reference`` along the tree of ``haps_info`` under the substitution model ``sub`` and
     the indel models ``ins`` / ``del_`` (``indels()`` or None), generated on the GPU.  Returns a ``Haplotypes`` object
     (substitution, insertion and deletion records; the tree as Newick text in ``.tree``, the call's figures in
@@ -646,7 +666,9 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     (substitutions are drawn exactly from P(t)).  ``n_threads`` and ``show_progress`` are accepted for compatibility.
     ``seed`` (keyword-only) addresses every draw; None draws one from numpy's global RNG.  With ``haps_gtrees`` each
     region follows its own tree (``.tree`` is None); ``table_budget`` (keyword-only) then bounds the bytes of threshold
-    tables built at once (0: the library's default) and does not change the result."""
+    tables built at once (0: the library's default) and does not change the result.  With ``haps_vcf`` the haplotypes
+    are the file's (``sub``, ``ins`` and ``del_`` must be None; ``n_threads`` host threads inflate it and copy the
+    records out); ``.tree`` is None and ``.stats`` holds the call's figures."""
     from . import _lib
     from .illumina import default_context
 
@@ -654,7 +676,16 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
     if not isinstance(reference, RefGenome):
         _bad(f, "reference", "a \"ref_genome\" object")
     if not isinstance(haps_info, HapsInfo):
-        _bad(f, "haps_info", "a \"haps_info\" object (from `haps_phylo`, `haps_theta` or `haps_gtrees`)")
+        _bad(f, "haps_info", "a \"haps_info\" object (from `haps_phylo`, `haps_theta`, `haps_gtrees` or `haps_vcf`)")
+    if isinstance(haps_info, HapsVcf):
+        if sub is not None or ins is not None or del_ is not None:
+            raise JackalopeError("\nFor `create_haplotypes` with `haps_vcf`, the haplotypes come from the file: "
+                                 "`sub`, `ins` and `del_` must be NULL.")
+        if not (_is_int(n_threads) and 1 <= n_threads <= 64):
+            _bad(f, "n_threads", "a single integer from 1 to 64")
+        if not (_is_int(batch_bytes) and batch_bytes >= 0):
+            _bad(f, "batch_bytes", "a single integer >= 0")
+        return _haps_from_vcf(reference, haps_info, int(n_threads), ctx or default_context(device), batch_bytes)
     if not isinstance(sub, SubModel):
         _bad(f, "sub", "a \"sub_info\" object (from one of the `sub_*` functions)")
     for par, x in (("ins", ins), ("del_", del_)):
@@ -722,6 +753,32 @@ def create_haplotypes(reference, haps_info, sub, ins=None, del_=None, epsilon=0.
         haps.stats.update(ist.as_dict())
     ctx._haps = haps
     return haps
+
+
+def _haps_from_vcf(reference, info, n_threads, ctx, batch_bytes):
+    from . import _lib
+    ctx.set_genome(reference)
+    p = _lib.VcfReadParams(info.path.encode(), n_threads, int(batch_bytes or 0))
+    st = _lib.VcfReadStats()
+    ctx._haps = None
+    ctx._check(ctx.lib.jlp_create_haplotypes_vcf(ctx.h, C.byref(p), C.byref(st)), "jlp_create_haplotypes_vcf")
+    names = [haplotype_name(ctx, h) for h in range(st.haplotypes)]
+    muts = [[haplotype_muts(ctx, h, c) for c in range(reference.n_chroms())] for h in range(len(names))]
+    haps = Haplotypes(reference, names, muts)
+    haps.tree = None
+    haps.stats = st.as_dict()
+    ctx._haps = haps
+    return haps
+
+
+def haplotype_name(ctx, h):
+    """The name the context holds for haplotype h (jlp_haplotype_name)."""
+    n = C.c_uint64()
+    buf = C.create_string_buffer(256)
+    if ctx.lib.jlp_haplotype_name(ctx.h, h, buf, 256, C.byref(n)) != 0 and n.value > 256:
+        buf = C.create_string_buffer(n.value)
+    ctx._check(ctx.lib.jlp_haplotype_name(ctx.h, h, buf, len(buf), C.byref(n)), "jlp_haplotype_name")
+    return buf.raw[:n.value].decode("utf-8", "surrogateescape")
 
 
 def indel_params(ins, del_, epsilon, pi):
