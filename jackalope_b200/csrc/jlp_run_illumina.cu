@@ -39,10 +39,14 @@ Compression compression_of(const jlp_illumina_params* P, SinkKind kind) {
     return z;
 }
 
+int ends_of(const jlp_illumina_params* P) { return P->paired || P->matepair ? 2 : 1; }
+// pairs of a duplicate pool: the pool closes at >= read_pool_size reads
+uint64_t pool_pairs(const jlp_illumina_params* P) { return (P->read_pool_size + ends_of(P) - 1) / ends_of(P); }
+
 // the argument checks the C++ layer of the reference performs, plus the ranges of the additions
 void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, SinkKind kind) {
     if (!P) throw ArgErr("params is NULL");
-    const int n_ends = P->paired || P->matepair ? 2 : 1;
+    const int n_ends = ends_of(P);
     if (c->chrom_off.size() < 2) throw ArgErr("no reference genome has been set");
     if (use_haps && c->haps.empty()) throw ArgErr("no haplotypes have been added");
     if (!c->have_prof[0]) throw ArgErr("no quality profile for read 1");
@@ -67,7 +71,7 @@ void check_params(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P,
 }
 
 LayoutSpec illumina_spec(const jlp_ctx* c, bool use_haps, const jlp_illumina_params* P) {
-    LayoutSpec S(use_haps, P, P->n_reads / (P->paired || P->matepair ? 2 : 1));
+    LayoutSpec S(use_haps, P, P->n_reads / ends_of(P));
     S.barcodes = P->barcodes;
     S.read_len = (uint32_t)c->tab[0].L;
     return S;
@@ -77,74 +81,45 @@ typedef std::vector<std::pair<uint64_t, uint64_t>> Ranges;
 typedef std::vector<std::array<uint64_t, 2>> PerJobBytes;
 
 // What a multi-GPU run tells each of its devices (jlp_ctx_create_multi); a plain call leaves everything empty.
-struct RunExtras {
+struct Piece {
     const Ranges* ranges = nullptr;       // [jobs] the pair range of every job this call generates (else: the shard of P)
-    PerJobBytes* sizes_out = nullptr;     // size pass: only count the FASTQ bytes per job and end of those ranges
     const PerJobBytes* base = nullptr;    // [jobs] where this call's bytes start in each job's files / in the memory sink
     bool shared_files = false;            // the files exist, created and sized by the caller: open without truncating, no EOF block
-    // [jobs] compressed multi-GPU runs: this call writes <name><suffix>, joined by the caller, who appends the BGZF
-    // end-of-file block
-    const std::vector<std::string>* job_suffix = nullptr;
-    PerJobBytes* zsizes_out = nullptr;    // the compressed bytes per job and end this call produced (device coder)
-    bool dry_files = false;               // generate and compress as for files, deliver nothing (sink NONE): the compressed size pass
+    const std::vector<std::string>* suffix = nullptr;   // [jobs] zlib: this call writes <name><suffix>, the caller joins them
 };
 
-// One Illumina run on device d, with the run's Layout (make_layout) and parameters checked (check_params) by the caller.
-void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* P, Layout Y, Output& sink, jlp_run_stats* stats,
-         const RunExtras& X = RunExtras()) {
-    const int n_ends = P->paired || P->matepair ? 2 : 1;
-    const bool matepair = P->matepair != 0;
-    if (use_haps) finish_upload(c, d);
-    const uint64_t h2d_before = d.h2d_bytes;
-    const Compression Z = compression_of(P, X.dry_files ? SINK_FILES : sink.kind);
-    const bool dev_z = Z.dev_z;
-    const bool sizes_only = X.sizes_out != nullptr;
-    if (X.zsizes_out) X.zsizes_out->assign(X.ranges ? X.ranges->size() : 0, std::array<uint64_t, 2>{0, 0});
+// the first and last group the pairs [lo, hi) of job read: those of the pairs, and through a duplicate chain's leader
+// possibly the one before (a leader lies at most pool_pairs - 1 pairs before its duplicate, never before the job's start)
+std::pair<size_t, size_t> groups_of(const Layout& Y, const jlp_illumina_params* P, const Job& job, uint64_t lo, uint64_t hi) {
+    const uint64_t first_pair = lo - std::min<uint64_t>(lo - job.lo, pool_pairs(P) - 1);
+    const size_t g_lo = (size_t)(std::upper_bound(Y.group_off.begin(), Y.group_off.end(), first_pair) - Y.group_off.begin()) - 1;
+    const size_t g_hi = std::min((size_t)(std::upper_bound(Y.group_off.begin(), Y.group_off.end(), hi - 1) - Y.group_off.begin()) - 1,
+                                 Y.groups.size() - 1);
+    return {std::min(g_lo, g_hi), g_hi};
+}
+
+// The groups' sequences on d: the reference's chromosomes, or the haplotype chromosomes the ranges touch (materialised now).
+void bind_sequences(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* P, Layout& Y, const Ranges& ranges) {
+    if (ranges.size() != Y.jobs.size()) throw std::runtime_error("internal: one range per job");
+    for (size_t k = 0; k < Y.jobs.size() && use_haps; k++) {
+        if (ranges[k].second <= ranges[k].first) continue;
+        const auto [g_lo, g_hi] = groups_of(Y, P, Y.jobs[k], ranges[k].first, ranges[k].second);
+        for (size_t g = g_lo; g <= g_hi; g++) ensure_hap_chrom(c, d, Y.group_hap[g], Y.group_chrom[g]);
+    }
+    for (size_t g = 0; g < Y.groups.size(); g++)
+        Y.groups[g].seq = use_haps ? d.hap_seq[Y.group_hap[g]][Y.group_chrom[g]] : d.genome.p + kPad + c->chrom_off[g];
+}
+
+// The kernels' parameters, with the fragment table, the groups, the string pool and a cleared status word uploaded to d
+GenParams gen_params(const jlp_ctx* c, Device& d, const jlp_illumina_params* P, const Layout& Y) {
+    const int n_ends = ends_of(P);
     const double insp[2] = {P->ins_prob1, P->ins_prob2}, delp[2] = {P->del_prob1, P->del_prob2};
-    const uint32_t L = (uint32_t)c->tab[0].L;
-
-    const std::vector<uint64_t>& group_off = Y.group_off;
-    std::vector<GroupDev>& groups = Y.groups;
-    const std::vector<Job>& jobs = Y.jobs;
-
-    // --- the pair range of every job this call generates
-    Ranges ranges;
-    if (X.ranges) ranges = *X.ranges;
-    else {
-        const uint32_t S = P->shard_count > 1 ? P->shard_count : 1, si = P->shard_count > 1 ? P->shard_index : 0;
-        for (const Job& j : jobs) { uint64_t lo, hi; shard_range(j.lo, j.hi, si, S, lo, hi); ranges.emplace_back(lo, hi); }
-    }
-    if (ranges.size() != jobs.size()) throw std::runtime_error("internal: one range per job");
-    const uint64_t pool_pairs = (P->read_pool_size + n_ends - 1) / n_ends;   // pool closes at >= read_pool_size reads
-    // groups a range reads: those of its pairs, and through a duplicate chain's leader possibly the one before
-    // (a leader lies at most pool_pairs - 1 pairs before its duplicate, never before the job's start)
-    auto groups_of = [&](const Job& job, uint64_t lo, uint64_t hi, size_t& g_lo, size_t& g_hi) {
-        const uint64_t first_pair = lo - std::min<uint64_t>(lo - job.lo, pool_pairs - 1);
-        g_lo = (size_t)(std::upper_bound(group_off.begin(), group_off.end(), first_pair) - group_off.begin()) - 1;
-        g_hi = (size_t)(std::upper_bound(group_off.begin(), group_off.end(), hi - 1) - group_off.begin()) - 1;
-        g_hi = std::min(g_hi, groups.size() - 1);
-        g_lo = std::min(g_lo, g_hi);
-    };
-    // --- sequences: the reference's chromosomes, or the haplotype chromosomes the ranges touch (materialised now)
-    if (!use_haps) {
-        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = d.genome.p + kPad + c->chrom_off[g];
-    } else {
-        for (size_t k = 0; k < jobs.size(); k++) {
-            if (ranges[k].second <= ranges[k].first) continue;
-            size_t g_lo, g_hi;
-            groups_of(jobs[k], ranges[k].first, ranges[k].second, g_lo, g_hi);
-            for (size_t g = g_lo; g <= g_hi; g++) ensure_hap_chrom(c, d, Y.group_hap[g], Y.group_chrom[g]);
-        }
-        for (size_t g = 0; g < groups.size(); g++) groups[g].seq = d.hap_seq[Y.group_hap[g]][Y.group_chrom[g]];
-    }
-
-    // --- thresholds
     GenParams gp;
     std::memset(&gp, 0, sizeof gp);
     gp.seed = P->seed;
     philox_round_keys(P->seed, gp.rk);
-    gp.n_ends = n_ends; gp.L = L; gp.matepair = matepair;
-    gp.pool_pairs = pool_pairs;
+    gp.n_ends = n_ends; gp.L = (uint32_t)c->tab[0].L; gp.matepair = P->matepair != 0;
+    gp.pool_pairs = pool_pairs(P);
     Thr td = thr_double_lt(P->prob_dup);
     gp.c_dup = td.thr; gp.dup_never = td.thr == 0;
     gp.c_rev = thr_ld_lt(0.5).thr;
@@ -163,33 +138,39 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
     std::vector<uint32_t> guide = frag_guide(frag);
     d.d_frag.upload(frag, d.s_compute);
     d.d_frag_guide.upload(guide, d.s_compute);
-    d.d_group_off.upload(group_off, d.s_compute);
-    d.d_groups.upload(groups, d.s_compute);
+    d.d_group_off.upload(Y.group_off, d.s_compute);
+    d.d_groups.upload(Y.groups, d.s_compute);
     d.d_strpool.upload(Y.strpool, d.s_compute);
     d.d_status.ensure(1);
     CK(cudaMemsetAsync(d.d_status.p, 0, sizeof(uint32_t), d.s_compute));
-    d.h2d_bytes += frag.size() * 8 + group_off.size() * 8 + groups.size() * sizeof(GroupDev) + Y.strpool.size();
+    d.h2d_bytes += frag.size() * 8 + Y.group_off.size() * 8 + Y.groups.size() * sizeof(GroupDev) + Y.strpool.size();
     gp.frag_cdf = d.d_frag.p; gp.frag_guide = d.d_frag_guide.p; gp.frag_n = (uint32_t)frag.size(); gp.frag_min = P->frag_len_min;
-    gp.group_off = d.d_group_off.p; gp.n_groups = (uint32_t)groups.size();
+    gp.group_off = d.d_group_off.p; gp.n_groups = (uint32_t)Y.groups.size();
     gp.groups = d.d_groups.p; gp.strpool = d.d_strpool.p; gp.status = d.d_status.p;
+    return gp;
+}
 
-    // --- batch buffers
+struct Batches { uint64_t B; uint32_t nblk; };   // pairs per batch, BGZF blocks of a file's batch
+
+// The pairs per batch, the read kernel's record buffers in gp, and every slot's buffers: placement and scan; FASTQ for
+// n_out files (none: no read kernel runs), pinned host copies of it (need_host); the device coder's (dev_z).
+Batches size_batches(Device& d, GenParams& gp, const Layout& Y, const Ranges& ranges, const jlp_illumina_params* P, int n_out,
+                     bool need_host, bool dev_z) {
     uint64_t max_range = 0;
     for (const auto& r : ranges) max_range = std::max(max_range, r.second - r.first);
     uint64_t B = P->batch_pairs ? P->batch_pairs : (1ull << 20);
     B = std::max<uint64_t>(1, std::min(B, max_range));
     uint32_t max_prefix = 0;
-    for (const GroupDev& g : groups) max_prefix = std::max(max_prefix, g.prefix_len);
-    const uint64_t max_rec = (uint64_t)max_prefix + 20 + 5 + 2ull * L + 4;
+    for (const GroupDev& g : Y.groups) max_prefix = std::max(max_prefix, g.prefix_len);
+    const uint64_t max_rec = (uint64_t)max_prefix + 20 + 5 + 2ull * gp.L + 4;
     B = std::max<uint64_t>(1, std::min<uint64_t>(B, 0xfff00000ull / max_rec));     // offsets inside a batch's output are 32 bits wide in k_reads
     gp.rec_buf = (uint32_t)((max_rec + 32 + 15) & ~15ull);   // a record at any 16-byte phase, and the 16 bytes the carry reads behind it
-    gp.tpl_buf = (L + 50u + 15u) & ~15u;        // the template, 16..31 bytes in front of it, 16 behind, the word over-read
-    gp.cod_buf = (L + 40u + 15u) & ~15u;        // base codes of a read's template (up to 2 more than the read with deletions), rounded up to the 16 of a lane
-    if (!sizes_only && !reads_fits(gp)) throw Unsupported("read_length " + std::to_string(L) + " (with these chromosome names) needs more shared memory per "
-                                                          "read pair than one SM has: the read kernel cannot hold such a record");
-    const uint64_t n_rec_max = B * n_ends;
+    gp.tpl_buf = (gp.L + 50u + 15u) & ~15u;     // the template, 16..31 bytes in front of it, 16 behind, the word over-read
+    gp.cod_buf = (gp.L + 40u + 15u) & ~15u;     // base codes of a read's template (up to 2 more than the read with deletions), rounded up to the 16 of a lane
+    if (n_out && !reads_fits(gp)) throw Unsupported("read_length " + std::to_string(gp.L) + " (with these chromosome names) needs more shared memory per "
+                                                    "read pair than one SM has: the read kernel cannot hold such a record");
+    const uint64_t n_rec_max = B * ends_of(P);
     const uint32_t nsb_max = (uint32_t)((B + kScanBlock - 1) / kScanBlock);
-    const bool need_host = sink.kind != SINK_NONE && !sizes_only;
     const uint32_t nblk = (uint32_t)((B * max_rec + kBgzfIn - 1) / kBgzfIn) + 1;
     for (Slot& s : d.slot) {
         s.plan.ensure(n_rec_max);
@@ -200,22 +181,75 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
         s.totals.ensure(4);
         s.h_totals.ensure(4);
         CK(cudaMemsetAsync(s.totals.p, 0, 4 * sizeof(uint64_t), d.s_compute));
-        for (int e = 0; e < n_ends && !sizes_only; e++) {
+        for (int e = 0; e < n_out; e++) {
             s.out[e].ensure(B * max_rec + 64);
             // compressed bytes of a batch never exceed its FASTQ bytes plus the members' framing (an incompressible block is stored)
             // (the same size with and without compression: pinning a gigabyte again for the first compressed call took seconds)
             if (need_host) s.h_out[e].ensure(B * max_rec + (size_t)nblk * 64 + 64);
         }
-        if (dev_z && !sizes_only) s.z.ensure(nblk, B * max_rec, n_ends);
+        if (dev_z) s.z.ensure(nblk, B * max_rec, ends_of(P));
         s.busy = false;
     }
+    return Batches{B, nblk};
+}
 
-    jlp_run_stats st;
-    std::memset(&st, 0, sizeof st);
+// A deferred genome upload: the compute stream waits for exactly the uploads of the chromosomes the batch [b0, b1) reads.
+// The first batch of this call's part [lo, hi) of the job copies, in the order the part reads them, all its chromosomes and
+// nothing else (with N GPUs each needs about 1/N of the genome); the rest stays on the host until some run asks for it.
+void wait_chromosomes(const jlp_ctx* c, Device& d, const Layout& Y, const jlp_illumina_params* P, const Job& job, uint64_t lo,
+                      uint64_t hi, uint64_t b0, uint64_t b1, std::vector<char>& waited) {
+    auto [g_lo, g_hi] = groups_of(Y, P, job, b0, b1);
+    g_hi = std::min(g_hi, d.chrom_ev.size() - 1);
+    g_lo = std::min(g_lo, g_hi);
+    if (b0 == lo) issue_upload(c, d, g_lo, std::min(groups_of(Y, P, job, lo, hi).second, d.chrom_ev.size() - 1));
+    issue_upload(c, d, g_lo, g_hi);
+    for (size_t g = g_lo; g <= g_hi; g++)
+        if (!waited[g]) { CK(cudaStreamWaitEvent(d.s_compute, d.chrom_ev[g], 0)); waited[g] = 1; }
+}
 
+// After a run's last batch: its time, the deferred upload's bookkeeping, the device's status word and the statistics.
+void finish(Device& d, jlp_run_stats& st, uint64_t h2d_before, jlp_run_stats* stats) {
+    CK(cudaEventRecord(d.ev_run[1], d.s_compute));
+    CK(cudaEventSynchronize(d.ev_run[1]));
+    st.run_ms = elapsed_ms(d.ev_run[0], d.ev_run[1]);
+    if (d.upload_pending) {
+        // the copies this run issued are done before the caller gets control back; chromosomes no
+        // shard of this run touched remain on the host (upload_src must stay valid, see the header)
+        CK(cudaStreamSynchronize(d.s_upload));
+        if (std::find(d.chrom_resident.begin(), d.chrom_resident.end(), 0) == d.chrom_resident.end()) {
+            d.upload_pending = false;
+            d.upload_src = nullptr;
+        }
+    }
+    uint32_t status = 0;
+    CK(cudaMemcpy(&status, d.d_status.p, sizeof status, cudaMemcpyDeviceToHost));
+    if (status & 1u) throw ArgErr("a barcode is at least as long as a read's template (fragment or chromosome too short)");
+    st.h2d_bytes = d.h2d_bytes - h2d_before;      // of this call (a deferred genome upload it performed included)
+    if (stats) *stats = st;
+}
+
+// One Illumina run on device d, with the run's Layout (make_layout) and parameters checked (check_params) by the caller.
+// Returns the device coder's bytes per job and file: into SINK_NONE with the files' Compression Z, a dry run sizes them.
+PerJobBytes run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* P, const Compression& Z, Layout Y,
+                Output& sink, jlp_run_stats* stats, const Piece& piece = Piece()) {
+    const int n_ends = ends_of(P);
+    const bool dev_z = Z.dev_z, need_host = sink.kind != SINK_NONE;
+    if (use_haps) finish_upload(c, d);
+    const uint64_t h2d_before = d.h2d_bytes;
+    Ranges ranges;
+    if (piece.ranges) ranges = *piece.ranges;
+    else {
+        const uint32_t S = P->shard_count > 1 ? P->shard_count : 1, si = P->shard_count > 1 ? P->shard_index : 0;
+        for (const Job& j : Y.jobs) { uint64_t lo, hi; shard_range(j.lo, j.hi, si, S, lo, hi); ranges.emplace_back(lo, hi); }
+    }
+    bind_sequences(c, d, use_haps, P, Y, ranges);
+    GenParams gp = gen_params(c, d, P, Y);
+    const Batches b = size_batches(d, gp, Y, ranges, P, n_ends, need_host, dev_z);
+    jlp_run_stats st{};
+    PerJobBytes zbytes(Y.jobs.size());
     sink.begin(Z, P->compress, P->n_threads, d.writers);
     Quiesce quiesce{d, &sink};
-    uint64_t job_index = 0;
+    size_t jk = 0;
     // stage 2 of a batch: its kernels are done -> statistics, then its FASTQ starts its way to the host
     // (queued right behind the previous batch's copy, so the bus never idles)
     auto issue_copy = [&](Slot& s) {
@@ -227,7 +261,7 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
         for (int e = 0; e < n_ends; e++) {
             s.tot[e] = s.h_totals.p[e]; st.bytes_out[e] += s.tot[e];
             s.ztot[e] = dev_z ? s.h_totals.p[2 + e] : 0; st.z_bytes[e] += s.ztot[e];
-            if (X.zsizes_out && job_index < X.zsizes_out->size()) (*X.zsizes_out)[job_index][e] += s.ztot[e];
+            zbytes[jk][e] += s.ztot[e];
         }
         st.pairs += s.pairs;
         st.batches++;
@@ -246,44 +280,21 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
             CK(cudaEventSynchronize(s.ev[4]));
             const uint8_t* data[2] = {s.h_out[0].p, s.h_out[1].p};
             const uint64_t n[2] = {dev_z ? s.ztot[0] : s.tot[0], dev_z ? s.ztot[1] : s.tot[1]};
-            sink.deliver(s.host, data, n, job_index, n_ends);
+            sink.deliver(s.host, data, n, jk, n_ends);
         }
         if (P->progress_cb) P->progress_cb(P->cb_user, (uint64_t)s.pairs * n_ends);
         s.busy = false;
     };
 
     std::vector<char> chrom_waited(d.chrom_ev.size(), 0);
-    if (sizes_only) X.sizes_out->assign(jobs.size(), std::array<uint64_t, 2>{0, 0});
-
-    for (size_t jk = 0; jk < jobs.size(); jk++) {
-        const Job& job = jobs[jk];
+    for (jk = 0; jk < Y.jobs.size(); jk++) {
+        const Job& job = Y.jobs[jk];
         const uint64_t lo = ranges[jk].first, hi = ranges[jk].second;
         if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();   // src/hts.h:536
-        if (X.ranges && hi <= lo) { job_index++; continue; }             // a multi-GPU device with no part in this job's files
-        if (!sizes_only) {
-            std::string names[2];
-            for (int e = 0; e < n_ends; e++)
-                names[e] = file_name(job, e, Z.want_gz, P) + (X.job_suffix ? (*X.job_suffix)[jk] : "");
-            sink.open_job(names, n_ends, X.base ? (*X.base)[jk].data() : nullptr, X.shared_files);
-        }
-        if (sizes_only) {
-            // size pass: placement and scan only; the totals come back batch by batch (a few hundred microseconds each)
-            for (uint64_t b0 = lo; b0 < hi; b0 += B) {
-                Slot& s = d.slot[0];
-                const uint32_t np = (uint32_t)std::min<uint64_t>(B, hi - b0);
-                gp.job_lo = job.lo; gp.job_hi = job.hi; gp.batch_lo = b0; gp.batch_pairs = np;
-                gp.plan = s.plan.p; gp.rec_len = s.rec_len.p; gp.rec_local = s.rec_local.p; gp.block_base = s.block_base.p;
-                gp.n_scan_blocks = (np + kScanBlock - 1) / kScanBlock;
-                CK(launch_place(gp, d.s_compute));
-                CK(launch_scan(s.rec_len.p, np * n_ends, n_ends, s.rec_local.p, s.block_tot.p, s.block_base.p, s.totals.p, d.s_compute));
-                CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
-                CK(cudaStreamSynchronize(d.s_compute));
-                for (int e = 0; e < n_ends; e++) (*X.sizes_out)[jk][e] += s.h_totals.p[e];
-                st.kernel_launches += 3; st.pairs += np; st.batches++;
-            }
-            job_index++;
-            continue;
-        }
+        if (piece.ranges && hi <= lo) continue;                         // a multi-GPU device with no part in this job's files
+        std::string names[2];
+        for (int e = 0; e < n_ends; e++) names[e] = file_name(job, e, Z.want_gz, P) + (piece.suffix ? (*piece.suffix)[jk] : "");
+        sink.open_job(names, n_ends, piece.base ? (*piece.base)[jk].data() : nullptr, piece.shared_files);
         // three batches in flight: batch b computes while b-1 crosses PCIe and b-2 is handed to the sink
         std::deque<Slot*> computing, copying;
         auto drain_one = [&]() {
@@ -291,27 +302,11 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
             else if (!computing.empty()) { issue_copy(*computing.front()); copying.push_back(computing.front()); computing.pop_front(); }
         };
         uint64_t bi = 0;
-        for (uint64_t b0 = lo; b0 < hi; b0 += B, bi++) {
+        for (uint64_t b0 = lo; b0 < hi; b0 += b.B, bi++) {
             Slot& s = d.slot[bi % 3];
             while (s.busy) drain_one();
-            const uint32_t np = (uint32_t)std::min<uint64_t>(B, hi - b0);
-            if (d.upload_pending && !use_haps) {
-                // make the compute stream wait for exactly the uploads of the chromosomes this batch reads
-                size_t g_lo, g_hi;
-                groups_of(job, b0, b0 + np, g_lo, g_hi);
-                g_hi = std::min(g_hi, d.chrom_ev.size() - 1);
-                g_lo = std::min(g_lo, g_hi);
-                if (b0 == lo) {
-                    // first batch of this call's part of the job: a deferred upload copies, in the order the part
-                    // will read them, all the chromosomes it reads and nothing else (with N GPUs each needs about
-                    // 1/N of the genome); the rest stays on the host until some run asks for it
-                    size_t g_end = (size_t)(std::upper_bound(group_off.begin(), group_off.end(), hi - 1) - group_off.begin()) - 1;
-                    issue_upload(c, d, g_lo, std::min(g_end, d.chrom_ev.size() - 1));
-                }
-                issue_upload(c, d, g_lo, g_hi);
-                for (size_t g = g_lo; g <= g_hi; g++)
-                    if (!chrom_waited[g]) { CK(cudaStreamWaitEvent(d.s_compute, d.chrom_ev[g], 0)); chrom_waited[g] = 1; }
-            }
+            const uint32_t np = (uint32_t)std::min<uint64_t>(b.B, hi - b0);
+            if (d.upload_pending && !use_haps) wait_chromosomes(c, d, Y, P, job, lo, hi, b0, b0 + np, chrom_waited);
             gp.job_lo = job.lo; gp.job_hi = job.hi; gp.batch_lo = b0; gp.batch_pairs = np;
             const uint32_t n_rec = np * n_ends;
             const uint32_t nsb = (np + kScanBlock - 1) / kScanBlock;
@@ -326,7 +321,7 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
             CK(launch_reads(gp, d.n_sm, d.s_compute));
             CK(cudaEventRecord(s.ev[3], d.s_compute));
             if (dev_z) {
-                CK(s.z.launch(s.out[0].p, s.out[1].p, s.totals.p, nblk, P->compress, d.s_compute));
+                CK(s.z.launch(s.out[0].p, s.out[1].p, s.totals.p, b.nblk, P->compress, d.s_compute));
                 st.kernel_launches += kBgzfLaunches;
             }
             CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
@@ -342,27 +337,47 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
         while (!computing.empty() || !copying.empty()) drain_one();
         for (Slot& s : d.slot) sink.settle(s.host);
         // a multi-GPU run appends the end-of-file block once, after joining the parts
-        sink.end_job(job_index, n_ends, !X.shared_files && !X.job_suffix);
-        job_index++;
+        sink.end_job(jk, n_ends, !piece.shared_files && !piece.suffix);
     }
-    CK(cudaEventRecord(d.ev_run[1], d.s_compute));
-    CK(cudaEventSynchronize(d.ev_run[1]));
-    st.run_ms = elapsed_ms(d.ev_run[0], d.ev_run[1]);
-    if (d.upload_pending) {
-        // the copies this run issued are done before the caller gets control back; chromosomes no
-        // shard of this run touched remain on the host (upload_src must stay valid, see the header)
-        CK(cudaStreamSynchronize(d.s_upload));
-        if (std::find(d.chrom_resident.begin(), d.chrom_resident.end(), 0) == d.chrom_resident.end()) {
-            d.upload_pending = false;
-            d.upload_src = nullptr;
+    finish(d, st, h2d_before, stats);
+    quiesce.armed = false;
+    return zbytes;
+}
+
+// The FASTQ bytes per job and file that run() writes on device d for the given ranges: placement and scan only, the
+// totals come back batch by batch (a few hundred microseconds each).
+PerJobBytes count_bytes(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* P, Layout Y, const Ranges& ranges,
+                        jlp_run_stats* stats) {
+    const int n_ends = ends_of(P);
+    if (use_haps) finish_upload(c, d);
+    const uint64_t h2d_before = d.h2d_bytes;
+    bind_sequences(c, d, use_haps, P, Y, ranges);
+    GenParams gp = gen_params(c, d, P, Y);
+    const Batches b = size_batches(d, gp, Y, ranges, P, 0, false, false);
+    jlp_run_stats st{};
+    PerJobBytes bytes(Y.jobs.size());
+    Output none;
+    none.begin(Compression(), P->compress, P->n_threads, d.writers);
+    Quiesce quiesce{d, &none};
+    Slot& s = d.slot[0];
+    for (size_t jk = 0; jk < Y.jobs.size(); jk++) {
+        if (P->abort_cb && P->abort_cb(P->cb_user)) throw Aborted();
+        for (uint64_t b0 = ranges[jk].first; b0 < ranges[jk].second; b0 += b.B) {
+            const uint32_t np = (uint32_t)std::min<uint64_t>(b.B, ranges[jk].second - b0);
+            gp.job_lo = Y.jobs[jk].lo; gp.job_hi = Y.jobs[jk].hi; gp.batch_lo = b0; gp.batch_pairs = np;
+            gp.plan = s.plan.p; gp.rec_len = s.rec_len.p; gp.rec_local = s.rec_local.p; gp.block_base = s.block_base.p;
+            gp.n_scan_blocks = (np + kScanBlock - 1) / kScanBlock;
+            CK(launch_place(gp, d.s_compute));
+            CK(launch_scan(s.rec_len.p, np * n_ends, n_ends, s.rec_local.p, s.block_tot.p, s.block_base.p, s.totals.p, d.s_compute));
+            CK(cudaMemcpyAsync(s.h_totals.p, s.totals.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, d.s_compute));
+            CK(cudaStreamSynchronize(d.s_compute));
+            for (int e = 0; e < n_ends; e++) bytes[jk][e] += s.h_totals.p[e];
+            st.kernel_launches += 3; st.pairs += np; st.batches++;
         }
     }
-    uint32_t status = 0;
-    CK(cudaMemcpy(&status, d.d_status.p, sizeof status, cudaMemcpyDeviceToHost));
-    if (status & 1u) throw ArgErr("a barcode is at least as long as a read's template (fragment or chromosome too short)");
-    st.h2d_bytes = d.h2d_bytes - h2d_before;      // of this call (a deferred genome upload it performed included)
-    if (stats) *stats = st;
+    finish(d, st, h2d_before, stats);
     quiesce.armed = false;
+    return bytes;
 }
 
 // ------------------------------------------------- one call, several GPUs ---
@@ -373,9 +388,9 @@ void run(const jlp_ctx* c, Device& d, bool use_haps, const jlp_illumina_params* 
 // space [0, n_pairs) is cut into near-equal contiguous pieces, one per device (a piece may cover several
 // haplotypes' jobs with sep_files, and a job may have several writers); every device runs the three-stage batch
 // pipeline of run() on its piece from its own host thread.  No data moves between the devices (no collective):
-//   plain FASTQ   a size pass (placement + scan only, a few hundred microseconds per batch) tells every device how
-//                 many bytes it will write per job and file, so the devices write into disjoint ranges of the
-//                 same, pre-sized R1 / R2 files (or of the caller's memory buffers) -- R1 and R2 stay aligned;
+//   plain FASTQ   a size pass (count_bytes) tells every device how many bytes it will write per job and file, so the
+//                 devices write into disjoint ranges of the same, pre-sized R1 / R2 files (or of the caller's memory
+//                 buffers) -- R1 and R2 stay aligned;
 //   compressed    by the device coder: the devices first generate and compress their pieces without delivering them
 //                 (a dry run: they are some fifty times faster than any sink), which gives every piece's compressed
 //                 size; then the files are pre-sized and every device writes its BGZF members straight to their
@@ -392,6 +407,99 @@ struct MultiShared {
 int multi_abort_cb(void* u) { return static_cast<MultiShared*>(u)->abort.load(std::memory_order_relaxed); }
 void multi_progress_cb(void* u, uint64_t reads) { static_cast<MultiShared*>(u)->progress.fetch_add(reads, std::memory_order_relaxed); }
 
+// Where each device's bytes start in each job's output, the devices in order, every job from 0 (files) or behind the one
+// before (concat: memory), from the bytes every device produces per job.  Returns where each job's bytes end.
+PerJobBytes offsets(const std::vector<PerJobBytes>& sizes, bool concat, std::vector<PerJobBytes>& base) {
+    const size_t nj = sizes[0].size();
+    base.assign(sizes.size(), PerJobBytes(nj));
+    PerJobBytes end(nj);
+    for (size_t k = 0; k < nj; k++)
+        for (int e = 0; e < 2; e++) {
+            uint64_t o = concat && k ? end[k - 1][e] : 0;
+            for (size_t r = 0; r < sizes.size(); r++) { base[r][k][e] = o; o += sizes[r][k][e]; }
+            end[k][e] = o;
+        }
+    return end;
+}
+
+// Every job's shared files created with their final size at once (no pages yet; pages are reserved slice by slice by the
+// devices' writer threads, see Output::deliver), bgzf_close's empty end-of-file block written now (gz); a file system
+// that cannot hold everything the run will write is reported here rather than half-way through.
+void create_sized(const Layout& Y, const jlp_illumina_params* P, const PerJobBytes& bytes, bool gz) {
+    const uint64_t tail = gz ? sizeof kBgzfEof : 0;
+    uint64_t need_bytes = 0;
+    for (size_t k = 0; k < Y.jobs.size(); k++)
+        for (int e = 0; e < ends_of(P); e++) {
+            const std::string name = file_name(Y.jobs[k], e, gz, P);
+            const uint64_t size = bytes[k][e] + tail;
+            const int fd = ::open(name.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
+            if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");      // src/io.h:288-290
+            need_bytes += size;
+            struct statvfs vfs;
+            const int rc = ::fstatvfs(fd, &vfs) == 0 && (uint64_t)vfs.f_bavail * vfs.f_frsize < need_bytes ? ENOSPC
+                           : ::ftruncate(fd, (off_t)size) == 0 ? 0 : errno;
+            const std::string w = rc ? std::strerror(rc) : pwrite_all(fd, kBgzfEof, tail, size - tail);
+            ::close(fd);
+            if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
+        }
+}
+
+// zlib output: the parts move behind the first device's bytes in device order (their offsets are known now), slices of
+// them copied by several threads at once; one end-of-file block per file (eof)
+void join_parts(jlp_ctx* c, const Layout& Y, const jlp_illumina_params* P, bool eof, const std::vector<Ranges>& ranges,
+                const std::vector<size_t>& first_dev) {
+    const size_t N = ranges.size();
+    struct CopyTask { int in_fd, out_fd; uint64_t in_off, out_off, len; };
+    std::vector<CopyTask> tasks;
+    std::vector<int> fds;
+    struct CloseAll { std::vector<int>& f; ~CloseAll() { for (int x : f) ::close(x); } } close_all{fds};
+    for (size_t k = 0; k < Y.jobs.size(); k++)
+        for (int e = 0; e < ends_of(P); e++) {
+            const std::string name = file_name(Y.jobs[k], e, true, P);
+            const int fd = ::open(name.c_str(), first_dev[k] < N ? O_RDWR : (O_RDWR | O_CREAT | O_TRUNC), 0644);
+            if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");
+            fds.push_back(fd);
+            struct stat sb;
+            if (::fstat(fd, &sb) != 0) throw IoErr("Error writing to file " + name + ": " + std::strerror(errno));
+            uint64_t pos = (uint64_t)sb.st_size;
+            for (size_t r = 0; r < N; r++) {
+                if (ranges[r][k].second <= ranges[r][k].first || r == first_dev[k]) continue;
+                const std::string part = name + ".part" + std::to_string(r);
+                const int in = ::open(part.c_str(), O_RDONLY);
+                if (in < 0 || ::fstat(in, &sb) != 0) { if (in >= 0) ::close(in); throw IoErr("cannot read " + part); }
+                fds.push_back(in);
+                const uint64_t slice = 64ull << 20;
+                for (uint64_t o = 0; o < (uint64_t)sb.st_size; o += slice)
+                    tasks.push_back(CopyTask{in, fd, o, pos + o, std::min<uint64_t>(slice, (uint64_t)sb.st_size - o)});
+                pos += (uint64_t)sb.st_size;
+            }
+            if (::ftruncate(fd, (off_t)(pos + (eof ? sizeof kBgzfEof : 0))) != 0)
+                throw IoErr("Error writing to file " + name + ": " + std::strerror(errno));
+            const std::string w = pwrite_all(fd, kBgzfEof, eof ? sizeof kBgzfEof : 0, pos);
+            if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
+        }
+    // a slice is copied through mappings of both files where that works (threads writing one file through
+    // write() / copy_file_range queue on its inode lock; page-cache pages filled through a mapping do not), else by
+    // copy_range; the writer threads of the first device do the copying
+    WriterPool& writers = c->dev[0]->writers;
+    std::atomic<int> pending{0};
+    writers.start(std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32)));
+    for (const CopyTask& t : tasks)
+        writers.submit(&pending, [t]() {
+            Mapping mo, mi;
+            std::string w;
+            if (map_range(t.out_fd, t.out_off, t.len, mo) && map_range(t.in_fd, t.in_off, t.len, mi, true))
+                std::memcpy(mo.at, mi.at, t.len);
+            else
+                w = copy_range(t.out_fd, t.out_off, t.in_fd, t.in_off, t.len);
+            mi.unmap();
+            mo.unmap();
+            return w;
+        });
+    const std::string w = writers.wait(pending);
+    if (!w.empty()) { writers.clear_error(); throw IoErr("Error joining the devices' parts: " + w); }
+}
+
 void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& sink, jlp_run_stats* stats) {
     if (sink.kind == SINK_STREAM)
         throw Unsupported("jlp_illumina_stream on a multi-GPU context: batches of several devices have no single order; "
@@ -400,16 +508,12 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
     const size_t N = c->dev.size();
     const Layout Y = make_layout(c, illumina_spec(c, use_haps, P));
     const size_t nj = Y.jobs.size();
-    const int n_ends = P->paired || P->matepair ? 2 : 1;
     const Compression Z = compression_of(P, sink.kind);
     if (Z.want_gz && Z.dev_z && sink.kind == SINK_MEMORY)
         throw Unsupported("compressed output into memory on a multi-GPU context");
     const bool sized = sink.kind == SINK_MEMORY || (sink.kind == SINK_FILES && !Z.want_gz);   // plain bytes at known offsets
-    // compressed by the device coder: the sizes come from a dry run (the devices generate and compress everything once
-    // without delivering it -- they are some fifty times faster than any sink), then every device writes its members
-    // straight to their final place; compressed by zlib on the host: part files, joined afterwards
-    const bool zsized = sink.kind == SINK_FILES && Z.want_gz && Z.dev_z;
-    const bool parts = sink.kind == SINK_FILES && Z.want_gz && !Z.dev_z;
+    const bool zsized = sink.kind == SINK_FILES && Z.want_gz && Z.dev_z;   // device coder: sized by a dry run
+    const bool parts = sink.kind == SINK_FILES && Z.want_gz && !Z.dev_z;   // zlib on the host: part files, joined afterwards
 
     // --- the devices' pieces of the pair-index space, per job
     std::vector<Ranges> ranges(N, Ranges(nj));
@@ -428,7 +532,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
     Pk.abort_cb = multi_abort_cb; Pk.progress_cb = multi_progress_cb; Pk.cb_user = &shared;
     Pk.n_threads = P->n_threads <= 1 ? 1 : std::max<uint64_t>(2, (P->n_threads + N - 1) / N);   // host writer threads per device
 
-    std::vector<jlp_run_stats> st(N);
+    std::vector<jlp_run_stats> st(N), pre(N);   // the run's, the size pass's (of which only the launches are reported)
     auto serve_callbacks = [&]() {
         const uint64_t n = shared.progress.exchange(0);
         if (n && P->progress_cb) P->progress_cb(P->cb_user, n);
@@ -452,68 +556,26 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
         if (shared.abort.load() == 2) throw Aborted();
     };
 
-    // a shared output file is created with its final size at once (no pages yet; pages are reserved slice by slice by the
-    // devices' writer threads, see Output::deliver), its last `tail` bytes written now; a file system that cannot hold
-    // everything the run will write is reported here rather than half-way through
-    uint64_t need_bytes = 0;
-    auto create_sized = [&](const std::string& name, uint64_t size, const uint8_t* tail, uint64_t tail_len) {
-        const int fd = ::open(name.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
-        if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");      // src/io.h:288-290
-        need_bytes += size;
-        struct statvfs vfs;
-        const int rc = ::fstatvfs(fd, &vfs) == 0 && (uint64_t)vfs.f_bavail * vfs.f_frsize < need_bytes ? ENOSPC
-                       : ::ftruncate(fd, (off_t)size) == 0 ? 0 : errno;
-        const std::string w = rc ? std::strerror(rc) : pwrite_all(fd, tail, tail_len, size - tail_len);
-        ::close(fd);
-        if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
-    };
-
-    // --- size pass
-    std::vector<PerJobBytes> sizes(N), base(N, PerJobBytes(nj, std::array<uint64_t, 2>{0, 0}));
-    std::vector<std::array<uint64_t, 2>> job_total(nj, std::array<uint64_t, 2>{0, 0});
-    uint64_t launches = 0;
+    // --- plain size pass
+    std::vector<PerJobBytes> base;
     if (sized) {
-        on_devices([&](Device& d, size_t r) {
-            Output none;
-            RunExtras X;
-            X.ranges = &ranges[r]; X.sizes_out = &sizes[r];
-            run(c, d, use_haps, &Pk, Y, none, &st[r], X);
-        }, false);
-        uint64_t mem_off[2] = {0, 0};
-        for (size_t k = 0; k < nj; k++)
-            for (int e = 0; e < n_ends; e++) {
-                uint64_t o = sink.kind == SINK_MEMORY ? mem_off[e] : 0;      // memory: the jobs' outputs are concatenated
-                for (size_t r = 0; r < N; r++) { base[r][k][e] = o; o += sizes[r][k][e]; }
-                job_total[k][e] = o - (sink.kind == SINK_MEMORY ? mem_off[e] : 0);
-                mem_off[e] += job_total[k][e];
-            }
-        for (size_t r = 0; r < N; r++) launches += st[r].kernel_launches;
-        if (sink.kind == SINK_FILES)
-            for (size_t k = 0; k < nj; k++)
-                for (int e = 0; e < n_ends; e++) create_sized(file_name(Y.jobs[k], e, false, P), job_total[k][e], nullptr, 0);
-        if (sink.kind == SINK_MEMORY) { sink.len[0] = mem_off[0]; sink.len[1] = mem_off[1]; }
+        std::vector<PerJobBytes> sizes(N);
+        on_devices([&](Device& d, size_t r) { sizes[r] = count_bytes(c, d, use_haps, &Pk, Y, ranges[r], &pre[r]); }, false);
+        const PerJobBytes end = offsets(sizes, sink.kind == SINK_MEMORY, base);    // memory: the jobs' outputs are concatenated
+        if (sink.kind == SINK_FILES) create_sized(Y, P, end, false);
+        if (sink.kind == SINK_MEMORY) { sink.len[0] = end.back()[0]; sink.len[1] = end.back()[1]; }
     }
 
-    // --- compressed size pass (device coder)
+    // --- device-BGZF dry run
     std::vector<PerJobBytes> zsizes(N), zcheck(N);
     if (zsized) {
         jlp_illumina_params Pdry = Pk;
         Pdry.progress_cb = nullptr;
         on_devices([&](Device& d, size_t r) {
             Output none;
-            RunExtras X;
-            X.ranges = &ranges[r]; X.zsizes_out = &zsizes[r]; X.dry_files = true;
-            run(c, d, use_haps, &Pdry, Y, none, &st[r], X);
+            zsizes[r] = run(c, d, use_haps, &Pdry, Z, Y, none, &pre[r], Piece{&ranges[r]});
         }, true);
-        for (size_t r = 0; r < N; r++) launches += st[r].kernel_launches;
-        for (size_t k = 0; k < nj; k++)
-            for (int e = 0; e < n_ends; e++) {
-                uint64_t o = 0;
-                for (size_t r = 0; r < N; r++) { base[r][k][e] = o; o += zsizes[r][k][e]; }
-                job_total[k][e] = o;
-                // bgzf_close: one empty block ends the file
-                create_sized(file_name(Y.jobs[k], e, true, P), o + sizeof kBgzfEof, kBgzfEof, sizeof kBgzfEof);
-            }
+        create_sized(Y, P, offsets(zsizes, false, base), true);
     }
 
     // --- the run proper
@@ -521,7 +583,7 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
         std::vector<std::string> names;
         ~Cleanup() { for (const std::string& n : names) ::unlink(n.c_str()); }
     } cleanup;
-    // compressed: for every job the first device with a part in it writes the file itself, the others write parts
+    // zlib: for every job the first device with a part in it writes <name> itself (no EOF block yet), device r <name>.part<r>
     std::vector<size_t> first_dev(nj, N);
     for (size_t k = 0; k < nj; k++)
         for (size_t r = N; r-- > 0;) if (ranges[r][k].second > ranges[r][k].first) first_dev[k] = r;
@@ -529,96 +591,33 @@ void run_multi(jlp_ctx* c, bool use_haps, const jlp_illumina_params* P, Output& 
         for (size_t r = 0; r < N; r++)
             for (size_t k = 0; k < nj; k++)
                 if (ranges[r][k].second > ranges[r][k].first && r != first_dev[k])
-                    for (int e = 0; e < n_ends; e++) cleanup.names.push_back(file_name(Y.jobs[k], e, true, P) + ".part" + std::to_string(r));
+                    for (int e = 0; e < ends_of(P); e++) cleanup.names.push_back(file_name(Y.jobs[k], e, true, P) + ".part" + std::to_string(r));
     on_devices([&](Device& d, size_t r) {
         Output sk(sink.kind);
         for (int e = 0; e < 2; e++) { sk.mem[e] = sink.mem[e]; sk.cap[e] = sink.cap[e]; }
-        RunExtras X;
-        X.ranges = &ranges[r];
-        if (sized) { X.base = &base[r]; X.shared_files = sink.kind == SINK_FILES; }
-        if (zsized) { X.base = &base[r]; X.shared_files = true; X.zsizes_out = &zcheck[r]; }
         std::vector<std::string> suffix;
-        if (parts) {
-            // per job: the job's first device writes <name> itself (no EOF block yet), every other one <name>.part<r>
-            X.job_suffix = &suffix;
-            for (size_t k = 0; k < nj; k++) suffix.push_back(r == first_dev[k] ? std::string() : ".part" + std::to_string(r));
-        }
-        run(c, d, use_haps, &Pk, Y, sk, &st[r], X);
+        for (size_t k = 0; k < nj && parts; k++) suffix.push_back(r == first_dev[k] ? std::string() : ".part" + std::to_string(r));
+        const Piece piece{&ranges[r], sized || zsized ? &base[r] : nullptr, sink.kind == SINK_FILES && (sized || zsized),
+                          parts ? &suffix : nullptr};
+        zcheck[r] = run(c, d, use_haps, &Pk, Z, Y, sk, &st[r], piece);
     }, true);
 
     if (zsized)         // the coder is deterministic; a difference between the two passes would have put members in the wrong place
         for (size_t r = 0; r < N; r++)
             if (zcheck[r] != zsizes[r]) throw std::runtime_error("internal: compressed sizes differ between the size pass and the run");
+    if (parts) join_parts(c, Y, P, Z.zmethod == DEFLATE_BGZF, ranges, first_dev);
 
-    // --- compressed: the parts move behind the first device's bytes in device order (their offsets are known now),
-    //     slices of them copied by several threads at once; one end-of-file block per file
-    if (parts) {
-        struct CopyTask { int in_fd, out_fd; uint64_t in_off, out_off, len; };
-        std::vector<CopyTask> tasks;
-        std::vector<int> fds;
-        struct CloseAll { std::vector<int>& f; ~CloseAll() { for (int x : f) ::close(x); } } close_all{fds};
-        const bool eof = Z.dev_z || Z.zmethod == DEFLATE_BGZF;
-        for (size_t k = 0; k < nj; k++)
-            for (int e = 0; e < n_ends; e++) {
-                const std::string name = file_name(Y.jobs[k], e, true, P);
-                const int fd = ::open(name.c_str(), first_dev[k] < N ? O_RDWR : (O_RDWR | O_CREAT | O_TRUNC), 0644);
-                if (fd < 0) throw IoErr("Unable to open file " + name + ".\n");
-                fds.push_back(fd);
-                struct stat sb;
-                if (::fstat(fd, &sb) != 0) throw IoErr("Error writing to file " + name + ": " + std::strerror(errno));
-                uint64_t pos = (uint64_t)sb.st_size;
-                for (size_t r = 0; r < N; r++) {
-                    if (ranges[r][k].second <= ranges[r][k].first || r == first_dev[k]) continue;
-                    const std::string part = name + ".part" + std::to_string(r);
-                    const int in = ::open(part.c_str(), O_RDONLY);
-                    if (in < 0 || ::fstat(in, &sb) != 0) { if (in >= 0) ::close(in); throw IoErr("cannot read " + part); }
-                    fds.push_back(in);
-                    const uint64_t slice = 64ull << 20;
-                    for (uint64_t o = 0; o < (uint64_t)sb.st_size; o += slice)
-                        tasks.push_back(CopyTask{in, fd, o, pos + o, std::min<uint64_t>(slice, (uint64_t)sb.st_size - o)});
-                    pos += (uint64_t)sb.st_size;
-                }
-                if (::ftruncate(fd, (off_t)(pos + (eof ? sizeof kBgzfEof : 0))) != 0)
-                    throw IoErr("Error writing to file " + name + ": " + std::strerror(errno));
-                if (eof) {
-                    const std::string w = pwrite_all(fd, kBgzfEof, sizeof kBgzfEof, pos);
-                    if (!w.empty()) throw IoErr("Error writing to file " + name + ": " + w);
-                }
-            }
-        // a slice is copied through mappings of both files where that works (threads writing one file through
-        // write() / copy_file_range queue on its inode lock; page-cache pages filled through a mapping do not), else by
-        // copy_range; the writer threads of the first device do the copying
-        WriterPool& writers = c->dev[0]->writers;
-        std::atomic<int> pending{0};
-        writers.start(std::min<size_t>(std::max<size_t>(tasks.size(), 1), std::min<uint64_t>(std::max<uint64_t>(P->n_threads, 4), 32)));
-        for (const CopyTask& t : tasks)
-            writers.submit(&pending, [t]() {
-                Mapping mo, mi;
-                std::string w;
-                if (map_range(t.out_fd, t.out_off, t.len, mo) && map_range(t.in_fd, t.in_off, t.len, mi, true))
-                    std::memcpy(mo.at, mi.at, t.len);
-                else
-                    w = copy_range(t.out_fd, t.out_off, t.in_fd, t.in_off, t.len);
-                mi.unmap();
-                mo.unmap();
-                return w;
-            });
-        const std::string w = writers.wait(pending);
-        if (!w.empty()) { writers.clear_error(); throw IoErr("Error joining the devices' parts: " + w); }
-    }
-
-    jlp_run_stats tot;
-    std::memset(&tot, 0, sizeof tot);
+    // --- the devices' statistics summed, their device times the slowest device's (they work side by side)
+    jlp_run_stats tot{};
     for (size_t r = 0; r < N; r++) {
-        tot.pairs += st[r].pairs; tot.batches += st[r].batches; tot.kernel_launches += st[r].kernel_launches;
-        for (int e = 0; e < 2; e++) { tot.bytes_out[e] += st[r].bytes_out[e]; tot.z_bytes[e] += st[r].z_bytes[e]; }
-        tot.d2h_bytes += st[r].d2h_bytes; tot.h2d_bytes += st[r].h2d_bytes;
-        // device time: the slowest device's (they work side by side)
-        tot.device_ms = std::max(tot.device_ms, st[r].device_ms); tot.place_ms = std::max(tot.place_ms, st[r].place_ms);
-        tot.reads_ms = std::max(tot.reads_ms, st[r].reads_ms); tot.bgzf_ms = std::max(tot.bgzf_ms, st[r].bgzf_ms);
-        tot.run_ms = std::max(tot.run_ms, st[r].run_ms);
+        const jlp_run_stats& s = st[r];
+        tot.pairs += s.pairs; tot.batches += s.batches; tot.kernel_launches += pre[r].kernel_launches + s.kernel_launches;
+        for (int e = 0; e < 2; e++) { tot.bytes_out[e] += s.bytes_out[e]; tot.z_bytes[e] += s.z_bytes[e]; }
+        tot.d2h_bytes += s.d2h_bytes; tot.h2d_bytes += s.h2d_bytes;
+        tot.device_ms = std::max(tot.device_ms, s.device_ms); tot.place_ms = std::max(tot.place_ms, s.place_ms);
+        tot.reads_ms = std::max(tot.reads_ms, s.reads_ms); tot.bgzf_ms = std::max(tot.bgzf_ms, s.bgzf_ms);
+        tot.run_ms = std::max(tot.run_ms, s.run_ms);
     }
-    tot.kernel_launches += launches;
     if (stats) *stats = tot;
 }
 
@@ -628,7 +627,7 @@ extern "C" {
 
 static void run_any(jlp_ctx* c, bool use_haps, const jlp_illumina_params* p, Output& s, jlp_run_stats* stats) {
     check_params(c, use_haps, p, s.kind);
-    if (c->dev.size() == 1) run(c, *c->dev[0], use_haps, p, make_layout(c, illumina_spec(c, use_haps, p)), s, stats);
+    if (c->dev.size() == 1) run(c, *c->dev[0], use_haps, p, compression_of(p, s.kind), make_layout(c, illumina_spec(c, use_haps, p)), s, stats);
     else run_multi(c, use_haps, p, s, stats);
 }
 
